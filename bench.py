@@ -359,11 +359,16 @@ def run_workload(cfg, args, world, rank, local_rank, dev, steps, warmup, with_ro
         flush.fill_(float(i))                        # L2 flush between timed iterations (outside the events)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        one_rollout(x0_dev, scheds[warmup + i])
+        xT = one_rollout(x0_dev, scheds[warmup + i])
         e1.record()
         evs.append((e0, e1))
     torch.cuda.synchronize()
     launches = lib.gnca_launch_count() - launches0
+    outputs = None
+    if args.dump_outputs:        # copied before the e2e / roofline passes below run further steps (training updates weights)
+        outputs = {"x_T": xT.detach().clone()}
+        if cfg["train"]:
+            outputs["weights"] = opt.flat.clone()
     sampler.stop_flag = True
     sampler.join()
     if world > 1:
@@ -436,7 +441,20 @@ def run_workload(cfg, args, world, rank, local_rank, dev, steps, warmup, with_ro
                                  x0_host.numel(), T, args)
 
     return {"value": value, "ms_per_step": dev_ms_max / steps, "e2e": e2e, "launches": int(launches), "roofline": roof,
-            "clocks": sampler.result(), "data": data, "dims": (C_, H, W, B, T)}
+            "clocks": sampler.result(), "data": data, "dims": (C_, H, W, B, T), "outputs": outputs}
+
+
+def dump_outputs(dirname, arrays, limit=64 << 20):
+    """Writes each array as DIR/<name>.npy in float32, `limit` bytes in all.  An array larger than its share is stored as
+    DIR/<name>_sample.npy: the flat elements at a fixed set of indices (seeded draw, sorted), the same in every run."""
+    os.makedirs(dirname, exist_ok=True)
+    share = limit // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() * 4 > share:
+            idx = torch.randint(t.numel(), (share // 4,), generator=torch.Generator().manual_seed(0)).unique()
+            t, name = t.reshape(-1)[idx.to(t.device)], name + "_sample"
+        np.save(os.path.join(dirname, name + ".npy"), t.cpu().numpy())
 
 
 def run_trainer(args, world, rank, local_rank, dev, steps, warmup, regime="short", scaling="weak", per_gpu=32,
@@ -580,6 +598,8 @@ def main():
     ap.add_argument("--no-train-extra", action="store_true", help="skip the fwd+bwd (c3) measurement of the default run")
     ap.add_argument("--T", type=int, default=0, help="development: override the number of CA steps per rollout")
     ap.add_argument("--B", type=int, default=0, help="development: override the per-GPU batch")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, float32, 64 MB at most")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     cfg = workload_cfg(args.workload)
@@ -605,13 +625,15 @@ def main():
     res = run_workload(cfg, args, world, rank, local_rank, dev, args.steps, args.warmup)
     C_, H, W, B, T = res["dims"]
     value, e2e, launches, roof, data = res["value"], res["e2e"], res["launches"], res["roofline"], res["data"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res["outputs"])
 
     # the other half of the metric ("fwd, fwd+bwd"): BASELINE configs[2] (and, for N > 1, configs[3]) through the trainer
     train = None
     if args.workload == "c2" and not args.no_train_extra:
-        ts = max(3, min(args.steps, 10))
+        ts = args.steps
         train = {"short": run_trainer(args, world, rank, local_rank, dev, ts, 3, "short", "weak"),
-                 "long": run_trainer(args, world, rank, local_rank, dev, 3, 3, "long", "weak")}
+                 "long": run_trainer(args, world, rank, local_rank, dev, ts, 3, "long", "weak")}
         if world > 1:    # configs[3]: damage curriculum, global batch 32 sharded 16 / 8 / 4 per GPU (strong) and 32 per GPU (weak)
             train["damage_weak"] = run_trainer(args, world, rank, local_rank, dev, ts, 3, "short", "weak", damage=True)
             train["damage_strong"] = run_trainer(args, world, rank, local_rank, dev, ts, 3, "short", "strong", damage=True)

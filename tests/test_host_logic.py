@@ -175,29 +175,6 @@ def test_words_sampler_reports_short_blocks_and_keeps_the_stream():
     assert random.getstate() == after
 
 
-def test_reference_staging_recipe():
-    """oracle/build_ref.py: when the reference checkout is present the seven hot-path files are staged verbatim into the
-    git-ignored oracle/_ref (the CPU arm / eager comparator of bench.py); the staged modules import and run one step."""
-    import filecmp
-    import os
-    import pytest
-    from oracle import build_ref
-    if not os.path.isdir("/root/reference/src"):
-        if not os.path.isdir(build_ref.DST):
-            pytest.skip("no reference checkout and nothing staged")
-    else:
-        assert build_ref.build(verbose=False)
-        for rel in build_ref.FILES:
-            assert filecmp.cmp(os.path.join("/root/reference/src", rel), os.path.join(build_ref.DST, rel), shallow=False), rel
-    import torch
-    import bench_ref
-    model, kind = bench_ref.make_reference_graph("cpu")
-    assert kind == "reference"
-    with torch.no_grad():
-        y = model(bench_ref.make_seed(2, "cpu"), fire_rate=0.5)
-    assert tuple(y.shape) == (2, 16, 40, 40) and bool(torch.isfinite(y).all())
-
-
 def test_history_allocation_is_quantised_in_steps():
     """rollout.py sizes the BPTT record buffer / dense history for T rounded up to 64 steps, so that rollouts of slightly
     different lengths reuse one cached block (a fresh 29 GB cudaMalloc per new maximum cost 70 ms in the long regime)."""
