@@ -11,7 +11,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 LIBDIR = os.path.join(PKG, "lib")
 LIB = os.path.join(LIBDIR, "libgnca.so")
-SOURCES = ["gnca_fwd.cu", "gnca_bwd.cu", "gnca_aux.cu", "gnca_rollout.cu", "gnca_resident.cu", "gnca_rep.cu", "gnca_rep_bwd.cu", "gnca_graph.cu", "gnca_update_tc.cu", "gnca_update_tc2.cu"]
+SOURCES = ["gnca_fwd.cu", "gnca_bwd.cu", "gnca_aux.cu", "gnca_rollout.cu", "gnca_resident.cu", "gnca_rep.cu", "gnca_rep_bwd.cu", "gnca_graph.cu", "gnca_update_tc.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v"]
 

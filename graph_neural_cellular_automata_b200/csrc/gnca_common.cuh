@@ -140,7 +140,6 @@ struct StepArgs {
   double* partials;                   // [B][nchunks][2]
   int nchunks, chunk;                 // k_update work split: cells per block and blocks per sample
   int npart;                          // GroupNorm partial slots per sample in `partials` (nchunks, or 3*nchunks: k_update_tc)
-  const float* stats_ready;           // [B][2] (mean, rstd) already finished by the update path (k_update_tc2) or null
   const uint32_t* actbits;            // [B][ceil(HW/32)] active (alive & fire) bits of this step written by k_compact, or null
   const uint32_t* alivebits;          // same layout: sender-alive bits (3x3 alpha max > graph_alpha_thr) of x_in, or null
   Offsets off;                        // host-supplied offsets (single step)

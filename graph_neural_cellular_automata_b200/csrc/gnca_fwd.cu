@@ -512,9 +512,7 @@ __global__ void __launch_bounds__(kThreads) k_apply(StepArgs a, Packed P, const 
 
   if (threadIdx.x < 32) {
     float mu = 0.f, rstd = 1.f;
-    if (gn && a.stats_ready) {                   // finished by the update path (k_tilestats)
-      mu = a.stats_ready[b * 2]; rstd = a.stats_ready[b * 2 + 1];
-    } else if (gn) {
+    if (gn) {
       double t1, t2;
       warp_reduce_partials(a, b, threadIdx.x, t1, t2);
       const double n = (double)C * (double)HW;
@@ -526,7 +524,7 @@ __global__ void __launch_bounds__(kThreads) k_apply(StepArgs a, Packed P, const 
     }
     if (threadIdx.x == 0) {
       s_stat[0] = mu; s_stat[1] = rstd;
-      if (blockIdx.x == 0 && a.stats && a.stats != a.stats_ready) { a.stats[b * 2] = mu; a.stats[b * 2 + 1] = rstd; }
+      if (blockIdx.x == 0 && a.stats) { a.stats[b * 2] = mu; a.stats[b * 2 + 1] = rstd; }
     }
   }
   __syncthreads();
@@ -675,7 +673,6 @@ FwdWorkspace carve_fwd_workspace(void* base, const gnca_model& m, int B, int H, 
   ws.rowsum = reinterpret_cast<float*>(p + o); o = align_up(o + (size_t)B * m.C * H * sizeof(float), 256);
   ws.attn_w = reinterpret_cast<float*>(p + o); o = align_up(o + (size_t)B * GNCA_MAX_K * sizeof(float), 256);
   ws.absmean = reinterpret_cast<float*>(p + o); o = align_up(o + (size_t)B * H * W * sizeof(float), 256);
-  ws.tc2 = p + o; o = align_up(o + update_tc2_workspace_bytes(B, H, W), 256);
   ws.actbits = reinterpret_cast<uint32_t*>(p + o); o = align_up(o + (size_t)B * ((H * W + 31) / 32) * sizeof(uint32_t), 256);
   ws.alivebits = reinterpret_cast<uint32_t*>(p + o); o = align_up(o + (size_t)B * ((H * W + 31) / 32) * sizeof(uint32_t), 256);
   ws.bytes = o;
@@ -702,7 +699,6 @@ static int launch_update(const gnca_model& m, const Packed& P, const float* pack
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   const size_t smem = UpdateSmem<C>::bytes(m.hidden, graph);
   dim3 g1(a.nchunks, a.B);
-  a.stats_ready = nullptr;
   a.actbits = nullptr;
   a.alivebits = nullptr;
   if (a.chunk == kChunkSmall) {
@@ -716,18 +712,13 @@ static int launch_update(const gnca_model& m, const Packed& P, const float* pack
   static_assert(kChunk == kTcChunk, "k_update_tc reads the chunk-local lists of k_compact<kChunk>");
   // Which k_update runs (read per launch so that one process can compare them: tests/test_gpu_scale.py):
   //   default        k_update_tc   compacted 128-cell tiles on the tensor cores (gnca_update_tc.cu)
-  //   GNCA_TC_V2=1   k_update_tc2  dense 8x16 tiles staged by TMA (gnca_update_tc2.cu) -- correct, but at fire 0.5 it runs
-  //                                twice the tiles through the serial tensor chain: 0.26 vs 0.21 ms per step at 256x256x32,
-  //                                profiles/r02_k_update_tc2.md
   //   GNCA_NO_TC=1   k_update      the round-1 FFMA kernel
-  const bool no_tc = getenv("GNCA_NO_TC") != nullptr, tc_v2 = getenv("GNCA_TC_V2") != nullptr;
+  const bool no_tc = getenv("GNCA_NO_TC") != nullptr;
   const bool use_tc = !no_tc && update_tc_supported(m, a);
-  if (use_tc && tc_v2 && update_tc2_supported(m, a)) return launch_update_tc2(m, P, packed, a, ws.tc2, st);
   a.npart = use_tc ? 3 * a.nchunks : a.nchunks;
   const size_t used = (size_t)a.B * a.npart * 2 * sizeof(double), have = (size_t)a.B * n_small * 2 * sizeof(double);
   const size_t need = ((size_t)a.B * a.nchunks + (size_t)a.B * (a.nchunks + 1)) * sizeof(int);
-  static const bool no_bal = getenv("GNCA_NO_BALANCE") != nullptr;            // development: the per-chunk kernel
-  if (!no_bal && a.nchunks <= kMaxBalChunks && used + need <= have) {
+  if (a.nchunks <= kMaxBalChunks && used + need <= have) {
     int* cnt = reinterpret_cast<int*>(reinterpret_cast<char*>(ws.partials) + used);
     int* prefix = cnt + (size_t)a.B * a.nchunks;
     uint16_t* glist = reinterpret_cast<uint16_t*>(ws.absmean);
@@ -828,9 +819,7 @@ __global__ void k_finalize_stats(StepArgs a, int C) {       // one warp per samp
   const int b = blockIdx.x, lane = threadIdx.x;
   if (b >= a.B || !a.stats) return;
   float mu = 0.f, rstd = 1.f;
-  if ((a.flags & GNCA_F_GROUPNORM) && a.stats_ready) {
-    mu = a.stats_ready[b * 2]; rstd = a.stats_ready[b * 2 + 1];
-  } else if (a.flags & GNCA_F_GROUPNORM) {
+  if (a.flags & GNCA_F_GROUPNORM) {
     double t1, t2;
     warp_reduce_partials(a, b, lane, t1, t2);
     const double n = (double)C * (double)a.H * (double)a.W;
@@ -856,7 +845,6 @@ int launch_step_recompute(const gnca_model& m, const Packed& P, const float* pac
   }
   { const int rc = launch_update<C>(m, P, packed, a, ws, st); if (rc) return rc; }
   GNCA_LAUNCH_CHECK();
-  if (a.stats_ready && a.stats_ready == a.stats) return 0;       // k_update_tc2 finished the statistics in place
   k_finalize_stats<<<a.B, 32, 0, st>>>(a, C);
   GNCA_LAUNCH_CHECK();
   return 0;

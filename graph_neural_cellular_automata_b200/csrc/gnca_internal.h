@@ -10,7 +10,6 @@ struct FwdWorkspace {
   float* rowsum;      // [B][C][H]
   float* attn_w;      // [B][MAX_K]
   float* absmean;     // [B][H][W]
-  void* tc2;          // tile masks / lists / partials of k_update_tc2 (update_tc2_workspace_bytes)
   uint32_t* actbits;  // [B][ceil(HW/32)] active bits of the step (k_compact -> k_apply)
   uint32_t* alivebits;   // [B][ceil(HW/32)] sender-alive bits of the step (k_compact -> k_update_tc)
   size_t bytes;
@@ -58,12 +57,6 @@ constexpr int kTcChunk = 1024;
 bool update_tc_supported(const gnca_model& m, const StepArgs& a);
 int launch_update_tc(const gnca_model& m, const Packed& P, const float* packed, StepArgs& a, const uint16_t* glist,
                      const int* prefix, cudaStream_t st);
-
-// dense-tile, TMA-staged tensor-core k_update (gnca_update_tc2.cu): H % 8 == 0, W % 16 == 0.  Finishes the GroupNorm
-// statistics itself: a.stats_ready points at (mean, rstd) per sample afterwards (written to a.stats when that is set).
-size_t update_tc2_workspace_bytes(int B, int H, int W);
-bool update_tc2_supported(const gnca_model& m, const StepArgs& a);
-int launch_update_tc2(const gnca_model& m, const Packed& P, const float* packed, StepArgs& a, void* ws, cudaStream_t st);
 
 // cluster-resident forward rollout (gnca_resident.cu); GNCA_ERR_UNSUPPORTED when the configuration has no
 // resident kernel (zero-padded graph shift, sample too large for the cluster's shared memory)

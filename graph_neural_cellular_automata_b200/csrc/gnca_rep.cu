@@ -27,6 +27,7 @@
 #include <type_traits>
 #include "gnca_common.cuh"
 #include "gnca_internal.h"
+#include "gnca_ptx.cuh"
 #include "gnca_rep.h"
 
 namespace cg = cooperative_groups;
@@ -60,9 +61,6 @@ struct RepArgs {
   int use_async;              // 1: st.async + mbarrier transaction counts between the CTAs, 0: two cluster barriers per step
 };
 
-__device__ __forceinline__ void cl_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
-__device__ __forceinline__ void cl_wait() { asm volatile("barrier.cluster.wait.aligned;" ::: "memory"); }
-
 #ifdef GNCA_PHASE_COUNTERS          /* build with -DGNCA_PHASE_COUNTERS for the per-phase cycle counters */
 #define REP_MARK(idx)                                                               \
   do {                                                                              \
@@ -76,7 +74,6 @@ __device__ __forceinline__ void cl_wait() { asm volatile("barrier.cluster.wait.a
 #define REP_MARK(idx) do { } while (0)
 #endif
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ uint32_t mapa_u32(uint32_t addr, int rank) {
   uint32_t o;
   asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(o) : "r"(addr), "r"(rank));
@@ -84,19 +81,6 @@ __device__ __forceinline__ uint32_t mapa_u32(uint32_t addr, int rank) {
 }
 __device__ __forceinline__ void st_cluster_f32(uint32_t addr, float v) {
   asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
-}
-__device__ __forceinline__ void mbar_init(uint32_t addr, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(addr), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t addr, uint32_t tx) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(addr), "r"(tx) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t addr, uint32_t parity) {
-  uint32_t ok = 0;
-  do {
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(ok) : "r"(addr), "r"(parity) : "memory");
-  } while (!ok);
 }
 // remote store that signals `bytes written` on an mbarrier of the destination CTA: the consumer waits for the
 // expected byte count instead of a cluster-wide barrier (and no MEMBAR on the producer side)
@@ -396,9 +380,9 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
   if (tid == 0) {
     mbar_init(mbarA, 1);
     mbar_init(mbarB, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   }
-  cl_arrive(); cl_wait();                        // every replica initialised before any remote store
+  cluster_arrive(); cluster_wait();              // every replica initialised before any remote store
 
   const int my_steps = a.steps ? min(a.steps[b], R.T) : R.T;
   long long t_prev = clock64();
@@ -761,10 +745,10 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
         }
       }
       REP_MARK(2);
-      cl_arrive();                                                            // ---- cluster barrier 1
+      cluster_arrive();                                                       // ---- cluster barrier 1
       sched_commit(cur);                  // step t+2 -> the buffer step t no longer needs (visible after later barriers)
       sched_fetch(t + 3);
-      cl_wait();
+      cluster_wait();
     } else {
       // my partial -> every peer (8 bytes each, counted on the peer's mbarrier A); a peer's partial arriving here also
       // says that peer has finished reading x_t, so its cells may be overwritten once all of them are in
@@ -871,7 +855,7 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
       mbar_wait(mbarB, (uint32_t)(t & 1));                                    // every peer's cells have landed here
       __syncthreads();                                                        // ... and my own warps' writes are done
     } else {
-      cl_arrive(); cl_wait();                                                 // ---- cluster barrier 2
+      cluster_arrive(); cluster_wait();                                       // ---- cluster barrier 2
     }
     REP_MARK(5);
 
@@ -918,7 +902,7 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
   if (R.hist) store_state(R.hist + (size_t)R.T * a.B * C * HW + sample_off, my_lo, my_hi);
   store_state(R.xT + sample_off, my_lo, my_hi);
   if (R.dbg && blockIdx.x == R.dbg_cta && tid < 24) R.dbg[tid] = s_dbg[tid];
-  cl_arrive(); cl_wait();      // nobody exits while a peer may still address its shared memory
+  cluster_arrive(); cluster_wait();      // nobody exits while a peer may still address its shared memory
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -27,6 +27,7 @@
 #include <type_traits>
 #include "gnca_common.cuh"
 #include "gnca_internal.h"
+#include "gnca_ptx.cuh"
 #include "gnca_rep.h"
 
 namespace cg = cooperative_groups;
@@ -81,11 +82,6 @@ __device__ __forceinline__ void bulk_store_512(float* gdst, const float* ssrc) {
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-__device__ __forceinline__ void cl_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;\n" ::: "memory");
-}
 
 template <int C>
 __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, const float* __restrict__ packed) {
@@ -168,7 +164,7 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
     }
   }
   __syncthreads();
-  cl_sync_all();
+  cluster_sync_acquire();
 
   const int my_steps = a.steps ? min(a.steps[b], R.T) : R.T;
   const int q = tid, qcell = 4 * tid;
@@ -336,7 +332,7 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
       }
     }
     REPB_MARK(4);
-    cl_sync_all();                                                            // ---- cluster barrier 1: S1/S2 partials, GZ visible
+    cluster_sync_acquire();                                                   // ---- cluster barrier 1: S1/S2 partials, GZ visible
     REPB_MARK(5);
     float s1n = 0.f, s2n = 0.f;
     if (gn) {
@@ -430,7 +426,7 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
 #pragma unroll
         for (int jj = 0; jj < 4; ++jj) { hmask |= acc1[m][jj] > 0.f ? (1u << (4 * m + jj)) : 0u; acc1[m][jj] = 0.f; }
       }
-      fence_proxy_async_smem();
+      fence_proxy_async();
       __syncwarp();
       if (issuer) bulk_store_512(hgh_row, myGH + lane * HID);
       if (lane < G) bulk_commit();
@@ -472,7 +468,7 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
         v.z = (hmask >> (4 * m + 2)) & 1u ? acc1[m][2] : 0.f; v.w = (hmask >> (4 * m + 3)) & 1u ? acc1[m][3] : 0.f;
         *reinterpret_cast<float4*>(myGH + m * HID + 4 * lane) = v;
       }
-      fence_proxy_async_smem();
+      fence_proxy_async();
       __syncwarp();
       if (issuer) bulk_store_512(hgh_row + HID, myGH + lane * HID);
       if (lane < G) bulk_commit();
@@ -518,7 +514,7 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
       }
     }
     REPB_MARK(6);
-    cl_sync_all();                                                            // ---- cluster barrier 2: RG visible
+    cluster_sync_acquire();                                                   // ---- cluster barrier 2: RG visible
     REPB_MARK(7);
     // ---- C: my band: g_t = gated g_{t+1} + perception^T (gy of active neighbours) + message^T (g_xs of receivers) --
     {
@@ -642,7 +638,7 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
     R.affpart[(size_t)blockIdx.x * 2 * C + tid] = ac;
   }
   if (lane < 8) bulk_wait_all();               // every h | gh row has reached global memory before the kernel ends
-  cl_sync_all();
+  cluster_sync_acquire();
 }
 
 // ------------------------------------------------------------------------------------------------

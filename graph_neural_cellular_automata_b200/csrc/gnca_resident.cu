@@ -20,6 +20,7 @@
 #include <type_traits>
 #include "gnca_common.cuh"
 #include "gnca_internal.h"
+#include "gnca_ptx.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -42,11 +43,10 @@ struct ResidentArgs {
   int damage_step;
   unsigned long long* dbg;    // optional phase-cycle counters (GNCA_PHASE_TIMING=<cta index>), else null
   int dbg_cta;
-  int dbg_repeat;             // development: bitmask of phases to execute twice (idempotent; cost = time delta)
-  int dbg_skip;               // development: bitmask of phases to skip (timing experiments only; results wrong)
 };
 
 // phase counters accumulate in shared memory (a global RMW per mark would sit on the critical path)
+#ifdef GNCA_PHASE_COUNTERS          /* build with -DGNCA_PHASE_COUNTERS for the per-phase cycle counters */
 #define GNCA_PHASE_MARK(idx)                                                        \
   do {                                                                              \
     if (R.dbg && tid == 0) {                                                        \
@@ -55,15 +55,9 @@ struct ResidentArgs {
       t_prev = _n;                                                                  \
     }                                                                               \
   } while (0)
-
-// Cluster barrier.  The arrive is a release (every DSMEM store issued before it is performed before a peer
-// passes the wait); the wait carries NO acquire: an acquire makes ptxas emit CCTL.IVALL, which invalidates the
-// whole L1 -- including the lines backing local memory (stack) -- at every barrier.  Nothing exchanged inside the
-// kernel travels through L1-cached global memory (peers communicate through shared::cluster stores only), so the
-// invalidation buys nothing here.
-__device__ __forceinline__ void cluster_barrier() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.aligned;\n" ::: "memory");
-}
+#else
+#define GNCA_PHASE_MARK(idx) do { } while (0)
+#endif
 
 // Out-of-line helpers: the per-step code of the resident kernel has to stay small enough for the instruction
 // caches (every phase is executed once per step by few warps, so cold-code fetch latency is on the critical path).
@@ -195,7 +189,7 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
   float* pAt = cluster.map_shared_rank(sAt, prev);
   float* nAt = cluster.map_shared_rank(sAt, next);
   __syncthreads();
-  cluster_barrier();
+  cluster_sync_no_acquire();
 
   const int my_steps = a.steps ? min(a.steps[b], R.T) : R.T;
   long long t_prev = clock64();
@@ -231,155 +225,150 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
     const bool msg_on = graph && gain_m != 0.f && a.k > 0;
 
     // ---- P1: alive & fire on own cells, deterministic compaction ------------------------------------------
-    for (int rep_ = 0; rep_ < ((R.dbg_repeat & 8) ? 2 : 1); ++rep_) {
-      int cnt = 0;
-      const int per = ((nown + kRThreads - 1) / kRThreads) * 32;     // own cells per warp (multiple of 32)
-      const int lo = warp * per;
-      for (int base = lo; base < lo + per; base += 32) {
-        const int oc = base + lane;
-        bool act = false;
-        if (oc < nown) {
-          const int orow = s_oy[oc], x = s_ox[oc];
-          act = alive_local(sA, HALO + orow, x, r0 + orow, a.alpha_thr) && fires(a, fr, b, (r0 + orow) * W + x);
-          s_slot[oc] = act ? 1 : -1;
-        }
-        cnt += __popc(__ballot_sync(0xffffffffu, act));
+    int cnt = 0;
+    const int per = ((nown + kRThreads - 1) / kRThreads) * 32;     // own cells per warp (multiple of 32)
+    const int lo = warp * per;
+    for (int base = lo; base < lo + per; base += 32) {
+      const int oc = base + lane;
+      bool act = false;
+      if (oc < nown) {
+        const int orow = s_oy[oc], x = s_ox[oc];
+        act = alive_local(sA, HALO + orow, x, r0 + orow, a.alpha_thr) && fires(a, fr, b, (r0 + orow) * W + x);
+        s_slot[oc] = act ? 1 : -1;
       }
-      if (lane == 0) s_wcount[warp] = cnt;
-      __syncthreads();
-      if (warp == 0) {                        // exclusive scan of the per-warp counts
-        const int v = lane < kRWarps ? s_wcount[lane] : 0;
-        int incl = v;
-#pragma unroll
-        for (int o = 1; o < kRWarps; o <<= 1) {
-          const int n = __shfl_up_sync(0xffffffffu, incl, o);
-          if (lane >= o) incl += n;
-        }
-        if (lane < kRWarps) s_wbase[lane] = incl - v;
-        if (lane == kRWarps - 1) s_wbase[kRWarps] = incl;
-      }
-      __syncthreads();
-      int pos = s_wbase[warp];
-      for (int base = lo; base < lo + per; base += 32) {
-        const int oc = base + lane;
-        const bool act = oc < nown && s_slot[oc] > 0;
-        const unsigned bal = __ballot_sync(0xffffffffu, act);
-        if (act) {
-          const int slot = pos + __popc(bal & ((1u << lane) - 1u));
-          s_actlist[slot] = oc;
-          s_slot[oc] = slot;
-        }
-        pos += __popc(bal);
-      }
-      __syncthreads();
+      cnt += __popc(__ballot_sync(0xffffffffu, act));
     }
+    if (lane == 0) s_wcount[warp] = cnt;
+    __syncthreads();
+    if (warp == 0) {                        // exclusive scan of the per-warp counts
+      const int v = lane < kRWarps ? s_wcount[lane] : 0;
+      int incl = v;
+#pragma unroll
+      for (int o = 1; o < kRWarps; o <<= 1) {
+        const int n = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += n;
+      }
+      if (lane < kRWarps) s_wbase[lane] = incl - v;
+      if (lane == kRWarps - 1) s_wbase[kRWarps] = incl;
+    }
+    __syncthreads();
+    int pos = s_wbase[warp];
+    for (int base = lo; base < lo + per; base += 32) {
+      const int oc = base + lane;
+      const bool act = oc < nown && s_slot[oc] > 0;
+      const unsigned bal = __ballot_sync(0xffffffffu, act);
+      if (act) {
+        const int slot = pos + __popc(bal & ((1u << lane) - 1u));
+        s_actlist[slot] = oc;
+        s_slot[oc] = slot;
+      }
+      pos += __popc(bal);
+    }
+    __syncthreads();
     const int nact = s_wbase[kRWarps];
     GNCA_PHASE_MARK(0);
     if (R.dbg && tid == 0) s_dbg[8] += nact;
 
     // ---- P2: perception + MLP + message on the active cells, in batches of MB ----------------------------
     float ps1 = 0.f, ps2 = 0.f;
-    for (int base = 0; base < ((R.dbg_skip & 1) ? 0 : nact); base += MB) {
+    for (int base = 0; base < nact; base += MB) {
       const int nb = min(MB, nact - base);
       const int G = nb > 32 ? 8 : 4;                    // cells per warp tile (layer 1 + layer 2 stay inside one warp)
       const int nbp = ((nb + G - 1) / G) * G;           // staged cells (zero padded to the tile)
       // 2a: sender table, one lane per (cell, offset): local index of the (alive) sender or -1
-      for (int rep_ = 0; rep_ < ((R.dbg_repeat & 1) ? 2 : 1); ++rep_) {
-        if (msg_on) {
-          for (int i = tid; i < nb * a.k; i += kRThreads) {
-            const int cl = i / a.k, oi = i - cl * a.k;
-            const int oc = s_actlist[base + cl];
-            const int orow = s_oy[oc], x = s_ox[oc], gy = r0 + orow;
-            const int dy = s_off[(t * a.k + oi) * 2], dx = s_off[(t * a.k + oi) * 2 + 1];
-            int gq = (gy - dy) % H; gq = gq < 0 ? gq + H : gq;       // sender's global row (torus)
-            int qx = (x - dx) % W; qx = qx < 0 ? qx + W : qx;
-            const int lq = HALO + orow - dy;                          // its local row (halo holds the wrap)
-            int q = lq * W + qx;
-            if (a2a && !alive_local(sA, lq, qx, gq, a.graph_alpha_thr)) q = -1;
-            s_q[cl * kk + oi] = q;
-          }
-          __syncthreads();
+      if (msg_on) {
+        for (int i = tid; i < nb * a.k; i += kRThreads) {
+          const int cl = i / a.k, oi = i - cl * a.k;
+          const int oc = s_actlist[base + cl];
+          const int orow = s_oy[oc], x = s_ox[oc], gy = r0 + orow;
+          const int dy = s_off[(t * a.k + oi) * 2], dx = s_off[(t * a.k + oi) * 2 + 1];
+          int gq = (gy - dy) % H; gq = gq < 0 ? gq + H : gq;       // sender's global row (torus)
+          int qx = (x - dx) % W; qx = qx < 0 ? qx + W : qx;
+          const int lq = HALO + orow - dy;                          // its local row (halo holds the wrap)
+          int q = lq * W + qx;
+          if (a2a && !alive_local(sA, lq, qx, gq, a.graph_alpha_thr)) q = -1;
+          s_q[cl * kk + oi] = q;
         }
-        // 2b: one half-warp per cell, lane = channel: perception (9 independent loads) and the gathered sender
-        //     state xs = sum_i w x(q_i) with the k loads issued back to back (invalid senders get weight 0)
-        const int hw = tid >> 4, l16 = tid & 15;
-        const float wuni = a.k > 0 ? 1.0f / (float)a.k : 0.f;
-        for (int cl = hw; cl < nbp; cl += kRThreads / 16) {
-          const bool valid = cl < nb;
-          int orow = 0, x = 0;
-          if (valid) { const int oc = s_actlist[base + cl]; orow = s_oy[oc]; x = s_ox[oc]; }
-          const int gy = r0 + orow;
-          const bool up = gy > 0, dn = gy < H - 1, lf = x > 0, rt = x < W - 1;
-          int nvalid = 0;
-          for (int c = l16; c < C; c += 16) {
-            float vid = 0.f, vsx = 0.f, vsy = 0.f, xs = 0.f;
-            if (valid) {
-              const float* pc = sX + (size_t)c * PL;
-              const float* p = pc + (HALO + orow) * W + x;
-              const float a00 = (up && lf) ? p[-W - 1] : 0.f, a01 = up ? p[-W] : 0.f, a02 = (up && rt) ? p[-W + 1] : 0.f;
-              const float a10 = lf ? p[-1] : 0.f, a12 = rt ? p[1] : 0.f;
-              const float a20 = (dn && lf) ? p[W - 1] : 0.f, a21 = dn ? p[W] : 0.f, a22 = (dn && rt) ? p[W + 1] : 0.f;
-              vid = p[0];
-              vsx = (a00 - a02) + 2.f * (a10 - a12) + (a20 - a22);
-              vsy = (a00 + 2.f * a01 + a02) - (a20 + 2.f * a21 + a22);
-              if (msg_on) {
-                nvalid = 0;
-                const int* qrow = s_q + cl * kk;
-                for (int o4 = 0; o4 < a.k; o4 += 4) {
-                  int q0, q1, q2, q3;
-                  if ((kk & 3) == 0) {
-                    const int4 qq = *reinterpret_cast<const int4*>(qrow + o4);
-                    q0 = qq.x; q1 = qq.y; q2 = qq.z; q3 = qq.w;
-                  } else {
-                    q0 = qrow[o4];
-                    q1 = (o4 + 1 < a.k) ? qrow[o4 + 1] : -1;
-                    q2 = (o4 + 2 < a.k) ? qrow[o4 + 2] : -1;
-                    q3 = (o4 + 3 < a.k) ? qrow[o4 + 3] : -1;
-                  }
-                  const float v0 = pc[max(q0, 0)], v1 = pc[max(q1, 0)], v2 = pc[max(q2, 0)], v3 = pc[max(q3, 0)];
-                  xs = fmaf(q0 >= 0 ? wuni : 0.f, v0, xs);
-                  xs = fmaf(q1 >= 0 ? wuni : 0.f, v1, xs);
-                  xs = fmaf(q2 >= 0 ? wuni : 0.f, v2, xs);
-                  xs = fmaf(q3 >= 0 ? wuni : 0.f, v3, xs);
-                  nvalid += (q0 >= 0) + (q1 >= 0) + (q2 >= 0) + (q3 >= 0);
+        __syncthreads();
+      }
+      // 2b: one half-warp per cell, lane = channel: perception (9 independent loads) and the gathered sender
+      //     state xs = sum_i w x(q_i) with the k loads issued back to back (invalid senders get weight 0)
+      const int hw = tid >> 4, l16 = tid & 15;
+      const float wuni = a.k > 0 ? 1.0f / (float)a.k : 0.f;
+      for (int cl = hw; cl < nbp; cl += kRThreads / 16) {
+        const bool valid = cl < nb;
+        int orow = 0, x = 0;
+        if (valid) { const int oc = s_actlist[base + cl]; orow = s_oy[oc]; x = s_ox[oc]; }
+        const int gy = r0 + orow;
+        const bool up = gy > 0, dn = gy < H - 1, lf = x > 0, rt = x < W - 1;
+        int nvalid = 0;
+        for (int c = l16; c < C; c += 16) {
+          float vid = 0.f, vsx = 0.f, vsy = 0.f, xs = 0.f;
+          if (valid) {
+            const float* pc = sX + (size_t)c * PL;
+            const float* p = pc + (HALO + orow) * W + x;
+            const float a00 = (up && lf) ? p[-W - 1] : 0.f, a01 = up ? p[-W] : 0.f, a02 = (up && rt) ? p[-W + 1] : 0.f;
+            const float a10 = lf ? p[-1] : 0.f, a12 = rt ? p[1] : 0.f;
+            const float a20 = (dn && lf) ? p[W - 1] : 0.f, a21 = dn ? p[W] : 0.f, a22 = (dn && rt) ? p[W + 1] : 0.f;
+            vid = p[0];
+            vsx = (a00 - a02) + 2.f * (a10 - a12) + (a20 - a22);
+            vsy = (a00 + 2.f * a01 + a02) - (a20 + 2.f * a21 + a22);
+            if (msg_on) {
+              nvalid = 0;
+              const int* qrow = s_q + cl * kk;
+              for (int o4 = 0; o4 < a.k; o4 += 4) {
+                int q0, q1, q2, q3;
+                if ((kk & 3) == 0) {
+                  const int4 qq = *reinterpret_cast<const int4*>(qrow + o4);
+                  q0 = qq.x; q1 = qq.y; q2 = qq.z; q3 = qq.w;
+                } else {
+                  q0 = qrow[o4];
+                  q1 = (o4 + 1 < a.k) ? qrow[o4 + 1] : -1;
+                  q2 = (o4 + 2 < a.k) ? qrow[o4 + 2] : -1;
+                  q3 = (o4 + 3 < a.k) ? qrow[o4 + 3] : -1;
                 }
+                const float v0 = pc[max(q0, 0)], v1 = pc[max(q1, 0)], v2 = pc[max(q2, 0)], v3 = pc[max(q3, 0)];
+                xs = fmaf(q0 >= 0 ? wuni : 0.f, v0, xs);
+                xs = fmaf(q1 >= 0 ? wuni : 0.f, v1, xs);
+                xs = fmaf(q2 >= 0 ? wuni : 0.f, v2, xs);
+                xs = fmaf(q3 >= 0 ? wuni : 0.f, v3, xs);
+                nvalid += (q0 >= 0) + (q1 >= 0) + (q2 >= 0) + (q3 >= 0);
               }
             }
-            Yt[c * MBP + cl] = vid;
-            Yt[(C + c) * MBP + cl] = vsx;
-            Yt[(2 * C + c) * MBP + cl] = vsy;
-            XSt[c * MBP + cl] = xs;
           }
-          if (l16 == 0) {
-            float as = 0.f;
-            for (int n = 0; n < nvalid; ++n) as += wuni;     // same summation as the streaming path
-            AS[cl] = as;
-          }
-          __syncwarp();     // nbp is even: both half-warps of a warp run this loop the same number of times
-          // message projection by the first CQ lanes of the half-warp:
-          //   MSGt[c][cl] = gain * tanh(bm[c]*as + sum_ci Wm[c][ci] xs[ci]) on the gated channels, else 0
-          if (l16 < CQ) {
-            const int cq = l16;
-            float agg[4] = {0.f, 0.f, 0.f, 0.f};
-            if (msg_on && valid && 4 * cq + 3 >= c_lo) {
-              const float as = AS[cl];
-              const float4 bmv = *reinterpret_cast<const float4*>(sbm + 4 * cq);
-              agg[0] = bmv.x * as; agg[1] = bmv.y * as; agg[2] = bmv.z * as; agg[3] = bmv.w * as;
-#pragma unroll 4
-              for (int ci = 0; ci < C; ++ci) {
-                const float xv = XSt[ci * MBP + cl];
-                const float4 w = *reinterpret_cast<const float4*>(sWmT + ci * C + 4 * cq);
-                agg[0] = fmaf(w.x, xv, agg[0]); agg[1] = fmaf(w.y, xv, agg[1]);
-                agg[2] = fmaf(w.z, xv, agg[2]); agg[3] = fmaf(w.w, xv, agg[3]);
-              }
-#pragma unroll
-              for (int cc = 0; cc < 4; ++cc) agg[cc] = (4 * cq + cc >= c_lo) ? tanhf(agg[cc]) * gain_m : 0.f;
-            }
-#pragma unroll
-            for (int cc = 0; cc < 4; ++cc) MSGt[(4 * cq + cc) * MBP + cl] = agg[cc];
-          }
+          Yt[c * MBP + cl] = vid;
+          Yt[(C + c) * MBP + cl] = vsx;
+          Yt[(2 * C + c) * MBP + cl] = vsy;
+          XSt[c * MBP + cl] = xs;
         }
-        if (rep_ == 0 && (R.dbg_repeat & 1)) __syncthreads();
+        if (l16 == 0) {
+          float as = 0.f;
+          for (int n = 0; n < nvalid; ++n) as += wuni;     // same summation as the streaming path
+          AS[cl] = as;
+        }
+        __syncwarp();     // nbp is even: both half-warps of a warp run this loop the same number of times
+        // message projection by the first CQ lanes of the half-warp:
+        //   MSGt[c][cl] = gain * tanh(bm[c]*as + sum_ci Wm[c][ci] xs[ci]) on the gated channels, else 0
+        if (l16 < CQ) {
+          const int cq = l16;
+          float agg[4] = {0.f, 0.f, 0.f, 0.f};
+          if (msg_on && valid && 4 * cq + 3 >= c_lo) {
+            const float as = AS[cl];
+            const float4 bmv = *reinterpret_cast<const float4*>(sbm + 4 * cq);
+            agg[0] = bmv.x * as; agg[1] = bmv.y * as; agg[2] = bmv.z * as; agg[3] = bmv.w * as;
+#pragma unroll 4
+            for (int ci = 0; ci < C; ++ci) {
+              const float xv = XSt[ci * MBP + cl];
+              const float4 w = *reinterpret_cast<const float4*>(sWmT + ci * C + 4 * cq);
+              agg[0] = fmaf(w.x, xv, agg[0]); agg[1] = fmaf(w.y, xv, agg[1]);
+              agg[2] = fmaf(w.z, xv, agg[2]); agg[3] = fmaf(w.w, xv, agg[3]);
+            }
+#pragma unroll
+            for (int cc = 0; cc < 4; ++cc) agg[cc] = (4 * cq + cc >= c_lo) ? tanhf(agg[cc]) * gain_m : 0.f;
+          }
+#pragma unroll
+          for (int cc = 0; cc < 4; ++cc) MSGt[(4 * cq + cc) * MBP + cl] = agg[cc];
+        }
       }
       __syncthreads();
       GNCA_PHASE_MARK(10);
@@ -477,19 +466,14 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
           __syncwarp();
         }
       };
-      for (int rep_ = 0; rep_ < ((R.dbg_repeat & 2) ? 2 : 1); ++rep_) {
-        float sv1 = ps1, sv2 = ps2;
-        if (G == 8) mlp_tile(std::integral_constant<int, 8>{}); else mlp_tile(std::integral_constant<int, 4>{});
-        if (rep_ == 0 && (R.dbg_repeat & 2)) { ps1 = sv1; ps2 = sv2; }
-      }
+      if (G == 8) mlp_tile(std::integral_constant<int, 8>{}); else mlp_tile(std::integral_constant<int, 4>{});
       __syncthreads();     // staging buffers are reused by the next batch
     }
     GNCA_PHASE_MARK(1);
 
     // ---- GroupNorm(1,C) statistics over the whole sample: block partial -> DSMEM all-gather ----------------
     float mu = 0.f, rstd = 1.f;
-    for (int rep_ = 0; rep_ < ((R.dbg_repeat & 512) ? 2 : 1); ++rep_)
-    if (gn && !(R.dbg_skip & 2)) {
+    if (gn) {
       // fp32 tree (warp shuffles -> 16 warps -> NC CTAs); every CTA reduces the same values in the same order
       const float f1 = warp_sum(ps1), f2 = warp_sum(ps2);
       if (lane == 0) { s_wredf[warp][0] = f1; s_wredf[warp][1] = f2; }
@@ -503,7 +487,7 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
         }
       }
       GNCA_PHASE_MARK(2);
-      cluster_barrier();                                                      // barrier 1
+      cluster_sync_no_acquire();                                              // barrier 1
       GNCA_PHASE_MARK(3);
       if (warp == 0) {
         float t1 = 0.f, t2 = 0.f;
@@ -533,7 +517,7 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
 
     // ---- P3: bounded update in place (own cells); idle update of the halo copies; pre-gate alpha rows -------
     // inactive own cells: x += idle_c (their masked pre-norm update is 0); lanes <-> consecutive cells
-    for (int item = warp; item < ((R.dbg_skip & 4) ? 0 : ((nown + 31) >> 5) * CQ); item += kRWarps) {
+    for (int item = warp; item < ((nown + 31) >> 5) * CQ; item += kRWarps) {
       const int cq = item & (CQ - 1), oc = (item >> LCQ) * 32 + lane;
       if (oc >= nown || s_slot[oc] >= 0) continue;
       float* px = sX + (size_t)(4 * cq) * PL + HALO * W + oc;
@@ -552,7 +536,7 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
       }
     }
     // active cells: x += gain * tanh(gn(u)); one lane per (slot, channel), lanes <-> consecutive slots
-    for (int item = warp; item < ((R.dbg_skip & 4) ? 0 : ((nact + 31) >> 5) * C); item += kRWarps) {
+    for (int item = warp; item < ((nact + 31) >> 5) * C; item += kRWarps) {
       const int c = item & (C - 1), sl = (item / C) * 32 + lane;
       if (sl >= nact) continue;
       const int oc = s_actlist[sl];
@@ -568,26 +552,21 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
         *px = v;
       }
     }
-    for (int rep_ = 0; rep_ < ((R.dbg_repeat & 256) ? 3 : 1); ++rep_)
     for (int item = warp; item < ((2 * HALO * W + 31) >> 5) * CQ; item += kRWarps) {   // halo cells, channels != 3
       const int cq = item & (CQ - 1), hc = (item >> LCQ) * 32 + lane;
       if (hc >= 2 * HALO * W) continue;
       const int off = hc < HALO * W ? hc : own * W + hc;                    // top halo | bottom halo
       float* px = sX + (size_t)(4 * cq) * PL + off;
-      const float sgn_ = (rep_ == 1) ? -1.f : 1.f;
 #pragma unroll
       for (int cc = 0; cc < 4; ++cc)
-        if (4 * cq + cc != 3) px[(size_t)cc * PL] += sgn_ * s_idle[4 * cq + cc];
+        if (4 * cq + cc != 3) px[(size_t)cc * PL] += s_idle[4 * cq + cc];
     }
     __syncthreads();
     GNCA_PHASE_MARK(5);
-    if (R.dbg_repeat & 32) cluster_barrier();
-    if (R.dbg_repeat & 64) { for (int q_ = 0; q_ < 10; ++q_) __syncthreads(); }
-    if (!(R.dbg_skip & 16)) cluster_barrier();                                // barrier 2
+    cluster_sync_no_acquire();                                                // barrier 2
     GNCA_PHASE_MARK(6);
     // ---- P4: post-alive gate on own cells; push gated alpha rows + active cells' channels to the halos -------
-    for (int rep_ = 0; rep_ < ((R.dbg_repeat & 16) ? 2 : 1); ++rep_)
-    for (int oc = tid; oc < ((R.dbg_skip & 8) ? 0 : nown); oc += kRThreads) {
+    for (int oc = tid; oc < nown; oc += kRThreads) {
       const int orow = s_oy[oc], x = s_ox[oc];
       const bool post = alive_local(sAt, 1 + orow, x, r0 + orow, a.alpha_thr);
       const float v = post ? sAt[W + oc] : 0.f;
@@ -612,14 +591,14 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
     }
     __syncthreads();
     GNCA_PHASE_MARK(7);
-    if (!(R.dbg_skip & 16)) cluster_barrier();                                // barrier 3
+    cluster_sync_no_acquire();                                                // barrier 3
     GNCA_PHASE_MARK(9);
   }
 
   if (R.hist) store_own(R.hist + (size_t)R.T * a.B * C * HW + sample_off);
   store_own(R.xT + sample_off);
   if (R.dbg && blockIdx.x == R.dbg_cta && tid < 16) R.dbg[tid] = s_dbg[tid];
-  cluster_barrier();     // nobody exits while a neighbour may still address its shared memory
+  cluster_sync_no_acquire();     // nobody exits while a neighbour may still address its shared memory
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -708,8 +687,6 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
               own, halo, MB, smem, nclusters);
     R.NC = NC; R.own_rows = own; R.halo = halo; R.MB = MB; R.plane_stride = plane_stride_of(own, halo, W);
     R.inv_n = 1.0 / ((double)C * (double)H * (double)W);
-    if (getenv("GNCA_SKIP")) R.dbg_skip = atoi(getenv("GNCA_SKIP"));
-    if (getenv("GNCA_REPEAT")) R.dbg_repeat = atoi(getenv("GNCA_REPEAT"));
     static unsigned long long* dbg_buf = nullptr;
     if (getenv("GNCA_PHASE_TIMING")) {
       if (!dbg_buf) cudaMalloc(&dbg_buf, 16 * sizeof(unsigned long long));

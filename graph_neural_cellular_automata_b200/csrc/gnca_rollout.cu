@@ -3,7 +3,6 @@
 //                       no host synchronisation inside the loop, so the whole call can sit in a CUDA graph.
 //   impl 2 (resident):  cluster kernel of gnca_resident.cu (state stays in shared memory across steps).
 // BPTT stores only x_t (x_hist); u, the hidden layer, masks and the message are recomputed in the backward.
-#include <cstdlib>
 #include "gnca_common.cuh"
 #include "gnca_internal.h"
 
@@ -98,9 +97,8 @@ int gnca_rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int H,
     // auto: small samples (the launch-latency-bound regime) go to the cluster-resident kernel
     const bool want = impl == 2 || impl == 3 || (size_t)H * W <= 16384;
     if (want) {
-      const char* kind = getenv("GNCA_RESIDENT_KIND");      // development: "band" forces the banded kernel
       int rc = GNCA_ERR_UNSUPPORTED;
-      if (impl != 3 && !(kind && kind[0] == 'b'))
+      if (impl != 3)
         rc = run_rep_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, x_hist_dev, stats_hist_dev, u_hist_dev,
                          nullptr, nullptr, r.ping, st);
       if (rc == GNCA_ERR_UNSUPPORTED)

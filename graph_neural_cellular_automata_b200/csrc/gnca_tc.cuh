@@ -1,4 +1,5 @@
-// tcgen05 / TMEM / mbarrier helpers (sm_100a inline PTX) shared by the tensor-core kernels of the library.
+// tcgen05 / TMEM helpers (sm_100a inline PTX) of the tensor-core kernels of the library; the mbarrier and fence
+// primitives they use are in gnca_ptx.cuh.
 //
 // Operand conventions used throughout (validated on a B200 by scratch/umma_probe.cu, profiles/r02_umma_probe.md):
 //  * kind::tf32, cta_group::1, M = 128: accumulator row m lives in TMEM lane m, column n in TMEM column base + n.
@@ -12,11 +13,10 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "gnca_ptx.cuh"
 
 namespace gnca {
 namespace tc {
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
 // float index of element (r, k) of an [R x K] operand in the canonical no-swizzle K-major layout (R % 8 == 0, K % 4 == 0)
 __host__ __device__ __forceinline__ int canon_idx(int r, int k, int K) {
@@ -50,23 +50,10 @@ __device__ __forceinline__ void mma_ss(uint32_t d_tmem, uint64_t adesc, uint64_t
 __device__ __forceinline__ void mma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" :: "r"(bar) : "memory");
 }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_init_fence() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  do {
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
-                 : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  } while (!ok);
-}
 __device__ __forceinline__ void fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-// generic-proxy writes to shared memory -> visible to the async proxy (UMMA operand reads)
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 // whole-warp: allocate / free `cols` TMEM columns (power of two >= 32); the base address lands in *slot (shared memory)
 __device__ __forceinline__ void tmem_alloc(uint32_t* slot, uint32_t cols) {

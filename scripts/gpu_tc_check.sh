@@ -1,7 +1,7 @@
 #!/bin/bash
-# scale-shape parity tests + the c5s bench line: TMA-tiled tensor-core k_update (default), compacted tensor-core (GNCA_TC_V1=1), FFMA (GNCA_NO_TC=1)
+# scale-shape parity tests + the c5s bench line: compacted tensor-core k_update (default), FFMA (GNCA_NO_TC=1)
 timeout 600 python -m pytest tests/test_gpu_scale.py tests/test_gpu_step.py -x -q -m gpu > gpurun_out/tc_scale_test.log 2>&1; tail -6 gpurun_out/tc_scale_test.log
-for v in GNCA_NONE=1 GNCA_TC_V2=1 GNCA_NO_TC=1; do
+for v in GNCA_NONE=1 GNCA_NO_TC=1; do
   env $v timeout 200 python bench.py --workload c5s --steps 5 --warmup 3 --no-cpu-baseline 2> gpurun_out/tc_c5s.err | python -c "
 import json,sys
 d=[json.loads(l) for l in sys.stdin if l.startswith('{')][-1]

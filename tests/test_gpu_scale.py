@@ -42,14 +42,12 @@ def _blobs(B):
     return x
 
 
-@pytest.mark.parametrize("kernel", ["tc", "tc2_tma", "ffma"])
+@pytest.mark.parametrize("kernel", ["tc", "ffma"])
 def test_one_step_vs_oracle_at_scale(kernel, monkeypatch):
-    """All three k_update variants of the large-problem path: compacted tensor-core tiles (default), dense TMA-staged
-    tensor-core tiles (GNCA_TC_V2=1), the round-1 FFMA kernel (GNCA_NO_TC=1)."""
-    monkeypatch.delenv("GNCA_TC_V2", raising=False); monkeypatch.delenv("GNCA_NO_TC", raising=False)
-    if kernel == "tc2_tma":
-        monkeypatch.setenv("GNCA_TC_V2", "1")
-    elif kernel == "ffma":
+    """Both k_update variants of the large-problem path: compacted tensor-core tiles (default), the round-1 FFMA kernel
+    (GNCA_NO_TC=1)."""
+    monkeypatch.delenv("GNCA_NO_TC", raising=False)
+    if kernel == "ffma":
         monkeypatch.setenv("GNCA_NO_TC", "1")
     m, p = _model()
     B = 5                                            # 5 * 64 chunks >= 2 * 148 blocks: the balanced large-problem path
@@ -113,7 +111,7 @@ def test_large_problem_path_at_the_grid_edges(Hh, Ww, B, kernel, monkeypatch):
     """The blobs of the tests above never touch the border.  Here the whole grid is alive except a dead band in the
     middle: every edge / corner cell runs the zero-halo perception (clamped taps + selects; the 8-byte tap pairs when W is
     even, the scalar taps at W = 75) and the torus wrap of the sender gather in the large-problem kernels."""
-    monkeypatch.delenv("GNCA_TC_V2", raising=False); monkeypatch.delenv("GNCA_NO_TC", raising=False)
+    monkeypatch.delenv("GNCA_NO_TC", raising=False)
     if kernel == "ffma":
         monkeypatch.setenv("GNCA_NO_TC", "1")
     torch.manual_seed(9); random.seed(9)
