@@ -194,21 +194,26 @@ __global__ void k_bwd_affine_reduce(BwdArgs A, float* __restrict__ gparams) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// Shared-memory plan of k_bwd_mlp.  WG = false stages W1T and W1 next to W2; WG = true reads those two from global memory
+// (L1-cached), for the C = 32 models with a hidden layer wide enough (>= 164 graph, >= 180 classic) that the staged plan
+// exceeds the 226 KB a block may use.
 template <int C>
 struct BwdSmem {
   using K = BwdCfg<C>;
-  static size_t floats(int hid, bool graph) {
-    size_t f = (size_t)3 * C * hid + pad4(hid) + (size_t)C * hid + (size_t)hid * 3 * C;   // W1T, b1, W2, W1
+  static size_t floats(int hid, bool graph, bool wg) {
+    size_t f = (wg ? 0 : (size_t)2 * 3 * C * hid) + pad4(hid) + (size_t)C * hid;            // [W1T, W1,] b1, W2
     f += C;                                                                                // gamma
     if (graph) f += C * C + C;                                                             // Wm, bm
     f += (size_t)(3 * C + C + 2 * hid) * K::NBP;                                           // Yt, GDt, Ht, GHt
     if (graph) f += (size_t)(3 * C + 2) * K::NBP;                                          // XSt, GAt, GXSt, AS, GB
     return f;
   }
-  static size_t bytes(int hid, bool graph) {
-    return floats(hid, graph) * sizeof(float) + kBChunk * sizeof(uint16_t) + K::NB * sizeof(int);
+  static size_t bytes(int hid, bool graph, bool wg) {
+    return floats(hid, graph, wg) * sizeof(float) + kBChunk * sizeof(uint16_t) + K::NB * sizeof(int);
   }
 };
+
+constexpr size_t kBwdSmemLimit = 226 * 1024;
 
 // Accumulation into a partial that ONE thread owns (this block's weight-gradient slot / this chunk's dL/dw slot): a
 // reduction without return value instead of load - add - store.  The thread does not wait for the L2 round trip (the
@@ -223,7 +228,7 @@ __device__ __forceinline__ float dot4(const float4& a, const float4& b) {
   return fmaf(a.x, b.x, fmaf(a.y, b.y, fmaf(a.z, b.z, a.w * b.w)));
 }
 
-template <int C, int CH>
+template <int C, int CH, bool WG>
 __global__ void __launch_bounds__(kBThreads, 2) k_bwd_mlp(BwdArgs A, Packed P, int hid, const float* __restrict__ packed) {
   using K = BwdCfg<C>;
   constexpr int NB = K::NB, NBP = K::NBP, TPC = K::TPC, CQ = K::CQ, C3 = 3 * C;
@@ -239,10 +244,17 @@ __global__ void __launch_bounds__(kBThreads, 2) k_bwd_mlp(BwdArgs A, Packed P, i
 
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* sW1T = reinterpret_cast<float*>(smem_raw);
-  float* sb1 = sW1T + C3 * hid;
+  float* sb1 = sW1T + (WG ? 0 : C3 * hid);
   float* sW2 = sb1 + pad4(hid);
   float* sW1 = sW2 + C * hid;
-  float* sgam = sW1 + hid * C3;
+  float* sgam = sW1 + (WG ? 0 : hid * C3);
+  // W1T / W1 rows as float4: shared memory, or the packed buffer in global memory (WG)
+  const float* W1T = WG ? packed + P.w1t : sW1T;
+  const float* W1 = WG ? packed + P.w1 : sW1;
+  auto w4 = [](const float* p) -> float4 {
+    if constexpr (WG) return __ldg(reinterpret_cast<const float4*>(p));
+    else return *reinterpret_cast<const float4*>(p);
+  };
   float* sWm = sgam + C;
   float* sbm = sWm + (graph ? C * C : 0);
   float* Yt = sbm + (graph ? C : 0);
@@ -262,10 +274,10 @@ __global__ void __launch_bounds__(kBThreads, 2) k_bwd_mlp(BwdArgs A, Packed P, i
   __shared__ int s_ody[GNCA_MAX_K], s_odx[GNCA_MAX_K];      // the step's sender offsets (reduced modulo the grid on a torus)
   __shared__ float s_owt[GNCA_MAX_K];                        // and the sample's weights
 
-  block_copy(sW1T, packed + P.w1t, C3 * hid);
+  if (!WG) block_copy(sW1T, packed + P.w1t, C3 * hid);
   block_copy(sb1, packed + P.b1, pad4(hid));
   block_copy(sW2, packed + P.w2, C * hid);
-  block_copy(sW1, packed + P.w1, hid * C3);
+  if (!WG) block_copy(sW1, packed + P.w1, hid * C3);
   if (threadIdx.x < C) sgam[threadIdx.x] = packed[P.gamma + threadIdx.x];
   if (graph) { block_copy(sWm, packed + P.wm, C * C); block_copy(sbm, packed + P.bm, C); }
   __syncthreads();
@@ -458,7 +470,7 @@ __global__ void __launch_bounds__(kBThreads, 2) k_bwd_mlp(BwdArgs A, Packed P, i
 #pragma unroll 4
           for (int k = 0; k < C3; ++k) {
             const float4 yv = *reinterpret_cast<const float4*>(Yt + k * NBP + 4 * cg);
-            const float4 w = *reinterpret_cast<const float4*>(sW1T + k * hid + j);
+            const float4 w = w4(W1T + k * hid + j);
             const float ym[4] = {yv.x, yv.y, yv.z, yv.w};
 #pragma unroll
             for (int m = 0; m < 4; ++m) {
@@ -508,7 +520,7 @@ __global__ void __launch_bounds__(kBThreads, 2) k_bwd_mlp(BwdArgs A, Packed P, i
 #pragma unroll 4
           for (int j = 0; j < hid; ++j) {
             const float4 gv = *reinterpret_cast<const float4*>(GHt + j * NBP + 4 * cg);
-            const float4 w = *reinterpret_cast<const float4*>(sW1 + j * C3 + 4 * kq);
+            const float4 w = w4(W1 + j * C3 + 4 * kq);
             const float gm[4] = {gv.x, gv.y, gv.z, gv.w};
 #pragma unroll
             for (int m = 0; m < 4; ++m) {
@@ -793,21 +805,10 @@ static BwdWorkspace carve_bwd(void* base, const gnca_model& m, int B, int H, int
 
 size_t bwd_workspace_bytes(const gnca_model& m, int B, int H, int W) { return carve_bwd(nullptr, m, B, H, W).bytes; }
 
-template <int C>
-static int launch_step_bwd(const gnca_model& m, const Packed& P, const float* packed, BwdArgs& A, float* gparams,
-                           cudaStream_t st) {
-  const StepArgs& a = A.s;
-  const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
-  dim3 g1(A.ntiles, a.B);
-  k_bwd_norm<C><<<g1, kBThreads, 0, st>>>(A, P, packed);
-  GNCA_LAUNCH_CHECK();
-  k_bwd_stats<C><<<a.B, 128, 0, st>>>(A, gparams);
-  GNCA_LAUNCH_CHECK();
-  k_bwd_affine_reduce<C><<<1, 64, 0, st>>>(A, gparams);
-  GNCA_LAUNCH_CHECK();
-  const size_t smem = BwdSmem<C>::bytes(m.hidden, graph);
-  if (smem > 226 * 1024) return GNCA_ERR_UNSUPPORTED;
-  // persistent blocks: as many as are resident at once (two per SM when the shared memory of a block allows it)
+// persistent blocks: as many as are resident at once (two per SM when the shared memory of a block allows it)
+template <int C, int CH, bool WG>
+static int launch_bwd_mlp(const gnca_model& m, const Packed& P, const float* packed, const BwdArgs& A, size_t smem,
+                          cudaStream_t st) {
   static int n_sm = 0;
   if (n_sm == 0) {
     int dev = 0;
@@ -815,22 +816,42 @@ static int launch_step_bwd(const gnca_model& m, const Packed& P, const float* pa
     GNCA_CHECK_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
   }
   int per_sm = 1;
+  GNCA_CHECK_CUDA(cudaFuncSetAttribute(k_bwd_mlp<C, CH, WG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bwd_mlp<C, CH, WG>, kBThreads, smem) != cudaSuccess || per_sm < 1) { cudaGetLastError(); per_sm = 1; }
+  const int nblk = min(A.n_items, min(kMaxBwdBlocks, per_sm * n_sm));
+  k_bwd_mlp<C, CH, WG><<<nblk, kBThreads, smem, st>>>(A, P, m.hidden, packed);
+  return 0;
+}
+
+template <int C>
+static int launch_step_bwd(const gnca_model& m, const Packed& P, const float* packed, BwdArgs& A, float* gparams,
+                           cudaStream_t st) {
+  const StepArgs& a = A.s;
+  const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
+  // the shared-memory plan is settled before the first launch: a rejected configuration leaves gparams untouched
+  const bool wg = BwdSmem<C>::bytes(m.hidden, graph, false) > kBwdSmemLimit;
+  const size_t smem = BwdSmem<C>::bytes(m.hidden, graph, wg);
+  if (smem > kBwdSmemLimit) return GNCA_ERR_UNSUPPORTED;
+  dim3 g1(A.ntiles, a.B);
+  k_bwd_norm<C><<<g1, kBThreads, 0, st>>>(A, P, packed);
+  GNCA_LAUNCH_CHECK();
+  k_bwd_stats<C><<<a.B, 128, 0, st>>>(A, gparams);
+  GNCA_LAUNCH_CHECK();
+  k_bwd_affine_reduce<C><<<1, 64, 0, st>>>(A, gparams);
+  GNCA_LAUNCH_CHECK();
   prof_begin(PROF_BWD_MLP, st);
-  if (A.bchunk == kBChunkSmall) {
-    GNCA_CHECK_CUDA(cudaFuncSetAttribute(k_bwd_mlp<C, kBChunkSmall>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bwd_mlp<C, kBChunkSmall>, kBThreads, smem) != cudaSuccess || per_sm < 1) { cudaGetLastError(); per_sm = 1; }
-    const int nblk = min(A.n_items, min(kMaxBwdBlocks, per_sm * n_sm));
-    k_bwd_mlp<C, kBChunkSmall><<<nblk, kBThreads, smem, st>>>(A, P, m.hidden, packed);
-  } else {
-    GNCA_CHECK_CUDA(cudaFuncSetAttribute(k_bwd_mlp<C, kBChunk>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bwd_mlp<C, kBChunk>, kBThreads, smem) != cudaSuccess || per_sm < 1) { cudaGetLastError(); per_sm = 1; }
-    const int nblk = min(A.n_items, min(kMaxBwdBlocks, per_sm * n_sm));
-    k_bwd_mlp<C, kBChunk><<<nblk, kBThreads, smem, st>>>(A, P, m.hidden, packed);
-  }
+  int rc;
+  if (A.bchunk == kBChunkSmall)
+    rc = wg ? launch_bwd_mlp<C, kBChunkSmall, true>(m, P, packed, A, smem, st)
+            : launch_bwd_mlp<C, kBChunkSmall, false>(m, P, packed, A, smem, st);
+  else
+    rc = wg ? launch_bwd_mlp<C, kBChunk, true>(m, P, packed, A, smem, st)
+            : launch_bwd_mlp<C, kBChunk, false>(m, P, packed, A, smem, st);
+  if (rc) return rc;
   prof_end(PROF_BWD_MLP, st);
   GNCA_LAUNCH_CHECK();
   if (A.gw_part) {
-    int rc = run_attn_bwd(m, P, packed, a, A.zp_rowsum, A.zp_scratch, A.nchunks, gparams, st, /*defer_reduce=*/true);
+    rc = run_attn_bwd(m, P, packed, a, A.zp_rowsum, A.zp_scratch, A.nchunks, gparams, st, /*defer_reduce=*/true);
     if (rc) return rc;
   }
   dim3 g3((a.H * a.W + 255) / 256, a.B);

@@ -144,6 +144,7 @@ int gnca_rollout_bwd(const gnca_model* m, const float* packed_dev, int B, int H,
     return GNCA_ERR_ARG;
   if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
   if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
   (void)impl;             // the backward currently always takes the streaming kernels (x_hist layout is shared)
   const bool saved = u_hist_dev != nullptr && stats_hist_dev != nullptr;   // else u and the statistics are recomputed
   const bool graph = (m->flags & GNCA_F_GRAPH) != 0;
@@ -204,6 +205,7 @@ int gnca_rollout_fwd_bptt(const gnca_model* m, const float* packed_dev, int B, i
   if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !bptt_dev || !workspace_dev) return GNCA_ERR_ARG;
   if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
   if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
   const size_t need = gnca_bptt_bytes(m, B, H, W, sched->T);
   if (need == 0) return GNCA_ERR_UNSUPPORTED;
   if (need > bptt_bytes) return GNCA_ERR_WORKSPACE;
@@ -232,6 +234,7 @@ int gnca_rollout_bwd_bptt(const gnca_model* m, const float* packed_dev, int B, i
   if (!m || !packed_dev || !sched || !bptt_dev || !gT_dev || !g0_dev || !gparams_dev || !workspace_dev) return GNCA_ERR_ARG;
   if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
   if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
   const size_t need = gnca_bptt_bytes(m, B, H, W, sched->T);
   if (need == 0) return GNCA_ERR_UNSUPPORTED;
   if (need > bptt_bytes) return GNCA_ERR_WORKSPACE;

@@ -105,12 +105,16 @@ def test_rollout_properties_at_scale():
     assert torch.isfinite(whole).all() and float((whole[:, 3] > 0.1).float().mean()) > 0.01
 
 
-@pytest.mark.parametrize("Hh,Ww,B", [(64, 64, 80), (48, 66, 80), (40, 75, 100)])
+_EDGE_CASES = [(64, 64, 80, 8), (48, 66, 80, 8), (40, 75, 100, 8), (64, 64, 80, 7), (40, 75, 100, 7)]
+
+
+@pytest.mark.parametrize("Hh,Ww,B,k", _EDGE_CASES, ids=[f"{h}-{w}-{b}" + ("" if k == 8 else f"-k{k}") for h, w, b, k in _EDGE_CASES])
 @pytest.mark.parametrize("kernel", ["tc", "ffma"])
-def test_large_problem_path_at_the_grid_edges(Hh, Ww, B, kernel, monkeypatch):
+def test_large_problem_path_at_the_grid_edges(Hh, Ww, B, k, kernel, monkeypatch):
     """The blobs of the tests above never touch the border.  Here the whole grid is alive except a dead band in the
     middle: every edge / corner cell runs the zero-halo perception (clamped taps + selects; the 8-byte tap pairs when W is
-    even, the scalar taps at W = 75) and the torus wrap of the sender gather in the large-problem kernels."""
+    even, the scalar taps at W = 75) and the torus wrap of the sender gather in the large-problem kernels.  k = 7 leaves
+    the last sender pair of the tensor-core gather half empty."""
     monkeypatch.delenv("GNCA_NO_TC", raising=False)
     if kernel == "ffma":
         monkeypatch.setenv("GNCA_NO_TC", "1")
@@ -126,7 +130,7 @@ def test_large_problem_path_at_the_grid_edges(Hh, Ww, B, kernel, monkeypatch):
     x[:, :, Hh // 2 - 4:Hh // 2 + 4, 5:Ww - 5] = 0.0                  # a dead band, not touching the border
     x[::3, 3] *= (torch.rand((B + 2) // 3, Hh, Ww) > 0.3).float()       # ragged alive sets on every third sample
     fu = torch.rand(B, 1, Hh, Ww)
-    chosen = [(4, -4), (-4, 4), (0, 3), (-3, 0), (1, 1), (-2, 4), (4, 0), (0, -4)]       # wraps on every side
+    chosen = [(4, -4), (-4, 4), (0, 3), (-3, 0), (1, 1), (-2, 4), (4, 0), (0, -4)][:k]   # wraps on every side
     cfg = O.StepConfig(update_gain=0.1, alpha_thr=0.1, graph=True, message_gain=0.3, hidden_only=True,
                        zero_padded_shift=False)
     ref = O.nca_step(x.double(), p, cfg, 0.5, fu.double(), chosen)
