@@ -59,16 +59,17 @@ int launch_update_tc(const gnca_model& m, const Packed& P, const float* packed, 
                      const int* prefix, cudaStream_t st);
 
 // cluster-resident forward rollout (gnca_resident.cu); GNCA_ERR_UNSUPPORTED when the configuration has no
-// resident kernel (zero-padded graph shift, sample too large for the cluster's shared memory)
+// resident kernel (zero-padded graph shift, sample too large for the cluster's shared memory).
+// hist: x_t of every step t % hist_every == 0 goes to slot t / hist_every ([T/hist_every+1][B][C][H][W]).
 int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                      const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
-                     float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st);
+                     float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st, int hist_every = 1);
 
 // replicated-state cluster rollout (gnca_rep.cu): every CTA of a sample's cluster holds the whole sample; first
 // choice of the resident path.  scratch: >= B*C*H*W floats of device memory (overflow of the in-smem u buffer).
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
-                float* u_hist, float* rec, uint32_t* masks, float* scratch, cudaStream_t st);
+                float* u_hist, float* rec, uint32_t* masks, float* scratch, cudaStream_t st, int hist_every = 1);
 // resident BPTT on the records of run_rep_fwd (gnca_rep_bwd.cu)
 size_t rep_bptt_bytes(const gnca_model& m, int B, int H, int W, int T);     // 0: configuration not supported
 void rep_bptt_carve(void* base, int B, int H, int W, int T, float** rec, uint32_t** masks, float** stats,

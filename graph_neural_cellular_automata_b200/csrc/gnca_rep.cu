@@ -47,7 +47,8 @@ struct RepArgs {
   const float* fire_u_base;   // [T][B][H][W] or null
   const float* x0;
   float* xT;
-  float* hist;                // [T+1][B][C][HW] or null
+  float* hist;                // [T/hist_every+1][B][C][HW] or null: x_t of the steps t % hist_every == 0, in slot t/hist_every
+  int hist_every;
   float* stats_hist;          // [T][B][2] or null
   float* u_hist;              // [T][B][C][HW] or null (dense layout, active cells only)
   float* rec;                 // [T][B][HW][kRecStride] or null: per-active-cell records for the resident backward
@@ -199,6 +200,10 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
     const int n = (hi - lo + 7) & ~7;
 #pragma unroll 1
     for (int i = tid; i < n * C; i += kPT) store_item(dst, lo, hi, i);
+  };
+  auto hist_at = [&](int t) -> float* {                       // history slot of x_t, or null when step t is not kept
+    if (!R.hist || t % R.hist_every != 0) return nullptr;
+    return R.hist + (size_t)(t / R.hist_every) * a.B * C * HW + sample_off;
   };
   {
     const int n8 = (HW + 7) & ~7;
@@ -407,7 +412,7 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
       prepare_from_state(t);
     }
     if (t >= my_steps) {                         // frozen sample (whole cluster agrees): state passes through
-      if (R.hist) store_state(R.hist + (size_t)t * a.B * C * HW + sample_off, my_lo, my_hi);
+      if (float* h = hist_at(t)) store_state(h, my_lo, my_hi);
       continue;
     }
     const float gain_m = s_gain[cur];
@@ -708,12 +713,12 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
     const bool dmg_now = R.damage.p && t == R.damage_step;
     auto side_jobs = [&](const bool fire, const bool hist) {
       const int nf = (t + 1 < R.T) ? n_fire_tasks : 0;
-      float* hdst = R.hist ? R.hist + (size_t)t * a.B * C * HW + sample_off : nullptr;
+      float* hdst = hist_at(t);
       if (fire) {
 #pragma unroll 1
         for (int task = kPW - 1 - warp; task < nf; task += kPW - 1) fire_task(task, t + 1, cur ^ 1, sparse_fire && t >= 1 && !dmg_now);
       }
-      if (hist) {
+      if (hist && hdst) {
 #pragma unroll 1
         for (int task = warp - 1; task < n_hist_tasks; task += kPW - 1) {
 #pragma unroll
@@ -899,7 +904,7 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
   }
 
   __syncthreads();
-  if (R.hist) store_state(R.hist + (size_t)R.T * a.B * C * HW + sample_off, my_lo, my_hi);
+  if (float* h = hist_at(R.T)) store_state(h, my_lo, my_hi);
   store_state(R.xT + sample_off, my_lo, my_hi);
   if (R.dbg && blockIdx.x == R.dbg_cta && tid < 24) R.dbg[tid] = s_dbg[tid];
   cluster_arrive(); cluster_wait();      // nobody exits while a peer may still address its shared memory
@@ -917,7 +922,8 @@ static size_t rep_smem_bytes(int C, int HW, int ucap, int listcap) {
 
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
-                float* u_hist, float* rec, uint32_t* masks, float* scratch /* >= B*C*H*W floats */, cudaStream_t st) {
+                float* u_hist, float* rec, uint32_t* masks, float* scratch /* >= B*C*H*W floats */, cudaStream_t st,
+                int hist_every) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (m.C != 16 || m.hidden != 128) return GNCA_ERR_UNSUPPORTED;
   if (H > kMaxRows || W > kMaxRows || H < 1 || W < 4 || (W & 3)) return GNCA_ERR_UNSUPPORTED;   // quads of 4 cells per row
@@ -942,7 +948,7 @@ int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B
   R.s.philox_offset = sched.philox_offset;
   R.fire_u_base = sched.fire_u;
   R.T = sched.T;
-  R.x0 = x0; R.xT = xT; R.hist = hist; R.stats_hist = stats_hist; R.u_hist = u_hist;
+  R.x0 = x0; R.xT = xT; R.hist = hist; R.hist_every = hist_every; R.stats_hist = stats_hist; R.u_hist = u_hist;
   R.rec = rec; R.masks = masks;
   R.damage = DamageView{sched.damage, sched.damage_layout}; R.damage_step = sched.damage_step;
   R.KP = k > 8 ? 16 : 8;

@@ -36,7 +36,8 @@ struct ResidentArgs {
   const float* fire_u_base;   // [T][B][H][W] or null
   const float* x0;
   float* xT;
-  float* hist;                // [T+1][B][C][HW] or null
+  float* hist;                // [T/hist_every+1][B][C][HW] or null: x_t of the steps t % hist_every == 0, in slot t/hist_every
+  int hist_every;
   float* stats_hist;          // [T][B][2] or null
   float* u_hist;              // [T][B][C][HW] or null: masked pre-norm update of the active cells (for the backward)
   DamageView damage;          // schedule.damage (dense or plane) or null
@@ -201,6 +202,9 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
       for (int oc = tid; oc < nown; oc += kRThreads)
         dst[(size_t)c * HW + r0 * W + oc] = sX[(size_t)c * PL + HALO * W + oc];
   };
+  auto store_hist = [&](int t) {        // x_t into its history slot when step t is kept
+    if (R.hist && t % R.hist_every == 0) store_own(R.hist + (size_t)(t / R.hist_every) * a.B * C * HW + sample_off);
+  };
   auto alive_local = [&](const float* plane, int lr, int x, int gy, float thr) {
     return alive_local_ool(plane, lr, x, gy, H, W, thr);
   };
@@ -216,7 +220,7 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
       }
       __syncthreads();
     }
-    if (R.hist) store_own(R.hist + (size_t)t * a.B * C * HW + sample_off);
+    store_hist(t);
     if (t >= my_steps) continue;               // frozen sample (whole cluster agrees): state passes through
     a.t = t;
     a.fire_u = R.fire_u_base ? R.fire_u_base + (size_t)t * a.B * HW : nullptr;
@@ -595,7 +599,7 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
     GNCA_PHASE_MARK(9);
   }
 
-  if (R.hist) store_own(R.hist + (size_t)R.T * a.B * C * HW + sample_off);
+  store_hist(R.T);
   store_own(R.xT + sample_off);
   if (R.dbg && blockIdx.x == R.dbg_cta && tid < 16) R.dbg[tid] = s_dbg[tid];
   cluster_sync_no_acquire();     // nobody exits while a neighbour may still address its shared memory
@@ -717,7 +721,7 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
 // entry used by gnca_rollout_fwd (impl 2 / auto)
 int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                      const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
-                     float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st) {
+                     float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st, int hist_every) {
   (void)ping; (void)pong; (void)alpha_tmp;
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (graph && !(m.flags & GNCA_F_TORUS) && sched.k > 0) return GNCA_ERR_UNSUPPORTED;   // zero-pad: streaming path
@@ -733,7 +737,7 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
   R.s.philox_offset = sched.philox_offset;
   R.fire_u_base = sched.fire_u;
   R.T = sched.T;
-  R.x0 = x0; R.xT = xT; R.hist = hist; R.stats_hist = stats_hist; R.u_hist = u_hist;
+  R.x0 = x0; R.xT = xT; R.hist = hist; R.hist_every = hist_every; R.stats_hist = stats_hist; R.u_hist = u_hist;
   R.damage = DamageView{sched.damage, sched.damage_layout}; R.damage_step = sched.damage_step;
   const int radius = sched.max_offset;       // largest |dy| / |dx| in the schedule: sets the halo depth
   switch (m.C) {

@@ -61,24 +61,11 @@ static void schedule_to_args(StepArgs& a, const gnca_schedule& s, int t, int B, 
   a.philox_offset = s.philox_offset;
 }
 
-}  // namespace gnca
-
-using namespace gnca;
-
-extern "C" {
-
-size_t gnca_rollout_workspace_bytes(const gnca_model* m, int B, int H, int W, int T) {
-  (void)T;
-  if (!m || B <= 0 || H <= 0 || W <= 0) return 0;
-  const size_t a = carve_rollout(nullptr, *m, B, H, W).bytes;
-  const size_t b = (m->C == 16) ? rep_bwd_workspace_bytes(*m, B, H, W) : 0;
-  return a > b ? a : b;
-}
-
-int gnca_rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
-                     const float* x0_dev, float* xT_dev, float* x_hist_dev, float* stats_hist_dev, float* u_hist_dev,
-                     void* workspace_dev,
-                     size_t workspace_bytes, int impl, void* stream) {
+// gnca_rollout_fwd with a strided history: x_t of every step t % every == 0 goes to x_hist slot t / every
+// (every == 1: the full [T+1] history of gnca_rollout_fwd).
+static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
+                       const float* x0_dev, float* xT_dev, float* x_hist_dev, int every, float* stats_hist_dev,
+                       float* u_hist_dev, void* workspace_dev, size_t workspace_bytes, int impl, void* stream) {
   if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !workspace_dev) return GNCA_ERR_ARG;
   if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
   if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
@@ -100,17 +87,18 @@ int gnca_rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int H,
       int rc = GNCA_ERR_UNSUPPORTED;
       if (impl != 3)
         rc = run_rep_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, x_hist_dev, stats_hist_dev, u_hist_dev,
-                         nullptr, nullptr, r.ping, st);
+                         nullptr, nullptr, r.ping, st, every);
       if (rc == GNCA_ERR_UNSUPPORTED)
         rc = run_resident_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, x_hist_dev, stats_hist_dev,
-                              u_hist_dev, r.ping, r.pong, r.alpha_tmp, st);
+                              u_hist_dev, r.ping, r.pong, r.alpha_tmp, st, every);
       if (rc != GNCA_ERR_UNSUPPORTED || impl == 2 || impl == 3) return rc;
     }
   }
 
-  // where x_t lives: x_hist slices when a history is requested, else ping/pong (x_T straight into xT_dev)
+  // where x_t lives: its x_hist slot when step t is kept, else ping/pong (x_T straight into xT_dev).  A step reads x_t
+  // and writes x_{t+1}: two history slots, or a slot and the ping/pong buffer of the other parity -- never one buffer.
   auto x_at = [&](int t) -> float* {
-    if (x_hist_dev) return x_hist_dev + (size_t)t * N;
+    if (x_hist_dev && t % every == 0) return x_hist_dev + (size_t)(t / every) * N;
     if (t == T) return xT_dev;
     return (t & 1) ? r.pong : r.ping;
   };
@@ -131,8 +119,73 @@ int gnca_rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int H,
     int rc = dispatch_step_fwd(*m, P, packed_dev, a, fws, nullptr, st);
     if (rc) return rc;
   }
-  if (x_hist_dev || T == 0)
+  if ((x_hist_dev && T % every == 0) || T == 0)
     GNCA_CHECK_CUDA(cudaMemcpyAsync(xT_dev, x_at(T), N * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  return 0;
+}
+
+}  // namespace gnca
+
+using namespace gnca;
+
+extern "C" {
+
+size_t gnca_rollout_workspace_bytes(const gnca_model* m, int B, int H, int W, int T) {
+  (void)T;
+  if (!m || B <= 0 || H <= 0 || W <= 0) return 0;
+  const size_t a = carve_rollout(nullptr, *m, B, H, W).bytes;
+  const size_t b = (m->C == 16) ? rep_bwd_workspace_bytes(*m, B, H, W) : 0;
+  return a > b ? a : b;
+}
+
+int gnca_rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
+                     const float* x0_dev, float* xT_dev, float* x_hist_dev, float* stats_hist_dev, float* u_hist_dev,
+                     void* workspace_dev, size_t workspace_bytes, int impl, void* stream) {
+  return rollout_fwd(m, packed_dev, B, H, W, sched, x0_dev, xT_dev, x_hist_dev, 1, stats_hist_dev, u_hist_dev,
+                     workspace_dev, workspace_bytes, impl, stream);
+}
+
+int gnca_record_frames(int T, int every) {
+  if (T < 0 || every <= 0) return GNCA_ERR_ARG;
+  return T / every + 1;
+}
+
+int gnca_rollout_record(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
+                        const float* x0_dev, float* xT_dev, int every, float* frames_dev, float* attn_dev,
+                        void* workspace_dev, size_t workspace_bytes, int impl, void* stream) {
+  if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !frames_dev || !workspace_dev) return GNCA_ERR_ARG;
+  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0 || every <= 0) return GNCA_ERR_ARG;
+  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  const bool graph = (m->flags & GNCA_F_GRAPH) != 0;
+  if (attn_dev && !graph) return GNCA_ERR_ARG;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
+  int rc = rollout_fwd(m, packed_dev, B, H, W, sched, x0_dev, xT_dev, frames_dev, every, nullptr, nullptr,
+                       workspace_dev, workspace_bytes, impl, stream);
+  if (rc || !attn_dev) return rc;
+  // Attention map of every recorded step t = f * every < T, from the frame (the state step t consumes) and step t's
+  // offsets -- the map gnca_step_fwd returns for that step.  Every sample gets one, frozen ones included, whatever the
+  // step's fire rate and message gain: the map depends on neither.
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t N = (size_t)B * m->C * H * W;
+  const Packed P = make_packed(m->C, m->hidden, m->d_model, graph);
+  const FwdWorkspace fws = carve_fwd_workspace(carve_rollout(workspace_dev, *m, B, H, W).step_ws, *m, B, H, W);
+  const bool zero_pad = !(m->flags & GNCA_F_TORUS);
+  for (int f = 0; (size_t)f * every < (size_t)sched->T; ++f) {
+    StepArgs a;
+    fill_step_args(a, *m, B, H, W);
+    schedule_to_args(a, *sched, f * every, B, H, W);
+    a.steps = nullptr;
+    a.fire_u = nullptr;
+    a.x_in = frames_dev + (size_t)f * N;
+    a.partials = fws.partials;
+    a.attn_w = nullptr;
+    if (zero_pad && a.k > 0) {
+      rc = run_attn_prepass(*m, P, packed_dev, a, fws, st);
+      if (rc) return rc;
+    }
+    rc = run_attn_map(*m, P, packed_dev, a, fws, attn_dev + (size_t)f * B * H * W, st);
+    if (rc) return rc;
+  }
   return 0;
 }
 

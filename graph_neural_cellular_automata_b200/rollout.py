@@ -319,3 +319,49 @@ def rollout(model, x0: torch.Tensor, schedule: Schedule, *, return_history: bool
     cfg = {"desc": model.model_desc(), "packed": model.packed_weights(), "schedule": schedule, "need_grad": need_grad,
            "history": bool(return_history), "impl": IMPL[impl]}
     return _RolloutFn.apply(x0, cfg, *ps)
+
+
+@dataclass
+class Trajectory:
+    """What `record_rollout` returns.  `states[f]` is x_{t[f]}, the state step t[f] consumes (after the schedule's
+    damage at `damage_step`); `attention[f]` is the attention map of step t[f] for every step t[f] < T (None when not
+    asked for); `x_T` is the final state, also when T is not a multiple of the stride."""
+    t: List[int]                            # recorded step indices 0, S, 2S, ... <= T
+    states: torch.Tensor                    # [F,B,C,H,W], F = T // S + 1
+    attention: Optional[torch.Tensor]       # [FA,B,H,W], FA = ceil(T / S)
+    x_T: torch.Tensor                       # [B,C,H,W]
+
+
+def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, attention: bool = False,
+                   impl: str = "auto") -> Trajectory:
+    """T steps from x0 under `schedule` in one library call (gnca_rollout_record), keeping x_t every `every` steps and,
+    with `attention=True`, the attention map `model.step(x_t, ..., return_attention=True)` gives for each kept step
+    t < T.  Watching a rollout this way keeps the fused rollout kernels; no gradient history or record buffer is
+    allocated, and the outputs are detached."""
+    every = int(every)
+    if every < 1:
+        raise ValueError(f"record_rollout: every must be >= 1, got {every}")
+    if attention and not getattr(model, "_is_graph", False):
+        raise ValueError("record_rollout: attention maps need a graph model (NeuralCAGraph)")
+    if not x0.is_cuda:
+        raise RuntimeError(f"record_rollout: x0 is on {x0.device}; CUDA (sm_100a) only, no CPU fallback")
+    desc = model.model_desc()
+    x0 = GF._require_cuda_f32(x0.detach(), "x0")
+    B, Cc, H, W = x0.shape
+    if Cc != desc.C:
+        raise ValueError(f"x0 has {Cc} channels, model has {desc.C}")
+    lib = _lib.load()
+    T = schedule.T
+    F = lib.gnca_record_frames(T, every)
+    if F < 0:
+        _lib.check(F, "gnca_record_frames")
+    FA = -(-T // every)
+    xT = torch.empty_like(x0)
+    frames = torch.empty(F, B, Cc, H, W, dtype=torch.float32, device=x0.device)
+    attn = torch.empty(FA, B, H, W, dtype=torch.float32, device=x0.device) if attention else None
+    ws = GF._WS.get(x0.device, lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, T))
+    cs = schedule.c_struct()
+    _lib.check(lib.gnca_rollout_record(C.byref(desc), GF._ptr(model.packed_weights()), B, H, W, C.byref(cs),
+                                       GF._ptr(x0), GF._ptr(xT), every, GF._ptr(frames), GF._ptr(attn), GF._ptr(ws),
+                                       ws.numel(), IMPL[impl], GF._stream()), "gnca_rollout_record")
+    return Trajectory(t=list(range(0, T + 1, every)), states=frames, attention=attn, x_T=xT)

@@ -10,6 +10,7 @@
  *   NeuralCA.forward                  src/modules/nca.py:64-105                  -> gnca_step_fwd/_bwd (GNCA_F_GRAPH clear)
  *   NeuralCAGraph.forward             src/modules/ncagraph.py:106-168            -> gnca_step_fwd/_bwd (GNCA_F_GRAPH set)
  *   the rollout loop                  src/training/train_graph_augmented_nca.py:302-324 -> gnca_rollout_fwd/_bwd
+ *   the recording loop                test_graph_augmented_regeneration.py:183-194     -> gnca_rollout_record
  *   loss_premult_rgba (+ its grad)    src/training/train_graph_augmented_nca.py:52-61,337-339 -> gnca_loss_premult_rgba
  *   grad normalise + Adam             src/training/train_graph_augmented_nca.py:370-375 -> gnca_normalize_adam
  *   multiplicative damage             src/utils/damage.py:16-98                  -> gnca_apply_mask
@@ -36,7 +37,7 @@
 extern "C" {
 #endif
 
-#define GNCA_VERSION 104
+#define GNCA_VERSION 105
 
 #define GNCA_ERR_ARG (-1)         /* null pointer / bad size */
 #define GNCA_ERR_UNSUPPORTED (-2) /* shape or flag combination without a kernel */
@@ -197,6 +198,26 @@ int gnca_rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int H,
                      const gnca_schedule* sched, const float* x0_dev, float* xT_dev,
                      float* x_hist_dev, float* stats_hist_dev, float* u_hist_dev,
                      void* workspace_dev, size_t workspace_bytes, int impl, void* stream);
+
+/*
+ * Recording rollout for inference: the T steps of gnca_rollout_fwd (same `impl`, dispatch and fallbacks, same
+ * GNCA_ERR_UNSUPPORTED combinations), keeping every `every`-th state and, optionally, the attention map of each kept step.
+ *   - frames: F = gnca_record_frames(T, every) = T / every + 1; frames_dev[f] ([F][B][C][H][W]) = x_{f*every}, the
+ *     state step f*every consumes (after the schedule's damage when f*every == damage_step).  A frozen sample
+ *     (steps[b] <= t) shows its frozen state.  xT_dev always receives x_T, whether or not T % every == 0.
+ *   - attention (attn_dev != NULL, graph models only): FA = ceil(T / every) maps, one per kept step f*every < T;
+ *     attn_dev[f] ([FA][B][H][W]) is exactly the attention map gnca_step_fwd returns for x_{f*every} with that step's
+ *     offsets (and, zero-padded shift, the per-sample softmax weights of that state).  It is computed for every
+ *     sample, frozen ones included, and depends on neither the fire rate nor the message gain of the step.
+ *   - T == 0: F = 1 (x_0) and FA = 0; every > T: F = 1.
+ * No BPTT buffers: the workspace is the one of gnca_rollout_workspace_bytes.  Argument errors (every <= 0, frames_dev
+ * NULL, attention on a classic model; k outside [0, GNCA_MAX_K] is GNCA_ERR_UNSUPPORTED) return before any launch.
+ */
+int gnca_record_frames(int T, int every); /* T / every + 1, or GNCA_ERR_ARG (T < 0, every <= 0) */
+int gnca_rollout_record(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                        const gnca_schedule* sched, const float* x0_dev, float* xT_dev,
+                        int every, float* frames_dev, float* attn_dev,
+                        void* workspace_dev, size_t workspace_bytes, int impl, void* stream);
 
 /* BPTT: given gT = dL/dx_T and the x_hist of the forward, produce g0 = dL/dx_0 and ACCUMULATE gparams. */
 int gnca_rollout_bwd(const gnca_model* m, const float* packed_dev, int B, int H, int W,
