@@ -13,7 +13,7 @@ LIB_PATH = os.path.join(_PKG, "lib", "libgnca.so")
 GNCA_F_GRAPH, GNCA_F_TORUS, GNCA_F_HIDDEN_ONLY, GNCA_F_ALIVE_TO_ALIVE, GNCA_F_GROUPNORM = 1, 2, 4, 8, 16
 GNCA_MAX_K = 64
 GNCA_ERR_ARG, GNCA_ERR_UNSUPPORTED = -1, -2
-GNCA_VERSION = 105
+GNCA_VERSION = 106
 
 
 class GncaModel(C.Structure):
@@ -80,6 +80,10 @@ EXPORTS = {
     "gnca_rollout_bwd": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
                                    C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
+    "gnca_rollout_bwd_frames": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                          C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                          C.c_int, C.c_void_p]),
     "gnca_bptt_bytes": (C.c_size_t, [C.POINTER(GncaModel), C.c_int, C.c_int, C.c_int, C.c_int]),
     "gnca_rollout_fwd_bptt": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
                                         C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
@@ -87,6 +91,13 @@ EXPORTS = {
     "gnca_rollout_bwd_bptt": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
                                         C.POINTER(GncaSchedule), C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
                                         C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "gnca_rollout_fwd_bptt_record": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                               C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                               C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "gnca_rollout_bwd_bptt_frames": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                               C.POINTER(GncaSchedule), C.c_void_p, C.c_size_t, C.c_int, C.c_void_p,
+                                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                               C.c_void_p]),
     "gnca_host_sample_indices": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "gnca_host_sample_offsets_words": (C.c_int, [C.c_char_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                  C.c_void_p, C.POINTER(C.c_int32)]),

@@ -9,7 +9,7 @@
 //                  five small GEMMs of the MLP backward with register tiles (FFMA); message backward;
 //                  weight-gradient partials per block (deterministic, no atomics).
 //   k_bwd_gather : dL/dx = gate path + perception transpose (gather from active neighbours) + message transpose
-//                  (gather from active receivers at +offset).
+//                  (gather from active receivers at +offset) + the gradient of a recorded frame of x, if any.
 //   k_bwd_reduce : gparams += sum over blocks of the partials.
 #include "gnca_common.cuh"
 #include "gnca_internal.h"
@@ -55,6 +55,7 @@ struct BwdArgs {
   AttnBwdScratch zp_scratch;
   float* gw_part;           // [B][nchunks][GNCA_MAX_K] dL/dw_i partials (zero-padded shift) or null
   const float* grow;        // [B][C][H] additive row term of dL/dx from the attention weights, or null
+  const float* gframe;      // [B][C][HW] dL/dx of a recorded frame (the state this step consumes), or null
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -684,9 +685,10 @@ __global__ void __launch_bounds__(256) k_bwd_gather(BwdArgs A) {
   if (cell >= HW) return;
   const float* go = A.gout + (size_t)b * C * HW + cell;
   float* gxp = A.gx + (size_t)b * C * HW + cell;
+  const float* gf = A.gframe ? A.gframe + (size_t)b * C * HW + cell : nullptr;
   if (!sample_active(a, b)) {
 #pragma unroll
-    for (int c = 0; c < C; ++c) gxp[(size_t)c * HW] = go[(size_t)c * HW];
+    for (int c = 0; c < C; ++c) gxp[(size_t)c * HW] = gf ? go[(size_t)c * HW] + gf[(size_t)c * HW] : go[(size_t)c * HW];
     return;
   }
   const int y = cell / W, x = cell - y * W;
@@ -750,6 +752,10 @@ __global__ void __launch_bounds__(256) k_bwd_gather(BwdArgs A) {
   if (A.grow) {
 #pragma unroll
     for (int c = 0; c < C; ++c) g[c] += A.grow[((size_t)b * C + c) * H + y];
+  }
+  if (gf) {
+#pragma unroll
+    for (int c = 0; c < C; ++c) g[c] += gf[(size_t)c * HW];
   }
 #pragma unroll
   for (int c = 0; c < C; ++c) gxp[(size_t)c * HW] = g[c];
@@ -874,7 +880,7 @@ int dispatch_step_bwd(const gnca_model& m, const Packed& P, const float* packed,
 
 int run_step_bwd(const gnca_model& m, const Packed& P, const float* packed, const StepArgs& a_in, const float* stats,
                  const float* gout, float* gx, float* gparams, const FwdWorkspace& fws, void* bwd_ws, bool zero_partials,
-                 bool reduce_partials, cudaStream_t st) {
+                 bool reduce_partials, cudaStream_t st, const float* gframe) {
   BwdWorkspace w = carve_bwd(bwd_ws, m, a_in.B, a_in.H, a_in.W);
   StepArgs a = a_in;
   // zero-padded shift: the per-sample softmax weights depend on x, Wq, Wk, scaling -> recompute them here and
@@ -895,7 +901,7 @@ int run_step_bwd(const gnca_model& m, const Packed& P, const float* packed, cons
   A.grow = zp ? w.attn.grow : nullptr;
   A.zp_rowsum = zp ? fws.rowsum : nullptr;
   A.zp_scratch = w.attn;
-  A.gout = gout; A.gx = gx; A.u = a.u; A.stats = stats;
+  A.gout = gout; A.gx = gx; A.u = a.u; A.stats = stats; A.gframe = gframe;
   A.actmask = w.actmask; A.postmask = w.postmask; A.gz = w.gz; A.gy = w.gy; A.gxs = w.gxs;
   A.tile_part = w.tile_part; A.sums = w.sums; A.wpart = w.wpart;
   A.ntiles = ((a.W + kBTileW - 1) / kBTileW) * ((a.H + kBTileH - 1) / kBTileH);

@@ -46,10 +46,11 @@ size_t graph_workspace_bytes(const gnca_model& m, int B, int H, int W);
 size_t bwd_workspace_bytes(const gnca_model& m, int B, int H, int W);
 // Backward of one step.  `a` describes the step (x_in, u, schedule...).  Weight-gradient partials live in the
 // workspace: zero_partials clears them first, reduce_partials folds them into gparams at the end (a rollout
-// clears at its first step and reduces after its last).
+// clears at its first step and reduces after its last).  gframe (optional, [B][C][H][W]) is added to gx: the gradient
+// of a recorded frame that is x_in itself.
 int run_step_bwd(const gnca_model& m, const Packed& P, const float* packed, const StepArgs& a, const float* stats,
                  const float* gout, float* gx, float* gparams, const FwdWorkspace& fws, void* bwd_ws, bool zero_partials,
-                 bool reduce_partials, cudaStream_t st);
+                 bool reduce_partials, cudaStream_t st, const float* gframe = nullptr);
 
 // tensor-core k_update (gnca_update_tc.cu): the balanced large-problem path for C in {16, 32}, hidden 128.
 // glist / prefix: the global active list of k_compact / k_scan.  Sets a.npart (3 partial slots per chunk).
@@ -70,7 +71,8 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                 float* u_hist, float* rec, uint32_t* masks, float* scratch, cudaStream_t st, int hist_every = 1);
-// resident BPTT on the records of run_rep_fwd (gnca_rep_bwd.cu)
+// resident BPTT on the records of run_rep_fwd (gnca_rep_bwd.cu).  g_frames (optional, [F][B][C][H][W]): dL/dx_{f*every}
+// added at step f * every (gnca_rollout_bwd_bptt_frames)
 size_t rep_bptt_bytes(const gnca_model& m, int B, int H, int W, int T);     // 0: configuration not supported
 void rep_bptt_carve(void* base, int B, int H, int W, int T, float** rec, uint32_t** masks, float** stats,
                     float** hgh = nullptr);
@@ -78,6 +80,6 @@ size_t rep_bwd_workspace_bytes(const gnca_model& m, int B, int H, int W);
 bool rep_bwd_supported(const gnca_model& m, int B, int H, int W, int k);    // a launch configuration of k_rep_bwd exists
 int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, void* bptt, const float* gT, float* g0, float* gparams, void* workspace,
-                cudaStream_t st);
+                cudaStream_t st, const float* g_frames = nullptr, int every = 1);
 
 }  // namespace gnca

@@ -83,8 +83,12 @@ __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.comm
 __device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
-template <int C>
-__global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, const float* __restrict__ packed) {
+// kFrames: gframes ([F][B][C][HW]) holds dL/dframe_f of the state step f * every consumes; it is added to g_t at
+// t = f * every (before that step's damage mask, since the frame is the post-damage state) and to g_T when T % every
+// == 0.  The instantiation without it is the one every plain BPTT launches (its parameters go unused).
+template <int C, bool kFrames>
+__global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, const float* __restrict__ packed,
+                                                   const float* __restrict__ gframes, int every) {
   static_assert(C == 16, "lane mapping: 2 cells x 16 channels per warp row");
   constexpr int C3 = 3 * C, HID = 128, CPL = 32 / C;
   cg::cluster_group cluster = cg::this_cluster();
@@ -158,7 +162,9 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
       const int cq = rest & 3, cgp = rest >> 2;
       const int cl = cgp * 8 + ci, ch = cq * 4 + c4;
       if (cl < nband) {
-        const float v = R.gT[sample_off + (size_t)ch * HW + band_lo + cl];
+        float v = R.gT[sample_off + (size_t)ch * HW + band_lo + cl];
+        if constexpr (kFrames)
+          if (R.T % every == 0) v += __ldg(gframes + ((size_t)(R.T / every) * a.B * C + (size_t)b * C + ch) * HW + band_lo + cl);
         sG[cl * C + ch] = v;
       }
     }
@@ -177,7 +183,23 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
 
   for (int t = R.T - 1; t >= 0; --t) {
     const bool dmg = R.damage.p && t == R.damage_step;
+    // dL/dframe of step t (my sample), or null when step t keeps no frame
+    const float* gfr = (kFrames && t % every == 0) ? gframes + ((size_t)(t / every) * a.B + b) * C * HW : nullptr;
     if (t >= my_steps) {                     // frozen: g passes through (the damage mask still multiplies x)
+      if constexpr (kFrames) {
+        if (dmg || gfr) {
+#pragma unroll 1
+          for (int i = tid; i < nband * C; i += kQT) {
+            const int cl = i / C, ch = i - cl * C;
+            float v = sG[i];
+            if (gfr) v += __ldg(gfr + (size_t)ch * HW + band_lo + cl);
+            if (dmg) v *= R.damage.at(b, ch, band_lo + cl, C, HW);
+            sG[i] = v;
+          }
+          __syncthreads();
+        }
+        continue;
+      }
       if (dmg) {
 #pragma unroll 1
         for (int i = tid; i < nband * C; i += kQT) {
@@ -601,6 +623,12 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
             g.z = fmaf(wuni, vr[i].z, g.z); g.w = fmaf(wuni, vr[i].w, g.w);
           }
         }
+        if constexpr (kFrames) {
+          if (gfr) {
+            const float* gf = gfr + (size_t)(4 * cq) * HW + cell;
+            g.x += __ldg(gf); g.y += __ldg(gf + HW); g.z += __ldg(gf + 2 * HW); g.w += __ldg(gf + 3 * HW);
+          }
+        }
         if (dmg) {
           g.x *= R.damage.at(b, 4 * cq, cell, C, HW); g.y *= R.damage.at(b, 4 * cq + 1, cell, C, HW);
           g.z *= R.damage.at(b, 4 * cq + 2, cell, C, HW); g.w *= R.damage.at(b, 4 * cq + 3, cell, C, HW);
@@ -854,7 +882,7 @@ static bool pick_rep_bwd_config(int B, int HW, cudaStream_t st, int* out_nc, int
       size_t smem = rep_bwd_smem_bytes(C, HW, NC, gmax);
       if (smem > 220 * 1024) { gmax = 4; smem = rep_bwd_smem_bytes(C, HW, NC, gmax); }
       if (smem > 220 * 1024) continue;
-      if (cudaFuncSetAttribute(k_rep_bwd<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
+      if (cudaFuncSetAttribute(k_rep_bwd<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
         cudaGetLastError();
         continue;
       }
@@ -865,7 +893,7 @@ static bool pick_rep_bwd_config(int B, int HW, cudaStream_t st, int* out_nc, int
       qa[0].val.clusterDim.x = NC; qa[0].val.clusterDim.y = 1; qa[0].val.clusterDim.z = 1;
       q.attrs = qa; q.numAttrs = 1;
       int ncl = 0;
-      if (cudaOccupancyMaxActiveClusters(&ncl, k_rep_bwd<16>, &q) != cudaSuccess || ncl < 1) {
+      if (cudaOccupancyMaxActiveClusters(&ncl, k_rep_bwd<16, false>, &q) != cudaSuccess || ncl < 1) {
         cudaGetLastError();
         continue;
       }
@@ -888,7 +916,7 @@ bool rep_bwd_supported(const gnca_model& m, int B, int H, int W, int k) {
 
 int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, void* bptt, const float* gT, float* g0, float* gparams, void* workspace,
-                cudaStream_t st) {
+                cudaStream_t st, const float* g_frames, int every) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (rep_bptt_bytes(m, B, H, W, sched.T) == 0) return GNCA_ERR_UNSUPPORTED;
   const int k = graph ? sched.k : 0;
@@ -923,7 +951,10 @@ int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B
   if (pick < 0) return GNCA_ERR_UNSUPPORTED;
   R.NC = pick; R.gmax = pick_gmax;
   if (getenv("GNCA_DEBUG")) fprintf(stderr, "[gnca] resident bwd: B=%d NC=%d smem=%zu\n", B, pick, pick_smem);
-  GNCA_CHECK_CUDA(cudaFuncSetAttribute(k_rep_bwd<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pick_smem));
+  // the frame-gradient instantiation has the register budget and shared memory of the plain one (same launch bounds,
+  // same carve), so the configuration picked for the plain kernel holds for it
+  const auto kern = g_frames ? k_rep_bwd<16, true> : k_rep_bwd<16, false>;
+  GNCA_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pick_smem));
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(B * pick);
   cfg.blockDim = dim3(kQT);
@@ -941,7 +972,7 @@ int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B
     R.dbg_cta = atoi(getenv("GNCA_PHASE_TIMING"));
   }
   prof_begin(PROF_RESIDENT_BWD, st);
-  cudaError_t e = cudaLaunchKernelEx(&cfg, k_rep_bwd<16>, R, P, packed);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, R, P, packed, g_frames, every);
   prof_end(PROF_RESIDENT_BWD, st);
   if (e != cudaSuccess) return (int)e;
   GNCA_LAUNCH_CHECK();

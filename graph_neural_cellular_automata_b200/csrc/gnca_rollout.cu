@@ -15,6 +15,24 @@ __global__ void k_mul_inplace(size_t n, float* __restrict__ x, DamageView d, int
   }
 }
 
+// out = a + b: dL/dx_T plus the gradient of the last frame when that frame is x_T (T % every == 0)
+__global__ void k_add(size_t n, float* __restrict__ out, const float* __restrict__ a, const float* __restrict__ b) {
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
+    out[i] = a[i] + b[i];
+}
+
+static int launch_add(size_t n, float* out, const float* a, const float* b, cudaStream_t st) {
+  k_add<<<(int)((n + 1023) / 1024 < 2368 ? (n + 1023) / 1024 : 2368), 256, 0, st>>>(n, out, a, b);
+  GNCA_LAUNCH_CHECK();
+  return 0;
+}
+
+// g0 of a rollout whose backward starts at step T: gT, plus dL/dframe_{T/every} when frame T / every is x_T
+static int fold_last_frame(size_t N, int T, int every, const float* g_frames, const float* gT, float* out,
+                           cudaStream_t st) {
+  return launch_add(N, out, gT, g_frames + (size_t)(T / every) * N, st);
+}
+
 struct RolloutWorkspace {
   float* ping;     // [B][C][H][W]
   float* pong;
@@ -124,6 +142,36 @@ static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int 
   return 0;
 }
 
+// gnca_rollout_fwd_bptt with a strided history: x_t of every step t % every == 0 goes to x_hist slot t / every
+static int rollout_fwd_bptt(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
+                            const float* x0_dev, float* xT_dev, float* x_hist_dev, int every, void* bptt_dev,
+                            size_t bptt_bytes, void* workspace_dev, size_t workspace_bytes, void* stream) {
+  if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !bptt_dev || !workspace_dev) return GNCA_ERR_ARG;
+  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
+  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
+  const size_t need = gnca_bptt_bytes(m, B, H, W, sched->T);
+  if (need == 0) return GNCA_ERR_UNSUPPORTED;
+  if (need > bptt_bytes) return GNCA_ERR_WORKSPACE;
+  RolloutWorkspace r = carve_rollout(workspace_dev, *m, B, H, W);
+  if (r.bytes > workspace_bytes) return GNCA_ERR_WORKSPACE;
+  const bool graph = (m->flags & GNCA_F_GRAPH) != 0;
+  // the records are only worth writing if the resident backward can consume them for this batch / shape
+  if (!rep_bwd_supported(*m, B, H, W, graph ? sched->k : 0)) return GNCA_ERR_UNSUPPORTED;
+  const Packed P = make_packed(m->C, m->hidden, m->d_model, graph);
+  float *rec, *stats;
+  uint32_t* masks;
+  rep_bptt_carve(bptt_dev, B, H, W, sched->T, &rec, &masks, &stats);
+  if (sched->T == 0) {
+    cudaMemcpyAsync(xT_dev, x0_dev, (size_t)B * m->C * H * W * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
+    if (x_hist_dev)
+      cudaMemcpyAsync(x_hist_dev, x0_dev, (size_t)B * m->C * H * W * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
+    return 0;
+  }
+  return run_rep_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, x_hist_dev, stats, nullptr, rec, masks, r.ping,
+                     (cudaStream_t)stream, every);
+}
+
 }  // namespace gnca
 
 using namespace gnca;
@@ -189,13 +237,15 @@ int gnca_rollout_record(const gnca_model* m, const float* packed_dev, int B, int
   return 0;
 }
 
-int gnca_rollout_bwd(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
-                     const float* x_hist_dev, const float* stats_hist_dev, const float* u_hist_dev,
-                     const float* gT_dev, float* g0_dev,
-                     float* gparams_dev, void* workspace_dev, size_t workspace_bytes, int impl, void* stream) {
+int gnca_rollout_bwd_frames(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                            const gnca_schedule* sched, const float* x_hist_dev, const float* stats_hist_dev,
+                            const float* u_hist_dev, int every, const float* g_frames_dev, const float* gT_dev,
+                            float* g0_dev, float* gparams_dev, void* workspace_dev, size_t workspace_bytes, int impl,
+                            void* stream) {
   if (!m || !packed_dev || !sched || !x_hist_dev || !gT_dev || !g0_dev || !gparams_dev || !workspace_dev)
     return GNCA_ERR_ARG;
   if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
+  if (g_frames_dev && every <= 0) return GNCA_ERR_ARG;
   if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
   if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
   (void)impl;             // the backward currently always takes the streaming kernels (x_hist layout is shared)
@@ -210,10 +260,16 @@ int gnca_rollout_bwd(const gnca_model* m, const float* packed_dev, int B, int H,
   char* bws = r.step_ws + fws.bytes;
   const int T = sched->T;
   if (T == 0) {
+    if (g_frames_dev) return fold_last_frame(N, T, every, g_frames_dev, gT_dev, g0_dev, st);
     GNCA_CHECK_CUDA(cudaMemcpyAsync(g0_dev, gT_dev, N * sizeof(float), cudaMemcpyDeviceToDevice, st));
     return 0;
   }
   const float* gcur = gT_dev;
+  if (g_frames_dev && T % every == 0) {          // g_b is not written before the second step (t = T - 2)
+    int rc = fold_last_frame(N, T, every, g_frames_dev, gT_dev, r.g_b, st);
+    if (rc) return rc;
+    gcur = r.g_b;
+  }
   for (int t = T - 1; t >= 0; --t) {
     StepArgs a;
     fill_step_args(a, *m, B, H, W);
@@ -233,7 +289,9 @@ int gnca_rollout_bwd(const gnca_model* m, const float* packed_dev, int B, int H,
       if (rc) return rc;
     }
     float* gnext = (t == 0) ? g0_dev : (((T - 1 - t) & 1) ? r.g_b : r.g_a);
-    rc = run_step_bwd(*m, P, packed_dev, a, stats_t, gcur, gnext, gparams_dev, fws, bws, t == T - 1, t == 0, st);
+    // the frame of step t is x_t after the damage: its gradient joins dL/dx_t before the damage mask multiplies it
+    const float* gframe = (g_frames_dev && t % every == 0) ? g_frames_dev + (size_t)(t / every) * N : nullptr;
+    rc = run_step_bwd(*m, P, packed_dev, a, stats_t, gcur, gnext, gparams_dev, fws, bws, t == T - 1, t == 0, st, gframe);
     if (rc) return rc;
     if (sched->damage && t == sched->damage_step) {
       k_mul_inplace<<<(int)((N + 1023) / 1024 < 2368 ? (N + 1023) / 1024 : 2368), 256, 0, st>>>(N, gnext, DamageView{sched->damage, sched->damage_layout}, m->C, H * W);
@@ -244,6 +302,14 @@ int gnca_rollout_bwd(const gnca_model* m, const float* packed_dev, int B, int H,
   return 0;
 }
 
+int gnca_rollout_bwd(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
+                     const float* x_hist_dev, const float* stats_hist_dev, const float* u_hist_dev,
+                     const float* gT_dev, float* g0_dev,
+                     float* gparams_dev, void* workspace_dev, size_t workspace_bytes, int impl, void* stream) {
+  return gnca_rollout_bwd_frames(m, packed_dev, B, H, W, sched, x_hist_dev, stats_hist_dev, u_hist_dev, 0, nullptr,
+                                 gT_dev, g0_dev, gparams_dev, workspace_dev, workspace_bytes, impl, stream);
+}
+
 
 /* ---- resident BPTT: records instead of the dense x_t / u_t history (gnca_rep.cu / gnca_rep_bwd.cu) ---- */
 size_t gnca_bptt_bytes(const gnca_model* m, int B, int H, int W, int T) {
@@ -252,40 +318,29 @@ size_t gnca_bptt_bytes(const gnca_model* m, int B, int H, int W, int T) {
   return rep_bptt_bytes(*m, B, H, W, T);
 }
 
+int gnca_rollout_fwd_bptt_record(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                                 const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                                 float* frames_dev, void* bptt_dev, size_t bptt_bytes, void* workspace_dev,
+                                 size_t workspace_bytes, void* stream) {
+  if (!frames_dev || every <= 0) return GNCA_ERR_ARG;
+  return rollout_fwd_bptt(m, packed_dev, B, H, W, sched, x0_dev, xT_dev, frames_dev, every, bptt_dev, bptt_bytes,
+                          workspace_dev, workspace_bytes, stream);
+}
+
 int gnca_rollout_fwd_bptt(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
                           const float* x0_dev, float* xT_dev, float* x_hist_dev, void* bptt_dev, size_t bptt_bytes,
                           void* workspace_dev, size_t workspace_bytes, void* stream) {
-  if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !bptt_dev || !workspace_dev) return GNCA_ERR_ARG;
-  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
-  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
-  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
-  const size_t need = gnca_bptt_bytes(m, B, H, W, sched->T);
-  if (need == 0) return GNCA_ERR_UNSUPPORTED;
-  if (need > bptt_bytes) return GNCA_ERR_WORKSPACE;
-  RolloutWorkspace r = carve_rollout(workspace_dev, *m, B, H, W);
-  if (r.bytes > workspace_bytes) return GNCA_ERR_WORKSPACE;
-  const bool graph = (m->flags & GNCA_F_GRAPH) != 0;
-  // the records are only worth writing if the resident backward can consume them for this batch / shape
-  if (!rep_bwd_supported(*m, B, H, W, graph ? sched->k : 0)) return GNCA_ERR_UNSUPPORTED;
-  const Packed P = make_packed(m->C, m->hidden, m->d_model, graph);
-  float *rec, *stats;
-  uint32_t* masks;
-  rep_bptt_carve(bptt_dev, B, H, W, sched->T, &rec, &masks, &stats);
-  if (sched->T == 0) {
-    cudaMemcpyAsync(xT_dev, x0_dev, (size_t)B * m->C * H * W * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
-    if (x_hist_dev)
-      cudaMemcpyAsync(x_hist_dev, x0_dev, (size_t)B * m->C * H * W * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
-    return 0;
-  }
-  return run_rep_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, x_hist_dev, stats, nullptr, rec, masks, r.ping,
-                     (cudaStream_t)stream);
+  return rollout_fwd_bptt(m, packed_dev, B, H, W, sched, x0_dev, xT_dev, x_hist_dev, 1, bptt_dev, bptt_bytes,
+                          workspace_dev, workspace_bytes, stream);
 }
 
-int gnca_rollout_bwd_bptt(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
-                          void* bptt_dev, size_t bptt_bytes, const float* gT_dev, float* g0_dev, float* gparams_dev,
-                          void* workspace_dev, size_t workspace_bytes, void* stream) {
+int gnca_rollout_bwd_bptt_frames(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                                 const gnca_schedule* sched, void* bptt_dev, size_t bptt_bytes, int every,
+                                 const float* g_frames_dev, const float* gT_dev, float* g0_dev, float* gparams_dev,
+                                 void* workspace_dev, size_t workspace_bytes, void* stream) {
   if (!m || !packed_dev || !sched || !bptt_dev || !gT_dev || !g0_dev || !gparams_dev || !workspace_dev) return GNCA_ERR_ARG;
   if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
+  if (g_frames_dev && every <= 0) return GNCA_ERR_ARG;
   if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
   if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
   const size_t need = gnca_bptt_bytes(m, B, H, W, sched->T);
@@ -295,11 +350,20 @@ int gnca_rollout_bwd_bptt(const gnca_model* m, const float* packed_dev, int B, i
   const bool graph = (m->flags & GNCA_F_GRAPH) != 0;
   const Packed P = make_packed(m->C, m->hidden, m->d_model, graph);
   if (sched->T == 0) {
-    cudaMemcpyAsync(g0_dev, gT_dev, (size_t)B * m->C * H * W * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
+    const size_t N = (size_t)B * m->C * H * W;
+    if (g_frames_dev) return fold_last_frame(N, 0, every, g_frames_dev, gT_dev, g0_dev, (cudaStream_t)stream);
+    cudaMemcpyAsync(g0_dev, gT_dev, N * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
     return 0;
   }
   return run_rep_bwd(*m, P, packed_dev, B, H, W, *sched, bptt_dev, gT_dev, g0_dev, gparams_dev, workspace_dev,
-                     (cudaStream_t)stream);
+                     (cudaStream_t)stream, g_frames_dev, every);
+}
+
+int gnca_rollout_bwd_bptt(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
+                          void* bptt_dev, size_t bptt_bytes, const float* gT_dev, float* g0_dev, float* gparams_dev,
+                          void* workspace_dev, size_t workspace_bytes, void* stream) {
+  return gnca_rollout_bwd_bptt_frames(m, packed_dev, B, H, W, sched, bptt_dev, bptt_bytes, 0, nullptr, gT_dev, g0_dev,
+                                      gparams_dev, workspace_dev, workspace_bytes, stream);
 }
 
 /* ---- host-side schedule construction: T x random.sample(range(n), k) on CPython's MT19937 state ----

@@ -183,10 +183,11 @@ class History:
     * records (`bptt`): the replicated-state kernel's per-active-cell records + bitmaps + statistics -- consumed by the
       cluster-resident backward (gnca_rollout_bwd_bptt); `x` is only filled when the caller asked for the history;
     * dense: x_t for every step and (optionally) the masked pre-norm update of the active cells + the GroupNorm
-      statistics, consumed by the streaming backward (gnca_rollout_bwd)."""
+      statistics, consumed by the streaming backward (gnca_rollout_bwd).
+    `frames` (forward with `every`): x_{f*every} in a buffer of its own, the differentiable states of `record_rollout`."""
 
-    def __init__(self, x, u=None, stats=None, bptt=None, shape=None):
-        self.x, self.u, self.stats, self.bptt = x, u, stats, bptt
+    def __init__(self, x, u=None, stats=None, bptt=None, shape=None, frames=None):
+        self.x, self.u, self.stats, self.bptt, self.frames = x, u, stats, bptt, frames
         self._shape = tuple(shape) if shape is not None else tuple(x.shape)
 
     @property
@@ -208,9 +209,11 @@ BPTT_MAX_BYTES = 48 << 30      # above this the record buffer is not worth it: d
 
 
 def rollout_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, *, history: bool, impl: int = 0,
-                    keep_u: bool = True, keep_x: bool = True):
+                    keep_u: bool = True, keep_x: bool = True, every: int = 0):
     """gnca_rollout_fwd without autograd: returns (x_T, History or None).  `keep_x=False`: the caller only needs the
-    history for the backward (the resident BPTT path then skips storing x_t)."""
+    history for the backward (the resident BPTT path then skips storing x_t).  `every > 0` (with `history`): the
+    History also carries the frames x_{f*every} of `record_rollout` -- on the record path the forward writes them in
+    place of the x_t history (gnca_rollout_fwd_bptt_record), on the dense path they are copied out of it."""
     x0 = GF._require_cuda_f32(x0, "x0")
     B, Cc, H, W = x0.shape
     if Cc != desc.C:
@@ -231,12 +234,21 @@ def rollout_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, *, history:
             if nb <= nb_q <= BPTT_MAX_BYTES and nb_q - nb <= _QUANT_SLACK_BYTES:
                 nb = nb_q
             bptt = torch.empty(nb, dtype=torch.uint8, device=x0.device)
-            hist = torch.empty(T + 1, B, Cc, H, W, dtype=torch.float32, device=x0.device) if keep_x else None
-            rc = lib.gnca_rollout_fwd_bptt(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(x0), GF._ptr(xT),
-                                           GF._ptr(hist), GF._ptr(bptt), nb, GF._ptr(ws), ws.numel(), GF._stream())
+            if every > 0:
+                hist = None
+                frames = torch.empty(T // every + 1, B, Cc, H, W, dtype=torch.float32, device=x0.device)
+                rc = lib.gnca_rollout_fwd_bptt_record(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(x0),
+                                                      GF._ptr(xT), every, GF._ptr(frames), GF._ptr(bptt), nb,
+                                                      GF._ptr(ws), ws.numel(), GF._stream())
+            else:
+                frames = None
+                hist = torch.empty(T + 1, B, Cc, H, W, dtype=torch.float32, device=x0.device) if keep_x else None
+                rc = lib.gnca_rollout_fwd_bptt(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(x0),
+                                               GF._ptr(xT), GF._ptr(hist), GF._ptr(bptt), nb, GF._ptr(ws), ws.numel(),
+                                               GF._stream())
             if rc != _lib.GNCA_ERR_UNSUPPORTED:
-                _lib.check(rc, "gnca_rollout_fwd_bptt")
-                return xT, History(hist, bptt=bptt, shape=(T + 1, B, Cc, H, W))
+                _lib.check(rc, "gnca_rollout_fwd_bptt_record" if every > 0 else "gnca_rollout_fwd_bptt")
+                return xT, History(hist, bptt=bptt, shape=(T + 1, B, Cc, H, W), frames=frames)
     hist = uh = sh = None
     if history:
         Tq = _round_up_steps(T)              # same quantised allocation for the dense history (prefix views)
@@ -249,12 +261,17 @@ def rollout_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, *, history:
     _lib.check(lib.gnca_rollout_fwd(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(x0), GF._ptr(xT),
                                     GF._ptr(hist), GF._ptr(sh), GF._ptr(uh), GF._ptr(ws), ws.numel(), int(impl),
                                     GF._stream()), "gnca_rollout_fwd")
-    return xT, (History(hist, uh, sh) if history else None)
+    if not history:
+        return xT, None
+    # the frames are a copy: editing them in place cannot corrupt the history the backward reads
+    return xT, History(hist, uh, sh, frames=hist[::every].clone() if every > 0 else None)
 
 
-def rollout_bwd_raw(desc, packed, hist, sched: Schedule, gT: torch.Tensor, *, gflat=None, impl: int = 0):
+def rollout_bwd_raw(desc, packed, hist, sched: Schedule, gT: torch.Tensor, *, gflat=None, impl: int = 0,
+                    g_frames: Optional[torch.Tensor] = None, every: int = 0):
     """gnca_rollout_bwd without autograd: returns (dL/dx_0, flat parameter gradient in canonical layout).
-    `gflat` (optional) is accumulated into."""
+    `gflat` (optional) is accumulated into.  `g_frames` (optional, [T // every + 1, B, C, H, W]): dL/dx_{f*every} of the
+    frames of the forward, added at their steps (gnca_rollout_bwd_frames / gnca_rollout_bwd_bptt_frames)."""
     if not isinstance(hist, History):
         hist = History(hist)
     _, B, Cc, H, W = hist.shape
@@ -267,14 +284,21 @@ def rollout_bwd_raw(desc, packed, hist, sched: Schedule, gT: torch.Tensor, *, gf
     nbytes = lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, sched.T)
     ws = GF._WS.get(gT.device, nbytes)
     cs = sched.c_struct()
+    if g_frames is not None:
+        g_frames = GF._require_cuda_f32(g_frames, "frame gradients")
+        if tuple(g_frames.shape) != (sched.T // every + 1, B, Cc, H, W):
+            raise ValueError(f"frame gradients have shape {tuple(g_frames.shape)}, expected "
+                             f"{(sched.T // every + 1, B, Cc, H, W)}")
     if hist.bptt is not None:
-        _lib.check(lib.gnca_rollout_bwd_bptt(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(hist.bptt),
-                                             hist.bptt.numel(), GF._ptr(gT), GF._ptr(g0), GF._ptr(gflat), GF._ptr(ws),
-                                             ws.numel(), GF._stream()), "gnca_rollout_bwd_bptt")
+        _lib.check(lib.gnca_rollout_bwd_bptt_frames(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs),
+                                                    GF._ptr(hist.bptt), hist.bptt.numel(), every, GF._ptr(g_frames),
+                                                    GF._ptr(gT), GF._ptr(g0), GF._ptr(gflat), GF._ptr(ws), ws.numel(),
+                                                    GF._stream()), "gnca_rollout_bwd_bptt_frames")
         return g0, gflat
-    _lib.check(lib.gnca_rollout_bwd(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(hist.x),
-                                    GF._ptr(hist.stats), GF._ptr(hist.u), GF._ptr(gT), GF._ptr(g0), GF._ptr(gflat),
-                                    GF._ptr(ws), ws.numel(), int(impl), GF._stream()), "gnca_rollout_bwd")
+    _lib.check(lib.gnca_rollout_bwd_frames(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(hist.x),
+                                           GF._ptr(hist.stats), GF._ptr(hist.u), every, GF._ptr(g_frames), GF._ptr(gT),
+                                           GF._ptr(g0), GF._ptr(gflat), GF._ptr(ws), ws.numel(), int(impl),
+                                           GF._stream()), "gnca_rollout_bwd_frames")
     return g0, gflat
 
 
@@ -321,6 +345,35 @@ def rollout(model, x0: torch.Tensor, schedule: Schedule, *, return_history: bool
     return _RolloutFn.apply(x0, cfg, *ps)
 
 
+class _RecordFn(torch.autograd.Function):
+    """record_rollout(..., differentiable=True): the frames and x_T as the outputs of one node; its backward is one
+    BPTT that adds dL/dframe_f at step f * every."""
+
+    @staticmethod
+    def forward(ctx, x0, cfg, *params):
+        xT, hist = rollout_fwd_raw(cfg["desc"], cfg["packed"], x0, cfg["schedule"], history=True, impl=cfg["impl"],
+                                   keep_x=False, every=cfg["every"])
+        ctx.set_materialize_grads(False)          # an unused output passes None: no zero tensor, no frame pass
+        ctx.cfg = cfg
+        ctx.param_shapes = [p.shape for p in params]
+        ctx.hist = hist
+        return hist.frames, xT
+
+    @staticmethod
+    def backward(ctx, g_states, g_xT):
+        cfg = ctx.cfg
+        if ctx.hist is None:
+            raise RuntimeError("record_rollout: the gradient history was already consumed by an earlier backward")
+        if g_xT is None:
+            g_xT = torch.zeros_like(ctx.hist.frames[0])
+        g0, gflat = rollout_bwd_raw(cfg["desc"], cfg["packed"], ctx.hist, cfg["schedule"], g_xT, impl=cfg["impl"],
+                                    g_frames=g_states, every=cfg["every"])
+        offs = GF.segment_offsets(cfg["desc"])
+        grads = [gflat[offs[i]:offs[i + 1]].view(ctx.param_shapes[i]) for i in range(len(ctx.param_shapes))]
+        ctx.hist = None
+        return (g0, None, *grads)
+
+
 @dataclass
 class Trajectory:
     """What `record_rollout` returns.  `states[f]` is x_{t[f]}, the state step t[f] consumes (after the schedule's
@@ -333,11 +386,17 @@ class Trajectory:
 
 
 def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, attention: bool = False,
-                   impl: str = "auto") -> Trajectory:
+                   impl: str = "auto", differentiable: bool = False) -> Trajectory:
     """T steps from x0 under `schedule` in one library call (gnca_rollout_record), keeping x_t every `every` steps and,
     with `attention=True`, the attention map `model.step(x_t, ..., return_attention=True)` gives for each kept step
     t < T.  Watching a rollout this way keeps the fused rollout kernels; no gradient history or record buffer is
-    allocated, and the outputs are detached."""
+    allocated, and the outputs are detached.
+
+    `differentiable=True` (with grad mode on and x0 or a parameter requiring grad): `states` and `x_T` are the outputs
+    of one autograd node, and a loss on any of them back-propagates to x0 and the parameters through one fused BPTT --
+    the gradients of T sequential `model.step` calls with the same schedule.  The BPTT history is the one `rollout()`
+    keeps for its backward.  `attention` stays detached (it costs one more, inference-only rollout).  Without grad the
+    call is exactly the detached recording."""
     every = int(every)
     if every < 1:
         raise ValueError(f"record_rollout: every must be >= 1, got {every}")
@@ -346,6 +405,19 @@ def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, a
     if not x0.is_cuda:
         raise RuntimeError(f"record_rollout: x0 is on {x0.device}; CUDA (sm_100a) only, no CPU fallback")
     desc = model.model_desc()
+    if differentiable:
+        ps = model.canonical_params()
+        if torch.is_grad_enabled() and (x0.requires_grad or any(p.requires_grad for p in ps)):
+            if x0.shape[1] != desc.C:
+                raise ValueError(f"x0 has {x0.shape[1]} channels, model has {desc.C}")
+            cfg = {"desc": desc, "packed": model.packed_weights(), "schedule": schedule, "impl": IMPL[impl],
+                   "every": every}
+            frames, xT = _RecordFn.apply(x0, cfg, *ps)
+            attn = None
+            if attention:
+                with torch.no_grad():
+                    attn = record_rollout(model, x0, schedule, every=every, attention=True, impl=impl).attention
+            return Trajectory(t=list(range(0, schedule.T + 1, every)), states=frames, attention=attn, x_T=xT)
     x0 = GF._require_cuda_f32(x0.detach(), "x0")
     B, Cc, H, W = x0.shape
     if Cc != desc.C:

@@ -11,6 +11,7 @@
  *   NeuralCAGraph.forward             src/modules/ncagraph.py:106-168            -> gnca_step_fwd/_bwd (GNCA_F_GRAPH set)
  *   the rollout loop                  src/training/train_graph_augmented_nca.py:302-324 -> gnca_rollout_fwd/_bwd
  *   the recording loop                test_graph_augmented_regeneration.py:183-194     -> gnca_rollout_record
+ *   losses on recorded states         (eager autograd through every x_t)               -> gnca_rollout_bwd_frames
  *   loss_premult_rgba (+ its grad)    src/training/train_graph_augmented_nca.py:52-61,337-339 -> gnca_loss_premult_rgba
  *   grad normalise + Adam             src/training/train_graph_augmented_nca.py:370-375 -> gnca_normalize_adam
  *   multiplicative damage             src/utils/damage.py:16-98                  -> gnca_apply_mask
@@ -37,7 +38,7 @@
 extern "C" {
 #endif
 
-#define GNCA_VERSION 105
+#define GNCA_VERSION 106
 
 #define GNCA_ERR_ARG (-1)         /* null pointer / bad size */
 #define GNCA_ERR_UNSUPPORTED (-2) /* shape or flag combination without a kernel */
@@ -227,6 +228,25 @@ int gnca_rollout_bwd(const gnca_model* m, const float* packed_dev, int B, int H,
                      void* workspace_dev, size_t workspace_bytes, int impl, void* stream);
 
 /*
+ * Differentiable frames: BPTT of a loss on the strided frames of a recording rollout (frame f = x_{f*every}, exactly the
+ * frames of gnca_rollout_record) and on x_T.  g_frames_dev ([F][B][C][H][W], F = gnca_record_frames(T, every)) holds
+ * dL/dframe_f; NULL is exactly gnca_rollout_bwd / gnca_rollout_bwd_bptt (which are these functions with NULL).
+ *   - At step t = f*every, dL/dx_t = (backward of step t) + dL/dframe_f.  The damage mask of damage_step multiplies that
+ *     SUM: the frame is the state after the damage.  A frozen sample (steps[b] <= t) passes g through and still
+ *     receives its frame gradients.
+ *   - When T % every == 0, frame F-1 and x_T hold equal values but are two outputs: their gradients add.  T == 0:
+ *     g0 = gT + g_frames[0].
+ * The result equals autograd through T sequential steps with the same schedule.  Argument errors return before any
+ * launch: `every <= 0` with a frame gradient, or a NULL required pointer, is GNCA_ERR_ARG; k outside [0, GNCA_MAX_K]
+ * is GNCA_ERR_UNSUPPORTED.  The workspaces are those of gnca_rollout_workspace_bytes.
+ */
+int gnca_rollout_bwd_frames(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                            const gnca_schedule* sched, const float* x_hist_dev, const float* stats_hist_dev,
+                            const float* u_hist_dev, int every, const float* g_frames_dev,
+                            const float* gT_dev, float* g0_dev, float* gparams_dev,
+                            void* workspace_dev, size_t workspace_bytes, int impl, void* stream);
+
+/*
  * Resident BPTT (16-channel / 128-hidden models, classic or torus graph, grids up to 2048 cells with W % 4 == 0).
  * Instead of the dense x_t / u_t history the forward keeps one compact record per ACTIVE cell and step (perception,
  * pre-norm update, gathered sender state ...) plus three bitmaps and the GroupNorm statistics per step, in the opaque
@@ -243,6 +263,17 @@ int gnca_rollout_bwd_bptt(const gnca_model* m, const float* packed_dev, int B, i
                           const gnca_schedule* sched, void* bptt_dev, size_t bptt_bytes, const float* gT_dev,
                           float* g0_dev, float* gparams_dev, void* workspace_dev, size_t workspace_bytes,
                           void* stream);
+/* The record-based forward of gnca_rollout_fwd_bptt keeping the frames of gnca_rollout_record instead of a full
+ * history: frames_dev[f] = x_{f*every} ([F][B][C][H][W], non-NULL, every > 0); xT_dev always receives x_T. */
+int gnca_rollout_fwd_bptt_record(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                                 const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                                 float* frames_dev, void* bptt_dev, size_t bptt_bytes, void* workspace_dev,
+                                 size_t workspace_bytes, void* stream);
+/* gnca_rollout_bwd_bptt with the frame gradients of gnca_rollout_bwd_frames */
+int gnca_rollout_bwd_bptt_frames(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                                 const gnca_schedule* sched, void* bptt_dev, size_t bptt_bytes, int every,
+                                 const float* g_frames_dev, const float* gT_dev, float* g0_dev, float* gparams_dev,
+                                 void* workspace_dev, size_t workspace_bytes, void* stream);
 
 /*
  * HOST function (no device work): T consecutive `random.sample(range(n), k)` draws of CPython's `random` module on
