@@ -12,7 +12,7 @@ LIB_PATH = os.path.join(_PKG, "lib", "libgnca.so")
 
 GNCA_F_GRAPH, GNCA_F_TORUS, GNCA_F_HIDDEN_ONLY, GNCA_F_ALIVE_TO_ALIVE, GNCA_F_GROUPNORM = 1, 2, 4, 8, 16
 GNCA_MAX_K = 64
-GNCA_ERR_ARG, GNCA_ERR_UNSUPPORTED = -1, -2
+GNCA_ERR_ARG, GNCA_ERR_UNSUPPORTED, GNCA_ERR_WORKSPACE = -1, -2, -3
 GNCA_VERSION = 106
 
 
@@ -84,6 +84,11 @@ EXPORTS = {
                                           C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
                                           C.c_int, C.c_void_p]),
+    "gnca_ckpt_segment_bytes": (C.c_size_t, [C.POINTER(GncaModel), C.c_int, C.c_int, C.c_int, C.c_int]),
+    "gnca_rollout_bwd_ckpt": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                        C.POINTER(GncaSchedule), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t,
+                                        C.c_void_p]),
     "gnca_bptt_bytes": (C.c_size_t, [C.POINTER(GncaModel), C.c_int, C.c_int, C.c_int, C.c_int]),
     "gnca_rollout_fwd_bptt": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
                                         C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,

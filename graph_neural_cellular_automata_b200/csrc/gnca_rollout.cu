@@ -79,6 +79,103 @@ static void schedule_to_args(StepArgs& a, const gnca_schedule& s, int t, int B, 
   a.philox_offset = s.philox_offset;
 }
 
+static int launch_damage(size_t N, float* x, const gnca_schedule& s, int C, int HW, cudaStream_t st) {
+  k_mul_inplace<<<(int)((N + 1023) / 1024 < 2368 ? (N + 1023) / 1024 : 2368), 256, 0, st>>>(N, x, DamageView{s.damage, s.damage_layout}, C, HW);
+  GNCA_LAUNCH_CHECK();
+  return 0;
+}
+
+// Where the backward finds the forward of the steps from t0 on: x_t0 at `x0`, x_t (t > t0) at rest[t - t0 - 1], u_t and
+// stats_t at slot t - t0 of `u` / `stats` (NULL: recomputed per step).  The dense history is {x_hist, x_hist + N, u_hist,
+// stats_hist, 0}; a checkpoint segment is {ckpt[j], its recomputed states, ..., j * every}.
+struct SavedSteps {
+  const float* x0;
+  const float* rest;
+  const float* u;
+  const float* stats;
+  int t0;
+};
+
+// g of the rollout's last state: gT, plus the last frame's gradient when that frame is x_T; T == 0 writes g0 directly
+static int bwd_begin(size_t N, int T, int every, const float* g_frames, const float* gT, float* g0,
+                     const RolloutWorkspace& r, const float** gcur, cudaStream_t st) {
+  *gcur = gT;
+  if (T == 0) {
+    if (g_frames) return fold_last_frame(N, T, every, g_frames, gT, g0, st);
+    GNCA_CHECK_CUDA(cudaMemcpyAsync(g0, gT, N * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    return 0;
+  }
+  if (g_frames && T % every == 0) {          // g_b is not written before the second step (t = T - 2)
+    int rc = fold_last_frame(N, T, every, g_frames, gT, r.g_b, st);
+    if (rc) return rc;
+    *gcur = r.g_b;
+  }
+  return 0;
+}
+
+// The per-step backward of steps t_hi - 1 down to t_lo of a T-step rollout.  *gcur enters as dL/dx_{t_hi} and leaves as
+// dL/dx_{t_lo}.  The gradient ping-pong and the weight-gradient partials follow the global t: the partials are zeroed at
+// t = T - 1 and reduced into gparams at t = 0, so a caller may split [0, T) into ranges run last to first.
+static int bwd_steps(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
+                     const gnca_schedule& s, const SavedSteps& sv, int t_lo, int t_hi, int every, const float* g_frames,
+                     const float** gcur, float* g0, float* gparams, const RolloutWorkspace& r, const FwdWorkspace& fws,
+                     char* bws, cudaStream_t st) {
+  const size_t N = (size_t)B * m.C * H * W;
+  const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
+  const int T = s.T;
+  for (int t = t_hi - 1; t >= t_lo; --t) {
+    StepArgs a;
+    fill_step_args(a, m, B, H, W);
+    schedule_to_args(a, s, t, B, H, W);
+    if (!graph) a.k = 0;
+    a.x_in = const_cast<float*>(t == sv.t0 ? sv.x0 : sv.rest + (size_t)(t - sv.t0 - 1) * N);
+    a.x_out = nullptr;
+    const float* stats_t = r.stats;
+    int rc = 0;
+    if (sv.u && sv.stats) {
+      a.u = const_cast<float*>(sv.u) + (size_t)(t - sv.t0) * N;
+      stats_t = sv.stats + (size_t)(t - sv.t0) * B * 2;
+    } else {
+      a.u = r.u;
+      a.stats = r.stats;
+      rc = dispatch_step_recompute(m, P, packed, a, fws, st);
+      if (rc) return rc;
+    }
+    float* gnext = (t == 0) ? g0 : (((T - 1 - t) & 1) ? r.g_b : r.g_a);
+    // the frame of step t is x_t after the damage: its gradient joins dL/dx_t before the damage mask multiplies it
+    const float* gframe = (g_frames && t % every == 0) ? g_frames + (size_t)(t / every) * N : nullptr;
+    rc = run_step_bwd(m, P, packed, a, stats_t, *gcur, gnext, gparams, fws, bws, t == T - 1, t == 0, st, gframe);
+    if (rc) return rc;
+    if (s.damage && t == s.damage_step) {
+      rc = launch_damage(N, gnext, s, m.C, H * W, st);
+      if (rc) return rc;
+    }
+    *gcur = gnext;
+  }
+  return 0;
+}
+
+// Segment buffer of gnca_rollout_bwd_ckpt: the recomputed x_t of a segment's steps after its first, then u_t and stats_t
+// of every step of the segment
+struct Segment {
+  float* x;       // [every - 1][B][C][H][W]
+  float* u;       // [every][B][C][H][W]
+  float* stats;   // [every][B][2]
+  size_t bytes;
+};
+
+static Segment carve_segment(void* base, const gnca_model& m, int B, int H, int W, int every) {
+  Segment s;
+  const size_t N = (size_t)B * m.C * H * W * sizeof(float);
+  char* p = reinterpret_cast<char*>(base);
+  size_t o = 0;
+  s.x = reinterpret_cast<float*>(p + o); o = al(o + (size_t)(every - 1) * N);
+  s.u = reinterpret_cast<float*>(p + o); o = al(o + (size_t)every * N);
+  s.stats = reinterpret_cast<float*>(p + o); o = al(o + (size_t)every * B * 2 * sizeof(float));
+  s.bytes = o;
+  return s;
+}
+
 // gnca_rollout_fwd with a strided history: x_t of every step t % every == 0 goes to x_hist slot t / every
 // (every == 1: the full [T+1] history of gnca_rollout_fwd).
 static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
@@ -123,8 +220,8 @@ static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int 
   GNCA_CHECK_CUDA(cudaMemcpyAsync(x_at(0), x0_dev, N * sizeof(float), cudaMemcpyDeviceToDevice, st));
   for (int t = 0; t < T; ++t) {
     if (sched->damage && t == sched->damage_step) {
-      k_mul_inplace<<<(int)((N + 1023) / 1024 < 2368 ? (N + 1023) / 1024 : 2368), 256, 0, st>>>(N, x_at(t), DamageView{sched->damage, sched->damage_layout}, m->C, H * W);
-      GNCA_LAUNCH_CHECK();
+      int rc = launch_damage(N, x_at(t), *sched, m->C, H * W, st);
+      if (rc) return rc;
     }
     StepArgs a;
     fill_step_args(a, *m, B, H, W);
@@ -249,7 +346,6 @@ int gnca_rollout_bwd_frames(const gnca_model* m, const float* packed_dev, int B,
   if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
   if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
   (void)impl;             // the backward currently always takes the streaming kernels (x_hist layout is shared)
-  const bool saved = u_hist_dev != nullptr && stats_hist_dev != nullptr;   // else u and the statistics are recomputed
   const bool graph = (m->flags & GNCA_F_GRAPH) != 0;
   cudaStream_t st = (cudaStream_t)stream;
   RolloutWorkspace r = carve_rollout(workspace_dev, *m, B, H, W);
@@ -257,47 +353,74 @@ int gnca_rollout_bwd_frames(const gnca_model* m, const float* packed_dev, int B,
   const size_t N = (size_t)B * m->C * H * W;
   const Packed P = make_packed(m->C, m->hidden, m->d_model, graph);
   FwdWorkspace fws = carve_fwd_workspace(r.step_ws, *m, B, H, W);
+  const int T = sched->T;
+  const float* gcur;
+  int rc = bwd_begin(N, T, every, g_frames_dev, gT_dev, g0_dev, r, &gcur, st);
+  if (rc || T == 0) return rc;
+  // u and the statistics are recomputed per step unless both histories are given
+  const SavedSteps sv{x_hist_dev, x_hist_dev + N, u_hist_dev, stats_hist_dev, 0};
+  return bwd_steps(*m, P, packed_dev, B, H, W, *sched, sv, 0, T, every, g_frames_dev, &gcur, g0_dev, gparams_dev, r, fws,
+                   r.step_ws + fws.bytes, st);
+}
+
+size_t gnca_ckpt_segment_bytes(const gnca_model* m, int B, int H, int W, int every) {
+  if (!m || B <= 0 || H <= 0 || W <= 0 || every <= 0) return 0;
+  return carve_segment(nullptr, *m, B, H, W, every).bytes;
+}
+
+int gnca_rollout_bwd_ckpt(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                          const gnca_schedule* sched, const float* ckpt_dev, int every,
+                          const float* g_frames_dev, const float* gT_dev, float* g0_dev, float* gparams_dev,
+                          void* segment_dev, size_t segment_bytes,
+                          void* workspace_dev, size_t workspace_bytes, void* stream) {
+  if (!m || !packed_dev || !sched || !ckpt_dev || !gT_dev || !g0_dev || !gparams_dev || !segment_dev || !workspace_dev)
+    return GNCA_ERR_ARG;
+  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0 || every <= 0) return GNCA_ERR_ARG;
+  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  const bool graph = (m->flags & GNCA_F_GRAPH) != 0;
+  if (sched->T > 0 && (!sched->fire_rate || (graph && !sched->message_gain))) return GNCA_ERR_ARG;
+  if (graph && sched->k > 0 && !sched->offsets) return GNCA_ERR_ARG;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
+  const Segment seg = carve_segment(segment_dev, *m, B, H, W, every);
+  if (seg.bytes > segment_bytes) return GNCA_ERR_WORKSPACE;
+  RolloutWorkspace r = carve_rollout(workspace_dev, *m, B, H, W);
+  if (r.bytes > workspace_bytes) return GNCA_ERR_WORKSPACE;
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t N = (size_t)B * m->C * H * W;
+  const Packed P = make_packed(m->C, m->hidden, m->d_model, graph);
+  // The recomputed forward writes only the segment, r.ping and the forward workspace: the weight-gradient partials in
+  // the backward workspace stay live from t = T - 1 to t = 0
+  FwdWorkspace fws = carve_fwd_workspace(r.step_ws, *m, B, H, W);
   char* bws = r.step_ws + fws.bytes;
   const int T = sched->T;
-  if (T == 0) {
-    if (g_frames_dev) return fold_last_frame(N, T, every, g_frames_dev, gT_dev, g0_dev, st);
-    GNCA_CHECK_CUDA(cudaMemcpyAsync(g0_dev, gT_dev, N * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    return 0;
-  }
-  const float* gcur = gT_dev;
-  if (g_frames_dev && T % every == 0) {          // g_b is not written before the second step (t = T - 2)
-    int rc = fold_last_frame(N, T, every, g_frames_dev, gT_dev, r.g_b, st);
-    if (rc) return rc;
-    gcur = r.g_b;
-  }
-  for (int t = T - 1; t >= 0; --t) {
-    StepArgs a;
-    fill_step_args(a, *m, B, H, W);
-    schedule_to_args(a, *sched, t, B, H, W);
-    if (!graph) a.k = 0;
-    a.x_in = x_hist_dev + (size_t)t * N;
-    a.x_out = nullptr;
-    const float* stats_t = r.stats;
-    int rc = 0;
-    if (saved) {
-      a.u = const_cast<float*>(u_hist_dev) + (size_t)t * N;
-      stats_t = stats_hist_dev + (size_t)t * B * 2;
-    } else {
-      a.u = r.u;
-      a.stats = r.stats;
-      rc = dispatch_step_recompute(*m, P, packed_dev, a, fws, st);
+  const float* gcur;
+  int rc = bwd_begin(N, T, every, g_frames_dev, gT_dev, g0_dev, r, &gcur, st);
+  if (rc || T == 0) return rc;
+  for (int j = (T - 1) / every; j >= 0; --j) {
+    const int t_lo = j * every, t_hi = t_lo + every < T ? t_lo + every : T;
+    const SavedSteps sv{ckpt_dev + (size_t)j * N, seg.x, seg.u, seg.stats, t_lo};
+    for (int t = t_lo; t < t_hi; ++t) {
+      float* x_in = const_cast<float*>(t == t_lo ? sv.x0 : seg.x + (size_t)(t - t_lo - 1) * N);
+      // a checkpoint is the state after the damage: only a damage step inside the segment is applied here
+      if (sched->damage && t == sched->damage_step && t != t_lo) {
+        rc = launch_damage(N, x_in, *sched, m->C, H * W, st);
+        if (rc) return rc;
+      }
+      StepArgs a;
+      fill_step_args(a, *m, B, H, W);
+      schedule_to_args(a, *sched, t, B, H, W);
+      if (!graph) a.k = 0;
+      a.x_in = x_in;
+      // the segment's last output (the next checkpoint, or x_T) is not needed by the backward
+      a.x_out = t + 1 < t_hi ? seg.x + (size_t)(t - t_lo) * N : r.ping;
+      a.u = seg.u + (size_t)(t - t_lo) * N;
+      a.stats = seg.stats + (size_t)(t - t_lo) * B * 2;
+      rc = dispatch_step_fwd(*m, P, packed_dev, a, fws, nullptr, st);
       if (rc) return rc;
     }
-    float* gnext = (t == 0) ? g0_dev : (((T - 1 - t) & 1) ? r.g_b : r.g_a);
-    // the frame of step t is x_t after the damage: its gradient joins dL/dx_t before the damage mask multiplies it
-    const float* gframe = (g_frames_dev && t % every == 0) ? g_frames_dev + (size_t)(t / every) * N : nullptr;
-    rc = run_step_bwd(*m, P, packed_dev, a, stats_t, gcur, gnext, gparams_dev, fws, bws, t == T - 1, t == 0, st, gframe);
+    rc = bwd_steps(*m, P, packed_dev, B, H, W, *sched, sv, t_lo, t_hi, every, g_frames_dev, &gcur, g0_dev, gparams_dev,
+                   r, fws, bws, st);
     if (rc) return rc;
-    if (sched->damage && t == sched->damage_step) {
-      k_mul_inplace<<<(int)((N + 1023) / 1024 < 2368 ? (N + 1023) / 1024 : 2368), 256, 0, st>>>(N, gnext, DamageView{sched->damage, sched->damage_layout}, m->C, H * W);
-      GNCA_LAUNCH_CHECK();
-    }
-    gcur = gnext;
   }
   return 0;
 }

@@ -328,18 +328,94 @@ class _RolloutFn(torch.autograd.Function):
         return (g0, None, *grads)
 
 
+class _CkptFn(torch.autograd.Function):
+    """Checkpointed BPTT: the forward keeps x_{j*every} (gnca_rollout_record on the streaming kernels) and returns them
+    with x_T; the backward recomputes one segment of `every` steps at a time from them (gnca_rollout_bwd_ckpt)."""
+
+    @staticmethod
+    def forward(ctx, x0, cfg, *params):
+        x0 = GF._require_cuda_f32(x0, "x0")
+        B, Cc, H, W = x0.shape
+        desc, sched, every = cfg["desc"], cfg["schedule"], cfg["every"]
+        if Cc != desc.C:
+            raise ValueError(f"x0 has {Cc} channels, model has {desc.C}")
+        lib = _lib.load()
+        xT = torch.empty_like(x0)
+        ckpt = torch.empty(sched.T // every + 1, B, Cc, H, W, dtype=torch.float32, device=x0.device)
+        ws = GF._WS.get(x0.device, lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, sched.T))
+        cs = sched.c_struct()
+        _lib.check(lib.gnca_rollout_record(C.byref(desc), GF._ptr(cfg["packed"]), B, H, W, C.byref(cs), GF._ptr(x0),
+                                           GF._ptr(xT), every, GF._ptr(ckpt), None, GF._ptr(ws), ws.numel(),
+                                           IMPL["streaming"], GF._stream()), "gnca_rollout_record")
+        ctx.set_materialize_grads(False)          # an unused output passes None: no zero tensor, no frame pass
+        ctx.cfg = cfg
+        ctx.param_shapes = [p.shape for p in params]
+        ctx.consumed = False
+        ctx.save_for_backward(ckpt)               # an in-place edit of a returned checkpoint makes the backward raise
+        return ckpt, xT
+
+    @staticmethod
+    def backward(ctx, g_ckpt, g_xT):
+        if ctx.consumed:
+            raise RuntimeError("rollout: the checkpoints were already consumed by an earlier backward")
+        (ckpt,) = ctx.saved_tensors
+        cfg = ctx.cfg
+        desc, sched, every = cfg["desc"], cfg["schedule"], cfg["every"]
+        _, B, Cc, H, W = ckpt.shape
+        lib = _lib.load()
+        g_xT = torch.zeros_like(ckpt[0]) if g_xT is None else GF._require_cuda_f32(g_xT, "grad_output")
+        if g_ckpt is not None:
+            g_ckpt = GF._require_cuda_f32(g_ckpt, "frame gradients")
+        g0 = torch.empty_like(ckpt[0])
+        gflat = torch.zeros(GF.param_layout(desc).total, dtype=torch.float32, device=ckpt.device)
+        segment = torch.empty(lib.gnca_ckpt_segment_bytes(C.byref(desc), B, H, W, every), dtype=torch.uint8,
+                              device=ckpt.device)
+        ws = GF._WS.get(ckpt.device, lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, sched.T))
+        cs = sched.c_struct()
+        _lib.check(lib.gnca_rollout_bwd_ckpt(C.byref(desc), GF._ptr(cfg["packed"]), B, H, W, C.byref(cs),
+                                             GF._ptr(ckpt), every, GF._ptr(g_ckpt), GF._ptr(g_xT), GF._ptr(g0),
+                                             GF._ptr(gflat), GF._ptr(segment), segment.numel(), GF._ptr(ws),
+                                             ws.numel(), GF._stream()), "gnca_rollout_bwd_ckpt")
+        ctx.consumed = True
+        offs = GF.segment_offsets(desc)
+        grads = [gflat[offs[i]:offs[i + 1]].view(ctx.param_shapes[i]) for i in range(len(ctx.param_shapes))]
+        return (g0, None, *grads)
+
+
+def _check_checkpoint_impl(impl: str, what: str) -> None:
+    if impl in ("resident", "banded"):
+        raise ValueError(f"{what}: checkpoints are recomputed with the streaming kernels, so impl={impl!r} cannot "
+                         "produce them; use impl='auto' or 'streaming'")
+
+
 IMPL = {"auto": 0, "streaming": 1, "resident": 2, "banded": 3}
 
 
-def rollout(model, x0: torch.Tensor, schedule: Schedule, *, return_history: bool = False, impl: str = "auto"):
+def rollout(model, x0: torch.Tensor, schedule: Schedule, *, checkpoint_every: Optional[int] = None,
+            return_history: bool = False, impl: str = "auto"):
     """x_T (and optionally the [T+1,B,C,H,W] history) of T steps from x0 under `schedule`.  Differentiable
-    w.r.t. x0 and the model parameters (BPTT stores x_t only and recomputes the rest)."""
+    w.r.t. x0 and the model parameters (BPTT stores x_t only and recomputes the rest).
+
+    `checkpoint_every=K` (with grad): the forward keeps only x_{jK} and the backward recomputes each K-step segment
+    from its checkpoint on the streaming kernels, so BPTT memory is T/K + 1 states plus one segment instead of the
+    2T + 1 states of the dense history.  The gradients equal those of the dense streaming BPTT.  Without grad it
+    changes nothing."""
+    if checkpoint_every is not None:
+        if int(checkpoint_every) < 1:
+            raise ValueError(f"rollout: checkpoint_every must be >= 1, got {checkpoint_every}")
+        if return_history:
+            raise ValueError("rollout: return_history=True keeps every state; it cannot be combined with checkpoint_every")
+        _check_checkpoint_impl(impl, "rollout")
     if not x0.is_cuda:
         raise RuntimeError(f"rollout: x0 is on {x0.device}; CUDA (sm_100a) only, no CPU fallback")
     ps = model.canonical_params()
     need_grad = torch.is_grad_enabled() and (x0.requires_grad or any(p.requires_grad for p in ps))
     if not need_grad and not return_history:        # inference: no autograd node, no history (same C call underneath)
         return rollout_fwd_raw(model.model_desc(), model.packed_weights(), x0, schedule, history=False, impl=IMPL[impl])[0]
+    if checkpoint_every is not None:
+        cfg = {"desc": model.model_desc(), "packed": model.packed_weights(), "schedule": schedule,
+               "every": int(checkpoint_every)}
+        return _CkptFn.apply(x0, cfg, *ps)[1]
     cfg = {"desc": model.model_desc(), "packed": model.packed_weights(), "schedule": schedule, "need_grad": need_grad,
            "history": bool(return_history), "impl": IMPL[impl]}
     return _RolloutFn.apply(x0, cfg, *ps)
@@ -386,7 +462,7 @@ class Trajectory:
 
 
 def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, attention: bool = False,
-                   impl: str = "auto", differentiable: bool = False) -> Trajectory:
+                   impl: str = "auto", differentiable: bool = False, checkpoint: bool = False) -> Trajectory:
     """T steps from x0 under `schedule` in one library call (gnca_rollout_record), keeping x_t every `every` steps and,
     with `attention=True`, the attention map `model.step(x_t, ..., return_attention=True)` gives for each kept step
     t < T.  Watching a rollout this way keeps the fused rollout kernels; no gradient history or record buffer is
@@ -396,10 +472,18 @@ def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, a
     of one autograd node, and a loss on any of them back-propagates to x0 and the parameters through one fused BPTT --
     the gradients of T sequential `model.step` calls with the same schedule.  The BPTT history is the one `rollout()`
     keeps for its backward.  `attention` stays detached (it costs one more, inference-only rollout).  Without grad the
-    call is exactly the detached recording."""
+    call is exactly the detached recording.
+
+    `checkpoint=True` (with `differentiable=True`): the recorded frames are the only history.  The backward recomputes
+    each `every`-step segment from its frame on the streaming kernels (rollout(..., checkpoint_every=every)), so memory
+    is the frames plus one segment.  Editing a returned frame in place makes the backward raise."""
     every = int(every)
     if every < 1:
         raise ValueError(f"record_rollout: every must be >= 1, got {every}")
+    if checkpoint:
+        if not differentiable:
+            raise ValueError("record_rollout: checkpoint=True needs differentiable=True")
+        _check_checkpoint_impl(impl, "record_rollout")
     if attention and not getattr(model, "_is_graph", False):
         raise ValueError("record_rollout: attention maps need a graph model (NeuralCAGraph)")
     if not x0.is_cuda:
@@ -412,7 +496,7 @@ def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, a
                 raise ValueError(f"x0 has {x0.shape[1]} channels, model has {desc.C}")
             cfg = {"desc": desc, "packed": model.packed_weights(), "schedule": schedule, "impl": IMPL[impl],
                    "every": every}
-            frames, xT = _RecordFn.apply(x0, cfg, *ps)
+            frames, xT = (_CkptFn if checkpoint else _RecordFn).apply(x0, cfg, *ps)
             attn = None
             if attention:
                 with torch.no_grad():

@@ -247,6 +247,32 @@ int gnca_rollout_bwd_frames(const gnca_model* m, const float* packed_dev, int B,
                             void* workspace_dev, size_t workspace_bytes, int impl, void* stream);
 
 /*
+ * Checkpointed BPTT: memory that does not grow with T on the streaming path.  The forward is gnca_rollout_record with
+ * impl = 1 (streaming): its frames x_{j*every} are the checkpoints.  They must come from the streaming kernels, because
+ * the backward recomputes every segment with them and relies on reproducing the forward bit for bit.  The backward
+ * keeps the checkpoints plus one segment: (every - 1) states, `every` pre-norm updates and `every` [B][2] statistics
+ * instead of the T + 1 states and T updates of the dense history.
+ *
+ * gnca_ckpt_segment_bytes: bytes of that segment buffer, each region 256-byte aligned; 0 on bad arguments.
+ *
+ * gnca_rollout_bwd_ckpt: ckpt_dev [T/every+1][B][C][H][W] = the frames gnca_rollout_record(..., every, impl = 1) wrote.
+ * Segments are processed last to first.  For each one, the forward of its steps is recomputed from its checkpoint into
+ * segment_dev, with the streaming kernels, the same schedule and the absolute step indices (Philox, steps[b], fire_u and
+ * the offsets key on them); a checkpoint at damage_step is already post-damage, a damage step inside a segment is applied
+ * to the recomputed state.  Then the per-step backward runs over the segment.  g_frames_dev (optional, same shape as
+ * ckpt_dev) has the semantics of gnca_rollout_bwd_frames.  The result equals gnca_rollout_bwd on the full streaming
+ * history.  gparams is ACCUMULATED.  Argument errors return before any launch: a NULL required pointer, every <= 0 or
+ * T < 0 is GNCA_ERR_ARG; a segment or workspace (gnca_rollout_workspace_bytes) too small is GNCA_ERR_WORKSPACE; k
+ * outside [0, GNCA_MAX_K] is GNCA_ERR_UNSUPPORTED.
+ */
+size_t gnca_ckpt_segment_bytes(const gnca_model* m, int B, int H, int W, int every);
+int gnca_rollout_bwd_ckpt(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                          const gnca_schedule* sched, const float* ckpt_dev, int every,
+                          const float* g_frames_dev, const float* gT_dev, float* g0_dev, float* gparams_dev,
+                          void* segment_dev, size_t segment_bytes,
+                          void* workspace_dev, size_t workspace_bytes, void* stream);
+
+/*
  * Resident BPTT (16-channel / 128-hidden models, classic or torus graph, grids up to 2048 cells with W % 4 == 0).
  * Instead of the dense x_t / u_t history the forward keeps one compact record per ACTIVE cell and step (perception,
  * pre-norm update, gathered sender state ...) plus three bitmaps and the GroupNorm statistics per step, in the opaque
