@@ -68,9 +68,13 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
 
 // replicated-state cluster rollout (gnca_rep.cu): every CTA of a sample's cluster holds the whole sample; first
 // choice of the resident path.  scratch: >= B*C*H*W floats of device memory (overflow of the in-smem u buffer).
+// t0: absolute step of the launch's first step, for a `sched` rebased to the launch (a checkpoint segment); only
+// sched.steps stays absolute.  The launch configuration depends on B and H*W only, so a segment launch reproduces the
+// steps of a whole-rollout launch bit for bit.
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
-                float* u_hist, float* rec, uint32_t* masks, float* scratch, cudaStream_t st, int hist_every = 1);
+                float* u_hist, float* rec, uint32_t* masks, float* scratch, cudaStream_t st, int hist_every = 1,
+                int t0 = 0);
 // resident BPTT on the records of run_rep_fwd (gnca_rep_bwd.cu).  g_frames (optional, [F][B][C][H][W]): dL/dx_{f*every}
 // added at step f * every (gnca_rollout_bwd_bptt_frames)
 size_t rep_bptt_bytes(const gnca_model& m, int B, int H, int W, int T);     // 0: configuration not supported
@@ -80,6 +84,6 @@ size_t rep_bwd_workspace_bytes(const gnca_model& m, int B, int H, int W);
 bool rep_bwd_supported(const gnca_model& m, int B, int H, int W, int k);    // a launch configuration of k_rep_bwd exists
 int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, void* bptt, const float* gT, float* g0, float* gparams, void* workspace,
-                cudaStream_t st, const float* g_frames = nullptr, int every = 1);
+                cudaStream_t st, const float* g_frames = nullptr, int every = 1, int t0 = 0);
 
 }  // namespace gnca

@@ -60,6 +60,10 @@ struct RepArgs {
   unsigned long long* dbg;
   int dbg_cta;
   int use_async;              // 1: st.async + mbarrier transaction counts between the CTAs, 0: two cluster barriers per step
+  // absolute step of the launch's local step 0 (a checkpoint segment starts at t0 = j * every).  The caller hands
+  // run_rep_fwd a schedule already rebased to the launch (arrays, fire_u, Philox counter, damage_step: segment_schedule
+  // in gnca_rollout.cu); the kernel needs t0 only for the per-sample step counts steps[b], which stay absolute
+  int t0;
 };
 
 #ifdef GNCA_PHASE_COUNTERS          /* build with -DGNCA_PHASE_COUNTERS for the per-phase cycle counters */
@@ -389,7 +393,7 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
   }
   cluster_arrive(); cluster_wait();              // every replica initialised before any remote store
 
-  const int my_steps = a.steps ? min(a.steps[b], R.T) : R.T;
+  const int my_steps = a.steps ? min(a.steps[b] - R.t0, R.T) : R.T;
   long long t_prev = clock64();
   float* myY = sY + warp * (C3 * 8);
   short* myq = sq + warp * (8 * 16);
@@ -923,7 +927,7 @@ static size_t rep_smem_bytes(int C, int HW, int ucap, int listcap) {
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                 float* u_hist, float* rec, uint32_t* masks, float* scratch /* >= B*C*H*W floats */, cudaStream_t st,
-                int hist_every) {
+                int hist_every, int t0) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (m.C != 16 || m.hidden != 128) return GNCA_ERR_UNSUPPORTED;
   if (H > kMaxRows || W > kMaxRows || H < 1 || W < 4 || (W & 3)) return GNCA_ERR_UNSUPPORTED;   // quads of 4 cells per row
@@ -948,6 +952,7 @@ int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B
   R.s.philox_offset = sched.philox_offset;
   R.fire_u_base = sched.fire_u;
   R.T = sched.T;
+  R.t0 = t0;
   R.x0 = x0; R.xT = xT; R.hist = hist; R.hist_every = hist_every; R.stats_hist = stats_hist; R.u_hist = u_hist;
   R.rec = rec; R.masks = masks;
   R.damage = DamageView{sched.damage, sched.damage_layout}; R.damage_step = sched.damage_step;

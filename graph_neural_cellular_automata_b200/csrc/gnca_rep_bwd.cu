@@ -56,6 +56,7 @@ struct RepBwdArgs {
   int damage_step;
   unsigned long long* dbg;    // optional phase-cycle counters (GNCA_PHASE_TIMING=<cta>)
   int dbg_cta;
+  int t0;                     // absolute step of local step 0 (see RepArgs::t0): only steps[b] is absolute
 };
 
 #ifdef GNCA_PHASE_COUNTERS          /* build with -DGNCA_PHASE_COUNTERS for the per-phase cycle counters */
@@ -172,7 +173,7 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
   __syncthreads();
   cluster_sync_acquire();
 
-  const int my_steps = a.steps ? min(a.steps[b], R.T) : R.T;
+  const int my_steps = a.steps ? min(a.steps[b] - R.t0, R.T) : R.T;
   const int q = tid, qcell = 4 * tid;
   const bool qv = q < NQ;
   const int qsh = 4 * (lane & 7), qword = min(q >> 3, kMaskWords - 1);
@@ -680,8 +681,9 @@ struct WgradArgs {
   const float* rec;
   const float* hgh;
   const uint32_t* masks;
-  const int32_t* steps;       // [B] or null
+  const int32_t* steps;       // [B] or null (absolute step counts)
   int T, B, HW, NW;
+  int t0;                     // absolute step of record step 0
   uint32_t flags;
   float* wpart;               // [gridDim.x][wtotal]
   int64_t wtotal;
@@ -726,7 +728,7 @@ __global__ void __launch_bounds__(kWT, 2) k_rep_wgrad(WgradArgs A) {
       int cnt = 0;
       if (seg < nseg) {
         const int t = seg / A.B, b = seg - t * A.B;
-        if (!(A.steps && A.steps[b] <= t)) {
+        if (!(A.steps && A.steps[b] - A.t0 <= t)) {
           const uint32_t* mk = A.masks + ((size_t)seg * 3 + 1) * kMaskWords;
           for (int i = 0; i < A.NW; ++i) cnt += __popc(__ldg(mk + i));
         }
@@ -916,7 +918,7 @@ bool rep_bwd_supported(const gnca_model& m, int B, int H, int W, int k) {
 
 int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, void* bptt, const float* gT, float* g0, float* gparams, void* workspace,
-                cudaStream_t st, const float* g_frames, int every) {
+                cudaStream_t st, const float* g_frames, int every, int t0) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (rep_bptt_bytes(m, B, H, W, sched.T) == 0) return GNCA_ERR_UNSUPPORTED;
   const int k = graph ? sched.k : 0;
@@ -940,6 +942,7 @@ int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B
   R.s.offsets_dev = sched.offsets;
   R.s.steps = sched.steps;
   R.T = sched.T;
+  R.t0 = t0;
   R.inv_n = (float)(1.0 / ((double)C * (double)H * (double)W));
   R.rec = rec; R.hgh = hgh; R.masks = masks; R.stats = stats; R.gT = gT; R.g0 = g0; R.GZ = GZ; R.RG = RG;
   R.affpart = affpart;
@@ -989,7 +992,7 @@ int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B
 
   // weight gradients from the records
   WgradArgs A{};
-  A.rec = rec; A.hgh = hgh; A.masks = masks; A.steps = sched.steps; A.T = sched.T; A.B = B; A.HW = HW; A.NW = (HW + 31) >> 5;
+  A.rec = rec; A.hgh = hgh; A.masks = masks; A.steps = sched.steps; A.T = sched.T; A.t0 = t0; A.B = B; A.HW = HW; A.NW = (HW + 31) >> 5;
   A.flags = m.flags; A.wpart = wpart; A.wtotal = L.total; A.L = L;
   int nseg = sched.T * B;
   int nblk = nseg < kMaxWgradBlocks ? nseg : kMaxWgradBlocks;

@@ -269,6 +269,56 @@ static int rollout_fwd_bptt(const gnca_model* m, const float* packed_dev, int B,
                      (cudaStream_t)stream, every);
 }
 
+// The schedule of steps [t0, t0 + n) as a launch of its own: per-step arrays and fire_u start at t0, the Philox counter
+// is advanced by the blocks of t0 steps (the resident kernels key block ((t*B + b)*HW >> 2) + q + philox_offset, and
+// H*W % 4 == 0 there, so this is exact), and damage_step becomes local.  `damage_at_start`: whether a damage step at t0
+// itself stays in the segment -- the backward must multiply its gradient, while a recomputed forward starts from a
+// checkpoint that is already post-damage.  steps[b] stays absolute (the kernels take t0 for it).
+static gnca_schedule segment_schedule(const gnca_schedule& s, int t0, int n, int B, int H, int W, bool damage_at_start) {
+  gnca_schedule r = s;
+  const size_t HW = (size_t)H * W;
+  r.T = n;
+  r.fire_rate = s.fire_rate ? s.fire_rate + t0 : nullptr;
+  r.message_gain = s.message_gain ? s.message_gain + t0 : nullptr;
+  r.offsets = s.offsets ? s.offsets + (size_t)t0 * s.k * 2 : nullptr;
+  r.fire_u = s.fire_u ? s.fire_u + (size_t)t0 * B * HW : nullptr;
+  r.philox_offset = s.philox_offset + (uint64_t)t0 * (uint64_t)B * (HW >> 2);
+  const int lo = damage_at_start ? t0 : t0 + 1;
+  if (s.damage && s.damage_step >= lo && s.damage_step < t0 + n) {
+    r.damage_step = s.damage_step - t0;
+  } else {
+    r.damage = nullptr;
+    r.damage_step = 0;
+  }
+  return r;
+}
+
+// Segment buffer of gnca_rollout_bwd_bptt_ckpt: the records of `every` steps (rep_bptt_carve layout of the segment's
+// step count), the gradient carried between segments, and x_T of the recomputed forward (not needed, but the kernel
+// writes it).  Neither may live in the rollout workspace: the resident backward's scratch (GZ, RG, partials) starts at
+// its base, where the recomputed forward also keeps its u overflow.
+struct RepSegment {
+  void* bptt;
+  size_t bptt_bytes;
+  float* g;       // [B][C][H][W]
+  float* xT;      // [B][C][H][W]
+  size_t bytes;
+};
+
+static RepSegment carve_rep_segment(void* base, const gnca_model& m, int B, int H, int W, int every) {
+  RepSegment s;
+  const size_t N = (size_t)B * m.C * H * W * sizeof(float);
+  char* p = reinterpret_cast<char*>(base);
+  size_t o = 0;
+  s.bptt = p;
+  s.bptt_bytes = rep_bptt_bytes(m, B, H, W, every);
+  o = al(o + s.bptt_bytes);
+  s.g = reinterpret_cast<float*>(p + o); o = al(o + N);
+  s.xT = reinterpret_cast<float*>(p + o); o = al(o + N);
+  s.bytes = o;
+  return s;
+}
+
 }  // namespace gnca
 
 using namespace gnca;
@@ -487,6 +537,90 @@ int gnca_rollout_bwd_bptt(const gnca_model* m, const float* packed_dev, int B, i
                           void* workspace_dev, size_t workspace_bytes, void* stream) {
   return gnca_rollout_bwd_bptt_frames(m, packed_dev, B, H, W, sched, bptt_dev, bptt_bytes, 0, nullptr, gT_dev, g0_dev,
                                       gparams_dev, workspace_dev, workspace_bytes, stream);
+}
+
+/* ---- checkpointed resident BPTT: x_{j*every} only; each segment's records are recomputed in the backward ---- */
+size_t gnca_bptt_ckpt_bytes(const gnca_model* m, int B, int H, int W, int every) {
+  if (!m || B <= 0 || H <= 0 || W <= 0 || every <= 0) return 0;
+  if (gnca_bptt_bytes(m, B, H, W, every) == 0) return 0;
+  return carve_rep_segment(nullptr, *m, B, H, W, every).bytes;
+}
+
+int gnca_rollout_fwd_bptt_ckpt(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                               const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every, float* ckpt_dev,
+                               void* workspace_dev, size_t workspace_bytes, void* stream) {
+  if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !ckpt_dev || !workspace_dev) return GNCA_ERR_ARG;
+  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0 || every <= 0) return GNCA_ERR_ARG;
+  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  const bool graph = (m->flags & GNCA_F_GRAPH) != 0;
+  if (sched->T > 0 && (!sched->fire_rate || (graph && !sched->message_gain))) return GNCA_ERR_ARG;
+  if (graph && sched->k > 0 && !sched->offsets) return GNCA_ERR_ARG;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
+  if (gnca_bptt_bytes(m, B, H, W, 1) == 0) return GNCA_ERR_UNSUPPORTED;
+  RolloutWorkspace r = carve_rollout(workspace_dev, *m, B, H, W);
+  if (r.bytes > workspace_bytes) return GNCA_ERR_WORKSPACE;
+  // checkpoints are only worth keeping if the resident backward can recompute from them for this batch / shape
+  if (!rep_bwd_supported(*m, B, H, W, graph ? sched->k : 0)) return GNCA_ERR_UNSUPPORTED;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (sched->T == 0) {
+    const size_t nb = (size_t)B * m->C * H * W * sizeof(float);
+    GNCA_CHECK_CUDA(cudaMemcpyAsync(xT_dev, x0_dev, nb, cudaMemcpyDeviceToDevice, st));
+    GNCA_CHECK_CUDA(cudaMemcpyAsync(ckpt_dev, x0_dev, nb, cudaMemcpyDeviceToDevice, st));
+    return 0;
+  }
+  const Packed P = make_packed(m->C, m->hidden, m->d_model, graph);
+  // the same kernel, scratch and launch configuration as the recompute of gnca_rollout_bwd_bptt_ckpt: no records
+  return run_rep_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, ckpt_dev, nullptr, nullptr, nullptr, nullptr,
+                     r.ping, st, every, 0);
+}
+
+int gnca_rollout_bwd_bptt_ckpt(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                               const gnca_schedule* sched, const float* ckpt_dev, int every, const float* gT_dev,
+                               float* g0_dev, float* gparams_dev, void* segment_dev, size_t segment_bytes,
+                               void* workspace_dev, size_t workspace_bytes, void* stream) {
+  if (!m || !packed_dev || !sched || !ckpt_dev || !gT_dev || !g0_dev || !gparams_dev || !segment_dev || !workspace_dev)
+    return GNCA_ERR_ARG;
+  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0 || every <= 0) return GNCA_ERR_ARG;
+  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  const bool graph = (m->flags & GNCA_F_GRAPH) != 0;
+  if (sched->T > 0 && (!sched->fire_rate || (graph && !sched->message_gain))) return GNCA_ERR_ARG;
+  if (graph && sched->k > 0 && !sched->offsets) return GNCA_ERR_ARG;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
+  const size_t need = gnca_bptt_ckpt_bytes(m, B, H, W, every);
+  if (need == 0) return GNCA_ERR_UNSUPPORTED;
+  if (need > segment_bytes) return GNCA_ERR_WORKSPACE;
+  RolloutWorkspace r = carve_rollout(workspace_dev, *m, B, H, W);
+  if (r.bytes > workspace_bytes || rep_bwd_workspace_bytes(*m, B, H, W) > workspace_bytes) return GNCA_ERR_WORKSPACE;
+  if (!rep_bwd_supported(*m, B, H, W, graph ? sched->k : 0)) return GNCA_ERR_UNSUPPORTED;
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t N = (size_t)B * m->C * H * W;
+  const int T = sched->T;
+  if (T == 0) {
+    GNCA_CHECK_CUDA(cudaMemcpyAsync(g0_dev, gT_dev, N * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    return 0;
+  }
+  const Packed P = make_packed(m->C, m->hidden, m->d_model, graph);
+  const RepSegment seg = carve_rep_segment(segment_dev, *m, B, H, W, every);
+  const int nseg = (T - 1) / every + 1;
+  // dL/dx_{j*every} goes to g0 for even j and to the segment's slot for odd j: segment 0 ends in g0, and no launch
+  // reads the buffer it writes
+  auto g_at = [&](int j) -> float* { return (j & 1) ? seg.g : g0_dev; };
+  for (int j = nseg - 1; j >= 0; --j) {
+    const int t0 = j * every, n = T - t0 < every ? T - t0 : every;
+    float *rec, *stats;
+    uint32_t* masks;
+    rep_bptt_carve(seg.bptt, B, H, W, n, &rec, &masks, &stats);
+    // the checkpoint is x_t0 after a damage at t0: the recompute applies only a damage step inside the segment
+    const gnca_schedule sf = segment_schedule(*sched, t0, n, B, H, W, false);
+    int rc = run_rep_fwd(*m, P, packed_dev, B, H, W, sf, ckpt_dev + (size_t)j * N, seg.xT, nullptr, stats, nullptr, rec,
+                         masks, r.ping, st, 1, t0);
+    if (rc) return rc;
+    const gnca_schedule sb = segment_schedule(*sched, t0, n, B, H, W, true);
+    rc = run_rep_bwd(*m, P, packed_dev, B, H, W, sb, seg.bptt, j == nseg - 1 ? gT_dev : g_at(j + 1), g_at(j),
+                     gparams_dev, workspace_dev, st, nullptr, 1, t0);
+    if (rc) return rc;
+  }
+  return 0;
 }
 
 /* ---- host-side schedule construction: T x random.sample(range(n), k) on CPython's MT19937 state ----

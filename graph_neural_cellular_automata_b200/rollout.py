@@ -184,10 +184,13 @@ class History:
       cluster-resident backward (gnca_rollout_bwd_bptt); `x` is only filled when the caller asked for the history;
     * dense: x_t for every step and (optionally) the masked pre-norm update of the active cells + the GroupNorm
       statistics, consumed by the streaming backward (gnca_rollout_bwd).
-    `frames` (forward with `every`): x_{f*every} in a buffer of its own, the differentiable states of `record_rollout`."""
+    `frames` (forward with `every`): x_{f*every} in a buffer of its own, the differentiable states of `record_rollout`.
+    `ckpt` (forward with a BPTT budget that called for checkpoints): x_{j*every} only, recomputed segment by segment on
+    the resident (`resident`) or the streaming kernels; `plan` is the bptt_plan result of that forward."""
 
-    def __init__(self, x, u=None, stats=None, bptt=None, shape=None, frames=None):
+    def __init__(self, x, u=None, stats=None, bptt=None, shape=None, frames=None, ckpt=None, every=0, resident=False):
         self.x, self.u, self.stats, self.bptt, self.frames = x, u, stats, bptt, frames
+        self.ckpt, self.every, self.resident, self.plan = ckpt, every, resident, None
         self._shape = tuple(shape) if shape is not None else tuple(x.shape)
 
     @property
@@ -208,52 +211,247 @@ def _round_up_steps(T: int, q: int = 64) -> int:
 BPTT_MAX_BYTES = 48 << 30      # above this the record buffer is not worth it: dense history + streaming backward
 
 
+def _record_bytes(lib, desc, B: int, H: int, W: int, T: int) -> int:
+    """Bytes of the record buffer the resident BPTT forward allocates for T steps, or 0 when `rollout()` takes the dense
+    history instead (configuration without records, T = 0, or more than BPTT_MAX_BYTES)."""
+    if T <= 0:
+        return 0
+    nb = lib.gnca_bptt_bytes(C.byref(desc), B, H, W, T)
+    if not 0 < nb <= BPTT_MAX_BYTES:
+        return 0
+    # the record buffer is GBs (T*B*H*W*1.4 KB worst case): sized for T rounded up to 64 steps, so that rollouts of
+    # slightly different lengths (per-iteration step counts of the trainer) ask the caching allocator for the SAME
+    # block instead of a fresh cudaMalloc whenever a new maximum shows up (70 ms for 29 GB in the long regime)
+    nb_q = lib.gnca_bptt_bytes(C.byref(desc), B, H, W, _round_up_steps(T))
+    if nb <= nb_q <= BPTT_MAX_BYTES and nb_q - nb <= _QUANT_SLACK_BYTES:
+        nb = nb_q
+    return nb
+
+
+def _dense_steps(T: int, n_state: int) -> int:
+    """Steps the dense history is allocated for (T rounded up like the record buffer, within the same slack)."""
+    Tq = _round_up_steps(T)
+    return T if (Tq - T) * n_state * 4 > _QUANT_SLACK_BYTES else Tq
+
+
+def _dense_bytes(B: int, Cc: int, H: int, W: int, T: int) -> int:
+    """Bytes of the dense history rollout_fwd_raw allocates: x_t of T + 1 steps, u_t and the statistics of T steps."""
+    n = B * Cc * H * W
+    Tq = _dense_steps(T, n)
+    return (Tq + 1) * n * 4 + ((Tq * n * 4 + Tq * B * 2 * 4) if T > 0 else 0)
+
+
+RESIDENT_MAX_K = 16      # offsets per step the resident kernels take (gnca_rep.cu, rep_bwd_supported)
+
+
+def _bptt_plan(desc, B: int, H: int, W: int, T: int, budget: int, impl: int, k: int = 0, resident_ok: bool = True):
+    """bptt_plan on a model descriptor, an impl code and the schedule's offsets per step k; `resident_ok=False` leaves
+    the resident branches out (the launch found no resident backward for the batch)."""
+    lib = _lib.load()
+    n_bytes = B * desc.C * H * W * 4
+    resident_ok = resident_ok and k <= RESIDENT_MAX_K
+    eligible = resident_ok and lib.gnca_bptt_ckpt_bytes(C.byref(desc), B, H, W, 1) > 0
+    if impl == IMPL["resident"] and not eligible:
+        raise ValueError("rollout: impl='resident' with bptt_budget needs the resident BPTT, which this model / shape "
+                         f"does not have (16 channels, hidden 128, classic or torus graph, H*W <= 2048, W % 4 == 0, "
+                         f"at most {RESIDENT_MAX_K} offsets per step)")
+    nrec = _record_bytes(lib, desc, B, H, W, T) if (impl in (IMPL["auto"], IMPL["resident"]) and resident_ok) else 0
+    if nrec:
+        today = ("records", None, nrec)
+    elif impl == IMPL["resident"]:
+        today = None                                   # the dense history belongs to the streaming backward
+    else:
+        today = ("dense", None, _dense_bytes(B, desc.C, H, W, T))
+    if today is not None and today[2] <= budget:
+        return today
+    branches = []
+    if eligible and impl in (IMPL["auto"], IMPL["resident"]):
+        branches.append(("resident_ckpt", lambda K: lib.gnca_bptt_ckpt_bytes(C.byref(desc), B, H, W, K)))
+    if impl in (IMPL["auto"], IMPL["streaming"]):
+        branches.append(("streaming_ckpt", lambda K: lib.gnca_ckpt_segment_bytes(C.byref(desc), B, H, W, K)))
+    smallest = today[2] if today is not None else None
+    for path, segment_bytes in branches:
+        # largest K first: the fewest segment launches (the recompute costs one forward whatever K is)
+        for K in range(max(T, 1), 0, -1):
+            need = (T // K + 1) * n_bytes + segment_bytes(K)
+            if need <= budget:
+                return path, K, need
+            smallest = need if smallest is None else min(smallest, need)
+    raise ValueError(f"rollout: bptt_budget={budget} bytes is too small for this rollout (B={B}, {H}x{W}, T={T}); "
+                     f"the smallest budget that works is {smallest} bytes")
+
+
+def bptt_plan(model, B: int, H: int, W: int, T: int, budget: int, impl: str = "auto", k: Optional[int] = None):
+    """Which BPTT history `rollout(..., bptt_budget=budget)` keeps for a B x C x H x W batch over T steps, without
+    touching the GPU: `(path, every, bytes)`.
+
+    * "records" / "dense": the history `rollout()` keeps without a budget (resident records, or the dense x_t / u_t
+      history of the streaming backward), when it fits; `every` is None.
+    * "resident_ckpt": x_{j*every} only, each segment's records recomputed on the resident kernels (models and shapes
+      that have the resident BPTT).
+    * "streaming_ckpt": x_{j*every} only, recomputed on the streaming kernels (`checkpoint_every`).
+    `every` is the largest stride whose checkpoints plus segment buffer fit; `bytes` is what the history takes (the
+    rollout workspace comes on top).  ValueError names the smallest budget that works when nothing fits.
+
+    `k`: offsets per step of the schedule (default: what `make_schedule` draws for the model, 0 for a classic model);
+    more than RESIDENT_MAX_K leaves the resident branches out, as in rollout().  rollout() takes this plan, except when
+    the resident backward finds no cluster launch configuration for the batch at run time: it then plans again
+    without the resident branches."""
+    if impl not in ("auto", "resident", "streaming"):
+        raise ValueError(f"bptt_plan: impl must be 'auto', 'resident' or 'streaming', got {impl!r}")
+    if int(budget) < 0:
+        raise ValueError(f"bptt_plan: budget must be >= 0, got {budget}")
+    if k is None:
+        g = getattr(model, "graph", None) if getattr(model, "_is_graph", False) else None
+        k = min(g.num_neighbors, len(g.offsets)) if g is not None else 0
+    return _bptt_plan(model.model_desc(), int(B), int(H), int(W), int(T), int(budget), IMPL[impl], int(k))
+
+
+def _ckpt_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, every: int, resident: bool):
+    """Checkpointing forward: (x_T, [T // every + 1, B, C, H, W] checkpoints), or None when the resident branch has no
+    backward for this launch (nothing was launched)."""
+    B, Cc, H, W = x0.shape
+    lib = _lib.load()
+    xT = torch.empty_like(x0)
+    ckpt = torch.empty(sched.T // every + 1, B, Cc, H, W, dtype=torch.float32, device=x0.device)
+    ws = GF._WS.get(x0.device, lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, sched.T))
+    cs = sched.c_struct()
+    if resident:
+        rc = lib.gnca_rollout_fwd_bptt_ckpt(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(x0),
+                                            GF._ptr(xT), every, GF._ptr(ckpt), GF._ptr(ws), ws.numel(), GF._stream())
+        if rc == _lib.GNCA_ERR_UNSUPPORTED:
+            return None
+        _lib.check(rc, "gnca_rollout_fwd_bptt_ckpt")
+    else:
+        _lib.check(lib.gnca_rollout_record(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(x0),
+                                           GF._ptr(xT), every, GF._ptr(ckpt), None, GF._ptr(ws), ws.numel(),
+                                           IMPL["streaming"], GF._stream()), "gnca_rollout_record")
+    return xT, ckpt
+
+
+def _ckpt_bwd_raw(desc, packed, ckpt: torch.Tensor, sched: Schedule, every: int, resident: bool, gT: torch.Tensor,
+                  gflat=None):
+    """Backward of _ckpt_fwd_raw: (dL/dx_0, flat parameter gradient), `gflat` accumulated into when given."""
+    _, B, Cc, H, W = ckpt.shape
+    lib = _lib.load()
+    gT = GF._require_cuda_f32(gT, "grad_output")
+    g0 = torch.empty_like(ckpt[0])
+    if gflat is None:
+        gflat = torch.zeros(GF.param_layout(desc).total, dtype=torch.float32, device=ckpt.device)
+    nseg = (lib.gnca_bptt_ckpt_bytes if resident else lib.gnca_ckpt_segment_bytes)(C.byref(desc), B, H, W, every)
+    segment = torch.empty(nseg, dtype=torch.uint8, device=ckpt.device)
+    ws = GF._WS.get(ckpt.device, lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, sched.T))
+    cs = sched.c_struct()
+    if resident:
+        _lib.check(lib.gnca_rollout_bwd_bptt_ckpt(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(ckpt),
+                                                  every, GF._ptr(gT), GF._ptr(g0), GF._ptr(gflat), GF._ptr(segment),
+                                                  segment.numel(), GF._ptr(ws), ws.numel(), GF._stream()),
+                   "gnca_rollout_bwd_bptt_ckpt")
+    else:
+        _lib.check(lib.gnca_rollout_bwd_ckpt(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(ckpt), every,
+                                             None, GF._ptr(gT), GF._ptr(g0), GF._ptr(gflat), GF._ptr(segment),
+                                             segment.numel(), GF._ptr(ws), ws.numel(), GF._stream()),
+                   "gnca_rollout_bwd_ckpt")
+    return g0, gflat
+
+
+def _budget_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, impl: int, budget: int, keep_u: bool):
+    """The forward of the path bptt_plan picks: (x_T, History, plan)."""
+    B, Cc, H, W = x0.shape
+    resident_ok = True
+    while True:
+        plan = _bptt_plan(desc, B, H, W, sched.T, budget, impl, sched.k, resident_ok)
+        path, every, _ = plan
+        if path == "records":
+            out = _records_fwd_raw(desc, packed, x0, sched, 0, keep_x=False)
+            if out is not None:
+                return out[0], out[1], plan
+        elif path == "dense":
+            # never the record attempt of rollout_fwd_raw: the plan chose the dense history because the records do not
+            # fit or have no backward for this launch, and their buffer alone could exceed the budget
+            xT, hist = _dense_fwd_raw(desc, packed, x0, sched, True, impl, keep_u, 0)
+            return xT, hist, plan
+        else:
+            resident = path == "resident_ckpt"
+            out = _ckpt_fwd_raw(desc, packed, x0, sched, every, resident)
+            if out is not None:
+                xT, ckpt = out
+                return xT, History(None, shape=(sched.T + 1, B, Cc, H, W), ckpt=ckpt, every=every,
+                                   resident=resident), plan
+        if impl == IMPL["resident"]:
+            raise ValueError("rollout: impl='resident' with bptt_budget, but the resident backward has no launch "
+                             f"configuration for this batch (B={B}, {H}x{W}, k={sched.k})")
+        resident_ok = False              # the resident backward does not take this launch: plan without it
+
+
+def _records_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, every: int, keep_x: bool):
+    """Resident BPTT forward with records: (x_T, History), or None when the configuration has no record path."""
+    B, Cc, H, W = x0.shape
+    lib = _lib.load()
+    T = sched.T
+    nb = _record_bytes(lib, desc, B, H, W, T)
+    if nb == 0:
+        return None
+    xT = torch.empty_like(x0)
+    ws = GF._WS.get(x0.device, lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, T))
+    cs = sched.c_struct()
+    bptt = torch.empty(nb, dtype=torch.uint8, device=x0.device)
+    if every > 0:
+        hist = None
+        frames = torch.empty(T // every + 1, B, Cc, H, W, dtype=torch.float32, device=x0.device)
+        rc = lib.gnca_rollout_fwd_bptt_record(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(x0),
+                                              GF._ptr(xT), every, GF._ptr(frames), GF._ptr(bptt), nb,
+                                              GF._ptr(ws), ws.numel(), GF._stream())
+    else:
+        frames = None
+        hist = torch.empty(T + 1, B, Cc, H, W, dtype=torch.float32, device=x0.device) if keep_x else None
+        rc = lib.gnca_rollout_fwd_bptt(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(x0),
+                                       GF._ptr(xT), GF._ptr(hist), GF._ptr(bptt), nb, GF._ptr(ws), ws.numel(),
+                                       GF._stream())
+    if rc == _lib.GNCA_ERR_UNSUPPORTED:
+        return None
+    _lib.check(rc, "gnca_rollout_fwd_bptt_record" if every > 0 else "gnca_rollout_fwd_bptt")
+    return xT, History(hist, bptt=bptt, shape=(T + 1, B, Cc, H, W), frames=frames)
+
+
 def rollout_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, *, history: bool, impl: int = 0,
-                    keep_u: bool = True, keep_x: bool = True, every: int = 0):
+                    keep_u: bool = True, keep_x: bool = True, every: int = 0, bptt_budget: Optional[int] = None):
     """gnca_rollout_fwd without autograd: returns (x_T, History or None).  `keep_x=False`: the caller only needs the
     history for the backward (the resident BPTT path then skips storing x_t).  `every > 0` (with `history`): the
     History also carries the frames x_{f*every} of `record_rollout` -- on the record path the forward writes them in
-    place of the x_t history (gnca_rollout_fwd_bptt_record), on the dense path they are copied out of it."""
+    place of the x_t history (gnca_rollout_fwd_bptt_record), on the dense path they are copied out of it.
+    `bptt_budget` (with `history`, without `every` or `keep_x`): the history takes at most that many bytes, on the
+    path bptt_plan picks (History.plan); None is exactly the call without it."""
     x0 = GF._require_cuda_f32(x0, "x0")
     B, Cc, H, W = x0.shape
     if Cc != desc.C:
         raise ValueError(f"x0 has {Cc} channels, model has {desc.C}")
+    if bptt_budget is not None and history:
+        if every > 0:
+            raise ValueError("rollout_fwd_raw: bptt_budget keeps no frames; it cannot be combined with every")
+        xT, hist, plan = _budget_fwd_raw(desc, packed, x0, sched, impl, int(bptt_budget), keep_u)
+        hist.plan = plan
+        return xT, hist
+    if history and impl in (0, 2) and sched.T > 0:
+        out = _records_fwd_raw(desc, packed, x0, sched, every, keep_x)
+        if out is not None:
+            return out
+    return _dense_fwd_raw(desc, packed, x0, sched, history, impl, keep_u, every)
+
+
+def _dense_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, history: bool, impl: int, keep_u: bool,
+                   every: int):
+    """gnca_rollout_fwd with the dense x_t / u_t history (or none): the path of rollout_fwd_raw without records."""
+    B, Cc, H, W = x0.shape
     lib = _lib.load()
     T = sched.T
     xT = torch.empty_like(x0)
     nbytes = lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, T)
     ws = GF._WS.get(x0.device, nbytes)
     cs = sched.c_struct()
-    if history and impl in (0, 2) and T > 0:
-        nb = lib.gnca_bptt_bytes(C.byref(desc), B, H, W, T)
-        if 0 < nb <= BPTT_MAX_BYTES:
-            # the record buffer is GBs (T*B*H*W*1.4 KB worst case): sized for T rounded up to 64 steps, so that rollouts of
-            # slightly different lengths (per-iteration step counts of the trainer) ask the caching allocator for the SAME
-            # block instead of a fresh cudaMalloc whenever a new maximum shows up (70 ms for 29 GB in the long regime)
-            nb_q = lib.gnca_bptt_bytes(C.byref(desc), B, H, W, _round_up_steps(T))
-            if nb <= nb_q <= BPTT_MAX_BYTES and nb_q - nb <= _QUANT_SLACK_BYTES:
-                nb = nb_q
-            bptt = torch.empty(nb, dtype=torch.uint8, device=x0.device)
-            if every > 0:
-                hist = None
-                frames = torch.empty(T // every + 1, B, Cc, H, W, dtype=torch.float32, device=x0.device)
-                rc = lib.gnca_rollout_fwd_bptt_record(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(x0),
-                                                      GF._ptr(xT), every, GF._ptr(frames), GF._ptr(bptt), nb,
-                                                      GF._ptr(ws), ws.numel(), GF._stream())
-            else:
-                frames = None
-                hist = torch.empty(T + 1, B, Cc, H, W, dtype=torch.float32, device=x0.device) if keep_x else None
-                rc = lib.gnca_rollout_fwd_bptt(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(x0),
-                                               GF._ptr(xT), GF._ptr(hist), GF._ptr(bptt), nb, GF._ptr(ws), ws.numel(),
-                                               GF._stream())
-            if rc != _lib.GNCA_ERR_UNSUPPORTED:
-                _lib.check(rc, "gnca_rollout_fwd_bptt_record" if every > 0 else "gnca_rollout_fwd_bptt")
-                return xT, History(hist, bptt=bptt, shape=(T + 1, B, Cc, H, W), frames=frames)
     hist = uh = sh = None
     if history:
-        Tq = _round_up_steps(T)              # same quantised allocation for the dense history (prefix views)
-        if (Tq - T) * B * Cc * H * W * 4 > _QUANT_SLACK_BYTES:
-            Tq = T
+        Tq = _dense_steps(T, B * Cc * H * W)   # same quantised allocation for the dense history (prefix views)
         hist = torch.empty(Tq + 1, B, Cc, H, W, dtype=torch.float32, device=x0.device)[:T + 1]
         if keep_u and T > 0:
             uh = torch.empty(Tq, B, Cc, H, W, dtype=torch.float32, device=x0.device)[:T]
@@ -274,6 +472,10 @@ def rollout_bwd_raw(desc, packed, hist, sched: Schedule, gT: torch.Tensor, *, gf
     frames of the forward, added at their steps (gnca_rollout_bwd_frames / gnca_rollout_bwd_bptt_frames)."""
     if not isinstance(hist, History):
         hist = History(hist)
+    if hist.ckpt is not None:
+        if g_frames is not None:
+            raise ValueError("rollout_bwd_raw: a checkpointed history (bptt_budget) takes no frame gradients")
+        return _ckpt_bwd_raw(desc, packed, hist.ckpt, sched, hist.every, hist.resident, gT, gflat)
     _, B, Cc, H, W = hist.shape
     gT = GF._require_cuda_f32(gT, "grad_output")
     lib = _lib.load()
@@ -382,6 +584,39 @@ class _CkptFn(torch.autograd.Function):
         return (g0, None, *grads)
 
 
+class _BudgetFn(torch.autograd.Function):
+    """rollout(..., bptt_budget=...): the forward keeps the history bptt_plan picks, the backward consumes it once.
+    Checkpoints are kept with save_for_backward, so an in-place edit of them makes the backward raise."""
+
+    @staticmethod
+    def forward(ctx, x0, cfg, *params):
+        xT, hist = rollout_fwd_raw(cfg["desc"], cfg["packed"], x0, cfg["schedule"], history=True, impl=cfg["impl"],
+                                   keep_x=False, bptt_budget=cfg["budget"])
+        ctx.cfg = cfg
+        ctx.param_shapes = [p.shape for p in params]
+        cfg["plan"] = hist.plan
+        ctx.has_ckpt = hist.ckpt is not None
+        if ctx.has_ckpt:
+            ctx.save_for_backward(hist.ckpt)
+            hist.ckpt = None
+        ctx.hist = hist
+        return xT
+
+    @staticmethod
+    def backward(ctx, gT):
+        cfg = ctx.cfg
+        if ctx.hist is None:
+            raise RuntimeError("rollout: the BPTT history was already consumed by an earlier backward")
+        hist = ctx.hist
+        if ctx.has_ckpt:
+            (hist.ckpt,) = ctx.saved_tensors
+        g0, gflat = rollout_bwd_raw(cfg["desc"], cfg["packed"], hist, cfg["schedule"], gT, impl=cfg["impl"])
+        ctx.hist = None
+        offs = GF.segment_offsets(cfg["desc"])
+        grads = [gflat[offs[i]:offs[i + 1]].view(ctx.param_shapes[i]) for i in range(len(ctx.param_shapes))]
+        return (g0, None, *grads)
+
+
 def _check_checkpoint_impl(impl: str, what: str) -> None:
     if impl in ("resident", "banded"):
         raise ValueError(f"{what}: checkpoints are recomputed with the streaming kernels, so impl={impl!r} cannot "
@@ -392,14 +627,28 @@ IMPL = {"auto": 0, "streaming": 1, "resident": 2, "banded": 3}
 
 
 def rollout(model, x0: torch.Tensor, schedule: Schedule, *, checkpoint_every: Optional[int] = None,
-            return_history: bool = False, impl: str = "auto"):
+            return_history: bool = False, impl: str = "auto", bptt_budget: Optional[int] = None):
     """x_T (and optionally the [T+1,B,C,H,W] history) of T steps from x0 under `schedule`.  Differentiable
     w.r.t. x0 and the model parameters (BPTT stores x_t only and recomputes the rest).
 
     `checkpoint_every=K` (with grad): the forward keeps only x_{jK} and the backward recomputes each K-step segment
     from its checkpoint on the streaming kernels, so BPTT memory is T/K + 1 states plus one segment instead of the
     2T + 1 states of the dense history.  The gradients equal those of the dense streaming BPTT.  Without grad it
-    changes nothing."""
+    changes nothing.
+
+    `bptt_budget=N` (bytes, with grad): the BPTT history takes at most N bytes; `bptt_plan` picks the path.  The
+    history `rollout()` keeps without a budget is kept unchanged when it fits (bit-identical results); else the
+    resident BPTT recomputes segments from checkpoints x_{jK} (same dL/dx_0 as the unsegmented resident BPTT), else
+    the streaming kernels do (`checkpoint_every`), each with the largest K that fits.  ValueError when nothing fits.
+    `impl="resident"` / `"streaming"` restrict the choice to that backward."""
+    if bptt_budget is not None:
+        if int(bptt_budget) < 0:
+            raise ValueError(f"rollout: bptt_budget must be >= 0 bytes, got {bptt_budget}")
+        if checkpoint_every is not None or return_history:
+            raise ValueError("rollout: bptt_budget chooses the history itself; it cannot be combined with "
+                             "checkpoint_every or return_history")
+        if impl not in ("auto", "resident", "streaming"):
+            raise ValueError(f"rollout: bptt_budget needs impl 'auto', 'resident' or 'streaming', got {impl!r}")
     if checkpoint_every is not None:
         if int(checkpoint_every) < 1:
             raise ValueError(f"rollout: checkpoint_every must be >= 1, got {checkpoint_every}")
@@ -416,6 +665,13 @@ def rollout(model, x0: torch.Tensor, schedule: Schedule, *, checkpoint_every: Op
         cfg = {"desc": model.model_desc(), "packed": model.packed_weights(), "schedule": schedule,
                "every": int(checkpoint_every)}
         return _CkptFn.apply(x0, cfg, *ps)[1]
+    if bptt_budget is not None:
+        desc = model.model_desc()
+        B, _, H, W = x0.shape
+        _bptt_plan(desc, B, H, W, schedule.T, int(bptt_budget), IMPL[impl], schedule.k)   # errors before any launch
+        cfg = {"desc": desc, "packed": model.packed_weights(), "schedule": schedule, "impl": IMPL[impl],
+               "budget": int(bptt_budget)}
+        return _BudgetFn.apply(x0, cfg, *ps)
     cfg = {"desc": model.model_desc(), "packed": model.packed_weights(), "schedule": schedule, "need_grad": need_grad,
            "history": bool(return_history), "impl": IMPL[impl]}
     return _RolloutFn.apply(x0, cfg, *ps)

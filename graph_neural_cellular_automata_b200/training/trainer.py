@@ -55,6 +55,9 @@ class TrainConfig:
     # pool_size / world slots and draws its share of the batch from them (SURVEY 8e: no state traffic at all; the batch is
     # then stratified over the ranks -- same marginal law per slot, not the reference's joint law)
     pool_sharding: str = "replicated"
+    # bytes the BPTT history of one iteration may take (rollout.bptt_plan picks the path and checkpoint stride);
+    # None keeps the history rollout() keeps without a budget
+    bptt_budget_bytes: Optional[int] = None
 
     @staticmethod
     def from_reference_config(cfg: dict) -> "TrainConfig":
@@ -71,7 +74,8 @@ class TrainConfig:
             random_reseed_prob=float(t.get("random_reseed_prob", 0.05)),
             message_gain=float(g.get("message_gain", 0.5)), message_rate=float(g.get("message_rate", 1.0)),
             message_every=int(g.get("message_every", 1)), scheduler_step_size=int(sch.get("step_size", 50)),
-            scheduler_gamma=float(sch.get("gamma", 0.7)), damage=dict(cfg.get("damage", {})))
+            scheduler_gamma=float(sch.get("gamma", 0.7)), damage=dict(cfg.get("damage", {})),
+            bptt_budget_bytes=None if t.get("bptt_budget_bytes") is None else int(t["bptt_budget_bytes"]))
 
 
 def scheduled_message_gain(epoch: int, base: float) -> float:
@@ -199,7 +203,8 @@ class GraphNCATrainer:
             x0 = sh.take(state).contiguous()
         desc, packed = self.model.model_desc(), self.model.packed_weights()
         impl = {"auto": 0, "streaming": 1, "resident": 2, "banded": 3}[cfg.rollout_impl]
-        xT, hist = rollout_fwd_raw(desc, packed, x0, sched, history=True, impl=impl, keep_x=False)
+        xT, hist = rollout_fwd_raw(desc, packed, x0, sched, history=True, impl=impl, keep_x=False,
+                                   bptt_budget=cfg.bptt_budget_bytes)
         per_local, gxT = premult_loss(xT, self.target, 1.0 / Bg)             # loss = mean over the GLOBAL batch
         _, gflat = rollout_bwd_raw(desc, packed, hist, sched, gxT, impl=impl)
         sh.allreduce_sum_(gflat)                                             # the one data-path collective

@@ -302,6 +302,41 @@ int gnca_rollout_bwd_bptt_frames(const gnca_model* m, const float* packed_dev, i
                                  void* workspace_dev, size_t workspace_bytes, void* stream);
 
 /*
+ * Checkpointed resident BPTT: the resident backward with memory that does not grow with T.  The forward keeps only the
+ * states x_{j*every}; the backward recomputes the records of one `every`-step segment at a time, last segment first,
+ * with the resident forward kernel, and runs the resident backward over them.  Eligible configurations are those of
+ * gnca_bptt_bytes (0 = not supported), and the launch must have a resident backward for the batch and shape.
+ *
+ * gnca_bptt_ckpt_bytes: bytes of the segment buffer: the records, bitmaps and statistics of `every` steps
+ * (gnca_bptt_bytes(m, B, H, W, every)), then one [B][C][H][W] gradient carried across segment boundaries and one
+ * [B][C][H][W] x_T scratch of the recompute, each 256-byte aligned.  0 on bad arguments or an ineligible configuration.
+ *
+ * gnca_rollout_fwd_bptt_ckpt: the T steps on the resident forward kernel, without records; ckpt_dev
+ * ([T/every+1][B][C][H][W], the frames of gnca_rollout_record) receives x_{j*every}, after the schedule's damage when
+ * j*every == damage_step; xT_dev receives x_T.  It uses the kernel and launch configuration of the recompute (they depend
+ * on B and H*W only), so the backward reproduces every step bit for bit.  GNCA_ERR_UNSUPPORTED where the resident
+ * backward does not exist for the model, batch or shape.
+ *
+ * gnca_rollout_bwd_bptt_ckpt: from the checkpoints of gnca_rollout_fwd_bptt_ckpt (same schedule and `every`) and
+ * gT = dL/dx_T, produce g0 = dL/dx_0 and ACCUMULATE gparams.  Segment j covers steps [j*every, min((j+1)*every, T)); its
+ * forward restarts from ckpt[j] at that absolute step (fire rates, gains, offsets, fire_u, the Philox counter and
+ * steps[b] keep their absolute indices), without re-applying a damage at the checkpoint; the backward still multiplies
+ * dL/dx by the mask at damage_step.  g0 equals the unsegmented gnca_rollout_bwd_bptt bit for bit; gparams match it up to
+ * the summation order.  There are no frame gradients on this path.  segment_dev: gnca_bptt_ckpt_bytes(every) bytes;
+ * workspace: gnca_rollout_workspace_bytes.  Argument errors return before any launch: a NULL required pointer,
+ * every <= 0 or T < 0 is GNCA_ERR_ARG; a segment or workspace too small is GNCA_ERR_WORKSPACE; k outside
+ * [0, GNCA_MAX_K] is GNCA_ERR_UNSUPPORTED.
+ */
+size_t gnca_bptt_ckpt_bytes(const gnca_model* m, int B, int H, int W, int every);
+int gnca_rollout_fwd_bptt_ckpt(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                               const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every, float* ckpt_dev,
+                               void* workspace_dev, size_t workspace_bytes, void* stream);
+int gnca_rollout_bwd_bptt_ckpt(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                               const gnca_schedule* sched, const float* ckpt_dev, int every, const float* gT_dev,
+                               float* g0_dev, float* gparams_dev, void* segment_dev, size_t segment_bytes,
+                               void* workspace_dev, size_t workspace_bytes, void* stream);
+
+/*
  * HOST function (no device work): T consecutive `random.sample(range(n), k)` draws of CPython's `random` module on
  * its own MT19937 state (`mt[624]`, `*mti` = random.getstate()[1][:624], [624]); state advanced in place so the caller
  * can `random.setstate` it back -- the python RNG stream stays exactly what T reference `forward` calls consume
