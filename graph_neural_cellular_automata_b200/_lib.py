@@ -103,6 +103,14 @@ EXPORTS = {
                                                C.POINTER(GncaSchedule), C.c_void_p, C.c_size_t, C.c_int, C.c_void_p,
                                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
                                                C.c_void_p]),
+    "gnca_bptt_zp_bytes": (C.c_size_t, [C.POINTER(GncaModel), C.c_int, C.c_int, C.c_int, C.c_int]),
+    "gnca_rollout_fwd_bptt_zp": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                           C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                           C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "gnca_rollout_bwd_bptt_zp": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                           C.POINTER(GncaSchedule), C.c_void_p, C.c_size_t, C.c_int, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                           C.c_void_p]),
     "gnca_bptt_ckpt_bytes": (C.c_size_t, [C.POINTER(GncaModel), C.c_int, C.c_int, C.c_int, C.c_int]),
     "gnca_rollout_fwd_bptt_ckpt": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
                                              C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,

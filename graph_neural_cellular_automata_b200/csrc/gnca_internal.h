@@ -71,19 +71,29 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
 // t0: absolute step of the launch's first step, for a `sched` rebased to the launch (a checkpoint segment); only
 // sched.steps stays absolute.  The launch configuration depends on B and H*W only, so a segment launch reproduces the
 // steps of a whole-rollout launch bit for bit.
+// zp (zero-padded graph shift only): with records, also the attention weights and row sums of every message step
+struct ZpRec;
+struct ZpBwd;
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                 float* u_hist, float* rec, uint32_t* masks, float* scratch, cudaStream_t st, int hist_every = 1,
-                int t0 = 0);
+                int t0 = 0, const ZpRec* zp = nullptr);
 // resident BPTT on the records of run_rep_fwd (gnca_rep_bwd.cu).  g_frames (optional, [F][B][C][H][W]): dL/dx_{f*every}
 // added at step f * every (gnca_rollout_bwd_bptt_frames)
 size_t rep_bptt_bytes(const gnca_model& m, int B, int H, int W, int T);     // 0: configuration not supported
 void rep_bptt_carve(void* base, int B, int H, int W, int T, float** rec, uint32_t** masks, float** stats,
                     float** hgh = nullptr);
 size_t rep_bwd_workspace_bytes(const gnca_model& m, int B, int H, int W);
-bool rep_bwd_supported(const gnca_model& m, int B, int H, int W, int k);    // a launch configuration of k_rep_bwd exists
+// a launch configuration of k_rep_bwd exists (zp: of the zero-padded-shift instantiation)
+bool rep_bwd_supported(const gnca_model& m, int B, int H, int W, int k, bool zp = false);
+// zp: the zero-padded graph shift's buffers (records of run_rep_fwd with a ZpRec); its Q/K/scaling gradients are
+// reduced into gparams after the sweep
 int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, void* bptt, const float* gT, float* g0, float* gparams, void* workspace,
-                cudaStream_t st, const float* g_frames = nullptr, int every = 1, int t0 = 0);
+                cudaStream_t st, const float* g_frames = nullptr, int every = 1, int t0 = 0, const ZpBwd* zp = nullptr);
+// zero-padded graph shift: the records of rep_bptt_bytes followed by x_t, the softmax weights, the row sums, bm . gm of
+// the active cells and the per-sample Q/K gradients (0: not supported)
+size_t rep_bptt_zp_bytes(const gnca_model& m, int B, int H, int W, int T);
+void rep_bptt_zp_carve(void* base, const gnca_model& m, int B, int H, int W, int T, float** x, ZpRec* rec, ZpBwd* bwd);
 
 }  // namespace gnca

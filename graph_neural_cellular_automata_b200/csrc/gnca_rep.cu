@@ -106,8 +106,9 @@ __device__ __forceinline__ uint32_t pack_nibbles(uint32_t nib, int lane) {
 // _shift2d_pad slices the x padding away again, so dx is a no-op -- and per-sample softmax weights over the k offsets
 // (graph_augmentation.py:114,136-154), recomputed from the resident state at the top of every step.  A separate
 // instantiation: the torus kernel (trainer, bench) is compiled exactly as before.
+// Z (ZP with records only, else unused): the softmax weights and row sums of every message step, for k_rep_bwd.
 template <int C, bool ZP>
-__global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const float* __restrict__ packed) {
+__global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const float* __restrict__ packed, ZpRec Z) {
   static_assert(C == 16, "lane mapping: 2 cells x 16 channels per warp row");
   constexpr int C3 = 3 * C, HID = 128;
   constexpr int CPL = 32 / C;                    // cells per lane row (2)
@@ -473,6 +474,11 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
           if (lane < 16) s_w[lane] = lane < k ? e / se : 0.f;
         }
         __syncthreads();
+        if (Z.w && rank == 0) {                                  // what the attention backward of this step reads
+          if (tid < 16) Z.w[((size_t)t * a.B + b) * 16 + tid] = s_w[tid];
+          float* zr = Z.rowsum + ((size_t)t * a.B + b) * C * H;
+          for (int i = tid; i < C * H; i += kPT) zr[i] = s_rowsum[i / H][i - (i / H) * H];
+        }
       }
     }
     REP_MARK(0);
@@ -927,14 +933,15 @@ static size_t rep_smem_bytes(int C, int HW, int ucap, int listcap) {
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                 float* u_hist, float* rec, uint32_t* masks, float* scratch /* >= B*C*H*W floats */, cudaStream_t st,
-                int hist_every, int t0) {
+                int hist_every, int t0, const ZpRec* zpr) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (m.C != 16 || m.hidden != 128) return GNCA_ERR_UNSUPPORTED;
   if (H > kMaxRows || W > kMaxRows || H < 1 || W < 4 || (W & 3)) return GNCA_ERR_UNSUPPORTED;   // quads of 4 cells per row
   if (H * W > 4 * kPT) return GNCA_ERR_UNSUPPORTED;                                            // one quad per thread
   const int k = graph ? sched.k : 0;
-  const bool zp = graph && k > 0 && !(m.flags & GNCA_F_TORUS);      // zero-padded shift: the ZP instantiation (forward only)
-  if (zp && (m.d_model > 32 || rec || masks)) return GNCA_ERR_UNSUPPORTED;      // BPTT records: torus only
+  const bool zp = graph && k > 0 && !(m.flags & GNCA_F_TORUS);      // zero-padded shift: the ZP instantiation
+  if (zp && m.d_model > 32) return GNCA_ERR_UNSUPPORTED;
+  if (zp && (rec || masks) && !zpr) return GNCA_ERR_UNSUPPORTED;     // its records are useless without w and the row sums
   if (k > 16) return GNCA_ERR_UNSUPPORTED;
   if (sched.fire_u && ((uintptr_t)sched.fire_u & 15)) return GNCA_ERR_UNSUPPORTED;    // float4 loads of the uniforms
   if (k > 0 && (sched.max_offset <= 0 || sched.max_offset >= H || sched.max_offset >= W)) return GNCA_ERR_UNSUPPORTED;
@@ -1021,8 +1028,9 @@ int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B
     R.dbg_cta = atoi(getenv("GNCA_PHASE_TIMING"));
   }
   prof_begin(PROF_RESIDENT_FWD, st);
-  cudaError_t e = zp ? cudaLaunchKernelEx(&cfg, k_rep_fwd<16, true>, R, P, packed)
-                     : cudaLaunchKernelEx(&cfg, k_rep_fwd<16, false>, R, P, packed);
+  const ZpRec Z = (zp && zpr && rec) ? *zpr : ZpRec{nullptr, nullptr};
+  cudaError_t e = zp ? cudaLaunchKernelEx(&cfg, k_rep_fwd<16, true>, R, P, packed, Z)
+                     : cudaLaunchKernelEx(&cfg, k_rep_fwd<16, false>, R, P, packed, Z);
   prof_end(PROF_RESIDENT_FWD, st);
   if (e != cudaSuccess) return (int)e;
   GNCA_LAUNCH_CHECK();

@@ -21,4 +21,24 @@ constexpr int kMaskWords = 64;
 // blocks of the batched weight-gradient kernel (two per SM)
 constexpr int kMaxWgradBlocks = 296;
 
+// Zero-padded graph shift (k_rep_fwd<16, true>): what the forward keeps beyond the records for the attention backward.
+// Rank 0 of a sample's cluster writes them on every step with the message on; other steps leave them unwritten.
+struct ZpRec {
+  float* w;                   // [T][B][16] softmax weight of offset i (0 for i >= k)
+  float* rowsum;              // [T][B][C][H] per-(channel, row) sums of x_t
+};
+// ... and what the resident backward (k_rep_bwd<16, kFrames, true>) reads and writes.
+struct ZpBwd {
+  const float* x;             // [T+1][B][C][HW] x_t, the state step t consumes (after the damage)
+  const float* w;             // ZpRec::w
+  const float* rowsum;        // ZpRec::rowsum
+  float* bg;                  // [B][HW] bm . gm of the active cells of the current step, by cell
+  float* pw;                  // [B][2dC + 2d + 1] per-sample wq | bq | wk | bk | scaling gradients (k_attn_bwd layout)
+  int d;                      // d_model
+};
+// floats of the backward's shared-memory tail for the attention backward (behind the plain carve)
+constexpr int kZpSmemFloats = 64 * 16 /*row sums*/ + 16 /*w*/ + 16 * 16 /*warp gw*/ + 8 * 16 /*cluster gw*/ +
+                              4 * 16 /*gL, logits, row range*/ + 16 /*bm*/ + 3 * 16 + 2 * 32 /*xbar, wkq, gxb, qp, gqp*/ +
+                              16 * 16 /*S*/ + 16 * 32 /*KP*/ + 64 /*row sums of gL*/ + 16 /*misc*/;
+
 }  // namespace gnca

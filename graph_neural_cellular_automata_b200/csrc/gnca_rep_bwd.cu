@@ -87,9 +87,15 @@ __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wa
 // kFrames: gframes ([F][B][C][HW]) holds dL/dframe_f of the state step f * every consumes; it is added to g_t at
 // t = f * every (before that step's damage mask, since the frame is the post-damage state) and to g_T when T % every
 // == 0.  The instantiation without it is the one every plain BPTT launches (its parameters go unused).
-template <int C, bool kFrames>
+// ZP: zero-padded graph shift (k_rep_fwd<16, true>, buffers in Z; Z is unused otherwise).  Senders (y - dy_i, x) with
+// the per-sample softmax weights w_i: the message transpose of phase C drops receivers outside the grid and weighs by
+// w_i, and on message steps it also sums dL/dw_i (sender side: A(s) [g_xs(r) . x_t(s) + bm . gm(r)]).  The k partials
+// are reduced over the cluster in a fixed order (third cluster barrier), then every CTA runs the softmax / pooled Q.K
+// backward of k_attn_bwd and adds its row term `grow` to its band of g_t; rank 0 accumulates the Q/K/scaling
+// gradients of the sample in Z.pw.
+template <int C, bool kFrames, bool ZP>
 __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, const float* __restrict__ packed,
-                                                   const float* __restrict__ gframes, int every) {
+                                                   const float* __restrict__ gframes, int every, ZpBwd Z) {
   static_assert(C == 16, "lane mapping: 2 cells x 16 channels per warp row");
   constexpr int C3 = 3 * C, HID = 128, CPL = 32 / C;
   cg::cluster_group cluster = cg::this_cluster();
@@ -122,6 +128,25 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
   float* sGH = sGD + kQW * C * GM;                            // [kQW][GM][HID] gh of the tile (permuted unit order)
   unsigned short* s_list = reinterpret_cast<unsigned short*>(sGH + kQW * GM * HID);  // [bandcap] my SHARE of the active cells
   unsigned short* s_blist = s_list + ((bandcap + 7) & ~7);                          // [bandcap] active cells of my BAND
+  // ZP: attention-backward scratch behind the band lists (kZpSmemFloats)
+  float* const zrs = reinterpret_cast<float*>(s_blist + ((bandcap + 7) & ~7));      // [C][H] row sums of x_t
+  float* const zw = zrs + 64 * 16;                                                  // [16] w_i
+  float* const zgww = zw + 16;                                                      // [kQW][16] dL/dw_i per warp
+  float* const zgwc = zgww + 16 * 16;                                               // [8][16] per CTA (pushed by the peers)
+  float* const zgL = zgwc + 8 * 16;                                                 // [16] dL/dw_i, then dL/dlogit_i
+  float* const zlg = zgL + 16;                                                      // [16] logits
+  int* const zrlo = reinterpret_cast<int*>(zlg + 16);                               // [16] kept rows of offset i
+  int* const zrhi = zrlo + 16;
+  float* const zbm = reinterpret_cast<float*>(zrhi + 16);                           // [C] bm
+  float* const zxbar = zbm + 16;                                                    // [C] mean of x_t
+  float* const zwkq = zxbar + 16;                                                   // [C] Wk^T qp
+  float* const zgxb = zwkq + 16;                                                    // [C] Wq^T gqp
+  float* const zqp = zgxb + 16;                                                     // [32] pooled query
+  float* const zgqp = zqp + 32;                                                     // [32] its gradient
+  float* const zS = zgqp + 32;                                                      // [16][C] row-range sums
+  float* const zKP = zS + 16 * 16;                                                  // [16][32] mean shifted keys
+  float* const zsL = zKP + 16 * 32;                                                 // [64] sum of dL/dlogit_i over offsets keeping row y
+  float* const zmisc = zsL + 64;                                                    // [0] dL/dscaling of the step
 
   __shared__ uint32_t s_bAS[kMaskWords], s_bAct[kMaskWords], s_bPost[kMaskWords];
   __shared__ __align__(16) int s_wtot[kQW];
@@ -149,6 +174,9 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
 #pragma unroll
   for (int cc = 0; cc < C; ++cc) if (tid < C) s_wmT[tid][cc] = graph ? packed[P.wm + cc * C + tid] : 0.f;
   const float gam_c = gn ? packed[P.gamma + c] : 1.f;
+  if constexpr (ZP) {
+    if (tid < C) zbm[tid] = packed[P.bm + tid];
+  }
 
   const size_t sample_off = (size_t)b * C * HW;
   float* GZs = R.GZ + (size_t)b * HW * C;
@@ -219,6 +247,9 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
     }
     if (tid >= 64 && tid < 64 + 2 * k) s_off[tid - 64] = a.offsets_dev[(size_t)t * k * 2 + (tid - 64)];
     if (tid == 96) s_gain = graph ? a.message_gain_dev[t] : 0.f;
+    if constexpr (ZP) {
+      if (tid >= 160 && tid < 176) zw[tid - 160] = Z.w[((size_t)t * a.B + b) * 16 + (tid - 160)];
+    }
     if (tid >= 128 && tid < 128 + C) {
       const int ch = tid - 128;
       float sc = 1.f, bi = 0.f;
@@ -393,6 +424,14 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
           gm = gd * gain_m * (1.f - th * th);
         }
         if (valid[r]) { rc[kRecU + c] = gd; rc[kRecTh + c] = gm; }           // record now holds gd | gm (weight gradients)
+        if constexpr (ZP) {                                                  // bm . gm of the cell (dL/dw_i, phase C)
+          if (msg_on) {
+            float bg = zbm[c] * gm;
+            bg += __shfl_xor_sync(0xffffffffu, bg, 8); bg += __shfl_xor_sync(0xffffffffu, bg, 4);
+            bg += __shfl_xor_sync(0xffffffffu, bg, 2); bg += __shfl_xor_sync(0xffffffffu, bg, 1);
+            if (c == 0 && valid[r]) Z.bg[(size_t)b * HW + cellr[r]] = bg;
+          }
+        }
         float acc = 0.f;                                                     // g_xs[c] = sum_cc Wm[cc][c] gm[cc]
         if (msg_on) {
 #pragma unroll
@@ -540,6 +579,9 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
     cluster_sync_acquire();                                                   // ---- cluster barrier 2: RG visible
     REPB_MARK(7);
     // ---- C: my band: g_t = gated g_{t+1} + perception^T (gy of active neighbours) + message^T (g_xs of receivers) --
+    float gwp[ZP ? 16 : 1];                  // ZP: this thread's share of dL/dw_i
+#pragma unroll
+    for (int i = 0; i < (ZP ? 16 : 1); ++i) gwp[i] = 0.f;
     {
       const float wuni = k > 0 ? 1.0f / (float)k : 0.f;
       auto actbit = [&](int cell) -> bool { return (s_bAct[cell >> 5] >> (cell & 31)) & 1u; };
@@ -580,6 +622,19 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
         int rcell[16];
         const bool sender = msg_on && (!a2a || ((s_bAS[cell >> 5] >> (cell & 31)) & 1u));
         if (sender) {
+          if constexpr (ZP) {
+            // receiver (y + dy_i, x): dx is a no-op, a receiver outside the grid does not exist
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+              rcell[i] = cell;
+              if (i < k) {
+                const int ry = py + (int)s_off[2 * i];
+                const bool inside = ry >= 0 && ry < H;
+                rcell[i] = inside ? ry * W + px : cell;
+                rm |= (inside && actbit(rcell[i])) ? (1u << i) : 0u;
+              }
+            }
+          } else {
 #pragma unroll
           for (int i = 0; i < 16; ++i) {
             rcell[i] = cell;
@@ -590,6 +645,7 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
               rcell[i] = ry * W + rx;
               rm |= actbit(rcell[i]) ? (1u << i) : 0u;
             }
+          }
           }
         }
         g.x += vid.x; g.y += vid.y; g.z += vid.z; g.w += vid.w;
@@ -618,10 +674,26 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
 #pragma unroll
           for (int i = 0; i < 16; ++i)
             vr[i] = (rm >> i) & 1u ? __ldcg(reinterpret_cast<const float4*>(RGs + (size_t)rcell[i] * 64 + 3 * C + 4 * cq)) : z4;
+          if constexpr (ZP) {
+            // x_t of my 4 channels of the sender, and bm . gm of the receivers (counted once, by the quad-0 thread)
+            const float* xs = Z.x + ((size_t)t * a.B + b) * C * HW + (size_t)(4 * cq) * HW + cell;
+            const float x0 = __ldcg(xs), x1 = __ldcg(xs + HW), x2 = __ldcg(xs + 2 * HW), x3 = __ldcg(xs + 3 * HW);
+            float bgr[16];
+#pragma unroll
+            for (int i = 0; i < 16; ++i) bgr[i] = (cq == 0 && ((rm >> i) & 1u)) ? __ldcg(Z.bg + (size_t)b * HW + rcell[i]) : 0.f;
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+              const float wi = zw[i];
+              g.x = fmaf(wi, vr[i].x, g.x); g.y = fmaf(wi, vr[i].y, g.y);
+              g.z = fmaf(wi, vr[i].z, g.z); g.w = fmaf(wi, vr[i].w, g.w);
+              gwp[i] += fmaf(vr[i].x, x0, fmaf(vr[i].y, x1, fmaf(vr[i].z, x2, fmaf(vr[i].w, x3, bgr[i]))));
+            }
+          } else {
 #pragma unroll
           for (int i = 0; i < 16; ++i) {
             g.x = fmaf(wuni, vr[i].x, g.x); g.y = fmaf(wuni, vr[i].y, g.y);
             g.z = fmaf(wuni, vr[i].z, g.z); g.w = fmaf(wuni, vr[i].w, g.w);
+          }
           }
         }
         if constexpr (kFrames) {
@@ -641,6 +713,135 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
     REPB_MARK(8);
     if (R.dbg && tid == 0) s_dbg[9] += n_my;
     (void)nact;
+    if constexpr (ZP) {
+      if (msg_on) {
+        // ---- dL/dw_i: lanes -> warps -> CTA -> every CTA of the cluster, each level in a fixed order ----------------
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {
+          const float v = warp_sum(gwp[i]);
+          if (lane == 0) zgww[warp * 16 + i] = v;
+        }
+        __syncthreads();
+        if (tid < 16) {
+          float v = 0.f;
+          for (int w = 0; w < kQW; ++w) v += zgww[w * 16 + tid];
+          for (int r = 0; r < NC; ++r) cluster.map_shared_rank(zgwc, r)[rank * 16 + tid] = v;
+        }
+        const float* rsg = Z.rowsum + ((size_t)t * a.B + b) * C * H;
+        for (int i = tid; i < C * H; i += kQT) zrs[i] = __ldcg(rsg + i);
+        cluster_sync_acquire();                                               // ---- cluster barrier 3: dL/dw_i partials
+        // ---- softmax / pooled Q.K backward of the step (k_attn_bwd), redundantly on every CTA -----------------------
+        const int d = Z.d;
+        const float invHW = 1.0f / (float)HW;
+        if (tid < k) {
+          float gw = 0.f;
+          for (int r = 0; r < NC; ++r) gw += zgwc[r * 16 + tid];
+          zgL[tid] = gw;
+          const int dy = (int)s_off[2 * tid];
+          const int lo = max(0, -dy), hi = min(H, H - dy);
+          zrlo[tid] = lo; zrhi[tid] = max(lo, hi);
+        }
+        __syncthreads();
+        if (tid < C) {
+          float sacc = 0.f;
+          for (int y = 0; y < H; ++y) sacc += zrs[tid * H + y];
+          zxbar[tid] = sacc * invHW;
+        }
+        for (int idx = tid; idx < k * C; idx += kQT) {
+          const int i = idx / C, cc = idx % C;
+          float sacc = 0.f;
+          for (int y = zrlo[i]; y < zrhi[i]; ++y) sacc += zrs[cc * H + y];
+          zS[idx] = sacc;
+        }
+        __syncthreads();
+        if (tid < d) {
+          float sacc = 0.f;
+          for (int cc = 0; cc < C; ++cc) sacc = fmaf(__ldg(packed + P.wq + tid * C + cc), zxbar[cc], sacc);
+          zqp[tid] = sacc + __ldg(packed + P.bq + tid);
+        }
+        for (int idx = tid; idx < k * d; idx += kQT) {
+          const int i = idx / d, j = idx % d;
+          float sacc = 0.f;
+          for (int cc = 0; cc < C; ++cc) sacc = fmaf(__ldg(packed + P.wk + j * C + cc), zS[i * C + cc], sacc);
+          zKP[i * 32 + j] = (sacc + (float)(zrhi[i] - zrlo[i]) * (float)W * __ldg(packed + P.bk + j)) * invHW;
+        }
+        __syncthreads();
+        if (tid < C) {
+          float sacc = 0.f;
+          for (int j = 0; j < d; ++j) sacc = fmaf(__ldg(packed + P.wk + j * C + tid), zqp[j], sacc);
+          zwkq[tid] = sacc;
+        }
+        if (tid >= 32 && tid < 32 + k) {
+          const int i = tid - 32;
+          float sacc = 0.f;
+          for (int j = 0; j < d; ++j) sacc = fmaf(zqp[j], zKP[i * 32 + j], sacc);
+          zlg[i] = sacc;
+        }
+        __syncthreads();
+        if (tid == 0) {                      // the forward's weights; logits only for dL/dscaling
+          float mx = -INFINITY;
+          for (int i = 0; i < k; ++i) mx = fmaxf(mx, zlg[i]);
+          const float sc = packed[P.scaling];
+          const float tau = fabsf(sc) + 1e-6f;
+          float dot = 0.f;
+          for (int i = 0; i < k; ++i) dot = fmaf(zw[i], zgL[i], dot);
+          float gtau = 0.f;
+          for (int i = 0; i < k; ++i) {
+            const float ga = zw[i] * (zgL[i] - dot);
+            gtau -= ga * ((zlg[i] - mx) / tau) / tau;
+            zgL[i] = ga / tau;               // dL/dlogit_i
+          }
+          zmisc[0] = gtau * (sc >= 0.f ? 1.f : -1.f);
+        }
+        __syncthreads();
+        if (tid < d) {
+          float sacc = 0.f;
+          for (int i = 0; i < k; ++i) sacc = fmaf(zgL[i], zKP[i * 32 + tid], sacc);
+          zgqp[tid] = sacc;
+        }
+        if (tid >= 64 && tid < 64 + H) {
+          const int y = tid - 64;
+          float sacc = 0.f;
+          for (int i = 0; i < k; ++i) if (y >= zrlo[i] && y < zrhi[i]) sacc += zgL[i];
+          zsL[y] = sacc;
+        }
+        __syncthreads();
+        if (tid < C) {
+          float sacc = 0.f;
+          for (int j = 0; j < d; ++j) sacc = fmaf(__ldg(packed + P.wq + j * C + tid), zgqp[j], sacc);
+          zgxb[tid] = sacc;
+        }
+        __syncthreads();
+        // grow = dL/dx_t through the pooled Q / K, for every cell alive or not; part of dL/dx_t, so the damage mask of
+        // step t multiplies it like the rest of g_t (phase C applied it to the rest)
+#pragma unroll 1
+        for (int i = tid; i < nband * C; i += kQT) {
+          const int cl = i / C, ch = i - cl * C;
+          const int cell = band_lo + cl;
+          float v = (zgxb[ch] + zwkq[ch] * zsL[cell / W]) * invHW;
+          if (dmg) v *= R.damage.at(b, ch, cell, C, HW);
+          sG[i] += v;
+        }
+        if (rank == 0) {                     // per-sample Q/K/scaling gradients, summed over the steps
+          float* pwb = Z.pw + (size_t)b * (2 * d * C + 2 * d + 1);
+          for (int idx = tid; idx < d * C; idx += kQT) {
+            const int j = idx / C, ch = idx % C;
+            pwb[idx] += zgqp[j] * zxbar[ch];
+            float sacc = 0.f;
+            for (int i = 0; i < k; ++i) sacc = fmaf(zgL[i], zS[i * C + ch], sacc);
+            pwb[d * C + d + idx] += zqp[j] * sacc * invHW;
+          }
+          for (int j = tid; j < d; j += kQT) {
+            pwb[d * C + j] += zgqp[j];
+            float sacc = 0.f;
+            for (int i = 0; i < k; ++i) sacc += zgL[i] * (float)(zrhi[i] - zrlo[i]);
+            pwb[2 * d * C + d + j] += zqp[j] * sacc * (float)W * invHW;
+          }
+          if (tid == 0) pwb[2 * d * C + 2 * d] += zmisc[0];
+        }
+        __syncthreads();
+      }
+    }
   }
 
   // dL/dx_0 (NCHW) from my band; per-CTA dgamma / dbeta partials
@@ -869,8 +1070,12 @@ size_t rep_bwd_workspace_bytes(const gnca_model& m, int B, int H, int W) {
 // cluster size / tile size / shared memory of k_rep_bwd for a batch: the largest NC in {8,4,2,1} whose bands start at a
 // quad boundary, that fits shared memory (220 KB dynamic + ~4 KB static) and keeps all B clusters co-resident; else the
 // smallest NC that fits (waves).  Returns false when nothing fits.
-static bool pick_rep_bwd_config(int B, int HW, cudaStream_t st, int* out_nc, int* out_gmax, size_t* out_smem) {
+static bool pick_rep_bwd_config(int B, int HW, cudaStream_t st, int* out_nc, int* out_gmax, size_t* out_smem,
+                                bool zp = false) {
   const int C = 16;
+  // the zero-padded-shift instantiation carries the attention-backward scratch behind the plain carve
+  const size_t zsm = zp ? (size_t)kZpSmemFloats * sizeof(float) : 0;
+  const void* kfn = zp ? (const void*)k_rep_bwd<16, false, true> : (const void*)k_rep_bwd<16, false, false>;
   const char* env_nc = getenv("GNCA_RESIDENT_NC");
   const int cands[4] = {8, 4, 2, 1};
   int pick = -1, pick_gmax = 8;
@@ -881,10 +1086,10 @@ static bool pick_rep_bwd_config(int B, int HW, cudaStream_t st, int* out_nc, int
       if (env_nc && atoi(env_nc) != NC) continue;
       if ((HW % (4 * NC)) != 0) continue;                 // bands start at a quad boundary
       int gmax = 8;
-      size_t smem = rep_bwd_smem_bytes(C, HW, NC, gmax);
-      if (smem > 220 * 1024) { gmax = 4; smem = rep_bwd_smem_bytes(C, HW, NC, gmax); }
+      size_t smem = rep_bwd_smem_bytes(C, HW, NC, gmax) + zsm;
+      if (smem > 220 * 1024) { gmax = 4; smem = rep_bwd_smem_bytes(C, HW, NC, gmax) + zsm; }
       if (smem > 220 * 1024) continue;
-      if (cudaFuncSetAttribute(k_rep_bwd<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
+      if (cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
         cudaGetLastError();
         continue;
       }
@@ -895,7 +1100,7 @@ static bool pick_rep_bwd_config(int B, int HW, cudaStream_t st, int* out_nc, int
       qa[0].val.clusterDim.x = NC; qa[0].val.clusterDim.y = 1; qa[0].val.clusterDim.z = 1;
       q.attrs = qa; q.numAttrs = 1;
       int ncl = 0;
-      if (cudaOccupancyMaxActiveClusters(&ncl, k_rep_bwd<16, false>, &q) != cudaSuccess || ncl < 1) {
+      if (cudaOccupancyMaxActiveClusters(&ncl, kfn, &q) != cudaSuccess || ncl < 1) {
         cudaGetLastError();
         continue;
       }
@@ -909,21 +1114,47 @@ static bool pick_rep_bwd_config(int B, int HW, cudaStream_t st, int* out_nc, int
   return true;
 }
 
-bool rep_bwd_supported(const gnca_model& m, int B, int H, int W, int k) {
+bool rep_bwd_supported(const gnca_model& m, int B, int H, int W, int k, bool zp) {
   if (rep_bptt_bytes(m, B, H, W, 1) == 0 || k > 16) return false;
   int nc, gmax;
   size_t smem;
-  return pick_rep_bwd_config(B, H * W, nullptr, &nc, &gmax, &smem);
+  return pick_rep_bwd_config(B, H * W, nullptr, &nc, &gmax, &smem, zp && k > 0);
+}
+
+static inline size_t zp_al(size_t v) { return (v + 255) & ~(size_t)255; }
+
+size_t rep_bptt_zp_bytes(const gnca_model& m, int B, int H, int W, int T) {
+  if (!(m.flags & GNCA_F_GRAPH) || (m.flags & GNCA_F_TORUS) || m.d_model < 1 || m.d_model > 32) return 0;
+  const size_t base = rep_bptt_bytes(m, B, H, W, T);
+  if (base == 0) return 0;
+  const size_t HW = (size_t)H * W, C = m.C, np = 2 * (size_t)m.d_model * C + 2 * (size_t)m.d_model + 1;
+  return zp_al(base) + zp_al((size_t)(T + 1) * B * C * HW * 4) + zp_al((size_t)T * B * 16 * 4) +
+         zp_al((size_t)T * B * C * H * 4) + zp_al((size_t)B * HW * 4) + zp_al((size_t)B * np * 4);
+}
+
+void rep_bptt_zp_carve(void* base, const gnca_model& m, int B, int H, int W, int T, float** x, ZpRec* rec, ZpBwd* bwd) {
+  const size_t HW = (size_t)H * W, C = m.C;
+  char* p = reinterpret_cast<char*>(base);
+  size_t o = zp_al(rep_bptt_bytes(m, B, H, W, T));
+  float* xs = reinterpret_cast<float*>(p + o); o += zp_al((size_t)(T + 1) * B * C * HW * 4);
+  float* w = reinterpret_cast<float*>(p + o); o += zp_al((size_t)T * B * 16 * 4);
+  float* rs = reinterpret_cast<float*>(p + o); o += zp_al((size_t)T * B * C * H * 4);
+  float* bg = reinterpret_cast<float*>(p + o); o += zp_al((size_t)B * HW * 4);
+  float* pw = reinterpret_cast<float*>(p + o);
+  if (x) *x = xs;
+  if (rec) *rec = ZpRec{w, rs};
+  if (bwd) *bwd = ZpBwd{xs, w, rs, bg, pw, m.d_model};
 }
 
 int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, void* bptt, const float* gT, float* g0, float* gparams, void* workspace,
-                cudaStream_t st, const float* g_frames, int every, int t0) {
+                cudaStream_t st, const float* g_frames, int every, int t0, const ZpBwd* zp) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (rep_bptt_bytes(m, B, H, W, sched.T) == 0) return GNCA_ERR_UNSUPPORTED;
   const int k = graph ? sched.k : 0;
-  if (graph && k > 0 && !(m.flags & GNCA_F_TORUS)) return GNCA_ERR_UNSUPPORTED;
+  if (graph && k > 0 && !(m.flags & GNCA_F_TORUS) && !zp) return GNCA_ERR_UNSUPPORTED;
   if (k > 16) return GNCA_ERR_UNSUPPORTED;
+  const bool zpk = zp && graph && k > 0 && !(m.flags & GNCA_F_TORUS);   // the attention backward runs
   const int C = 16, HW = H * W;
   float *rec, *stats, *hgh;
   uint32_t* masks;
@@ -950,13 +1181,17 @@ int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B
 
   int pick = -1, pick_gmax = 8;
   size_t pick_smem = 0;
-  if (!pick_rep_bwd_config(B, HW, st, &pick, &pick_gmax, &pick_smem)) pick = -1;
+  if (!pick_rep_bwd_config(B, HW, st, &pick, &pick_gmax, &pick_smem, zpk)) pick = -1;
   if (pick < 0) return GNCA_ERR_UNSUPPORTED;
   R.NC = pick; R.gmax = pick_gmax;
   if (getenv("GNCA_DEBUG")) fprintf(stderr, "[gnca] resident bwd: B=%d NC=%d smem=%zu\n", B, pick, pick_smem);
   // the frame-gradient instantiation has the register budget and shared memory of the plain one (same launch bounds,
   // same carve), so the configuration picked for the plain kernel holds for it
-  const auto kern = g_frames ? k_rep_bwd<16, true> : k_rep_bwd<16, false>;
+  const auto kern = zpk ? (g_frames ? k_rep_bwd<16, true, true> : k_rep_bwd<16, false, true>)
+                        : (g_frames ? k_rep_bwd<16, true, false> : k_rep_bwd<16, false, false>);
+  const ZpBwd Z = zpk ? *zp : ZpBwd{};
+  const int np = 2 * m.d_model * C + 2 * m.d_model + 1;
+  if (zpk) GNCA_CHECK_CUDA(cudaMemsetAsync(Z.pw, 0, (size_t)B * np * sizeof(float), st));
   GNCA_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pick_smem));
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(B * pick);
@@ -975,7 +1210,7 @@ int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B
     R.dbg_cta = atoi(getenv("GNCA_PHASE_TIMING"));
   }
   prof_begin(PROF_RESIDENT_BWD, st);
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, R, P, packed, g_frames, every);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, R, P, packed, g_frames, every, Z);
   prof_end(PROF_RESIDENT_BWD, st);
   if (e != cudaSuccess) return (int)e;
   GNCA_LAUNCH_CHECK();
@@ -1006,6 +1241,7 @@ int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B
   GNCA_LAUNCH_CHECK();
   k_rep_wreduce<<<(int)((L.total + 255) / 256), 256, 0, st>>>(nblk, L.total, wpart, B * pick, C, affpart, L, gparams);
   GNCA_LAUNCH_CHECK();
+  if (zpk) return run_attn_param_reduce(m, B, AttnBwdScratch{nullptr, nullptr, Z.pw}, gparams, st);
   return 0;
 }
 

@@ -5,6 +5,7 @@
 // BPTT stores only x_t (x_hist); u, the hidden layer, masks and the message are recomputed in the backward.
 #include "gnca_common.cuh"
 #include "gnca_internal.h"
+#include "gnca_rep.h"
 
 namespace gnca {
 
@@ -537,6 +538,91 @@ int gnca_rollout_bwd_bptt(const gnca_model* m, const float* packed_dev, int B, i
                           void* workspace_dev, size_t workspace_bytes, void* stream) {
   return gnca_rollout_bwd_bptt_frames(m, packed_dev, B, H, W, sched, bptt_dev, bptt_bytes, 0, nullptr, gT_dev, g0_dev,
                                       gparams_dev, workspace_dev, workspace_bytes, stream);
+}
+
+/* ---- resident BPTT of the zero-padded graph shift: records plus x_t, softmax weights and row sums ---- */
+size_t gnca_bptt_zp_bytes(const gnca_model* m, int B, int H, int W, int T) {
+  if (!m || B <= 0 || H <= 0 || W <= 0 || T < 0) return 0;
+  if (!model_supported(*m)) return 0;
+  return rep_bptt_zp_bytes(*m, B, H, W, T);
+}
+
+int gnca_rollout_fwd_bptt_zp(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                             const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every, float* frames_dev,
+                             void* bptt_dev, size_t bptt_bytes, void* workspace_dev, size_t workspace_bytes,
+                             void* stream) {
+  if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !bptt_dev || !workspace_dev) return GNCA_ERR_ARG;
+  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
+  if (frames_dev && every <= 0) return GNCA_ERR_ARG;
+  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  if (sched->T > 0 && (!sched->fire_rate || !sched->message_gain)) return GNCA_ERR_ARG;
+  if (sched->k > 0 && !sched->offsets) return GNCA_ERR_ARG;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
+  const size_t need = gnca_bptt_zp_bytes(m, B, H, W, sched->T);
+  if (need == 0) return GNCA_ERR_UNSUPPORTED;
+  if (need > bptt_bytes) return GNCA_ERR_WORKSPACE;
+  RolloutWorkspace r = carve_rollout(workspace_dev, *m, B, H, W);
+  if (r.bytes > workspace_bytes) return GNCA_ERR_WORKSPACE;
+  if (!rep_bwd_supported(*m, B, H, W, sched->k, true)) return GNCA_ERR_UNSUPPORTED;
+  const int T = sched->T;
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t N = (size_t)B * m->C * H * W;
+  float *rec, *stats, *xs;
+  uint32_t* masks;
+  ZpRec zr;
+  rep_bptt_carve(bptt_dev, B, H, W, T, &rec, &masks, &stats);
+  rep_bptt_zp_carve(bptt_dev, *m, B, H, W, T, &xs, &zr, nullptr);
+  if (T == 0) {
+    GNCA_CHECK_CUDA(cudaMemcpyAsync(xT_dev, x0_dev, N * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    if (frames_dev) GNCA_CHECK_CUDA(cudaMemcpyAsync(frames_dev, x0_dev, N * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    return 0;
+  }
+  // x_t of every step is what the backward reads (the dL/dw_i sums); the frames are a copy of every `every`-th state (a
+  // copy, not a view: a caller editing a frame in place cannot corrupt what the backward reads).  The full history
+  // (every = 1) is one contiguous copy; a strided 2D copy is avoided because every * state bytes can exceed the
+  // largest pitch the copy engine takes.
+  const Packed P = make_packed(m->C, m->hidden, m->d_model, true);
+  int rc = run_rep_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, xs, stats, nullptr, rec, masks, r.ping, st, 1,
+                       0, &zr);
+  if (rc || !frames_dev) return rc;
+  if (every == 1) {
+    GNCA_CHECK_CUDA(cudaMemcpyAsync(frames_dev, xs, (size_t)(T + 1) * N * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    return 0;
+  }
+  for (int f = 0; (size_t)f * every <= (size_t)T; ++f)
+    GNCA_CHECK_CUDA(cudaMemcpyAsync(frames_dev + (size_t)f * N, xs + (size_t)f * every * N, N * sizeof(float),
+                                    cudaMemcpyDeviceToDevice, st));
+  return 0;
+}
+
+int gnca_rollout_bwd_bptt_zp(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                             const gnca_schedule* sched, void* bptt_dev, size_t bptt_bytes, int every,
+                             const float* g_frames_dev, const float* gT_dev, float* g0_dev, float* gparams_dev,
+                             void* workspace_dev, size_t workspace_bytes, void* stream) {
+  if (!m || !packed_dev || !sched || !bptt_dev || !gT_dev || !g0_dev || !gparams_dev || !workspace_dev) return GNCA_ERR_ARG;
+  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
+  if (g_frames_dev && every <= 0) return GNCA_ERR_ARG;
+  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  if (sched->T > 0 && !sched->message_gain) return GNCA_ERR_ARG;
+  if (sched->k > 0 && !sched->offsets) return GNCA_ERR_ARG;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
+  const size_t need = gnca_bptt_zp_bytes(m, B, H, W, sched->T);
+  if (need == 0) return GNCA_ERR_UNSUPPORTED;
+  if (need > bptt_bytes) return GNCA_ERR_WORKSPACE;
+  if (rep_bwd_workspace_bytes(*m, B, H, W) > workspace_bytes) return GNCA_ERR_WORKSPACE;
+  if (!rep_bwd_supported(*m, B, H, W, sched->k, true)) return GNCA_ERR_UNSUPPORTED;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (sched->T == 0) {
+    const size_t N = (size_t)B * m->C * H * W;
+    if (g_frames_dev) return fold_last_frame(N, 0, every, g_frames_dev, gT_dev, g0_dev, st);
+    GNCA_CHECK_CUDA(cudaMemcpyAsync(g0_dev, gT_dev, N * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    return 0;
+  }
+  ZpBwd zb;
+  rep_bptt_zp_carve(bptt_dev, *m, B, H, W, sched->T, nullptr, nullptr, &zb);
+  const Packed P = make_packed(m->C, m->hidden, m->d_model, true);
+  return run_rep_bwd(*m, P, packed_dev, B, H, W, *sched, bptt_dev, gT_dev, g0_dev, gparams_dev, workspace_dev, st,
+                     g_frames_dev, every, 0, &zb);
 }
 
 /* ---- checkpointed resident BPTT: x_{j*every} only; each segment's records are recomputed in the backward ---- */

@@ -181,15 +181,18 @@ def make_schedule(model, B: int, H: int, W: int, T: int, *, fire_rate: Union[flo
 class History:
     """What the forward keeps for BPTT.  Two formats:
     * records (`bptt`): the replicated-state kernel's per-active-cell records + bitmaps + statistics -- consumed by the
-      cluster-resident backward (gnca_rollout_bwd_bptt); `x` is only filled when the caller asked for the history;
+      cluster-resident backward (gnca_rollout_bwd_bptt); `x` is only filled when the caller asked for the history.
+      `zp`: the zero-padded graph shift's buffer (gnca_bptt_zp_bytes: the records plus x_t, the attention weights and
+      row sums), consumed by gnca_rollout_bwd_bptt_zp;
     * dense: x_t for every step and (optionally) the masked pre-norm update of the active cells + the GroupNorm
       statistics, consumed by the streaming backward (gnca_rollout_bwd).
     `frames` (forward with `every`): x_{f*every} in a buffer of its own, the differentiable states of `record_rollout`.
     `ckpt` (forward with a BPTT budget that called for checkpoints): x_{j*every} only, recomputed segment by segment on
     the resident (`resident`) or the streaming kernels; `plan` is the bptt_plan result of that forward."""
 
-    def __init__(self, x, u=None, stats=None, bptt=None, shape=None, frames=None, ckpt=None, every=0, resident=False):
-        self.x, self.u, self.stats, self.bptt, self.frames = x, u, stats, bptt, frames
+    def __init__(self, x, u=None, stats=None, bptt=None, shape=None, frames=None, ckpt=None, every=0, resident=False,
+                 zp=False):
+        self.x, self.u, self.stats, self.bptt, self.frames, self.zp = x, u, stats, bptt, frames, zp
         self.ckpt, self.every, self.resident, self.plan = ckpt, every, resident, None
         self._shape = tuple(shape) if shape is not None else tuple(x.shape)
 
@@ -211,18 +214,20 @@ def _round_up_steps(T: int, q: int = 64) -> int:
 BPTT_MAX_BYTES = 48 << 30      # above this the record buffer is not worth it: dense history + streaming backward
 
 
-def _record_bytes(lib, desc, B: int, H: int, W: int, T: int) -> int:
+def _record_bytes(lib, desc, B: int, H: int, W: int, T: int, nbytes=None) -> int:
     """Bytes of the record buffer the resident BPTT forward allocates for T steps, or 0 when `rollout()` takes the dense
-    history instead (configuration without records, T = 0, or more than BPTT_MAX_BYTES)."""
+    history instead (configuration without records, T = 0, or more than BPTT_MAX_BYTES).  `nbytes`: the size function
+    of the buffer (default gnca_bptt_bytes; gnca_bptt_zp_bytes for the zero-padded graph shift)."""
     if T <= 0:
         return 0
-    nb = lib.gnca_bptt_bytes(C.byref(desc), B, H, W, T)
+    nbytes = nbytes or lib.gnca_bptt_bytes
+    nb = nbytes(C.byref(desc), B, H, W, T)
     if not 0 < nb <= BPTT_MAX_BYTES:
         return 0
     # the record buffer is GBs (T*B*H*W*1.4 KB worst case): sized for T rounded up to 64 steps, so that rollouts of
     # slightly different lengths (per-iteration step counts of the trainer) ask the caching allocator for the SAME
     # block instead of a fresh cudaMalloc whenever a new maximum shows up (70 ms for 29 GB in the long regime)
-    nb_q = lib.gnca_bptt_bytes(C.byref(desc), B, H, W, _round_up_steps(T))
+    nb_q = nbytes(C.byref(desc), B, H, W, _round_up_steps(T))
     if nb <= nb_q <= BPTT_MAX_BYTES and nb_q - nb <= _QUANT_SLACK_BYTES:
         nb = nb_q
     return nb
@@ -296,7 +301,11 @@ def bptt_plan(model, B: int, H: int, W: int, T: int, budget: int, impl: str = "a
     `k`: offsets per step of the schedule (default: what `make_schedule` draws for the model, 0 for a classic model);
     more than RESIDENT_MAX_K leaves the resident branches out, as in rollout().  rollout() takes this plan, except when
     the resident backward finds no cluster launch configuration for the batch at run time: it then plans again
-    without the resident branches."""
+    without the resident branches.
+
+    Zero-padded graph shift models: the plan is over the dense history and streaming checkpoints only.  The resident
+    zero-pad BPTT that rollout() takes without a budget (gnca_bptt_zp_bytes) has no checkpointed form, so under a budget
+    these models keep the dense history when it fits."""
     if impl not in ("auto", "resident", "streaming"):
         raise ValueError(f"bptt_plan: impl must be 'auto', 'resident' or 'streaming', got {impl!r}")
     if int(budget) < 0:
@@ -385,17 +394,33 @@ def _budget_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, impl: int, 
 
 
 def _records_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, every: int, keep_x: bool):
-    """Resident BPTT forward with records: (x_T, History), or None when the configuration has no record path."""
+    """Resident BPTT forward with records: (x_T, History), or None when the configuration has no record path.  Zero-padded
+    graph shift models keep the buffer of gnca_bptt_zp_bytes instead (History.zp)."""
     B, Cc, H, W = x0.shape
     lib = _lib.load()
     T = sched.T
     nb = _record_bytes(lib, desc, B, H, W, T)
+    zp = nb == 0 and sched.k <= RESIDENT_MAX_K
+    if zp:
+        nb = _record_bytes(lib, desc, B, H, W, T, lib.gnca_bptt_zp_bytes)
     if nb == 0:
         return None
     xT = torch.empty_like(x0)
     ws = GF._WS.get(x0.device, lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, T))
     cs = sched.c_struct()
     bptt = torch.empty(nb, dtype=torch.uint8, device=x0.device)
+    if zp:
+        # one call for both: the frames (or the full history, every = 1) are copies of the x_t the buffer keeps
+        hist = torch.empty(T + 1, B, Cc, H, W, dtype=torch.float32, device=x0.device) if keep_x and every <= 0 else None
+        frames = torch.empty(T // every + 1, B, Cc, H, W, dtype=torch.float32, device=x0.device) if every > 0 else None
+        out = frames if every > 0 else hist
+        rc = lib.gnca_rollout_fwd_bptt_zp(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(x0),
+                                          GF._ptr(xT), every if every > 0 else 1, GF._ptr(out), GF._ptr(bptt), nb,
+                                          GF._ptr(ws), ws.numel(), GF._stream())
+        if rc == _lib.GNCA_ERR_UNSUPPORTED:
+            return None
+        _lib.check(rc, "gnca_rollout_fwd_bptt_zp")
+        return xT, History(hist, bptt=bptt, shape=(T + 1, B, Cc, H, W), frames=frames, zp=True)
     if every > 0:
         hist = None
         frames = torch.empty(T // every + 1, B, Cc, H, W, dtype=torch.float32, device=x0.device)
@@ -491,6 +516,12 @@ def rollout_bwd_raw(desc, packed, hist, sched: Schedule, gT: torch.Tensor, *, gf
         if tuple(g_frames.shape) != (sched.T // every + 1, B, Cc, H, W):
             raise ValueError(f"frame gradients have shape {tuple(g_frames.shape)}, expected "
                              f"{(sched.T // every + 1, B, Cc, H, W)}")
+    if hist.bptt is not None and hist.zp:
+        _lib.check(lib.gnca_rollout_bwd_bptt_zp(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(hist.bptt),
+                                                hist.bptt.numel(), every, GF._ptr(g_frames), GF._ptr(gT), GF._ptr(g0),
+                                                GF._ptr(gflat), GF._ptr(ws), ws.numel(), GF._stream()),
+                   "gnca_rollout_bwd_bptt_zp")
+        return g0, gflat
     if hist.bptt is not None:
         _lib.check(lib.gnca_rollout_bwd_bptt_frames(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs),
                                                     GF._ptr(hist.bptt), hist.bptt.numel(), every, GF._ptr(g_frames),

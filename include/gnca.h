@@ -302,6 +302,40 @@ int gnca_rollout_bwd_bptt_frames(const gnca_model* m, const float* packed_dev, i
                                  void* workspace_dev, size_t workspace_bytes, void* stream);
 
 /*
+ * Resident BPTT of the zero-padded graph shift (the graph default: GNCA_F_GRAPH without GNCA_F_TORUS), for
+ * 16-channel / 128-hidden models with d_model <= 32, at most 16 offsets per step, grids up to 2048 cells with W % 4 == 0.
+ * gnca_bptt_bytes stays 0 for these models; this path has its own buffer and entry points.
+ *
+ * gnca_bptt_zp_bytes: bytes of `bptt_dev`: the records, bitmaps and statistics of gnca_bptt_bytes, then x_t of every
+ * step ([T+1][B][C][H][W]), the softmax weights and per-(channel, row) sums of x_t of every step with the message on,
+ * one per-cell scratch and the per-sample Q/K/scaling gradients.  0 for a classic or torus model, an unsupported
+ * model or shape, or bad arguments.
+ *
+ * gnca_rollout_fwd_bptt_zp: the T steps on the resident zero-pad forward kernel, keeping that buffer.  frames_dev
+ * (optional, [T/every+1][B][C][H][W]) receives x_{f*every} (every > 0; every = 1 is the full history); xT_dev always
+ * receives x_T, bit-equal to gnca_rollout_fwd.  GNCA_ERR_UNSUPPORTED (before any launch) where the forward or the
+ * backward has no resident kernel for the batch, shape or offsets (a grid no taller or wider than the largest offset).
+ *
+ * gnca_rollout_bwd_bptt_zp: from that buffer (same schedule), gT = dL/dx_T and the optional frame gradients of
+ * gnca_rollout_bwd_bptt_frames, produce g0 = dL/dx_0 and ACCUMULATE gparams, the attention's wq, bq, wk, bk and
+ * scaling included.  One cluster-resident launch propagates dL/dx through the message, the softmax weights and the
+ * pooled query / keys; the weight gradients follow as in gnca_rollout_bwd_bptt.  Workspace: gnca_rollout_workspace_bytes.
+ *
+ * Argument errors return before any launch: a NULL required pointer, B, H or W <= 0, T < 0, or every <= 0 with frames
+ * is GNCA_ERR_ARG; a buffer or workspace too small is GNCA_ERR_WORKSPACE; k outside [0, GNCA_MAX_K] or an unsupported
+ * configuration is GNCA_ERR_UNSUPPORTED.
+ */
+size_t gnca_bptt_zp_bytes(const gnca_model* m, int B, int H, int W, int T);
+int gnca_rollout_fwd_bptt_zp(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                             const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every, float* frames_dev,
+                             void* bptt_dev, size_t bptt_bytes, void* workspace_dev, size_t workspace_bytes,
+                             void* stream);
+int gnca_rollout_bwd_bptt_zp(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                             const gnca_schedule* sched, void* bptt_dev, size_t bptt_bytes, int every,
+                             const float* g_frames_dev, const float* gT_dev, float* g0_dev, float* gparams_dev,
+                             void* workspace_dev, size_t workspace_bytes, void* stream);
+
+/*
  * Checkpointed resident BPTT: the resident backward with memory that does not grow with T.  The forward keeps only the
  * states x_{j*every}; the backward recomputes the records of one `every`-step segment at a time, last segment first,
  * with the resident forward kernel, and runs the resident backward over them.  Eligible configurations are those of
