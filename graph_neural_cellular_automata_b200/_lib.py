@@ -118,6 +118,10 @@ EXPORTS = {
     "gnca_rollout_bwd_bptt_ckpt": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
                                              C.POINTER(GncaSchedule), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "gnca_rollout_bwd_bptt_ckpt_frames": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                    C.POINTER(GncaSchedule), C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                                    C.c_void_p, C.c_size_t, C.c_void_p]),
     "gnca_host_sample_indices": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "gnca_host_sample_offsets_words": (C.c_int, [C.c_char_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                  C.c_void_p, C.POINTER(C.c_int32)]),

@@ -87,10 +87,12 @@ size_t rep_bwd_workspace_bytes(const gnca_model& m, int B, int H, int W);
 // a launch configuration of k_rep_bwd exists (zp: of the zero-padded-shift instantiation)
 bool rep_bwd_supported(const gnca_model& m, int B, int H, int W, int k, bool zp = false);
 // zp: the zero-padded graph shift's buffers (records of run_rep_fwd with a ZpRec); its Q/K/scaling gradients are
-// reduced into gparams after the sweep
+// reduced into gparams after the sweep.  gT_frame = false: g_frames' frame at sched.T is not added to gT (a checkpoint
+// segment, where it is the next segment's first frame)
 int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, void* bptt, const float* gT, float* g0, float* gparams, void* workspace,
-                cudaStream_t st, const float* g_frames = nullptr, int every = 1, int t0 = 0, const ZpBwd* zp = nullptr);
+                cudaStream_t st, const float* g_frames = nullptr, int every = 1, int t0 = 0, const ZpBwd* zp = nullptr,
+                bool gT_frame = true);
 // zero-padded graph shift: the records of rep_bptt_bytes followed by x_t, the softmax weights, the row sums, bm . gm of
 // the active cells and the per-sample Q/K gradients (0: not supported)
 size_t rep_bptt_zp_bytes(const gnca_model& m, int B, int H, int W, int T);

@@ -54,6 +54,10 @@ struct RepBwdArgs {
   float* affpart;             // [B*NC][2C] dgamma | dbeta partials
   DamageView damage;
   int damage_step;
+  // kFrames: add frame T / every to g_T when T % every == 0.  0 in a checkpoint segment, whose frame at T is the next
+  // segment's first, added there already.  It sits in the padding before `dbg`, so the struct keeps its size and every
+  // later kernel parameter its offset: the instantiations without frames compile to the same SASS as without the field
+  int gT_frame;
   unsigned long long* dbg;    // optional phase-cycle counters (GNCA_PHASE_TIMING=<cta>)
   int dbg_cta;
   int t0;                     // absolute step of local step 0 (see RepArgs::t0): only steps[b] is absolute
@@ -85,8 +89,8 @@ __device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bu
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
 // kFrames: gframes ([F][B][C][HW]) holds dL/dframe_f of the state step f * every consumes; it is added to g_t at
-// t = f * every (before that step's damage mask, since the frame is the post-damage state) and to g_T when T % every
-// == 0.  The instantiation without it is the one every plain BPTT launches (its parameters go unused).
+// t = f * every (before that step's damage mask, since the frame is the post-damage state) and, with R.gT_frame, to g_T
+// when T % every == 0.  The instantiation without it is the one every plain BPTT launches (its parameters go unused).
 // ZP: zero-padded graph shift (k_rep_fwd<16, true>, buffers in Z; Z is unused otherwise).  Senders (y - dy_i, x) with
 // the per-sample softmax weights w_i: the message transpose of phase C drops receivers outside the grid and weighs by
 // w_i, and on message steps it also sums dL/dw_i (sender side: A(s) [g_xs(r) . x_t(s) + bm . gm(r)]).  The k partials
@@ -193,7 +197,7 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
       if (cl < nband) {
         float v = R.gT[sample_off + (size_t)ch * HW + band_lo + cl];
         if constexpr (kFrames)
-          if (R.T % every == 0) v += __ldg(gframes + ((size_t)(R.T / every) * a.B * C + (size_t)b * C + ch) * HW + band_lo + cl);
+          if (R.gT_frame && R.T % every == 0) v += __ldg(gframes + ((size_t)(R.T / every) * a.B * C + (size_t)b * C + ch) * HW + band_lo + cl);
         sG[cl * C + ch] = v;
       }
     }
@@ -1148,7 +1152,7 @@ void rep_bptt_zp_carve(void* base, const gnca_model& m, int B, int H, int W, int
 
 int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, void* bptt, const float* gT, float* g0, float* gparams, void* workspace,
-                cudaStream_t st, const float* g_frames, int every, int t0, const ZpBwd* zp) {
+                cudaStream_t st, const float* g_frames, int every, int t0, const ZpBwd* zp, bool gT_frame) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (rep_bptt_bytes(m, B, H, W, sched.T) == 0) return GNCA_ERR_UNSUPPORTED;
   const int k = graph ? sched.k : 0;
@@ -1174,6 +1178,7 @@ int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B
   R.s.steps = sched.steps;
   R.T = sched.T;
   R.t0 = t0;
+  R.gT_frame = gT_frame ? 1 : 0;
   R.inv_n = (float)(1.0 / ((double)C * (double)H * (double)W));
   R.rec = rec; R.hgh = hgh; R.masks = masks; R.stats = stats; R.gT = gT; R.g0 = g0; R.GZ = GZ; R.RG = RG;
   R.affpart = affpart;

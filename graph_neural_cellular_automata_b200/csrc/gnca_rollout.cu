@@ -660,19 +660,21 @@ int gnca_rollout_fwd_bptt_ckpt(const gnca_model* m, const float* packed_dev, int
                      r.ping, st, every, 0);
 }
 
-int gnca_rollout_bwd_bptt_ckpt(const gnca_model* m, const float* packed_dev, int B, int H, int W,
-                               const gnca_schedule* sched, const float* ckpt_dev, int every, const float* gT_dev,
-                               float* g0_dev, float* gparams_dev, void* segment_dev, size_t segment_bytes,
-                               void* workspace_dev, size_t workspace_bytes, void* stream) {
-  if (!m || !packed_dev || !sched || !ckpt_dev || !gT_dev || !g0_dev || !gparams_dev || !segment_dev || !workspace_dev)
+int gnca_rollout_bwd_bptt_ckpt_frames(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                                      const gnca_schedule* sched, const float* frames_dev, int every, int ckpt_every,
+                                      const float* g_frames_dev, const float* gT_dev, float* g0_dev, float* gparams_dev,
+                                      void* segment_dev, size_t segment_bytes, void* workspace_dev,
+                                      size_t workspace_bytes, void* stream) {
+  if (!m || !packed_dev || !sched || !frames_dev || !gT_dev || !g0_dev || !gparams_dev || !segment_dev || !workspace_dev)
     return GNCA_ERR_ARG;
-  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0 || every <= 0) return GNCA_ERR_ARG;
+  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0 || every <= 0 || ckpt_every <= 0) return GNCA_ERR_ARG;
+  if (ckpt_every % every != 0) return GNCA_ERR_ARG;
   if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
   const bool graph = (m->flags & GNCA_F_GRAPH) != 0;
   if (sched->T > 0 && (!sched->fire_rate || (graph && !sched->message_gain))) return GNCA_ERR_ARG;
   if (graph && sched->k > 0 && !sched->offsets) return GNCA_ERR_ARG;
   if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
-  const size_t need = gnca_bptt_ckpt_bytes(m, B, H, W, every);
+  const size_t need = gnca_bptt_ckpt_bytes(m, B, H, W, ckpt_every);
   if (need == 0) return GNCA_ERR_UNSUPPORTED;
   if (need > segment_bytes) return GNCA_ERR_WORKSPACE;
   RolloutWorkspace r = carve_rollout(workspace_dev, *m, B, H, W);
@@ -682,31 +684,54 @@ int gnca_rollout_bwd_bptt_ckpt(const gnca_model* m, const float* packed_dev, int
   const size_t N = (size_t)B * m->C * H * W;
   const int T = sched->T;
   if (T == 0) {
+    if (g_frames_dev) return fold_last_frame(N, 0, every, g_frames_dev, gT_dev, g0_dev, st);
     GNCA_CHECK_CUDA(cudaMemcpyAsync(g0_dev, gT_dev, N * sizeof(float), cudaMemcpyDeviceToDevice, st));
     return 0;
   }
   const Packed P = make_packed(m->C, m->hidden, m->d_model, graph);
-  const RepSegment seg = carve_rep_segment(segment_dev, *m, B, H, W, every);
-  const int nseg = (T - 1) / every + 1;
-  // dL/dx_{j*every} goes to g0 for even j and to the segment's slot for odd j: segment 0 ends in g0, and no launch
+  const RepSegment seg = carve_rep_segment(segment_dev, *m, B, H, W, ckpt_every);
+  const int nseg = (T - 1) / ckpt_every + 1;
+  const size_t per_ckpt = (size_t)(ckpt_every / every);           // frames between consecutive checkpoints
+  // dL/dx_{j*ckpt_every} goes to g0 for even j and to the segment's slot for odd j: segment 0 ends in g0, and no launch
   // reads the buffer it writes
   auto g_at = [&](int j) -> float* { return (j & 1) ? seg.g : g0_dev; };
+  // The last frame, when it is x_T, goes into g_T here, once: each segment's backward leaves it out of its own g_T
+  // (there it would be the next segment's first frame, added already).  g_at(nseg) is the buffer the last segment
+  // does not write.
+  const float* gT = gT_dev;
+  if (g_frames_dev && T % every == 0) {
+    int rc = fold_last_frame(N, T, every, g_frames_dev, gT_dev, g_at(nseg), st);
+    if (rc) return rc;
+    gT = g_at(nseg);
+  }
   for (int j = nseg - 1; j >= 0; --j) {
-    const int t0 = j * every, n = T - t0 < every ? T - t0 : every;
+    const int t0 = j * ckpt_every, n = T - t0 < ckpt_every ? T - t0 : ckpt_every;
     float *rec, *stats;
     uint32_t* masks;
     rep_bptt_carve(seg.bptt, B, H, W, n, &rec, &masks, &stats);
     // the checkpoint is x_t0 after a damage at t0: the recompute applies only a damage step inside the segment
     const gnca_schedule sf = segment_schedule(*sched, t0, n, B, H, W, false);
-    int rc = run_rep_fwd(*m, P, packed_dev, B, H, W, sf, ckpt_dev + (size_t)j * N, seg.xT, nullptr, stats, nullptr, rec,
-                         masks, r.ping, st, 1, t0);
+    int rc = run_rep_fwd(*m, P, packed_dev, B, H, W, sf, frames_dev + (size_t)j * per_ckpt * N, seg.xT, nullptr, stats,
+                         nullptr, rec, masks, r.ping, st, 1, t0);
     if (rc) return rc;
+    // frames t0 / every ... of the segment are added at their local steps t % every == 0 (t0 is a multiple of every)
     const gnca_schedule sb = segment_schedule(*sched, t0, n, B, H, W, true);
-    rc = run_rep_bwd(*m, P, packed_dev, B, H, W, sb, seg.bptt, j == nseg - 1 ? gT_dev : g_at(j + 1), g_at(j),
-                     gparams_dev, workspace_dev, st, nullptr, 1, t0);
+    const float* gfr = g_frames_dev ? g_frames_dev + (size_t)(t0 / every) * N : nullptr;
+    rc = run_rep_bwd(*m, P, packed_dev, B, H, W, sb, seg.bptt, j == nseg - 1 ? gT : g_at(j + 1), g_at(j),
+                     gparams_dev, workspace_dev, st, gfr, every, t0, nullptr, false);
     if (rc) return rc;
   }
   return 0;
+}
+
+int gnca_rollout_bwd_bptt_ckpt(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                               const gnca_schedule* sched, const float* ckpt_dev, int every, const float* gT_dev,
+                               float* g0_dev, float* gparams_dev, void* segment_dev, size_t segment_bytes,
+                               void* workspace_dev, size_t workspace_bytes, void* stream) {
+  // the checkpoints are the frames of stride `every`, each one a checkpoint
+  return gnca_rollout_bwd_bptt_ckpt_frames(m, packed_dev, B, H, W, sched, ckpt_dev, every, every, nullptr, gT_dev,
+                                           g0_dev, gparams_dev, segment_dev, segment_bytes, workspace_dev,
+                                           workspace_bytes, stream);
 }
 
 /* ---- host-side schedule construction: T x random.sample(range(n), k) on CPython's MT19937 state ----

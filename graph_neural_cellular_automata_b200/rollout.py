@@ -187,13 +187,16 @@ class History:
     * dense: x_t for every step and (optionally) the masked pre-norm update of the active cells + the GroupNorm
       statistics, consumed by the streaming backward (gnca_rollout_bwd).
     `frames` (forward with `every`): x_{f*every} in a buffer of its own, the differentiable states of `record_rollout`.
-    `ckpt` (forward with a BPTT budget that called for checkpoints): x_{j*every} only, recomputed segment by segment on
-    the resident (`resident`) or the streaming kernels; `plan` is the bptt_plan result of that forward."""
+    `ckpt` (forward with a BPTT budget that called for checkpoints): x_{f*every} only, recomputed segment by segment on
+    the resident (`resident`) or the streaming kernels from every (ckpt_every / every)-th of them, so segments are
+    `ckpt_every` steps long (default `every`; a multiple of it when the frames of `record_rollout` are the checkpoints);
+    `plan` is the bptt_plan result of that forward."""
 
     def __init__(self, x, u=None, stats=None, bptt=None, shape=None, frames=None, ckpt=None, every=0, resident=False,
-                 zp=False):
+                 zp=False, ckpt_every=None):
         self.x, self.u, self.stats, self.bptt, self.frames, self.zp = x, u, stats, bptt, frames, zp
         self.ckpt, self.every, self.resident, self.plan = ckpt, every, resident, None
+        self.ckpt_every = ckpt_every or every
         self._shape = tuple(shape) if shape is not None else tuple(x.shape)
 
     @property
@@ -249,15 +252,18 @@ def _dense_bytes(B: int, Cc: int, H: int, W: int, T: int) -> int:
 RESIDENT_MAX_K = 16      # offsets per step the resident kernels take (gnca_rep.cu, rep_bwd_supported)
 
 
-def _bptt_plan(desc, B: int, H: int, W: int, T: int, budget: int, impl: int, k: int = 0, resident_ok: bool = True):
+def _bptt_plan(desc, B: int, H: int, W: int, T: int, budget: int, impl: int, k: int = 0, resident_ok: bool = True,
+               every: Optional[int] = None):
     """bptt_plan on a model descriptor, an impl code and the schedule's offsets per step k; `resident_ok=False` leaves
-    the resident branches out (the launch found no resident backward for the batch)."""
+    the resident branches out (the launch found no resident backward for the batch).  `every`: the plan of
+    record_rollout(..., bptt_budget=...) with frames every `every` steps."""
     lib = _lib.load()
     n_bytes = B * desc.C * H * W * 4
+    who = "rollout" if every is None else "record_rollout"
     resident_ok = resident_ok and k <= RESIDENT_MAX_K
     eligible = resident_ok and lib.gnca_bptt_ckpt_bytes(C.byref(desc), B, H, W, 1) > 0
     if impl == IMPL["resident"] and not eligible:
-        raise ValueError("rollout: impl='resident' with bptt_budget needs the resident BPTT, which this model / shape "
+        raise ValueError(f"{who}: impl='resident' with bptt_budget needs the resident BPTT, which this model / shape "
                          f"does not have (16 channels, hidden 128, classic or torus graph, H*W <= 2048, W % 4 == 0, "
                          f"at most {RESIDENT_MAX_K} offsets per step)")
     nrec = _record_bytes(lib, desc, B, H, W, T) if (impl in (IMPL["auto"], IMPL["resident"]) and resident_ok) else 0
@@ -275,6 +281,19 @@ def _bptt_plan(desc, B: int, H: int, W: int, T: int, budget: int, impl: int, k: 
     if impl in (IMPL["auto"], IMPL["streaming"]):
         branches.append(("streaming_ckpt", lambda K: lib.gnca_ckpt_segment_bytes(C.byref(desc), B, H, W, K)))
     smallest = today[2] if today is not None else None
+    if every is not None:
+        # the frames are the checkpoints, so only the segment buffer comes on top of them.  Resident segments span a
+        # whole number of frames: the largest such K that fits, from the first multiple of `every` that covers T (one
+        # segment) down; streaming segments are one frame interval long (gnca_rollout_bwd_ckpt).
+        for path, segment_bytes in branches:
+            Ks = range(-(-max(T, 1) // every) * every, 0, -every) if path == "resident_ckpt" else (every,)
+            for K in Ks:
+                need = segment_bytes(K)
+                if need <= budget:
+                    return path, K, need
+                smallest = need if smallest is None else min(smallest, need)
+        raise ValueError(f"record_rollout: bptt_budget={budget} bytes is too small for this recording (B={B}, {H}x{W}, "
+                         f"T={T}, every={every}); the smallest budget that works is {smallest} bytes")
     for path, segment_bytes in branches:
         # largest K first: the fewest segment launches (the recompute costs one forward whatever K is)
         for K in range(max(T, 1), 0, -1):
@@ -286,7 +305,8 @@ def _bptt_plan(desc, B: int, H: int, W: int, T: int, budget: int, impl: int, k: 
                      f"the smallest budget that works is {smallest} bytes")
 
 
-def bptt_plan(model, B: int, H: int, W: int, T: int, budget: int, impl: str = "auto", k: Optional[int] = None):
+def bptt_plan(model, B: int, H: int, W: int, T: int, budget: int, impl: str = "auto", k: Optional[int] = None, *,
+              every: Optional[int] = None):
     """Which BPTT history `rollout(..., bptt_budget=budget)` keeps for a B x C x H x W batch over T steps, without
     touching the GPU: `(path, every, bytes)`.
 
@@ -305,15 +325,28 @@ def bptt_plan(model, B: int, H: int, W: int, T: int, budget: int, impl: str = "a
 
     Zero-padded graph shift models: the plan is over the dense history and streaming checkpoints only.  The resident
     zero-pad BPTT that rollout() takes without a budget (gnca_bptt_zp_bytes) has no checkpointed form, so under a budget
-    these models keep the dense history when it fits."""
+    these models keep the dense history when it fits.
+
+    `every=S` (keyword only): the plan of `record_rollout(..., every=S, differentiable=True, bptt_budget=budget)`, whose
+    frames x_{f*S} are returned whatever the plan, so `bytes` counts what the BPTT keeps beyond them and x_T:
+    * "records" / "dense": the history record_rollout keeps without a budget, when it fits;
+    * ("resident_ckpt", K, segment bytes): the frames are the checkpoints; K is the largest multiple of S whose resident
+      segment buffer (gnca_bptt_ckpt_bytes) fits;
+    * ("streaming_ckpt", S, segment bytes): the frames are the checkpoints of the streaming kernels, exactly
+      record_rollout(..., checkpoint=True).
+    Zero-padded graph shift models take the dense history or the streaming checkpoints here too.  ValueError names the
+    smallest budget that works when nothing fits."""
     if impl not in ("auto", "resident", "streaming"):
         raise ValueError(f"bptt_plan: impl must be 'auto', 'resident' or 'streaming', got {impl!r}")
     if int(budget) < 0:
         raise ValueError(f"bptt_plan: budget must be >= 0, got {budget}")
+    if every is not None and int(every) < 1:
+        raise ValueError(f"bptt_plan: every must be >= 1, got {every}")
     if k is None:
         g = getattr(model, "graph", None) if getattr(model, "_is_graph", False) else None
         k = min(g.num_neighbors, len(g.offsets)) if g is not None else 0
-    return _bptt_plan(model.model_desc(), int(B), int(H), int(W), int(T), int(budget), IMPL[impl], int(k))
+    return _bptt_plan(model.model_desc(), int(B), int(H), int(W), int(T), int(budget), IMPL[impl], int(k),
+                      every=None if every is None else int(every))
 
 
 def _ckpt_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, every: int, resident: bool):
@@ -339,57 +372,65 @@ def _ckpt_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, every: int, r
 
 
 def _ckpt_bwd_raw(desc, packed, ckpt: torch.Tensor, sched: Schedule, every: int, resident: bool, gT: torch.Tensor,
-                  gflat=None):
-    """Backward of _ckpt_fwd_raw: (dL/dx_0, flat parameter gradient), `gflat` accumulated into when given."""
+                  gflat=None, g_frames=None, ckpt_every: Optional[int] = None):
+    """Backward of _ckpt_fwd_raw: (dL/dx_0, flat parameter gradient), `gflat` accumulated into when given.  `ckpt` holds
+    x_{f*every}; segments are `ckpt_every` steps long (default `every`; resident only: a multiple of it, starting at
+    every (ckpt_every / every)-th frame).  `g_frames` (optional, the shape of `ckpt`): dL/dx_{f*every}, added at the
+    frames' steps."""
     _, B, Cc, H, W = ckpt.shape
+    ckpt_every = ckpt_every or every
     lib = _lib.load()
     gT = GF._require_cuda_f32(gT, "grad_output")
     g0 = torch.empty_like(ckpt[0])
     if gflat is None:
         gflat = torch.zeros(GF.param_layout(desc).total, dtype=torch.float32, device=ckpt.device)
-    nseg = (lib.gnca_bptt_ckpt_bytes if resident else lib.gnca_ckpt_segment_bytes)(C.byref(desc), B, H, W, every)
+    nseg = (lib.gnca_bptt_ckpt_bytes if resident else lib.gnca_ckpt_segment_bytes)(C.byref(desc), B, H, W, ckpt_every)
     segment = torch.empty(nseg, dtype=torch.uint8, device=ckpt.device)
     ws = GF._WS.get(ckpt.device, lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, sched.T))
     cs = sched.c_struct()
     if resident:
-        _lib.check(lib.gnca_rollout_bwd_bptt_ckpt(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(ckpt),
-                                                  every, GF._ptr(gT), GF._ptr(g0), GF._ptr(gflat), GF._ptr(segment),
-                                                  segment.numel(), GF._ptr(ws), ws.numel(), GF._stream()),
-                   "gnca_rollout_bwd_bptt_ckpt")
+        _lib.check(lib.gnca_rollout_bwd_bptt_ckpt_frames(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs),
+                                                         GF._ptr(ckpt), every, ckpt_every, GF._ptr(g_frames),
+                                                         GF._ptr(gT), GF._ptr(g0), GF._ptr(gflat), GF._ptr(segment),
+                                                         segment.numel(), GF._ptr(ws), ws.numel(), GF._stream()),
+                   "gnca_rollout_bwd_bptt_ckpt_frames")
     else:
         _lib.check(lib.gnca_rollout_bwd_ckpt(C.byref(desc), GF._ptr(packed), B, H, W, C.byref(cs), GF._ptr(ckpt), every,
-                                             None, GF._ptr(gT), GF._ptr(g0), GF._ptr(gflat), GF._ptr(segment),
-                                             segment.numel(), GF._ptr(ws), ws.numel(), GF._stream()),
+                                             GF._ptr(g_frames), GF._ptr(gT), GF._ptr(g0), GF._ptr(gflat),
+                                             GF._ptr(segment), segment.numel(), GF._ptr(ws), ws.numel(), GF._stream()),
                    "gnca_rollout_bwd_ckpt")
     return g0, gflat
 
 
-def _budget_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, impl: int, budget: int, keep_u: bool):
-    """The forward of the path bptt_plan picks: (x_T, History, plan)."""
+def _budget_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, impl: int, budget: int, keep_u: bool,
+                    every: int = 0):
+    """The forward of the path bptt_plan picks: (x_T, History, plan).  `every > 0`: the plan of record_rollout, and the
+    History carries the frames x_{f*every} (on the checkpoint paths they are the checkpoints)."""
     B, Cc, H, W = x0.shape
     resident_ok = True
     while True:
-        plan = _bptt_plan(desc, B, H, W, sched.T, budget, impl, sched.k, resident_ok)
-        path, every, _ = plan
+        plan = _bptt_plan(desc, B, H, W, sched.T, budget, impl, sched.k, resident_ok, every or None)
+        path, K, _ = plan
         if path == "records":
-            out = _records_fwd_raw(desc, packed, x0, sched, 0, keep_x=False)
+            out = _records_fwd_raw(desc, packed, x0, sched, every, keep_x=False)
             if out is not None:
                 return out[0], out[1], plan
         elif path == "dense":
             # never the record attempt of rollout_fwd_raw: the plan chose the dense history because the records do not
             # fit or have no backward for this launch, and their buffer alone could exceed the budget
-            xT, hist = _dense_fwd_raw(desc, packed, x0, sched, True, impl, keep_u, 0)
+            xT, hist = _dense_fwd_raw(desc, packed, x0, sched, True, impl, keep_u, every)
             return xT, hist, plan
         else:
             resident = path == "resident_ckpt"
-            out = _ckpt_fwd_raw(desc, packed, x0, sched, every, resident)
+            out = _ckpt_fwd_raw(desc, packed, x0, sched, every or K, resident)
             if out is not None:
                 xT, ckpt = out
-                return xT, History(None, shape=(sched.T + 1, B, Cc, H, W), ckpt=ckpt, every=every,
-                                   resident=resident), plan
+                return xT, History(None, shape=(sched.T + 1, B, Cc, H, W), ckpt=ckpt, every=every or K,
+                                   resident=resident, frames=ckpt if every else None, ckpt_every=K), plan
         if impl == IMPL["resident"]:
-            raise ValueError("rollout: impl='resident' with bptt_budget, but the resident backward has no launch "
-                             f"configuration for this batch (B={B}, {H}x{W}, k={sched.k})")
+            raise ValueError(f"{'record_rollout' if every else 'rollout'}: impl='resident' with bptt_budget, but the "
+                             "resident backward has no launch configuration for this batch "
+                             f"(B={B}, {H}x{W}, k={sched.k})")
         resident_ok = False              # the resident backward does not take this launch: plan without it
 
 
@@ -445,16 +486,15 @@ def rollout_fwd_raw(desc, packed, x0: torch.Tensor, sched: Schedule, *, history:
     history for the backward (the resident BPTT path then skips storing x_t).  `every > 0` (with `history`): the
     History also carries the frames x_{f*every} of `record_rollout` -- on the record path the forward writes them in
     place of the x_t history (gnca_rollout_fwd_bptt_record), on the dense path they are copied out of it.
-    `bptt_budget` (with `history`, without `every` or `keep_x`): the history takes at most that many bytes, on the
-    path bptt_plan picks (History.plan); None is exactly the call without it."""
+    `bptt_budget` (with `history`, without `keep_x`): the history takes at most that many bytes, on the path bptt_plan
+    picks (History.plan; with `every`, the plan of bptt_plan(..., every=every), whose checkpoints are the frames); None
+    is exactly the call without it."""
     x0 = GF._require_cuda_f32(x0, "x0")
     B, Cc, H, W = x0.shape
     if Cc != desc.C:
         raise ValueError(f"x0 has {Cc} channels, model has {desc.C}")
     if bptt_budget is not None and history:
-        if every > 0:
-            raise ValueError("rollout_fwd_raw: bptt_budget keeps no frames; it cannot be combined with every")
-        xT, hist, plan = _budget_fwd_raw(desc, packed, x0, sched, impl, int(bptt_budget), keep_u)
+        xT, hist, plan = _budget_fwd_raw(desc, packed, x0, sched, impl, int(bptt_budget), keep_u, every)
         hist.plan = plan
         return xT, hist
     if history and impl in (0, 2) and sched.T > 0:
@@ -499,8 +539,12 @@ def rollout_bwd_raw(desc, packed, hist, sched: Schedule, gT: torch.Tensor, *, gf
         hist = History(hist)
     if hist.ckpt is not None:
         if g_frames is not None:
-            raise ValueError("rollout_bwd_raw: a checkpointed history (bptt_budget) takes no frame gradients")
-        return _ckpt_bwd_raw(desc, packed, hist.ckpt, sched, hist.every, hist.resident, gT, gflat)
+            g_frames = GF._require_cuda_f32(g_frames, "frame gradients")
+            if g_frames.shape != hist.ckpt.shape:
+                raise ValueError(f"frame gradients have shape {tuple(g_frames.shape)}, expected "
+                                 f"{tuple(hist.ckpt.shape)}")
+        return _ckpt_bwd_raw(desc, packed, hist.ckpt, sched, hist.every, hist.resident, gT, gflat, g_frames,
+                             hist.ckpt_every)
     _, B, Cc, H, W = hist.shape
     gT = GF._require_cuda_f32(gT, "grad_output")
     lib = _lib.load()
@@ -710,26 +754,37 @@ def rollout(model, x0: torch.Tensor, schedule: Schedule, *, checkpoint_every: Op
 
 class _RecordFn(torch.autograd.Function):
     """record_rollout(..., differentiable=True): the frames and x_T as the outputs of one node; its backward is one
-    BPTT that adds dL/dframe_f at step f * every."""
+    BPTT that adds dL/dframe_f at step f * every.  With cfg["budget"] the history is the one bptt_plan(..., every=every)
+    picks (ctx.plan); frames that are checkpoints are kept with save_for_backward, so editing one in place makes the
+    backward raise."""
 
     @staticmethod
     def forward(ctx, x0, cfg, *params):
         xT, hist = rollout_fwd_raw(cfg["desc"], cfg["packed"], x0, cfg["schedule"], history=True, impl=cfg["impl"],
-                                   keep_x=False, every=cfg["every"])
+                                   keep_x=False, every=cfg["every"], bptt_budget=cfg.get("budget"))
         ctx.set_materialize_grads(False)          # an unused output passes None: no zero tensor, no frame pass
         ctx.cfg = cfg
         ctx.param_shapes = [p.shape for p in params]
+        ctx.plan = hist.plan
+        frames = hist.frames
+        ctx.has_ckpt = hist.ckpt is not None
+        if ctx.has_ckpt:
+            ctx.save_for_backward(frames)
+            hist.ckpt = hist.frames = None
         ctx.hist = hist
-        return hist.frames, xT
+        return frames, xT
 
     @staticmethod
     def backward(ctx, g_states, g_xT):
         cfg = ctx.cfg
         if ctx.hist is None:
             raise RuntimeError("record_rollout: the gradient history was already consumed by an earlier backward")
+        hist = ctx.hist
+        if ctx.has_ckpt:
+            (hist.ckpt,) = ctx.saved_tensors
         if g_xT is None:
-            g_xT = torch.zeros_like(ctx.hist.frames[0])
-        g0, gflat = rollout_bwd_raw(cfg["desc"], cfg["packed"], ctx.hist, cfg["schedule"], g_xT, impl=cfg["impl"],
+            g_xT = torch.zeros_like(hist.ckpt[0] if ctx.has_ckpt else hist.frames[0])
+        g0, gflat = rollout_bwd_raw(cfg["desc"], cfg["packed"], hist, cfg["schedule"], g_xT, impl=cfg["impl"],
                                     g_frames=g_states, every=cfg["every"])
         offs = GF.segment_offsets(cfg["desc"])
         grads = [gflat[offs[i]:offs[i + 1]].view(ctx.param_shapes[i]) for i in range(len(ctx.param_shapes))]
@@ -749,7 +804,8 @@ class Trajectory:
 
 
 def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, attention: bool = False,
-                   impl: str = "auto", differentiable: bool = False, checkpoint: bool = False) -> Trajectory:
+                   impl: str = "auto", differentiable: bool = False, checkpoint: bool = False,
+                   bptt_budget: Optional[int] = None) -> Trajectory:
     """T steps from x0 under `schedule` in one library call (gnca_rollout_record), keeping x_t every `every` steps and,
     with `attention=True`, the attention map `model.step(x_t, ..., return_attention=True)` gives for each kept step
     t < T.  Watching a rollout this way keeps the fused rollout kernels; no gradient history or record buffer is
@@ -763,10 +819,30 @@ def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, a
 
     `checkpoint=True` (with `differentiable=True`): the recorded frames are the only history.  The backward recomputes
     each `every`-step segment from its frame on the streaming kernels (rollout(..., checkpoint_every=every)), so memory
-    is the frames plus one segment.  Editing a returned frame in place makes the backward raise."""
+    is the frames plus one segment.  Editing a returned frame in place makes the backward raise.
+
+    `bptt_budget=N` (bytes, with `differentiable=True`): what the BPTT keeps beyond the returned frames and x_T takes at
+    most N bytes, on the path `bptt_plan(..., every=every)` picks.  The history the call keeps without a budget is kept
+    when it fits (bit-identical results); else the frames are the checkpoints of the resident BPTT, which recomputes
+    segments of the largest multiple of `every` steps whose buffer fits (dL/dx_0 bit-equal to the unbudgeted resident
+    path, parameter gradients up to the summation order); else those of the streaming kernels, exactly
+    `checkpoint=True`.  ValueError names the smallest budget that works when nothing fits.  Zero-padded graph shift
+    models keep the dense history when it fits and otherwise take the streaming checkpoints, as in
+    rollout(..., bptt_budget=N).  `impl="resident"` / `"streaming"` restrict the choice to that backward.  Frames that
+    are checkpoints make the backward raise when edited in place.  Without grad the call is the detached recording."""
     every = int(every)
     if every < 1:
         raise ValueError(f"record_rollout: every must be >= 1, got {every}")
+    if bptt_budget is not None:
+        if checkpoint:
+            raise ValueError("record_rollout: bptt_budget chooses the history itself; it cannot be combined with "
+                             "checkpoint=True")
+        if not differentiable:
+            raise ValueError("record_rollout: bptt_budget needs differentiable=True")
+        if impl not in ("auto", "resident", "streaming"):
+            raise ValueError(f"record_rollout: bptt_budget needs impl 'auto', 'resident' or 'streaming', got {impl!r}")
+        if int(bptt_budget) < 0:
+            raise ValueError(f"record_rollout: bptt_budget must be >= 0 bytes, got {bptt_budget}")
     if checkpoint:
         if not differentiable:
             raise ValueError("record_rollout: checkpoint=True needs differentiable=True")
@@ -783,6 +859,11 @@ def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, a
                 raise ValueError(f"x0 has {x0.shape[1]} channels, model has {desc.C}")
             cfg = {"desc": desc, "packed": model.packed_weights(), "schedule": schedule, "impl": IMPL[impl],
                    "every": every}
+            if bptt_budget is not None:
+                B, _, H, W = x0.shape
+                # errors before any launch
+                _bptt_plan(desc, B, H, W, schedule.T, int(bptt_budget), IMPL[impl], schedule.k, every=every)
+                cfg["budget"] = int(bptt_budget)
             frames, xT = (_CkptFn if checkpoint else _RecordFn).apply(x0, cfg, *ps)
             attn = None
             if attention:

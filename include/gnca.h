@@ -356,10 +356,20 @@ int gnca_rollout_bwd_bptt_zp(const gnca_model* m, const float* packed_dev, int B
  * forward restarts from ckpt[j] at that absolute step (fire rates, gains, offsets, fire_u, the Philox counter and
  * steps[b] keep their absolute indices), without re-applying a damage at the checkpoint; the backward still multiplies
  * dL/dx by the mask at damage_step.  g0 equals the unsegmented gnca_rollout_bwd_bptt bit for bit; gparams match it up to
- * the summation order.  There are no frame gradients on this path.  segment_dev: gnca_bptt_ckpt_bytes(every) bytes;
- * workspace: gnca_rollout_workspace_bytes.  Argument errors return before any launch: a NULL required pointer,
- * every <= 0 or T < 0 is GNCA_ERR_ARG; a segment or workspace too small is GNCA_ERR_WORKSPACE; k outside
- * [0, GNCA_MAX_K] is GNCA_ERR_UNSUPPORTED.
+ * the summation order.  segment_dev: gnca_bptt_ckpt_bytes(every) bytes; workspace: gnca_rollout_workspace_bytes.
+ * Argument errors return before any launch: a NULL required pointer, every <= 0 or T < 0 is GNCA_ERR_ARG; a segment
+ * or workspace too small is GNCA_ERR_WORKSPACE; k outside [0, GNCA_MAX_K] is GNCA_ERR_UNSUPPORTED.  It is
+ * gnca_rollout_bwd_bptt_ckpt_frames with frames_dev = ckpt_dev, ckpt_every = every and no frame gradients.
+ *
+ * gnca_rollout_bwd_bptt_ckpt_frames: the same backward with frame gradients, for a loss on recorded frames.  frames_dev
+ * ([T/every+1][B][C][H][W]) holds x_{f*every}, written by gnca_rollout_fwd_bptt_ckpt(..., every, frames_dev); the
+ * checkpoints are frames_dev[j * ckpt_every / every], so segments are ckpt_every steps long.  g_frames_dev (optional,
+ * same shape) holds dL/dx_{f*every}: segment j adds frames [t0/every, (t0+n)/every) at their steps, before the damage
+ * mask, with the semantics of gnca_rollout_bwd_bptt_frames; when T % every == 0 the last frame is x_T and is added to
+ * gT once, before the last segment.  T = 0 gives g0 = gT + g_frames[0].  segment_dev: gnca_bptt_ckpt_bytes(ckpt_every)
+ * bytes.  A ckpt_every that is not a positive multiple of every is GNCA_ERR_ARG; the other argument errors are those
+ * of gnca_rollout_bwd_bptt_ckpt, and a configuration without the checkpointed resident BPTT (gnca_bptt_ckpt_bytes
+ * = 0, e.g. the zero-padded graph shift) is GNCA_ERR_UNSUPPORTED, all before any launch.
  */
 size_t gnca_bptt_ckpt_bytes(const gnca_model* m, int B, int H, int W, int every);
 int gnca_rollout_fwd_bptt_ckpt(const gnca_model* m, const float* packed_dev, int B, int H, int W,
@@ -369,6 +379,11 @@ int gnca_rollout_bwd_bptt_ckpt(const gnca_model* m, const float* packed_dev, int
                                const gnca_schedule* sched, const float* ckpt_dev, int every, const float* gT_dev,
                                float* g0_dev, float* gparams_dev, void* segment_dev, size_t segment_bytes,
                                void* workspace_dev, size_t workspace_bytes, void* stream);
+int gnca_rollout_bwd_bptt_ckpt_frames(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                                      const gnca_schedule* sched, const float* frames_dev, int every, int ckpt_every,
+                                      const float* g_frames_dev, const float* gT_dev, float* g0_dev, float* gparams_dev,
+                                      void* segment_dev, size_t segment_bytes, void* workspace_dev,
+                                      size_t workspace_bytes, void* stream);
 
 /*
  * HOST function (no device work): T consecutive `random.sample(range(n), k)` draws of CPython's `random` module on
