@@ -77,6 +77,11 @@ EXPORTS = {
     "gnca_rollout_record": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
                                       C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                       C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
+    "gnca_metrics_scratch_bytes": (C.c_size_t, [C.POINTER(GncaModel), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "gnca_rollout_metrics": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                       C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_float,
+                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_int,
+                                       C.c_void_p]),
     "gnca_rollout_bwd": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
                                    C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),

@@ -59,12 +59,27 @@ bool update_tc_supported(const gnca_model& m, const StepArgs& a);
 int launch_update_tc(const gnca_model& m, const Packed& P, const float* packed, StepArgs& a, const uint16_t* glist,
                      const int* prefix, cudaStream_t st);
 
+// Per-frame metrics of gnca_rollout_metrics, written by the forward kernels at every step t % every == 0 (and at T when
+// T % every == 0): one partial of 4 doubles per (frame, sample, part) -- part = the CTA's rank in the cluster kernels,
+// a block of k_frame_metrics on the streaming path -- summed over the parts in part order by run_metrics_reduce.
+struct FrameMetrics {
+  const float* target;   // [4][H][W] premultiplied RGBA
+  double* part;          // [F][B][P][4] (gnca_metrics_scratch_bytes)
+  double* sums;          // [F][B][2] premultiplied-RGBA and clipped-RGB squared-error sums
+  int* counts;           // [F][B][2] pixel-perfect and alive cells
+  float eps;
+  int every;
+};
+// sums / counts of `rows` (frame, sample) pairs from their P partials (gnca_rollout.cu)
+int run_metrics_reduce(int rows, int P, const double* part, double* sums, int* counts, cudaStream_t st);
+
 // cluster-resident forward rollout (gnca_resident.cu); GNCA_ERR_UNSUPPORTED when the configuration has no
 // resident kernel (zero-padded graph shift, sample too large for the cluster's shared memory).
 // hist: x_t of every step t % hist_every == 0 goes to slot t / hist_every ([T/hist_every+1][B][C][H][W]).
 int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                      const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
-                     float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st, int hist_every = 1);
+                     float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st, int hist_every = 1,
+                     const FrameMetrics* met = nullptr);
 
 // replicated-state cluster rollout (gnca_rep.cu): every CTA of a sample's cluster holds the whole sample; first
 // choice of the resident path.  scratch: >= B*C*H*W floats of device memory (overflow of the in-smem u buffer).
@@ -72,12 +87,13 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
 // sched.steps stays absolute.  The launch configuration depends on B and H*W only, so a segment launch reproduces the
 // steps of a whole-rollout launch bit for bit.
 // zp (zero-padded graph shift only): with records, also the attention weights and row sums of every message step
+// met: the per-frame metrics of the steps t % met->every == 0 (a whole rollout, t0 = 0)
 struct ZpRec;
 struct ZpBwd;
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                 float* u_hist, float* rec, uint32_t* masks, float* scratch, cudaStream_t st, int hist_every = 1,
-                int t0 = 0, const ZpRec* zp = nullptr);
+                int t0 = 0, const ZpRec* zp = nullptr, const FrameMetrics* met = nullptr);
 // resident BPTT on the records of run_rep_fwd (gnca_rep_bwd.cu).  g_frames (optional, [F][B][C][H][W]): dL/dx_{f*every}
 // added at step f * every (gnca_rollout_bwd_bptt_frames)
 size_t rep_bptt_bytes(const gnca_model& m, int B, int H, int W, int T);     // 0: configuration not supported

@@ -27,6 +27,7 @@
 #include <type_traits>
 #include "gnca_common.cuh"
 #include "gnca_internal.h"
+#include "gnca_metrics.cuh"
 #include "gnca_ptx.cuh"
 #include "gnca_rep.h"
 
@@ -102,13 +103,44 @@ __device__ __forceinline__ uint32_t pack_nibbles(uint32_t nib, int lane) {
   return w;
 }
 
+// Frame metrics of x_t (cell-major sX, alpha plane sAg) over cells [lo, hi), spread over warps [w0, kPW): each warp
+// leaves its partial as 4 doubles at the head of its own perception tile in sY, which is free from the end of its tiles
+// to the next step's tiles.  rep_met_flush (one thread, after a barrier) adds them in warp order.
+__device__ __forceinline__ void rep_met_cells(const FrameMetrics& M, const float* sX, const float* sAg, float* sY, int lo,
+                                              int hi, int HW, float thr, int w0) {
+  constexpr int C = 16, kTile = 3 * C * 8;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  MetAcc acc{0.0, 0.0, 0, 0};
+#pragma unroll 1
+  for (int cell = lo + (warp - w0) * 32 + lane; cell < hi; cell += (kPW - w0) * 32) {
+    const float4 v = *reinterpret_cast<const float4*>(sX + (size_t)cell * C);
+    met_cell(acc, v.x, v.y, v.z, sAg[cell], M.target, cell, HW, M.eps, thr);
+  }
+  met_warp_sum(acc);
+  if (lane == 0) met_put(reinterpret_cast<double*>(sY + warp * kTile), acc);
+}
+__device__ __forceinline__ void rep_met_flush(const float* sY, int w0, double* dst) {
+  met_sum_parts(dst, reinterpret_cast<const double*>(sY), w0, kPW, 3 * 16 * 8 / 2);
+}
+// a whole frame by all warps, outside the tile phase of a step
+__device__ __forceinline__ void rep_met_frame(const FrameMetrics& M, const float* sX, const float* sAg, float* sY, int lo,
+                                              int hi, int HW, float thr, double* dst) {
+  rep_met_cells(M, sX, sAg, sY, lo, hi, HW, thr, 0);
+  __syncthreads();
+  if (threadIdx.x == 0) rep_met_flush(sY, 0, dst);
+  __syncthreads();
+}
+
 // ZP: zero-padded graph shift (the module default, graph_augmentation.py:85-92): senders (y - dy, x) -- the reference's
 // _shift2d_pad slices the x padding away again, so dx is a no-op -- and per-sample softmax weights over the k offsets
 // (graph_augmentation.py:114,136-154), recomputed from the resident state at the top of every step.  A separate
 // instantiation: the torus kernel (trainer, bench) is compiled exactly as before.
 // Z (ZP with records only, else unused): the softmax weights and row sums of every message step, for k_rep_bwd.
-template <int C, bool ZP>
-__global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const float* __restrict__ packed, ZpRec Z) {
+// MET (gnca_rollout_metrics): at every step t % M.every == 0 each CTA reduces the cells it stores for the history,
+// [my_lo, my_hi), against M.target and writes one partial per (frame, sample, rank); M is unused otherwise.
+template <int C, bool ZP, bool MET>
+__global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const float* __restrict__ packed, ZpRec Z,
+                                                     FrameMetrics M) {
   static_assert(C == 16, "lane mapping: 2 cells x 16 channels per warp row");
   constexpr int C3 = 3 * C, HID = 128;
   constexpr int CPL = 32 / C;                    // cells per lane row (2)
@@ -226,6 +258,9 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
   const int my_lo = (HW * rank) >> lnc, my_hi = (HW * (rank + 1)) >> lnc;
   const int hist_items = ((my_hi - my_lo + 7) & ~7) * C;
   const int n_fire_tasks = (NQ + 31) >> 5, n_hist_tasks = R.hist ? (hist_items + 255) >> 8 : 0;
+  // frame metrics: the partial of this CTA's cells of frame t goes to part[frame][b][rank]
+  double* met_dst = MET ? M.part + ((size_t)b * NC + rank) * 4 : nullptr;
+  const size_t met_frame_stride = MET ? (size_t)a.B * NC * 4 : 0;
 
   // ---- schedule: registers hold step t+2 while step t runs; smem buffers hold t and t+1 ---------------------
   float nx_fr = 0.f, nx_gain = 0.f;
@@ -418,6 +453,8 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
     }
     if (t >= my_steps) {                         // frozen sample (whole cluster agrees): state passes through
       if (float* h = hist_at(t)) store_state(h, my_lo, my_hi);
+      if constexpr (MET)
+        if (t % M.every == 0) rep_met_frame(M, sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr, met_dst + (t / M.every) * met_frame_stride);
       continue;
     }
     const float gain_m = s_gain[cur];
@@ -738,6 +775,7 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
           }
         }
       }
+      if constexpr (MET) if (hist && t % M.every == 0) rep_met_cells(M, sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr, 1);
     };
     const bool had_tile = n_my <= 32 ? (2 * warp < n_my) : n_my <= 64 ? (4 * warp < n_my) : (((n_my * warp) >> 4) < ((n_my * (warp + 1)) >> 4));
     const bool fire_early = !use_async || !had_tile;
@@ -750,6 +788,8 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
       if (lane == 0) { s_wred[warp][0] = f1; s_wred[warp][1] = f2; }
     }
     __syncthreads();
+    if constexpr (MET)
+      if (tid == 32 && t % M.every == 0) rep_met_flush(sY, 1, met_dst + (t / M.every) * met_frame_stride);
     if (!use_async) {
       if (gn && warp == 0) {
         float t1 = lane < kPW ? s_wred[lane][0] : 0.f, t2 = lane < kPW ? s_wred[lane][1] : 0.f;
@@ -915,6 +955,8 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
 
   __syncthreads();
   if (float* h = hist_at(R.T)) store_state(h, my_lo, my_hi);
+  if constexpr (MET)
+    if (R.T % M.every == 0) rep_met_frame(M, sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr, met_dst + (R.T / M.every) * met_frame_stride);
   store_state(R.xT + sample_off, my_lo, my_hi);
   if (R.dbg && blockIdx.x == R.dbg_cta && tid < 24) R.dbg[tid] = s_dbg[tid];
   cluster_arrive(); cluster_wait();      // nobody exits while a peer may still address its shared memory
@@ -933,7 +975,7 @@ static size_t rep_smem_bytes(int C, int HW, int ucap, int listcap) {
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                 float* u_hist, float* rec, uint32_t* masks, float* scratch /* >= B*C*H*W floats */, cudaStream_t st,
-                int hist_every, int t0, const ZpRec* zpr) {
+                int hist_every, int t0, const ZpRec* zpr, const FrameMetrics* met) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (m.C != 16 || m.hidden != 128) return GNCA_ERR_UNSUPPORTED;
   if (H > kMaxRows || W > kMaxRows || H < 1 || W < 4 || (W & 3)) return GNCA_ERR_UNSUPPORTED;   // quads of 4 cells per row
@@ -965,7 +1007,10 @@ int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B
   R.damage = DamageView{sched.damage, sched.damage_layout}; R.damage_step = sched.damage_step;
   R.KP = k > 8 ? 16 : 8;
   R.zd = zp ? m.d_model : 0;
-  const void* kfn = zp ? (const void*)k_rep_fwd<16, true> : (const void*)k_rep_fwd<16, false>;
+  // the metrics instantiations have the same shared memory and register cap as the plain ones: the same launch
+  // configuration, so x_T is bit-equal to the rollout without metrics
+  const void* kfn = zp ? (met ? (const void*)k_rep_fwd<16, true, true> : (const void*)k_rep_fwd<16, true, false>)
+                       : (met ? (const void*)k_rep_fwd<16, false, true> : (const void*)k_rep_fwd<16, false, false>);
   R.HWp = 4 * (((HW >> 2) + 31) & ~31) + 16;      // planes padded to whole warps of quads + one scratch quad
   R.inv_n = (float)(1.0 / ((double)C * (double)H * (double)W));
 
@@ -1029,11 +1074,18 @@ int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B
   }
   prof_begin(PROF_RESIDENT_FWD, st);
   const ZpRec Z = (zp && zpr && rec) ? *zpr : ZpRec{nullptr, nullptr};
-  cudaError_t e = zp ? cudaLaunchKernelEx(&cfg, k_rep_fwd<16, true>, R, P, packed, Z)
-                     : cudaLaunchKernelEx(&cfg, k_rep_fwd<16, false>, R, P, packed, Z);
+  const FrameMetrics M = met ? *met : FrameMetrics{};
+  cudaError_t e = zp ? (met ? cudaLaunchKernelEx(&cfg, k_rep_fwd<16, true, true>, R, P, packed, Z, M)
+                            : cudaLaunchKernelEx(&cfg, k_rep_fwd<16, true, false>, R, P, packed, Z, M))
+                     : (met ? cudaLaunchKernelEx(&cfg, k_rep_fwd<16, false, true>, R, P, packed, Z, M)
+                            : cudaLaunchKernelEx(&cfg, k_rep_fwd<16, false, false>, R, P, packed, Z, M));
   prof_end(PROF_RESIDENT_FWD, st);
   if (e != cudaSuccess) return (int)e;
   GNCA_LAUNCH_CHECK();
+  if (met) {
+    const int rc = run_metrics_reduce((R.T / met->every + 1) * B, pick, met->part, met->sums, met->counts, st);
+    if (rc) return rc;
+  }
   if (R.dbg) {
     unsigned long long h[24];
     cudaStreamSynchronize(st);

@@ -20,6 +20,7 @@
 #include <type_traits>
 #include "gnca_common.cuh"
 #include "gnca_internal.h"
+#include "gnca_metrics.cuh"
 #include "gnca_ptx.cuh"
 
 namespace cg = cooperative_groups;
@@ -88,9 +89,11 @@ __device__ __noinline__ bool alive_local_ool(const float* plane, int lr, int x, 
   return m > thr;
 }
 
-template <int C>
+// MET (gnca_rollout_metrics): at every step t % M.every == 0 each CTA reduces its own rows (the cells store_own writes)
+// against M.target and writes one partial per (frame, sample, rank); M is unused otherwise.
+template <int C, bool MET>
 __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, Packed P, int hid,
-                                                               const float* __restrict__ packed) {
+                                                               const float* __restrict__ packed, FrameMetrics M) {
   cg::cluster_group cluster = cg::this_cluster();
   constexpr int C3 = 3 * C;
   constexpr int CQ = C / 4;                                     // channel quads (power of two)
@@ -205,6 +208,23 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
   auto store_hist = [&](int t) {        // x_t into its history slot when step t is kept
     if (R.hist && t % R.hist_every == 0) store_own(R.hist + (size_t)(t / R.hist_every) * a.B * C * HW + sample_off);
   };
+  // frame metrics of x_t over the own rows; the warps' partials go through the head of the hidden-layer staging
+  // buffer Ht, which is free outside P2
+  auto met_frame = [&](int t) {
+    MetAcc acc{0.0, 0.0, 0, 0};
+#pragma unroll 1
+    for (int oc = tid; oc < nown; oc += kRThreads) {
+      const float* px = sX + HALO * W + oc;
+      met_cell(acc, px[0], px[PL], px[2 * (size_t)PL], px[3 * (size_t)PL], M.target, r0 * W + oc, HW, M.eps,
+               a.alpha_thr);
+    }
+    met_warp_sum(acc);
+    double* s_met = reinterpret_cast<double*>(Ht);
+    if (lane == 0) met_put(s_met + warp * 4, acc);
+    __syncthreads();
+    if (tid == 0) met_sum_parts(M.part + (((size_t)(t / M.every) * a.B + b) * NC + rank) * 4, s_met, 0, kRWarps, 4);
+    __syncthreads();
+  };
   auto alive_local = [&](const float* plane, int lr, int x, int gy, float thr) {
     return alive_local_ool(plane, lr, x, gy, H, W, thr);
   };
@@ -221,6 +241,7 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
       __syncthreads();
     }
     store_hist(t);
+    if constexpr (MET) if (t % M.every == 0) met_frame(t);
     if (t >= my_steps) continue;               // frozen sample (whole cluster agrees): state passes through
     a.t = t;
     a.fire_u = R.fire_u_base ? R.fire_u_base + (size_t)t * a.B * HW : nullptr;
@@ -600,6 +621,7 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
   }
 
   store_hist(R.T);
+  if constexpr (MET) if (R.T % M.every == 0) met_frame(R.T);
   store_own(R.xT + sample_off);
   if (R.dbg && blockIdx.x == R.dbg_cta && tid < 16) R.dbg[tid] = s_dbg[tid];
   cluster_sync_no_acquire();     // nobody exits while a neighbour may still address its shared memory
@@ -627,7 +649,7 @@ static size_t resident_smem_bytes(int C, int hid, bool graph, int own, int halo,
 
 template <int C>
 static int launch_resident(const gnca_model& m, const Packed& P, const float* packed, ResidentArgs& R, int B, int radius,
-                           cudaStream_t st) {
+                           cudaStream_t st, const FrameMetrics* met) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   const int H = R.s.H, W = R.s.W;
   if (m.hidden != 128 || C < 4 || W > 255) return GNCA_ERR_UNSUPPORTED;   // layer 1 + 2 of a tile live in one warp: 32 lanes x 4 units
@@ -640,6 +662,8 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
   // Cluster size: the largest NC in {8,4,2,1} whose bands are at least `halo` rows, that fits shared memory and
   // keeps ALL B clusters co-resident (B <= cudaOccupancyMaxActiveClusters); if the batch is too large for that,
   // the smallest NC that fits (most clusters per wave) and the launch runs in waves.
+  // the metrics instantiation has the plain one's shared memory and register cap: the same launch configuration
+  auto kfn = met ? k_resident_fwd<C, true> : k_resident_fwd<C, false>;
   const int cands[4] = {8, 4, 2, 1};
   int pick = -1, pick_MB = 0, pick_nclusters = 0;
   size_t pick_smem = 0;
@@ -654,7 +678,7 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
       if (smem > 226 * 1024) { MB = 32; smem = resident_smem_bytes(C, m.hidden, graph, own, halo, W, MB, R.s.k, R.T); }
       if (smem > 226 * 1024) { MB = 16; smem = resident_smem_bytes(C, m.hidden, graph, own, halo, W, MB, R.s.k, R.T); }   // 40x40x32
       if (smem > 226 * 1024) continue;
-      GNCA_CHECK_CUDA(cudaFuncSetAttribute(k_resident_fwd<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      GNCA_CHECK_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       cudaLaunchConfig_t q{};
       q.gridDim = dim3(B * NC); q.blockDim = dim3(kRThreads); q.dynamicSmemBytes = smem; q.stream = st;
       cudaLaunchAttribute qa[1];
@@ -662,7 +686,7 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
       qa[0].val.clusterDim.x = NC; qa[0].val.clusterDim.y = 1; qa[0].val.clusterDim.z = 1;
       q.attrs = qa; q.numAttrs = 1;
       int nclusters = 0;
-      if (cudaOccupancyMaxActiveClusters(&nclusters, k_resident_fwd<C>, &q) != cudaSuccess || nclusters < 1) {
+      if (cudaOccupancyMaxActiveClusters(&nclusters, kfn, &q) != cudaSuccess || nclusters < 1) {
         cudaGetLastError();
         continue;
       }
@@ -675,7 +699,7 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
   {
     const int NC = pick, own = H / NC, MB = pick_MB;
     const size_t smem = pick_smem;
-    GNCA_CHECK_CUDA(cudaFuncSetAttribute(k_resident_fwd<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    GNCA_CHECK_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(B * NC);
     cfg.blockDim = dim3(kRThreads);
@@ -699,10 +723,14 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
       R.dbg_cta = atoi(getenv("GNCA_PHASE_TIMING"));
     }
     prof_begin(PROF_RESIDENT_FWD, st);
-    cudaError_t e = cudaLaunchKernelEx(&cfg, k_resident_fwd<C>, R, P, m.hidden, packed);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, kfn, R, P, m.hidden, packed, met ? *met : FrameMetrics{});
     prof_end(PROF_RESIDENT_FWD, st);
     if (e != cudaSuccess) return (int)e;
     GNCA_LAUNCH_CHECK();
+    if (met) {
+      const int rc = run_metrics_reduce((R.T / met->every + 1) * B, NC, met->part, met->sums, met->counts, st);
+      if (rc) return rc;
+    }
     if (R.dbg) {   // development only: synchronous read-back of the phase counters of CTA 0
       unsigned long long h[16];
       cudaStreamSynchronize(st);
@@ -721,7 +749,8 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
 // entry used by gnca_rollout_fwd (impl 2 / auto)
 int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                      const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
-                     float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st, int hist_every) {
+                     float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st, int hist_every,
+                     const FrameMetrics* met) {
   (void)ping; (void)pong; (void)alpha_tmp;
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (graph && !(m.flags & GNCA_F_TORUS) && sched.k > 0) return GNCA_ERR_UNSUPPORTED;   // zero-pad: streaming path
@@ -741,10 +770,10 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
   R.damage = DamageView{sched.damage, sched.damage_layout}; R.damage_step = sched.damage_step;
   const int radius = sched.max_offset;       // largest |dy| / |dx| in the schedule: sets the halo depth
   switch (m.C) {
-    case 4: return launch_resident<4>(m, P, packed, R, B, radius, st);
-    case 8: return launch_resident<8>(m, P, packed, R, B, radius, st);
-    case 16: return launch_resident<16>(m, P, packed, R, B, radius, st);
-    case 32: return launch_resident<32>(m, P, packed, R, B, radius, st);
+    case 4: return launch_resident<4>(m, P, packed, R, B, radius, st, met);
+    case 8: return launch_resident<8>(m, P, packed, R, B, radius, st, met);
+    case 16: return launch_resident<16>(m, P, packed, R, B, radius, st, met);
+    case 32: return launch_resident<32>(m, P, packed, R, B, radius, st, met);
   }
   return GNCA_ERR_UNSUPPORTED;
 }

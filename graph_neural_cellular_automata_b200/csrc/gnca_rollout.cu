@@ -5,6 +5,7 @@
 // BPTT stores only x_t (x_hist); u, the hidden layer, masks and the message are recomputed in the backward.
 #include "gnca_common.cuh"
 #include "gnca_internal.h"
+#include "gnca_metrics.cuh"
 #include "gnca_rep.h"
 
 namespace gnca {
@@ -20,6 +21,59 @@ __global__ void k_mul_inplace(size_t n, float* __restrict__ x, DamageView d, int
 __global__ void k_add(size_t n, float* __restrict__ out, const float* __restrict__ a, const float* __restrict__ b) {
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
     out[i] = a[i] + b[i];
+}
+
+// Frame metrics of one state buffer x ([B][C][HW]) on the streaming path: block (p, b) reduces cells
+// [p * cells, (p + 1) * cells) of sample b into part[b][p] -- the first level of a two-level reduction whose second is
+// k_metrics_reduce, both in a fixed order.
+constexpr int kMetThreads = 256;
+constexpr int kMetCells = 4096;                    // cells per block of k_frame_metrics
+
+static inline int frame_metrics_parts(int HW) { return (HW + kMetCells - 1) / kMetCells; }
+
+__global__ void __launch_bounds__(kMetThreads) k_frame_metrics(const float* __restrict__ x, int C, int HW,
+                                                                const float* __restrict__ tgt, float eps, float thr,
+                                                                double* __restrict__ part) {
+  const int p = blockIdx.x, P = gridDim.x, b = blockIdx.y;
+  const int lo = p * kMetCells, hi = min(HW, lo + kMetCells);
+  const float* xb = x + (size_t)b * C * HW;
+  MetAcc acc{0.0, 0.0, 0, 0};
+  for (int cell = lo + (int)threadIdx.x; cell < hi; cell += kMetThreads)
+    met_cell(acc, xb[cell], xb[HW + cell], xb[2 * (size_t)HW + cell], xb[3 * (size_t)HW + cell], tgt, cell, HW, eps,
+             thr);
+  met_warp_sum(acc);
+  __shared__ double s_met[kMetThreads / 32][4];
+  if ((threadIdx.x & 31) == 0) met_put(s_met[threadIdx.x >> 5], acc);
+  __syncthreads();
+  if (threadIdx.x == 0) met_sum_parts(part + ((size_t)b * P + p) * 4, &s_met[0][0], 0, kMetThreads / 32, 4);
+}
+
+// sums / counts of each (frame, sample) row from its P partials, in part order
+__global__ void k_metrics_reduce(int rows, int P, const double* __restrict__ part, double* __restrict__ sums,
+                                 int* __restrict__ counts) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= rows) return;
+  double s[4];
+  met_sum_parts(s, part + (size_t)r * P * 4, 0, P, 4);
+  sums[2 * (size_t)r] = s[0];
+  sums[2 * (size_t)r + 1] = s[1];
+  counts[2 * (size_t)r] = (int)s[2];
+  counts[2 * (size_t)r + 1] = (int)s[3];
+}
+
+int run_metrics_reduce(int rows, int P, const double* part, double* sums, int* counts, cudaStream_t st) {
+  k_metrics_reduce<<<(rows + 127) / 128, 128, 0, st>>>(rows, P, part, sums, counts);
+  GNCA_LAUNCH_CHECK();
+  return 0;
+}
+
+// metrics of frame f (the state x) on the streaming path
+static int frame_metrics(const FrameMetrics& met, const float* x, int f, int B, int C, int HW, float thr,
+                         cudaStream_t st) {
+  const int P = frame_metrics_parts(HW);
+  k_frame_metrics<<<dim3(P, B), kMetThreads, 0, st>>>(x, C, HW, met.target, met.eps, thr, met.part);
+  GNCA_LAUNCH_CHECK();
+  return run_metrics_reduce(B, P, met.part, met.sums + (size_t)f * B * 2, met.counts + (size_t)f * B * 2, st);
 }
 
 static int launch_add(size_t n, float* out, const float* a, const float* b, cudaStream_t st) {
@@ -179,9 +233,11 @@ static Segment carve_segment(void* base, const gnca_model& m, int B, int H, int 
 
 // gnca_rollout_fwd with a strided history: x_t of every step t % every == 0 goes to x_hist slot t / every
 // (every == 1: the full [T+1] history of gnca_rollout_fwd).
+// met: the per-frame metrics of gnca_rollout_metrics (stride met->every), by the kernel that runs the steps
 static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
                        const float* x0_dev, float* xT_dev, float* x_hist_dev, int every, float* stats_hist_dev,
-                       float* u_hist_dev, void* workspace_dev, size_t workspace_bytes, int impl, void* stream) {
+                       float* u_hist_dev, void* workspace_dev, size_t workspace_bytes, int impl, void* stream,
+                       const FrameMetrics* met = nullptr) {
   if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !workspace_dev) return GNCA_ERR_ARG;
   if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
   if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
@@ -203,10 +259,10 @@ static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int 
       int rc = GNCA_ERR_UNSUPPORTED;
       if (impl != 3)
         rc = run_rep_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, x_hist_dev, stats_hist_dev, u_hist_dev,
-                         nullptr, nullptr, r.ping, st, every);
+                         nullptr, nullptr, r.ping, st, every, 0, nullptr, met);
       if (rc == GNCA_ERR_UNSUPPORTED)
         rc = run_resident_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, x_hist_dev, stats_hist_dev,
-                              u_hist_dev, r.ping, r.pong, r.alpha_tmp, st, every);
+                              u_hist_dev, r.ping, r.pong, r.alpha_tmp, st, every, met);
       if (rc != GNCA_ERR_UNSUPPORTED || impl == 2 || impl == 3) return rc;
     }
   }
@@ -224,6 +280,10 @@ static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int 
       int rc = launch_damage(N, x_at(t), *sched, m->C, H * W, st);
       if (rc) return rc;
     }
+    if (met && t % met->every == 0) {
+      int rc = frame_metrics(*met, x_at(t), t / met->every, B, m->C, H * W, m->alpha_thr, st);
+      if (rc) return rc;
+    }
     StepArgs a;
     fill_step_args(a, *m, B, H, W);
     schedule_to_args(a, *sched, t, B, H, W);
@@ -237,6 +297,7 @@ static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int 
   }
   if ((x_hist_dev && T % every == 0) || T == 0)
     GNCA_CHECK_CUDA(cudaMemcpyAsync(xT_dev, x_at(T), N * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  if (met && T % met->every == 0) return frame_metrics(*met, xT_dev, T / met->every, B, m->C, H * W, m->alpha_thr, st);
   return 0;
 }
 
@@ -383,6 +444,31 @@ int gnca_rollout_record(const gnca_model* m, const float* packed_dev, int B, int
     if (rc) return rc;
   }
   return 0;
+}
+
+size_t gnca_metrics_scratch_bytes(const gnca_model* m, int B, int H, int W, int T, int every) {
+  if (!m || B <= 0 || H <= 0 || W <= 0 || T < 0 || every <= 0 || m->C < 4) return 0;
+  // the cluster kernels keep one partial per rank (<= 8) of every frame; the streaming path reuses one frame's blocks
+  const size_t F = (size_t)(T / every + 1);
+  const size_t cluster = F * B * 8, streaming = (size_t)B * frame_metrics_parts(H * W);
+  return (cluster > streaming ? cluster : streaming) * 4 * sizeof(double);
+}
+
+int gnca_rollout_metrics(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
+                         const float* x0_dev, float* xT_dev, int every, const float* target_dev, float eps,
+                         double* sums_dev, int32_t* counts_dev, void* scratch_dev, size_t scratch_bytes,
+                         void* workspace_dev, size_t workspace_bytes, int impl, void* stream) {
+  if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !target_dev || !sums_dev || !counts_dev || !scratch_dev ||
+      !workspace_dev)
+    return GNCA_ERR_ARG;
+  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0 || every <= 0 || m->C < 4) return GNCA_ERR_ARG;
+  if (!(eps >= 0.f)) return GNCA_ERR_ARG;
+  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
+  if (gnca_metrics_scratch_bytes(m, B, H, W, sched->T, every) > scratch_bytes) return GNCA_ERR_WORKSPACE;
+  const FrameMetrics met{target_dev, reinterpret_cast<double*>(scratch_dev), sums_dev, counts_dev, eps, every};
+  return rollout_fwd(m, packed_dev, B, H, W, sched, x0_dev, xT_dev, nullptr, 1, nullptr, nullptr, workspace_dev,
+                     workspace_bytes, impl, stream, &met);
 }
 
 int gnca_rollout_bwd_frames(const gnca_model* m, const float* packed_dev, int B, int H, int W,

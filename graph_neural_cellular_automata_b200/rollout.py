@@ -889,3 +889,66 @@ def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, a
                                        GF._ptr(x0), GF._ptr(xT), every, GF._ptr(frames), GF._ptr(attn), GF._ptr(ws),
                                        ws.numel(), IMPL[impl], GF._stream()), "gnca_rollout_record")
     return Trajectory(t=list(range(0, T + 1, every)), states=frames, attention=attn, x_T=xT)
+
+
+@dataclass
+class Monitor:
+    """What `monitor_rollout` returns.  Row f of every [F,B] tensor is frame f of `record_rollout(..., every=S)`:
+    x_{t[f]}, after the schedule's damage at `damage_step`, frozen for a sample with steps[b] <= t[f]."""
+    t: List[int]                            # step indices 0, S, 2S, ... <= T
+    loss: torch.Tensor                      # [F,B] f32: premultiplied-RGBA MSE against the target
+    psnr: torch.Tensor                      # [F,B] f32: utils.metrics.psnr_rgb
+    pixel_perfect: torch.Tensor             # [F,B] f32: utils.metrics.pixel_perfect(frame, target, eps)
+    alive: torch.Tensor                     # [F,B] int64: cells with alpha > model.alpha_thr (no dilation)
+    x_T: torch.Tensor                       # [B,C,H,W]
+
+
+def monitor_rollout(model, x0: torch.Tensor, schedule: Schedule, target: torch.Tensor, *, every: int,
+                    impl: str = "auto", eps: float = 0.05) -> Monitor:
+    """Quality curves of a rollout without its states: the T steps of `rollout()` (same `impl` and dispatch, the same
+    x_T) in one library call (gnca_rollout_metrics), reducing every `every`-th state against `target` ([4,H,W]
+    premultiplied RGBA on x0's device) where the kernel holds it.  Memory is F*B*24 bytes of results plus at most
+    F*B*256 bytes of per-CTA partials, instead of the F*B*C*H*W*4 bytes of `record_rollout` frames.  Inference only: the outputs are
+    detached and no BPTT buffer is allocated, whatever the grad mode.  PSNR is 10*log10(1 / mse) of the clipped RGB
+    from the kernel's sum; a frame equal to the target gives +inf, as utils.metrics.psnr_rgb does."""
+    every = int(every)
+    if every < 1:
+        raise ValueError(f"monitor_rollout: every must be >= 1, got {every}")
+    eps = float(eps)
+    if not eps >= 0.0:
+        raise ValueError(f"monitor_rollout: eps must be >= 0, got {eps}")
+    if impl not in IMPL:
+        raise ValueError(f"monitor_rollout: impl must be one of {sorted(IMPL)}, got {impl!r}")
+    desc = model.model_desc()
+    if x0.dim() != 4:
+        raise ValueError(f"monitor_rollout: x0 must be [B, C, H, W], got {list(x0.shape)}")
+    B, Cc, H, W = x0.shape
+    if Cc != desc.C:
+        raise ValueError(f"x0 has {Cc} channels, model has {desc.C}")
+    if desc.C < 4:
+        raise ValueError(f"monitor_rollout: the metrics read RGBA (channels 0-3); the model has {desc.C} channels")
+    if tuple(target.shape) != (4, H, W):
+        raise ValueError(f"monitor_rollout: target must be [4, {H}, {W}] (premultiplied RGBA), got "
+                         f"{list(target.shape)}")
+    x0 = GF._require_cuda_f32(x0.detach(), "x0")
+    target = GF._require_cuda_f32(target.detach(), "target")
+    if target.device != x0.device:
+        raise ValueError(f"monitor_rollout: target is on {target.device}, x0 on {x0.device}")
+    lib = _lib.load()
+    T = schedule.T
+    F = T // every + 1
+    xT = torch.empty_like(x0)
+    sums = torch.empty(F, B, 2, dtype=torch.float64, device=x0.device)
+    counts = torch.empty(F, B, 2, dtype=torch.int32, device=x0.device)
+    scratch = torch.empty(lib.gnca_metrics_scratch_bytes(C.byref(desc), B, H, W, T, every), dtype=torch.uint8,
+                          device=x0.device)
+    ws = GF._WS.get(x0.device, lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, T))
+    cs = schedule.c_struct()
+    _lib.check(lib.gnca_rollout_metrics(C.byref(desc), GF._ptr(model.packed_weights()), B, H, W, C.byref(cs),
+                                        GF._ptr(x0), GF._ptr(xT), every, GF._ptr(target), eps, GF._ptr(sums),
+                                        GF._ptr(counts), GF._ptr(scratch), scratch.numel(), GF._ptr(ws), ws.numel(),
+                                        IMPL[impl], GF._stream()), "gnca_rollout_metrics")
+    HW = H * W
+    return Monitor(t=list(range(0, T + 1, every)), loss=(sums[..., 0] / (4 * HW)).float(),
+                   psnr=(10.0 * torch.log10(1.0 / (sums[..., 1] / (3 * HW)))).float(),
+                   pixel_perfect=(counts[..., 0].double() / HW).float(), alive=counts[..., 1].long(), x_T=xT)

@@ -220,6 +220,28 @@ int gnca_rollout_record(const gnca_model* m, const float* packed_dev, int B, int
                         int every, float* frames_dev, float* attn_dev,
                         void* workspace_dev, size_t workspace_bytes, int impl, void* stream);
 
+/*
+ * Monitoring rollout: the T steps of gnca_rollout_fwd (same `impl`, dispatch and GNCA_ERR_UNSUPPORTED combinations;
+ * xT_dev receives the same x_T), reducing each frame gnca_rollout_record would keep against a target instead of
+ * keeping it.  Frame f (F = gnca_record_frames(T, every)) is x_{f*every}, as in gnca_rollout_record; per frame and
+ * sample, with p = the premultiplied RGBA of the frame (rgb * alpha, alpha = channel 3) and d = p - target:
+ *   - sums_dev[F][B][2]   = { sum of d^2 over the 4 channels and H*W cells,
+ *                             sum of (clip(p, 0, 1) - clip(target, 0, 1))^2 over the 3 RGB channels };
+ *   - counts_dev[F][B][2] = { cells with |d| < eps on all 4 channels, cells with alpha > m->alpha_thr }.
+ * target_dev: [4][H][W] fp32, premultiplied.  The products and differences are rounded one operation at a time (no
+ * FMA), the squares are summed in double over a fixed partition in a fixed order: two calls give bit-identical sums.
+ * scratch_dev: gnca_metrics_scratch_bytes(m, B, H, W, T, every) bytes (0: bad arguments); the workspace is the one of
+ * gnca_rollout_workspace_bytes.  No BPTT buffer.  Argument errors (a NULL pointer, every <= 0, eps < 0, C < 4) are
+ * GNCA_ERR_ARG, a scratch or workspace too small is GNCA_ERR_WORKSPACE, k outside [0, GNCA_MAX_K] is
+ * GNCA_ERR_UNSUPPORTED, all before any launch.
+ */
+size_t gnca_metrics_scratch_bytes(const gnca_model* m, int B, int H, int W, int T, int every);
+int gnca_rollout_metrics(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                         const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                         const float* target_dev, float eps, double* sums_dev, int32_t* counts_dev,
+                         void* scratch_dev, size_t scratch_bytes, void* workspace_dev, size_t workspace_bytes,
+                         int impl, void* stream);
+
 /* BPTT: given gT = dL/dx_T and the x_hist of the forward, produce g0 = dL/dx_0 and ACCUMULATE gparams. */
 int gnca_rollout_bwd(const gnca_model* m, const float* packed_dev, int B, int H, int W,
                      const gnca_schedule* sched, const float* x_hist_dev, const float* stats_hist_dev,
