@@ -82,6 +82,13 @@ EXPORTS = {
                                        C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_float,
                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_int,
                                        C.c_void_p]),
+    "gnca_rollout_record_models": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                             C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                             C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
+    "gnca_rollout_metrics_models": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                              C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                              C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p,
+                                              C.c_size_t, C.c_int, C.c_void_p]),
     "gnca_rollout_bwd": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
                                    C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),

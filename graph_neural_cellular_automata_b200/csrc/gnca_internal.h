@@ -73,13 +73,21 @@ struct FrameMetrics {
 // sums / counts of `rows` (frame, sample) pairs from their P partials (gnca_rollout.cu)
 int run_metrics_reduce(int rows, int P, const double* part, double* sums, int* counts, cudaStream_t st);
 
+// A stack of same-architecture models in one launch of the cluster kernels (gnca_rollout_record_models /
+// gnca_rollout_metrics_models): `packed` is [n_models][stride] and sample b runs model b / per_model.  Each kernel
+// rebases `packed` once, before staging the weights into shared memory.  stride = 0: one model for the whole batch.
+struct ModelStack {
+  int stride;      // floats between two models' packed buffers (Packed::total)
+  int per_model;   // samples per model (B / n_models)
+};
+
 // cluster-resident forward rollout (gnca_resident.cu); GNCA_ERR_UNSUPPORTED when the configuration has no
 // resident kernel (zero-padded graph shift, sample too large for the cluster's shared memory).
 // hist: x_t of every step t % hist_every == 0 goes to slot t / hist_every ([T/hist_every+1][B][C][H][W]).
 int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                      const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                      float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st, int hist_every = 1,
-                     const FrameMetrics* met = nullptr);
+                     const FrameMetrics* met = nullptr, ModelStack ms = ModelStack{0, 0});
 
 // replicated-state cluster rollout (gnca_rep.cu): every CTA of a sample's cluster holds the whole sample; first
 // choice of the resident path.  scratch: >= B*C*H*W floats of device memory (overflow of the in-smem u buffer).
@@ -88,12 +96,14 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
 // steps of a whole-rollout launch bit for bit.
 // zp (zero-padded graph shift only): with records, also the attention weights and row sums of every message step
 // met: the per-frame metrics of the steps t % met->every == 0 (a whole rollout, t0 = 0)
+// ms: a stack of models, one per block of ms.per_model samples (inference only: no records)
 struct ZpRec;
 struct ZpBwd;
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                 float* u_hist, float* rec, uint32_t* masks, float* scratch, cudaStream_t st, int hist_every = 1,
-                int t0 = 0, const ZpRec* zp = nullptr, const FrameMetrics* met = nullptr);
+                int t0 = 0, const ZpRec* zp = nullptr, const FrameMetrics* met = nullptr,
+                ModelStack ms = ModelStack{0, 0});
 // resident BPTT on the records of run_rep_fwd (gnca_rep_bwd.cu).  g_frames (optional, [F][B][C][H][W]): dL/dx_{f*every}
 // added at step f * every (gnca_rollout_bwd_bptt_frames)
 size_t rep_bptt_bytes(const gnca_model& m, int B, int H, int W, int T);     // 0: configuration not supported

@@ -65,6 +65,9 @@ struct RepArgs {
   // run_rep_fwd a schedule already rebased to the launch (arrays, fire_u, Philox counter, damage_step: segment_schedule
   // in gnca_rollout.cu); the kernel needs t0 only for the per-sample step counts steps[b], which stay absolute
   int t0;
+  // a stack of models (ModelStack): sample b stages its weights from packed + (b / model_per) * model_stride;
+  // model_stride = 0: every sample runs the model at `packed`
+  int model_stride, model_per;
 };
 
 #ifdef GNCA_PHASE_COUNTERS          /* build with -DGNCA_PHASE_COUNTERS for the per-phase cycle counters */
@@ -195,7 +198,8 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
   __shared__ unsigned long long s_dbg[24];
   if (tid < 24) s_dbg[tid] = 0;
 
-  // ---- weights -> smem ---------------------------------------------------------------------------------------
+  // ---- weights -> smem (the only reads of `packed`) -------------------------------------------------------------
+  if (R.model_stride) packed += (size_t)(b / R.model_per) * R.model_stride;
 #pragma unroll 1
   for (int i = tid; i < C3 * HID; i += kPT) {
     const int kk = i / HID, jp = i - kk * HID;                 // jp = l*4 + jj  <->  true unit l + 32*jj
@@ -975,7 +979,7 @@ static size_t rep_smem_bytes(int C, int HW, int ucap, int listcap) {
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                 float* u_hist, float* rec, uint32_t* masks, float* scratch /* >= B*C*H*W floats */, cudaStream_t st,
-                int hist_every, int t0, const ZpRec* zpr, const FrameMetrics* met) {
+                int hist_every, int t0, const ZpRec* zpr, const FrameMetrics* met, ModelStack ms) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (m.C != 16 || m.hidden != 128) return GNCA_ERR_UNSUPPORTED;
   if (H > kMaxRows || W > kMaxRows || H < 1 || W < 4 || (W & 3)) return GNCA_ERR_UNSUPPORTED;   // quads of 4 cells per row
@@ -1007,6 +1011,7 @@ int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B
   R.damage = DamageView{sched.damage, sched.damage_layout}; R.damage_step = sched.damage_step;
   R.KP = k > 8 ? 16 : 8;
   R.zd = zp ? m.d_model : 0;
+  R.model_stride = ms.stride; R.model_per = ms.per_model;
   // the metrics instantiations have the same shared memory and register cap as the plain ones: the same launch
   // configuration, so x_T is bit-equal to the rollout without metrics
   const void* kfn = zp ? (met ? (const void*)k_rep_fwd<16, true, true> : (const void*)k_rep_fwd<16, true, false>)

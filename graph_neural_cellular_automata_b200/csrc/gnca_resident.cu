@@ -91,9 +91,12 @@ __device__ __noinline__ bool alive_local_ool(const float* plane, int lr, int x, 
 
 // MET (gnca_rollout_metrics): at every step t % M.every == 0 each CTA reduces its own rows (the cells store_own writes)
 // against M.target and writes one partial per (frame, sample, rank); M is unused otherwise.
-template <int C, bool MET>
+// MS (a stack of models, gnca_rollout_*_models): sample b stages its weights from packed + (b / S.per_model) * S.stride;
+// S is unused otherwise.  A compile-time flag: a runtime field moves the register allocation of the plain kernels.
+template <int C, bool MET, bool MS>
 __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, Packed P, int hid,
-                                                               const float* __restrict__ packed, FrameMetrics M) {
+                                                               const float* __restrict__ packed, FrameMetrics M,
+                                                               ModelStack S) {
   cg::cluster_group cluster = cg::this_cluster();
   constexpr int C3 = 3 * C;
   constexpr int CQ = C / 4;                                     // channel quads (power of two)
@@ -146,6 +149,8 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
 
   // ---- weights -> smem.  Hidden units are permuted so that lane l of a warp owns units {g*128 + l + 32*jj}:
   //      its 4 weights of one input k are one float4, and the warp's stores of h are bank-conflict free.
+  //      These are the only reads of `packed`.
+  if constexpr (MS) packed += (size_t)(b / S.per_model) * S.stride;
 #pragma unroll 1
   for (int i = tid; i < C3 * hid; i += kRThreads) {
     const int k = i / hid, jp = i - k * hid;                   // jp = g*128 + l*4 + jj
@@ -649,7 +654,7 @@ static size_t resident_smem_bytes(int C, int hid, bool graph, int own, int halo,
 
 template <int C>
 static int launch_resident(const gnca_model& m, const Packed& P, const float* packed, ResidentArgs& R, int B, int radius,
-                           cudaStream_t st, const FrameMetrics* met) {
+                           cudaStream_t st, const FrameMetrics* met, ModelStack S) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   const int H = R.s.H, W = R.s.W;
   if (m.hidden != 128 || C < 4 || W > 255) return GNCA_ERR_UNSUPPORTED;   // layer 1 + 2 of a tile live in one warp: 32 lanes x 4 units
@@ -663,7 +668,9 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
   // keeps ALL B clusters co-resident (B <= cudaOccupancyMaxActiveClusters); if the batch is too large for that,
   // the smallest NC that fits (most clusters per wave) and the launch runs in waves.
   // the metrics instantiation has the plain one's shared memory and register cap: the same launch configuration
-  auto kfn = met ? k_resident_fwd<C, true> : k_resident_fwd<C, false>;
+  const bool stack = S.stride != 0;
+  auto kfn = stack ? (met ? k_resident_fwd<C, true, true> : k_resident_fwd<C, false, true>)
+                   : (met ? k_resident_fwd<C, true, false> : k_resident_fwd<C, false, false>);
   const int cands[4] = {8, 4, 2, 1};
   int pick = -1, pick_MB = 0, pick_nclusters = 0;
   size_t pick_smem = 0;
@@ -723,7 +730,7 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
       R.dbg_cta = atoi(getenv("GNCA_PHASE_TIMING"));
     }
     prof_begin(PROF_RESIDENT_FWD, st);
-    cudaError_t e = cudaLaunchKernelEx(&cfg, kfn, R, P, m.hidden, packed, met ? *met : FrameMetrics{});
+    cudaError_t e = cudaLaunchKernelEx(&cfg, kfn, R, P, m.hidden, packed, met ? *met : FrameMetrics{}, S);
     prof_end(PROF_RESIDENT_FWD, st);
     if (e != cudaSuccess) return (int)e;
     GNCA_LAUNCH_CHECK();
@@ -750,7 +757,7 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
 int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                      const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                      float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st, int hist_every,
-                     const FrameMetrics* met) {
+                     const FrameMetrics* met, ModelStack ms) {
   (void)ping; (void)pong; (void)alpha_tmp;
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (graph && !(m.flags & GNCA_F_TORUS) && sched.k > 0) return GNCA_ERR_UNSUPPORTED;   // zero-pad: streaming path
@@ -770,10 +777,10 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
   R.damage = DamageView{sched.damage, sched.damage_layout}; R.damage_step = sched.damage_step;
   const int radius = sched.max_offset;       // largest |dy| / |dx| in the schedule: sets the halo depth
   switch (m.C) {
-    case 4: return launch_resident<4>(m, P, packed, R, B, radius, st, met);
-    case 8: return launch_resident<8>(m, P, packed, R, B, radius, st, met);
-    case 16: return launch_resident<16>(m, P, packed, R, B, radius, st, met);
-    case 32: return launch_resident<32>(m, P, packed, R, B, radius, st, met);
+    case 4: return launch_resident<4>(m, P, packed, R, B, radius, st, met, ms);
+    case 8: return launch_resident<8>(m, P, packed, R, B, radius, st, met, ms);
+    case 16: return launch_resident<16>(m, P, packed, R, B, radius, st, met, ms);
+    case 32: return launch_resident<32>(m, P, packed, R, B, radius, st, met, ms);
   }
   return GNCA_ERR_UNSUPPORTED;
 }

@@ -234,10 +234,12 @@ static Segment carve_segment(void* base, const gnca_model& m, int B, int H, int 
 // gnca_rollout_fwd with a strided history: x_t of every step t % every == 0 goes to x_hist slot t / every
 // (every == 1: the full [T+1] history of gnca_rollout_fwd).
 // met: the per-frame metrics of gnca_rollout_metrics (stride met->every), by the kernel that runs the steps
+// ms: a stack of models (gnca_rollout_*_models): the steps run on a cluster kernel or not at all, since only those stage
+// their weights per sample.  T = 0 reads no weight and takes the copy path below.
 static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
                        const float* x0_dev, float* xT_dev, float* x_hist_dev, int every, float* stats_hist_dev,
                        float* u_hist_dev, void* workspace_dev, size_t workspace_bytes, int impl, void* stream,
-                       const FrameMetrics* met = nullptr) {
+                       const FrameMetrics* met = nullptr, const ModelStack* ms = nullptr) {
   if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !workspace_dev) return GNCA_ERR_ARG;
   if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
   if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
@@ -254,16 +256,17 @@ static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int 
   const int T = sched->T;
   if (impl != 1 && T > 0) {
     // auto: small samples (the launch-latency-bound regime) go to the cluster-resident kernel
-    const bool want = impl == 2 || impl == 3 || (size_t)H * W <= 16384;
+    const bool want = impl == 2 || impl == 3 || ms || (size_t)H * W <= 16384;
     if (want) {
+      const ModelStack one{0, 0};
       int rc = GNCA_ERR_UNSUPPORTED;
       if (impl != 3)
         rc = run_rep_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, x_hist_dev, stats_hist_dev, u_hist_dev,
-                         nullptr, nullptr, r.ping, st, every, 0, nullptr, met);
+                         nullptr, nullptr, r.ping, st, every, 0, nullptr, met, ms ? *ms : one);
       if (rc == GNCA_ERR_UNSUPPORTED)
         rc = run_resident_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, x_hist_dev, stats_hist_dev,
-                              u_hist_dev, r.ping, r.pong, r.alpha_tmp, st, every, met);
-      if (rc != GNCA_ERR_UNSUPPORTED || impl == 2 || impl == 3) return rc;
+                              u_hist_dev, r.ping, r.pong, r.alpha_tmp, st, every, met, ms ? *ms : one);
+      if (rc != GNCA_ERR_UNSUPPORTED || impl == 2 || impl == 3 || ms) return rc;
     }
   }
 
@@ -469,6 +472,51 @@ int gnca_rollout_metrics(const gnca_model* m, const float* packed_dev, int B, in
   const FrameMetrics met{target_dev, reinterpret_cast<double*>(scratch_dev), sums_dev, counts_dev, eps, every};
   return rollout_fwd(m, packed_dev, B, H, W, sched, x0_dev, xT_dev, nullptr, 1, nullptr, nullptr, workspace_dev,
                      workspace_bytes, impl, stream, &met);
+}
+
+/* ---- a stack of same-architecture models in one launch: sample b runs model b / (B / n_models) ---- */
+// the argument checks of the two stacked entry points that gnca_rollout_record / gnca_rollout_metrics do not make
+static int model_stack(const gnca_model& m, int n_models, int B, int impl, ModelStack* ms) {
+  if (n_models < 1 || B % n_models != 0 || impl < 0 || impl > 3) return GNCA_ERR_ARG;
+  if (impl == 1) return GNCA_ERR_UNSUPPORTED;        // the streaming kernels stage weights per tile, not per sample
+  ms->stride = make_packed(m.C, m.hidden, m.d_model, (m.flags & GNCA_F_GRAPH) != 0).total;
+  ms->per_model = B / n_models;
+  return 0;
+}
+
+int gnca_rollout_record_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                               const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                               float* frames_dev, void* workspace_dev, size_t workspace_bytes, int impl, void* stream) {
+  if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !frames_dev || !workspace_dev) return GNCA_ERR_ARG;
+  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0 || every <= 0) return GNCA_ERR_ARG;
+  ModelStack ms;
+  int rc = model_stack(*m, n_models, B, impl, &ms);
+  if (rc) return rc;
+  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
+  return rollout_fwd(m, packed_dev, B, H, W, sched, x0_dev, xT_dev, frames_dev, every, nullptr, nullptr, workspace_dev,
+                     workspace_bytes, impl, stream, nullptr, &ms);
+}
+
+int gnca_rollout_metrics_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                                const float* target_dev, float eps, double* sums_dev, int32_t* counts_dev,
+                                void* scratch_dev, size_t scratch_bytes, void* workspace_dev, size_t workspace_bytes,
+                                int impl, void* stream) {
+  if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !target_dev || !sums_dev || !counts_dev || !scratch_dev ||
+      !workspace_dev)
+    return GNCA_ERR_ARG;
+  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0 || every <= 0 || m->C < 4) return GNCA_ERR_ARG;
+  if (!(eps >= 0.f)) return GNCA_ERR_ARG;
+  ModelStack ms;
+  int rc = model_stack(*m, n_models, B, impl, &ms);
+  if (rc) return rc;
+  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
+  if (gnca_metrics_scratch_bytes(m, B, H, W, sched->T, every) > scratch_bytes) return GNCA_ERR_WORKSPACE;
+  const FrameMetrics met{target_dev, reinterpret_cast<double*>(scratch_dev), sums_dev, counts_dev, eps, every};
+  return rollout_fwd(m, packed_dev, B, H, W, sched, x0_dev, xT_dev, nullptr, 1, nullptr, nullptr, workspace_dev,
+                     workspace_bytes, impl, stream, &met, &ms);
 }
 
 int gnca_rollout_bwd_frames(const gnca_model* m, const float* packed_dev, int B, int H, int W,

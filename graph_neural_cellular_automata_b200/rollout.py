@@ -579,6 +579,45 @@ def rollout_bwd_raw(desc, packed, hist, sched: Schedule, gT: torch.Tensor, *, gf
     return g0, gflat
 
 
+def _model_stack(models, x0: torch.Tensor, what: str, impl: str):
+    """(desc, models as a list, M) of a list of same-architecture models: the model-stacked calls of
+    record_rollout / monitor_rollout.  ValueError, before any launch, for an empty list, models that differ in their
+    descriptor, graph offsets or neighbour count, or device, models on another device than x0, a batch that is not a
+    multiple of M, and impl='streaming' (the streaming kernels stage weights per tile, not per sample)."""
+    models = list(models)
+    if not models:
+        raise ValueError(f"{what}: the list of models is empty")
+    if impl == "streaming":
+        raise ValueError(f"{what}: a list of models runs on the cluster kernels only; impl='streaming' cannot take it")
+    desc = models[0].model_desc()
+    dev = next(models[0].parameters()).device
+    g0 = getattr(models[0], "graph", None) if getattr(models[0], "_is_graph", False) else None
+    for i, m in enumerate(models[1:], 1):
+        d = m.model_desc()
+        for name, _ in desc._fields_:
+            if getattr(d, name) != getattr(desc, name):
+                raise ValueError(f"{what}: model {i} differs from model 0 in {name} ({getattr(d, name)} vs "
+                                 f"{getattr(desc, name)}); a stack shares one architecture")
+        g = getattr(m, "graph", None) if getattr(m, "_is_graph", False) else None
+        if g0 is not None and (list(g.offsets) != list(g0.offsets) or g.num_neighbors != g0.num_neighbors):
+            raise ValueError(f"{what}: model {i} differs from model 0 in graph.offsets or num_neighbors; a stack "
+                             "shares one schedule")
+        if next(m.parameters()).device != dev:
+            raise ValueError(f"{what}: model {i} is on {next(m.parameters()).device}, model 0 on {dev}")
+    if dev != x0.device:
+        raise ValueError(f"{what}: the models are on {dev}, x0 on {x0.device}")
+    M = len(models)
+    if x0.dim() != 4 or x0.shape[0] % M != 0:
+        raise ValueError(f"{what}: x0 must be [M*B, C, H, W] with the batch a multiple of the {M} models, got "
+                         f"{list(x0.shape)}")
+    return desc, models, M
+
+
+def _stack_packed(models) -> torch.Tensor:
+    """[M, packed_total]: the cached packed_weights() of every model, one row each"""
+    return torch.stack([m.packed_weights() for m in models])
+
+
 class _RolloutFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x0, cfg, *params):
@@ -829,10 +868,27 @@ def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, a
     `checkpoint=True`.  ValueError names the smallest budget that works when nothing fits.  Zero-padded graph shift
     models keep the dense history when it fits and otherwise take the streaming checkpoints, as in
     rollout(..., bptt_budget=N).  `impl="resident"` / `"streaming"` restrict the choice to that backward.  Frames that
-    are checkpoints make the backward raise when edited in place.  Without grad the call is the detached recording."""
+    are checkpoints make the backward raise when edited in place.  Without grad the call is the detached recording.
+
+    `model` may be a list of M models of one architecture (same `model_desc()`, graph offsets and neighbour count, one
+    device), e.g. the saved checkpoints of a training run: one launch runs them side by side (gnca_rollout_record_models),
+    each sample's cluster with its own model's weights.  x0 is [M*B, C, H, W], model-major, and the outputs keep their
+    fields with the sample axis M*B long: model i's frames are `states[:, i*B:(i+1)*B]`, its final states
+    `x_T[i*B:(i+1)*B]`.  Build the schedule with `make_schedule(models[0], M*B, ...)`: every model then sees the same
+    offsets, fire draws and damage, which is the controlled experiment a checkpoint comparison wants.  Inference only, on
+    the cluster kernels: `differentiable`, `attention`, `checkpoint`, `bptt_budget` and impl='streaming' raise
+    ValueError, and a shape neither cluster kernel takes raises the library's RuntimeError."""
     every = int(every)
     if every < 1:
         raise ValueError(f"record_rollout: every must be >= 1, got {every}")
+    stack = isinstance(model, (list, tuple))
+    if stack:
+        for name, on in (("differentiable=True", differentiable), ("attention=True", attention),
+                         ("checkpoint=True", checkpoint), ("bptt_budget", bptt_budget is not None)):
+            if on:
+                raise ValueError(f"record_rollout: {name} does not take a list of models (the stacked call is "
+                                 "inference only)")
+        desc, models, M = _model_stack(model, x0, "record_rollout", impl)
     if bptt_budget is not None:
         if checkpoint:
             raise ValueError("record_rollout: bptt_budget chooses the history itself; it cannot be combined with "
@@ -851,7 +907,8 @@ def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, a
         raise ValueError("record_rollout: attention maps need a graph model (NeuralCAGraph)")
     if not x0.is_cuda:
         raise RuntimeError(f"record_rollout: x0 is on {x0.device}; CUDA (sm_100a) only, no CPU fallback")
-    desc = model.model_desc()
+    if not stack:
+        desc = model.model_desc()
     if differentiable:
         ps = model.canonical_params()
         if torch.is_grad_enabled() and (x0.requires_grad or any(p.requires_grad for p in ps)):
@@ -885,6 +942,12 @@ def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, a
     attn = torch.empty(FA, B, H, W, dtype=torch.float32, device=x0.device) if attention else None
     ws = GF._WS.get(x0.device, lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, T))
     cs = schedule.c_struct()
+    if stack:
+        _lib.check(lib.gnca_rollout_record_models(C.byref(desc), GF._ptr(_stack_packed(models)), M, B, H, W,
+                                                  C.byref(cs), GF._ptr(x0), GF._ptr(xT), every, GF._ptr(frames),
+                                                  GF._ptr(ws), ws.numel(), IMPL[impl], GF._stream()),
+                   "gnca_rollout_record_models")
+        return Trajectory(t=list(range(0, T + 1, every)), states=frames, attention=None, x_T=xT)
     _lib.check(lib.gnca_rollout_record(C.byref(desc), GF._ptr(model.packed_weights()), B, H, W, C.byref(cs),
                                        GF._ptr(x0), GF._ptr(xT), every, GF._ptr(frames), GF._ptr(attn), GF._ptr(ws),
                                        ws.numel(), IMPL[impl], GF._stream()), "gnca_rollout_record")
@@ -910,7 +973,14 @@ def monitor_rollout(model, x0: torch.Tensor, schedule: Schedule, target: torch.T
     premultiplied RGBA on x0's device) where the kernel holds it.  Memory is F*B*24 bytes of results plus at most
     F*B*256 bytes of per-CTA partials, instead of the F*B*C*H*W*4 bytes of `record_rollout` frames.  Inference only: the outputs are
     detached and no BPTT buffer is allocated, whatever the grad mode.  PSNR is 10*log10(1 / mse) of the clipped RGB
-    from the kernel's sum; a frame equal to the target gives +inf, as utils.metrics.psnr_rgb does."""
+    from the kernel's sum; a frame equal to the target gives +inf, as utils.metrics.psnr_rgb does.
+
+    `model` may be a list of M models of one architecture, as in `record_rollout`: one launch
+    (gnca_rollout_metrics_models), x0 [M*B, C, H, W] model-major, every [F, M*B] curve and x_T with the sample axis M*B
+    long, model i's curves at `[:, i*B:(i+1)*B]`.  Build the schedule with `make_schedule(models[0], M*B, ...)` so that
+    every model sees the same offsets, fire draws and damage.  impl='streaming' raises ValueError; a shape neither
+    cluster kernel takes raises the library's RuntimeError.  Picking the best epoch of a run by pixel-perfection after
+    damage is one such call over its checkpoints."""
     every = int(every)
     if every < 1:
         raise ValueError(f"monitor_rollout: every must be >= 1, got {every}")
@@ -919,7 +989,11 @@ def monitor_rollout(model, x0: torch.Tensor, schedule: Schedule, target: torch.T
         raise ValueError(f"monitor_rollout: eps must be >= 0, got {eps}")
     if impl not in IMPL:
         raise ValueError(f"monitor_rollout: impl must be one of {sorted(IMPL)}, got {impl!r}")
-    desc = model.model_desc()
+    stack = isinstance(model, (list, tuple))
+    if stack:
+        desc, models, M = _model_stack(model, x0, "monitor_rollout", impl)
+    else:
+        desc = model.model_desc()
     if x0.dim() != 4:
         raise ValueError(f"monitor_rollout: x0 must be [B, C, H, W], got {list(x0.shape)}")
     B, Cc, H, W = x0.shape
@@ -944,10 +1018,17 @@ def monitor_rollout(model, x0: torch.Tensor, schedule: Schedule, target: torch.T
                           device=x0.device)
     ws = GF._WS.get(x0.device, lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, T))
     cs = schedule.c_struct()
-    _lib.check(lib.gnca_rollout_metrics(C.byref(desc), GF._ptr(model.packed_weights()), B, H, W, C.byref(cs),
-                                        GF._ptr(x0), GF._ptr(xT), every, GF._ptr(target), eps, GF._ptr(sums),
-                                        GF._ptr(counts), GF._ptr(scratch), scratch.numel(), GF._ptr(ws), ws.numel(),
-                                        IMPL[impl], GF._stream()), "gnca_rollout_metrics")
+    if stack:
+        _lib.check(lib.gnca_rollout_metrics_models(C.byref(desc), GF._ptr(_stack_packed(models)), M, B, H, W,
+                                                   C.byref(cs), GF._ptr(x0), GF._ptr(xT), every, GF._ptr(target), eps,
+                                                   GF._ptr(sums), GF._ptr(counts), GF._ptr(scratch), scratch.numel(),
+                                                   GF._ptr(ws), ws.numel(), IMPL[impl], GF._stream()),
+                   "gnca_rollout_metrics_models")
+    else:
+        _lib.check(lib.gnca_rollout_metrics(C.byref(desc), GF._ptr(model.packed_weights()), B, H, W, C.byref(cs),
+                                            GF._ptr(x0), GF._ptr(xT), every, GF._ptr(target), eps, GF._ptr(sums),
+                                            GF._ptr(counts), GF._ptr(scratch), scratch.numel(), GF._ptr(ws),
+                                            ws.numel(), IMPL[impl], GF._stream()), "gnca_rollout_metrics")
     HW = H * W
     return Monitor(t=list(range(0, T + 1, every)), loss=(sums[..., 0] / (4 * HW)).float(),
                    psnr=(10.0 * torch.log10(1.0 / (sums[..., 1] / (3 * HW)))).float(),

@@ -242,6 +242,30 @@ int gnca_rollout_metrics(const gnca_model* m, const float* packed_dev, int B, in
                          void* scratch_dev, size_t scratch_bytes, void* workspace_dev, size_t workspace_bytes,
                          int impl, void* stream);
 
+/*
+ * Many models in one rollout: gnca_rollout_record / gnca_rollout_metrics for a stack of n_models models that share the
+ * descriptor `m`, the schedule and (metrics) the target -- e.g. the saved checkpoints of one training run.
+ * packed_dev is [n_models][packed_total] (gnca_param_layout().packed_total floats per model, each buffer from
+ * gnca_pack_weights).  B counts all samples and must be a multiple of n_models: sample b runs model b / (B / n_models),
+ * so x0, frames, x_T, sums and counts keep their single-model shapes with the model-major B.  Each sample's cluster stages
+ * its own model's weights, so the M * B samples fill the GPU the way one large batch does.
+ *   - impl: 0 (auto) = the replicated-state kernel where it runs, else the banded one; 2 / 3 as in gnca_rollout_fwd.
+ *     impl 1 (streaming) is GNCA_ERR_UNSUPPORTED, and so is a shape or model neither cluster kernel takes: there is no
+ *     fallback to the streaming kernels.  T == 0 launches no step.
+ *   - No attention maps and no BPTT.  With n_models == 1 the results are bit-identical to the single-model call on the
+ *     same impl; model i's block equals the single-model call with model i on the same B, schedule and impl.
+ * Argument errors return before any launch: those of gnca_rollout_record / gnca_rollout_metrics, n_models < 1,
+ * B % n_models != 0 or impl outside [0, 3] are GNCA_ERR_ARG.  Scratch and workspace sizes are those of the total B.
+ */
+int gnca_rollout_record_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                               const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                               float* frames_dev, void* workspace_dev, size_t workspace_bytes, int impl, void* stream);
+int gnca_rollout_metrics_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                                const float* target_dev, float eps, double* sums_dev, int32_t* counts_dev,
+                                void* scratch_dev, size_t scratch_bytes, void* workspace_dev, size_t workspace_bytes,
+                                int impl, void* stream);
+
 /* BPTT: given gT = dL/dx_T and the x_hist of the forward, produce g0 = dL/dx_0 and ACCUMULATE gparams. */
 int gnca_rollout_bwd(const gnca_model* m, const float* packed_dev, int B, int H, int W,
                      const gnca_schedule* sched, const float* x_hist_dev, const float* stats_hist_dev,
