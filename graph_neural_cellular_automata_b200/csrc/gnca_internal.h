@@ -15,6 +15,10 @@ struct FwdWorkspace {
   size_t bytes;
 };
 
+// Largest dynamic shared memory a launch of `kfn` may ask for on the current device: the opt-in limit per block less the
+// kernel's static shared memory, at most 226 KB.  Cached per (kernel, device); 0 when the attributes cannot be read.
+size_t dynamic_smem_cap(const void* kfn);
+
 FwdWorkspace carve_fwd_workspace(void* base, const gnca_model& m, int B, int H, int W);
 void fill_step_args(StepArgs& a, const gnca_model& m, int B, int H, int W);
 int set_host_offsets(StepArgs& a, const int32_t* offsets_host, int k);

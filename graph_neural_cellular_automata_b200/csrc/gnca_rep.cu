@@ -24,6 +24,9 @@
 #include <cooperative_groups.h>
 #include <cstdio>
 #include <cstdlib>
+#include <map>
+#include <mutex>
+#include <utility>
 #include <type_traits>
 #include "gnca_common.cuh"
 #include "gnca_internal.h"
@@ -967,6 +970,28 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
 }
 
 // ------------------------------------------------------------------------------------------------
+size_t dynamic_smem_cap(const void* kfn) {
+  static std::mutex mu;
+  static std::map<std::pair<const void*, int>, size_t> cache;
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) { cudaGetLastError(); return 0; }
+  std::lock_guard<std::mutex> lock(mu);
+  const auto key = std::make_pair(kfn, dev);
+  const auto it = cache.find(key);
+  if (it != cache.end()) return it->second;
+  cudaFuncAttributes fa{};
+  int optin = 0;
+  if (cudaFuncGetAttributes(&fa, kfn) != cudaSuccess ||
+      cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess) {
+    cudaGetLastError();
+    return 0;
+  }
+  const size_t limit = (size_t)optin > fa.sharedSizeBytes ? (size_t)optin - fa.sharedSizeBytes : 0;
+  const size_t cap = limit < (size_t)226 * 1024 ? limit : (size_t)226 * 1024;
+  cache.emplace(key, cap);
+  return cap;
+}
+
 static size_t rep_smem_bytes(int C, int HW, int ucap, int listcap) {
   const int HWp = 4 * (((HW >> 2) + 31) & ~31) + 16;
   size_t f = (size_t)3 * C * 128 + 128 + 128 * kW2S + (size_t)HW * C + 2 * (size_t)HWp + (size_t)kPW * 3 * C * 8 +
@@ -1021,6 +1046,9 @@ int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B
 
   const char* env_nc = getenv("GNCA_RESIDENT_NC");
   const bool debug = getenv("GNCA_DEBUG") != nullptr;
+  // the dynamic carve shares the opt-in limit with the kernel's static shared memory (6 KB, 15 KB for the ZP
+  // instantiation): near 2048 cells the dynamic cap of 226 KB alone would ask for more than a block may have
+  const size_t cap = dynamic_smem_cap(kfn);
   const int cands[4] = {8, 4, 2, 1};
   int pick = -1, pick_ucap = 0, pick_list = 0, pick_ncl = 0;
   size_t pick_smem = 0;
@@ -1031,8 +1059,8 @@ int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B
       const int share = (HW + NC - 1) / NC + 1;
       int ucap = share < 384 ? share : 384;
       size_t smem = rep_smem_bytes(C, HW, ucap, share);
-      while (smem > 226 * 1024 && ucap > 128) { ucap -= 64; smem = rep_smem_bytes(C, HW, ucap, share); }
-      if (smem > 226 * 1024) continue;
+      while (smem > cap && ucap > 128) { ucap -= 64; smem = rep_smem_bytes(C, HW, ucap, share); }
+      if (smem > cap) continue;
       if (ucap < share && !scratch) continue;
       GNCA_CHECK_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       cudaLaunchConfig_t q{};

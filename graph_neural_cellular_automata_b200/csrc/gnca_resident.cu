@@ -136,8 +136,8 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
   int* s_actlist = s_q + MB * kk;                       // [nown] own-cell index of active cells (compacted)
   int* s_slot = s_actlist + nown;                       // [nown] slot in the active list or -1
   unsigned char* s_oy = reinterpret_cast<unsigned char*>(s_slot + nown);   // [nown] own row of an own cell
-  unsigned char* s_ox = s_oy + nown;                                        // [nown] column
-  float* s_fr = reinterpret_cast<float*>(s_ox + ((nown + 15) & ~15));      // [T] fire rate per step
+  unsigned char* s_ox = s_oy + ((nown + 15) & ~15);                         // [nown] column
+  float* s_fr = reinterpret_cast<float*>(s_ox + ((nown + 15) & ~15));      // [T] fire rate per step (16B aligned)
   float* s_gain = s_fr + R.T;                                               // [T] message gain per step
   signed char* s_off = reinterpret_cast<signed char*>(s_gain + R.T);        // [T][k][2] offsets
   __shared__ float s_partsf[8][2];           // (sum u, sum u^2) of every CTA of the cluster, pushed by its owner
@@ -647,7 +647,7 @@ static size_t resident_smem_bytes(int C, int hid, bool graph, int own, int halo,
   f += (size_t)3 * C * MBP + (size_t)C * MBP + MBP + (size_t)C * MBP + (size_t)hid * MBP;
   f += (size_t)C * own * W;
   size_t bytes = f * sizeof(float);
-  bytes += (size_t)MB * (k > 0 ? k : 1) * sizeof(int) + 2 * (size_t)own * W * sizeof(int) + 2 * (size_t)own * W;
+  bytes += (size_t)MB * (k > 0 ? k : 1) * sizeof(int) + 2 * (size_t)own * W * sizeof(int) + 2 * (size_t)((own * W + 15) & ~15);
   bytes += 16 + (size_t)T * 8 + (size_t)T * k * 2;        // schedule: fire rate, gain, offsets
   return bytes + 64;
 }
@@ -671,6 +671,8 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
   const bool stack = S.stride != 0;
   auto kfn = stack ? (met ? k_resident_fwd<C, true, true> : k_resident_fwd<C, false, true>)
                    : (met ? k_resident_fwd<C, true, false> : k_resident_fwd<C, false, false>);
+  // the dynamic carve shares the opt-in limit with the kernel's static shared memory (about 1.1 KB at C = 32)
+  const size_t cap = dynamic_smem_cap((const void*)kfn);
   const int cands[4] = {8, 4, 2, 1};
   int pick = -1, pick_MB = 0, pick_nclusters = 0;
   size_t pick_smem = 0;
@@ -682,9 +684,9 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
       const int own = H / NC;
       int MB = 64;
       size_t smem = resident_smem_bytes(C, m.hidden, graph, own, halo, W, MB, R.s.k, R.T);
-      if (smem > 226 * 1024) { MB = 32; smem = resident_smem_bytes(C, m.hidden, graph, own, halo, W, MB, R.s.k, R.T); }
-      if (smem > 226 * 1024) { MB = 16; smem = resident_smem_bytes(C, m.hidden, graph, own, halo, W, MB, R.s.k, R.T); }   // 40x40x32
-      if (smem > 226 * 1024) continue;
+      if (smem > cap) { MB = 32; smem = resident_smem_bytes(C, m.hidden, graph, own, halo, W, MB, R.s.k, R.T); }
+      if (smem > cap) { MB = 16; smem = resident_smem_bytes(C, m.hidden, graph, own, halo, W, MB, R.s.k, R.T); }   // 40x40x32
+      if (smem > cap) continue;
       GNCA_CHECK_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       cudaLaunchConfig_t q{};
       q.gridDim = dim3(B * NC); q.blockDim = dim3(kRThreads); q.dynamicSmemBytes = smem; q.stream = st;
