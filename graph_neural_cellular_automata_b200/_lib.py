@@ -123,6 +123,15 @@ EXPORTS = {
                                            C.POINTER(GncaSchedule), C.c_void_p, C.c_size_t, C.c_int, C.c_void_p,
                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
                                            C.c_void_p]),
+    "gnca_rollout_workspace_models_bytes": (C.c_size_t, [C.POINTER(GncaModel), C.c_int, C.c_int, C.c_int, C.c_int,
+                                                         C.c_int]),
+    **{name: (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(GncaSchedule),
+                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p])
+       for name in ("gnca_rollout_fwd_bptt_models", "gnca_rollout_fwd_bptt_zp_models")},
+    **{name: (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(GncaSchedule),
+                        C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                        C.c_void_p])
+       for name in ("gnca_rollout_bwd_bptt_models", "gnca_rollout_bwd_bptt_zp_models")},
     "gnca_bptt_ckpt_bytes": (C.c_size_t, [C.POINTER(GncaModel), C.c_int, C.c_int, C.c_int, C.c_int]),
     "gnca_rollout_fwd_bptt_ckpt": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
                                              C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,

@@ -297,9 +297,15 @@ __global__ void k_attn_bwd(StepArgs a, Packed P, int C, int d, const float* __re
   }
 }
 
+// MS: blockIdx.y = model of a stack: B is its sample count, its rows of pw and its gparams row
+template <bool MS>
 __global__ void k_attn_param_reduce(int B, int C, int d, gnca_layout L, const float* __restrict__ pw,
                                     float* __restrict__ gparams) {
   const int n = 2 * d * C + 2 * d + 1;
+  if constexpr (MS) {
+    pw += (size_t)blockIdx.y * B * n;
+    gparams += (size_t)blockIdx.y * L.total;
+  }
   for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += gridDim.x * blockDim.x) {
     float s = 0.f;
     for (int b0 = 0; b0 < B; b0 += 8) {          // 8 loads in flight, added in sample order
@@ -362,8 +368,10 @@ int run_attn_bwd(const gnca_model& m, const Packed& P, const float* packed, cons
   return 0;
 }
 
-int run_attn_param_reduce(const gnca_model& m, int B, const AttnBwdScratch& sc, float* gparams, cudaStream_t st) {
-  k_attn_param_reduce<<<4, 256, 0, st>>>(B, m.C, m.d_model, make_layout(m), sc.pw, gparams);
+int run_attn_param_reduce(const gnca_model& m, int B, const AttnBwdScratch& sc, float* gparams, cudaStream_t st,
+                          int n_models) {
+  const auto kern = n_models > 1 ? k_attn_param_reduce<true> : k_attn_param_reduce<false>;
+  kern<<<dim3(4, n_models), 256, 0, st>>>(B / n_models, m.C, m.d_model, make_layout(m), sc.pw, gparams);
   GNCA_LAUNCH_CHECK();
   return 0;
 }

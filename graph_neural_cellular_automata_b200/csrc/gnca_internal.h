@@ -44,7 +44,9 @@ size_t attn_bwd_scratch_bytes(const gnca_model& m, int B, int H, int nparts);
 AttnBwdScratch carve_attn_bwd(void* base, const gnca_model& m, int B, int H, int nparts);
 int run_attn_bwd(const gnca_model& m, const Packed& P, const float* packed, const StepArgs& a, const float* rowsum,
                  const AttnBwdScratch& sc, int nparts, float* gparams, cudaStream_t st, bool defer_reduce);
-int run_attn_param_reduce(const gnca_model& m, int B, const AttnBwdScratch& sc, float* gparams, cudaStream_t st);
+// n_models > 1: a stack (B / n_models samples per model), model i's sum into gparams + i * layout.total
+int run_attn_param_reduce(const gnca_model& m, int B, const AttnBwdScratch& sc, float* gparams, cudaStream_t st,
+                          int n_models = 1);
 
 size_t graph_workspace_bytes(const gnca_model& m, int B, int H, int W);
 size_t bwd_workspace_bytes(const gnca_model& m, int B, int H, int W);
@@ -100,7 +102,7 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
 // steps of a whole-rollout launch bit for bit.
 // zp (zero-padded graph shift only): with records, also the attention weights and row sums of every message step
 // met: the per-frame metrics of the steps t % met->every == 0 (a whole rollout, t0 = 0)
-// ms: a stack of models, one per block of ms.per_model samples (inference only: no records)
+// ms: a stack of models, one per block of ms.per_model samples, with or without records
 struct ZpRec;
 struct ZpBwd;
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
@@ -113,16 +115,18 @@ int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B
 size_t rep_bptt_bytes(const gnca_model& m, int B, int H, int W, int T);     // 0: configuration not supported
 void rep_bptt_carve(void* base, int B, int H, int W, int T, float** rec, uint32_t** masks, float** stats,
                     float** hgh = nullptr);
-size_t rep_bwd_workspace_bytes(const gnca_model& m, int B, int H, int W);
+// n_models: the weight-gradient partials of a stack (at least one block per model)
+size_t rep_bwd_workspace_bytes(const gnca_model& m, int B, int H, int W, int n_models = 1);
 // a launch configuration of k_rep_bwd exists (zp: of the zero-padded-shift instantiation)
 bool rep_bwd_supported(const gnca_model& m, int B, int H, int W, int k, bool zp = false);
 // zp: the zero-padded graph shift's buffers (records of run_rep_fwd with a ZpRec); its Q/K/scaling gradients are
 // reduced into gparams after the sweep.  gT_frame = false: g_frames' frame at sched.T is not added to gT (a checkpoint
 // segment, where it is the next segment's first frame)
+// ms: a stack of models (no frame gradients): gparams is [n_models][layout.total], model i's gradients in row i
 int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, void* bptt, const float* gT, float* g0, float* gparams, void* workspace,
                 cudaStream_t st, const float* g_frames = nullptr, int every = 1, int t0 = 0, const ZpBwd* zp = nullptr,
-                bool gT_frame = true);
+                bool gT_frame = true, ModelStack ms = ModelStack{0, 0});
 // zero-padded graph shift: the records of rep_bptt_bytes followed by x_t, the softmax weights, the row sums, bm . gm of
 // the active cells and the per-sample Q/K gradients (0: not supported)
 size_t rep_bptt_zp_bytes(const gnca_model& m, int B, int H, int W, int T);

@@ -97,9 +97,14 @@ __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wa
 // are reduced over the cluster in a fixed order (third cluster barrier), then every CTA runs the softmax / pooled Q.K
 // backward of k_attn_bwd and adds its row term `grow` to its band of g_t; rank 0 accumulates the Q/K/scaling
 // gradients of the sample in Z.pw.
-template <int C, bool kFrames, bool ZP>
+// MS (a stack of models, gnca_rollout_bwd_bptt_*_models): sample b reads its weights from packed + (b / S.per_model) *
+// S.stride.  `packed` is rebased once at entry, so every later read (gamma / beta in the step loop, the attention
+// parameters of ZP) goes through the rebased pointer.  A compile-time flag with a trailing parameter, not a RepBwdArgs
+// field: the kernel runs at its register cap, and the instantiations without MS keep their SASS.
+template <int C, bool kFrames, bool ZP, bool MS = false>
 __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, const float* __restrict__ packed,
-                                                   const float* __restrict__ gframes, int every, ZpBwd Z) {
+                                                   const float* __restrict__ gframes, int every, ZpBwd Z,
+                                                   ModelStack S) {
   static_assert(C == 16, "lane mapping: 2 cells x 16 channels per warp row");
   constexpr int C3 = 3 * C, HID = 128, CPL = 32 / C;
   cg::cluster_group cluster = cg::this_cluster();
@@ -165,6 +170,7 @@ __global__ void __launch_bounds__(kQT, 1) k_rep_bwd(RepBwdArgs R, Packed P, cons
   if (threadIdx.x < 16) s_dbg[threadIdx.x] = 0;
   long long t_prev = clock64();
 
+  if constexpr (MS) packed += (size_t)(b / S.per_model) * S.stride;
 #pragma unroll 1
   for (int i = tid; i < C3 * HID; i += kQT) {
     const int kk = i / HID, jp = i - kk * HID;
@@ -893,6 +899,9 @@ struct WgradArgs {
   float* wpart;               // [gridDim.x][wtotal]
   int64_t wtotal;
   gnca_layout L;
+  // a stack of models: samples [i*per, (i+1)*per) run model i, and blocks [i*nbm, (i+1)*nbm) sum its records only.
+  // (read by the MS instantiation only)
+  int per, nbm;
 };
 
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
@@ -904,7 +913,7 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 
 // dW1 += gh (x) y, db1 += gh, dW2 += gd (x) h, dWm += gm (x) xs, dbm += gm * as over all records: operands are read
 // record-major straight from the cp.async buffers (a thread's 4 hidden units are one float4 of the permuted h / gh rows).
-template <int C>
+template <int C, bool MS>
 __global__ void __launch_bounds__(kWT, 2) k_rep_wgrad(WgradArgs A) {
   constexpr int C3 = 3 * C, HID = 128, NB = kWNB;
   constexpr int TK = 6, KG = C3 / TK;          // dW1 tile: 4 hidden units (one permuted float4) x 6 consecutive inputs
@@ -925,13 +934,24 @@ __global__ void __launch_bounds__(kWT, 2) k_rep_wgrad(WgradArgs A) {
   const int cp2 = tid % (C / 2), jg2 = tid / (C / 2);   // dW2: channels 2 cp2, 2 cp2 + 1, units jg2 + 32 jj
   const int mc = tid / C, mci = tid % C;                // dWm[mc][mci]
 
-  const int nseg = A.T * A.B;
-  for (int seg0 = blockIdx.x; seg0 < nseg; seg0 += gridDim.x * kWMaxSeg) {
+  // MS: my model's segments (t, b), b in [model*per, (model+1)*per), in the local order ls = t*per + (b - model*per); I
+  // take ls = lb, lb + nbm, ...  With one model that is the partition of the plain instantiation (ls = t*B + b), which
+  // keeps the single-model code without the mapping
+  const unsigned nbm = MS ? (unsigned)A.nbm : gridDim.x;
+  const int model = MS ? (int)blockIdx.x / A.nbm : 0;
+  const int lb = MS ? (int)blockIdx.x - model * A.nbm : blockIdx.x;
+  const int nseg = A.T * (MS ? A.per : A.B);
+  auto gseg = [&](int ls) {
+    if constexpr (MS) { const int t = ls / A.per; return t * A.B + model * A.per + (ls - t * A.per); }
+    return ls;
+  };
+  for (int seg0 = lb; seg0 < nseg; seg0 += nbm * kWMaxSeg) {
     __syncthreads();
     for (int si = tid; si < kWMaxSeg; si += kWT) {        // record counts of my segments (popcount of the active bitmap)
-      const int seg = seg0 + si * gridDim.x;
+      const int ls = seg0 + si * nbm;
       int cnt = 0;
-      if (seg < nseg) {
+      if (ls < nseg) {
+        const int seg = gseg(ls);
         const int t = seg / A.B, b = seg - t * A.B;
         if (!(A.steps && A.steps[b] - A.t0 <= t)) {
           const uint32_t* mk = A.masks + ((size_t)seg * 3 + 1) * kMaskWords;
@@ -945,7 +965,7 @@ __global__ void __launch_bounds__(kWT, 2) k_rep_wgrad(WgradArgs A) {
     auto skip_empty = [&](int& s_, int& b_) { while (s_ < kWMaxSeg && b_ >= s_cnt[s_]) { ++s_; b_ = 0; } };
     auto issue = [&](int s_, int b_, int buf) {
       if (s_ < kWMaxSeg) {
-        const int seg = seg0 + s_ * gridDim.x;
+        const int seg = gseg(seg0 + s_ * nbm);
         const int nb = min(NB, s_cnt[s_] - b_);
         const float* src = A.rec + ((size_t)seg * A.HW + b_) * kRecStride;
         const float* srch = A.hgh + ((size_t)seg * A.HW + b_) * kHghStride;
@@ -1019,11 +1039,18 @@ __global__ void __launch_bounds__(kWT, 2) k_rep_wgrad(WgradArgs A) {
   }
 }
 
-// gparams[i] += sum over blocks of wpart[blk][i] (fixed order); + dgamma / dbeta partials of the resident kernel
+// gparams[i] += sum over blocks of wpart[blk][i] (fixed order); + dgamma / dbeta partials of the resident kernel.
+// MS: blockIdx.y = model of a stack: its nblk partials, its naff affine partials (its samples' CTAs) and its gparams row
+template <bool MS>
 __global__ void k_rep_wreduce(int nblk, int64_t total, const float* __restrict__ wpart, int naff, int C,
                               const float* __restrict__ affpart, gnca_layout L, float* __restrict__ gparams) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
+  if constexpr (MS) {
+    wpart += (size_t)blockIdx.y * nblk * total;
+    affpart += (size_t)blockIdx.y * naff * 2 * C;
+    gparams += (size_t)blockIdx.y * total;
+  }
   float acc = 0.f;
   for (int bl = 0; bl < nblk; ++bl) acc += wpart[(size_t)bl * total + i];
   if (i >= L.gamma && i < L.gamma + C) for (int r = 0; r < naff; ++r) acc += affpart[(size_t)r * 2 * C + (i - L.gamma)];
@@ -1063,11 +1090,18 @@ void rep_bptt_carve(void* base, int B, int H, int W, int T, float** rec, uint32_
   *stats = reinterpret_cast<float*>(p + o);
 }
 
-size_t rep_bwd_workspace_bytes(const gnca_model& m, int B, int H, int W) {
+// a stack of n_models runs wgrad_blocks_per_model blocks per model: at most kMaxWgradBlocks in all, and at least one each
+static int wgrad_blocks_per_model(int T, int per, int n_models) {
+  const int seg = T * per, cap = kMaxWgradBlocks / n_models;
+  const int n = seg < cap ? seg : cap;
+  return n < 1 ? 1 : n;
+}
+
+size_t rep_bwd_workspace_bytes(const gnca_model& m, int B, int H, int W, int n_models) {
   const size_t HW = (size_t)H * W, C = m.C;
   size_t f = (size_t)B * HW * C /*GZ*/ + (size_t)B * HW * 64 /*RG*/ + (size_t)B * 8 * 2 * C;
   const gnca_layout L = make_layout(m);
-  f += (size_t)kMaxWgradBlocks * (size_t)L.total;
+  f += (size_t)(n_models > kMaxWgradBlocks ? n_models : kMaxWgradBlocks) * (size_t)L.total;
   return f * sizeof(float) + 1024;
 }
 
@@ -1152,9 +1186,11 @@ void rep_bptt_zp_carve(void* base, const gnca_model& m, int B, int H, int W, int
 
 int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, void* bptt, const float* gT, float* g0, float* gparams, void* workspace,
-                cudaStream_t st, const float* g_frames, int every, int t0, const ZpBwd* zp, bool gT_frame) {
+                cudaStream_t st, const float* g_frames, int every, int t0, const ZpBwd* zp, bool gT_frame,
+                ModelStack ms) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (rep_bptt_bytes(m, B, H, W, sched.T) == 0) return GNCA_ERR_UNSUPPORTED;
+  if (ms.stride && g_frames) return GNCA_ERR_UNSUPPORTED;      // a stack has no frame gradients
   const int k = graph ? sched.k : 0;
   if (graph && k > 0 && !(m.flags & GNCA_F_TORUS) && !zp) return GNCA_ERR_UNSUPPORTED;
   if (k > 16) return GNCA_ERR_UNSUPPORTED;
@@ -1192,7 +1228,9 @@ int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B
   if (getenv("GNCA_DEBUG")) fprintf(stderr, "[gnca] resident bwd: B=%d NC=%d smem=%zu\n", B, pick, pick_smem);
   // the frame-gradient instantiation has the register budget and shared memory of the plain one (same launch bounds,
   // same carve), so the configuration picked for the plain kernel holds for it
-  const auto kern = zpk ? (g_frames ? k_rep_bwd<16, true, true> : k_rep_bwd<16, false, true>)
+  // so does the stacked one (MS)
+  const auto kern = ms.stride ? (zpk ? k_rep_bwd<16, false, true, true> : k_rep_bwd<16, false, false, true>)
+                  : zpk ? (g_frames ? k_rep_bwd<16, true, true> : k_rep_bwd<16, false, true>)
                         : (g_frames ? k_rep_bwd<16, true, false> : k_rep_bwd<16, false, false>);
   const ZpBwd Z = zpk ? *zp : ZpBwd{};
   const int np = 2 * m.d_model * C + 2 * m.d_model + 1;
@@ -1215,7 +1253,7 @@ int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B
     R.dbg_cta = atoi(getenv("GNCA_PHASE_TIMING"));
   }
   prof_begin(PROF_RESIDENT_BWD, st);
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, R, P, packed, g_frames, every, Z);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, R, P, packed, g_frames, every, Z, ms);
   prof_end(PROF_RESIDENT_BWD, st);
   if (e != cudaSuccess) return (int)e;
   GNCA_LAUNCH_CHECK();
@@ -1234,19 +1272,24 @@ int run_rep_bwd(const gnca_model& m, const Packed& P, const float* packed, int B
   WgradArgs A{};
   A.rec = rec; A.hgh = hgh; A.masks = masks; A.steps = sched.steps; A.T = sched.T; A.t0 = t0; A.B = B; A.HW = HW; A.NW = (HW + 31) >> 5;
   A.flags = m.flags; A.wpart = wpart; A.wtotal = L.total; A.L = L;
-  int nseg = sched.T * B;
-  int nblk = nseg < kMaxWgradBlocks ? nseg : kMaxWgradBlocks;
-  if (nblk < 1) nblk = 1;
+  // a stack: one group of blocks per model, each group summing that model's segments only (one model: the whole batch)
+  const int n_models = ms.stride ? B / ms.per_model : 1;
+  A.per = ms.stride ? ms.per_model : B;
+  A.nbm = wgrad_blocks_per_model(sched.T, A.per, n_models);
+  const int nblk = n_models * A.nbm;
   GNCA_CHECK_CUDA(cudaMemsetAsync(wpart, 0, (size_t)nblk * L.total * sizeof(float), st));
   const size_t wsmem = 2 * (size_t)kWNB * (kRecStride + kHghStride) * sizeof(float);
-  GNCA_CHECK_CUDA(cudaFuncSetAttribute(k_rep_wgrad<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
+  const auto wkern = ms.stride ? k_rep_wgrad<16, true> : k_rep_wgrad<16, false>;
+  GNCA_CHECK_CUDA(cudaFuncSetAttribute(wkern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
   prof_begin(PROF_BWD_MLP, st);
-  k_rep_wgrad<16><<<nblk, kWT, wsmem, st>>>(A);
+  wkern<<<nblk, kWT, wsmem, st>>>(A);
   prof_end(PROF_BWD_MLP, st);
   GNCA_LAUNCH_CHECK();
-  k_rep_wreduce<<<(int)((L.total + 255) / 256), 256, 0, st>>>(nblk, L.total, wpart, B * pick, C, affpart, L, gparams);
+  const auto rkern = ms.stride ? k_rep_wreduce<true> : k_rep_wreduce<false>;
+  rkern<<<dim3((unsigned)((L.total + 255) / 256), n_models), 256, 0, st>>>(A.nbm, L.total, wpart, A.per * pick, C,
+                                                                          affpart, L, gparams);
   GNCA_LAUNCH_CHECK();
-  if (zpk) return run_attn_param_reduce(m, B, AttnBwdScratch{nullptr, nullptr, Z.pw}, gparams, st);
+  if (zpk) return run_attn_param_reduce(m, B, AttnBwdScratch{nullptr, nullptr, Z.pw}, gparams, st, n_models);
   return 0;
 }
 

@@ -759,6 +759,110 @@ int gnca_rollout_bwd_bptt_zp(const gnca_model* m, const float* packed_dev, int B
                      g_frames_dev, every, 0, &zb);
 }
 
+/* ---- resident BPTT of a stack of same-architecture models: sample b runs model b / (B / n_models) ---- */
+size_t gnca_rollout_workspace_models_bytes(const gnca_model* m, int n_models, int B, int H, int W, int T) {
+  if (!m || n_models < 1 || B <= 0 || H <= 0 || W <= 0) return 0;
+  const size_t a = gnca_rollout_workspace_bytes(m, B, H, W, T);
+  const size_t b = (m->C == 16) ? rep_bwd_workspace_bytes(*m, B, H, W, n_models) : 0;
+  return a > b ? a : b;
+}
+
+// the checks of the four stacked BPTT entry points after their pointer checks, all before any launch.  zp: the
+// zero-padded graph shift's buffer (gnca_bptt_zp_bytes), else the records of gnca_bptt_bytes
+static int bptt_models_check(const gnca_model* m, int n_models, int B, int H, int W, const gnca_schedule* sched,
+                             bool zp, size_t bptt_bytes, size_t workspace_bytes, ModelStack* ms) {
+  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
+  const int rc = model_stack(*m, n_models, B, 0, ms);
+  if (rc) return rc;
+  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  const bool graph = (m->flags & GNCA_F_GRAPH) != 0;
+  if (sched->T > 0 && (!sched->fire_rate || (graph && !sched->message_gain))) return GNCA_ERR_ARG;
+  if (graph && sched->k > 0 && !sched->offsets) return GNCA_ERR_ARG;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
+  const size_t need = zp ? gnca_bptt_zp_bytes(m, B, H, W, sched->T) : gnca_bptt_bytes(m, B, H, W, sched->T);
+  if (need == 0) return GNCA_ERR_UNSUPPORTED;
+  if (need > bptt_bytes) return GNCA_ERR_WORKSPACE;
+  if (gnca_rollout_workspace_models_bytes(m, n_models, B, H, W, sched->T) > workspace_bytes) return GNCA_ERR_WORKSPACE;
+  // no streaming fallback: the records are only written when the resident backward takes this batch and shape
+  if (!rep_bwd_supported(*m, B, H, W, graph ? sched->k : 0, zp)) return GNCA_ERR_UNSUPPORTED;
+  return 0;
+}
+
+static int fwd_bptt_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                           const gnca_schedule* sched, const float* x0_dev, float* xT_dev, void* bptt_dev,
+                           size_t bptt_bytes, void* workspace_dev, size_t workspace_bytes, void* stream, bool zp) {
+  if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !bptt_dev || !workspace_dev) return GNCA_ERR_ARG;
+  ModelStack ms;
+  const int rc = bptt_models_check(m, n_models, B, H, W, sched, zp, bptt_bytes, workspace_bytes, &ms);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int T = sched->T;
+  if (T == 0) {
+    GNCA_CHECK_CUDA(cudaMemcpyAsync(xT_dev, x0_dev, (size_t)B * m->C * H * W * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    return 0;
+  }
+  RolloutWorkspace r = carve_rollout(workspace_dev, *m, B, H, W);
+  const Packed P = make_packed(m->C, m->hidden, m->d_model, (m->flags & GNCA_F_GRAPH) != 0);
+  float *rec, *stats, *xs = nullptr;
+  uint32_t* masks;
+  ZpRec zr;
+  rep_bptt_carve(bptt_dev, B, H, W, T, &rec, &masks, &stats);
+  if (zp) rep_bptt_zp_carve(bptt_dev, *m, B, H, W, T, &xs, &zr, nullptr);
+  return run_rep_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, xs, stats, nullptr, rec, masks, r.ping, st, 1,
+                     0, zp ? &zr : nullptr, nullptr, ms);
+}
+
+static int bwd_bptt_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                           const gnca_schedule* sched, void* bptt_dev, size_t bptt_bytes, const float* gT_dev,
+                           float* g0_dev, float* gparams_dev, void* workspace_dev, size_t workspace_bytes, void* stream,
+                           bool zp) {
+  if (!m || !packed_dev || !sched || !bptt_dev || !gT_dev || !g0_dev || !gparams_dev || !workspace_dev)
+    return GNCA_ERR_ARG;
+  ModelStack ms;
+  const int rc = bptt_models_check(m, n_models, B, H, W, sched, zp, bptt_bytes, workspace_bytes, &ms);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (sched->T == 0) {
+    GNCA_CHECK_CUDA(cudaMemcpyAsync(g0_dev, gT_dev, (size_t)B * m->C * H * W * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    return 0;
+  }
+  const Packed P = make_packed(m->C, m->hidden, m->d_model, (m->flags & GNCA_F_GRAPH) != 0);
+  ZpBwd zb;
+  if (zp) rep_bptt_zp_carve(bptt_dev, *m, B, H, W, sched->T, nullptr, nullptr, &zb);
+  return run_rep_bwd(*m, P, packed_dev, B, H, W, *sched, bptt_dev, gT_dev, g0_dev, gparams_dev, workspace_dev, st,
+                     nullptr, 1, 0, zp ? &zb : nullptr, true, ms);
+}
+
+int gnca_rollout_fwd_bptt_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                 const gnca_schedule* sched, const float* x0_dev, float* xT_dev, void* bptt_dev,
+                                 size_t bptt_bytes, void* workspace_dev, size_t workspace_bytes, void* stream) {
+  return fwd_bptt_models(m, packed_dev, n_models, B, H, W, sched, x0_dev, xT_dev, bptt_dev, bptt_bytes, workspace_dev,
+                         workspace_bytes, stream, false);
+}
+
+int gnca_rollout_bwd_bptt_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                 const gnca_schedule* sched, void* bptt_dev, size_t bptt_bytes, const float* gT_dev,
+                                 float* g0_dev, float* gparams_dev, void* workspace_dev, size_t workspace_bytes,
+                                 void* stream) {
+  return bwd_bptt_models(m, packed_dev, n_models, B, H, W, sched, bptt_dev, bptt_bytes, gT_dev, g0_dev, gparams_dev,
+                         workspace_dev, workspace_bytes, stream, false);
+}
+
+int gnca_rollout_fwd_bptt_zp_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                    const gnca_schedule* sched, const float* x0_dev, float* xT_dev, void* bptt_dev,
+                                    size_t bptt_bytes, void* workspace_dev, size_t workspace_bytes, void* stream) {
+  return fwd_bptt_models(m, packed_dev, n_models, B, H, W, sched, x0_dev, xT_dev, bptt_dev, bptt_bytes, workspace_dev,
+                         workspace_bytes, stream, true);
+}
+
+int gnca_rollout_bwd_bptt_zp_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                    const gnca_schedule* sched, void* bptt_dev, size_t bptt_bytes, const float* gT_dev,
+                                    float* g0_dev, float* gparams_dev, void* workspace_dev, size_t workspace_bytes,
+                                    void* stream) {
+  return bwd_bptt_models(m, packed_dev, n_models, B, H, W, sched, bptt_dev, bptt_bytes, gT_dev, g0_dev, gparams_dev,
+                         workspace_dev, workspace_bytes, stream, true);
+}
+
 /* ---- checkpointed resident BPTT: x_{j*every} only; each segment's records are recomputed in the backward ---- */
 size_t gnca_bptt_ckpt_bytes(const gnca_model* m, int B, int H, int W, int every) {
   if (!m || B <= 0 || H <= 0 || W <= 0 || every <= 0) return 0;

@@ -579,11 +579,12 @@ def rollout_bwd_raw(desc, packed, hist, sched: Schedule, gT: torch.Tensor, *, gf
     return g0, gflat
 
 
-def _model_stack(models, x0: torch.Tensor, what: str, impl: str):
-    """(desc, models as a list, M) of a list of same-architecture models: the model-stacked calls of
+def _model_stack(models, x0: Optional[torch.Tensor], what: str, impl: str):
+    """(desc, models as a list, M) of a list of same-architecture models: the model-stacked calls of rollout /
     record_rollout / monitor_rollout.  ValueError, before any launch, for an empty list, models that differ in their
     descriptor, graph offsets or neighbour count, or device, models on another device than x0, a batch that is not a
-    multiple of M, and impl='streaming' (the streaming kernels stage weights per tile, not per sample)."""
+    multiple of M, and impl='streaming' (the streaming kernels stage weights per tile, not per sample).  x0=None checks
+    the models only."""
     models = list(models)
     if not models:
         raise ValueError(f"{what}: the list of models is empty")
@@ -604,9 +605,11 @@ def _model_stack(models, x0: torch.Tensor, what: str, impl: str):
                              "shares one schedule")
         if next(m.parameters()).device != dev:
             raise ValueError(f"{what}: model {i} is on {next(m.parameters()).device}, model 0 on {dev}")
+    M = len(models)
+    if x0 is None:
+        return desc, models, M
     if dev != x0.device:
         raise ValueError(f"{what}: the models are on {dev}, x0 on {x0.device}")
-    M = len(models)
     if x0.dim() != 4 or x0.shape[0] % M != 0:
         raise ValueError(f"{what}: x0 must be [M*B, C, H, W] with the batch a multiple of the {M} models, got "
                          f"{list(x0.shape)}")
@@ -616,6 +619,62 @@ def _model_stack(models, x0: torch.Tensor, what: str, impl: str):
 def _stack_packed(models) -> torch.Tensor:
     """[M, packed_total]: the cached packed_weights() of every model, one row each"""
     return torch.stack([m.packed_weights() for m in models])
+
+
+def stack_bptt_bytes(desc, B: int, H: int, W: int, T: int, k: int = 0) -> Tuple[int, bool]:
+    """(bytes, zp) of the record buffer `rollout(models, ...)` allocates for a stack on a B x C x H x W batch (B counts
+    the samples of all models) over T steps with k offsets per step; zp: the zero-padded graph shift's buffer
+    (gnca_bptt_zp_bytes), else gnca_bptt_bytes.  That is what the single-model call keeps for the same batch, but a
+    stack has no dense streaming history to fall back to, so ValueError, naming the bytes, where the single-model call
+    would take it: above BPTT_MAX_BYTES, or outside the resident BPTT's envelope."""
+    lib = _lib.load()
+    zp = bool(desc.flags & _lib.GNCA_F_GRAPH) and not (desc.flags & _lib.GNCA_F_TORUS)
+    nbytes = lib.gnca_bptt_zp_bytes if zp else lib.gnca_bptt_bytes
+    nb = nbytes(C.byref(desc), B, H, W, T) if k <= RESIDENT_MAX_K else 0
+    if nb == 0:
+        raise ValueError(f"rollout: a list of models trains on the resident BPTT only, which this model / shape does not "
+                         f"have (16 channels, hidden 128, H*W <= 2048, W % 4 == 0, at most {RESIDENT_MAX_K} offsets per "
+                         f"step, d_model <= 32 for the zero-padded shift); got B={B}, {H}x{W}, k={k}")
+    if nb > BPTT_MAX_BYTES:
+        raise ValueError(f"rollout: the records of this stack take {nb} bytes (B={B}, {H}x{W}, T={T}), more than "
+                         f"BPTT_MAX_BYTES = {BPTT_MAX_BYTES}; a stack has no streaming backward to fall back to, so "
+                         "train fewer models, samples or steps per call")
+    return _record_bytes(lib, desc, B, H, W, T, nbytes) or nb, zp
+
+
+def rollout_models_fwd_raw(desc, packed: torch.Tensor, x0: torch.Tensor, sched: Schedule):
+    """Resident BPTT forward of a stack (gnca_rollout_fwd_bptt_models, or its _zp form) without autograd: (x_T, History).
+    packed: [M, packed_total]; x0: [M*B, C, H, W], model-major."""
+    x0 = GF._require_cuda_f32(x0, "x0")
+    B, Cc, H, W = x0.shape
+    if Cc != desc.C:
+        raise ValueError(f"x0 has {Cc} channels, model has {desc.C}")
+    M, T = packed.shape[0], sched.T
+    nb, zp = stack_bptt_bytes(desc, B, H, W, T, sched.k)           # errors before any allocation or launch
+    lib = _lib.load()
+    xT = torch.empty_like(x0)
+    ws = GF._WS.get(x0.device, lib.gnca_rollout_workspace_models_bytes(C.byref(desc), M, B, H, W, T))
+    bptt = torch.empty(nb, dtype=torch.uint8, device=x0.device)
+    name = "gnca_rollout_fwd_bptt_zp_models" if zp else "gnca_rollout_fwd_bptt_models"
+    _lib.check(getattr(lib, name)(C.byref(desc), GF._ptr(packed), M, B, H, W, C.byref(sched.c_struct()), GF._ptr(x0),
+                                  GF._ptr(xT), GF._ptr(bptt), nb, GF._ptr(ws), ws.numel(), GF._stream()), name)
+    return xT, History(None, bptt=bptt, shape=(T + 1, B, Cc, H, W), zp=zp)
+
+
+def rollout_models_bwd_raw(desc, packed: torch.Tensor, hist: History, sched: Schedule, gT: torch.Tensor):
+    """Backward of rollout_models_fwd_raw: (dL/dx_0, [M, param_total] parameter gradients, row i model i's)."""
+    M = packed.shape[0]
+    _, B, Cc, H, W = hist.shape
+    gT = GF._require_cuda_f32(gT, "grad_output")
+    lib = _lib.load()
+    g0 = torch.empty(B, Cc, H, W, dtype=torch.float32, device=gT.device)
+    gflat = torch.zeros(M, GF.param_layout(desc).total, dtype=torch.float32, device=gT.device)
+    ws = GF._WS.get(gT.device, lib.gnca_rollout_workspace_models_bytes(C.byref(desc), M, B, H, W, sched.T))
+    name = "gnca_rollout_bwd_bptt_zp_models" if hist.zp else "gnca_rollout_bwd_bptt_models"
+    _lib.check(getattr(lib, name)(C.byref(desc), GF._ptr(packed), M, B, H, W, C.byref(sched.c_struct()),
+                                  GF._ptr(hist.bptt), hist.bptt.numel(), GF._ptr(gT), GF._ptr(g0), GF._ptr(gflat),
+                                  GF._ptr(ws), ws.numel(), GF._stream()), name)
+    return g0, gflat
 
 
 class _RolloutFn(torch.autograd.Function):
@@ -731,6 +790,29 @@ class _BudgetFn(torch.autograd.Function):
         return (g0, None, *grads)
 
 
+class _RolloutModelsFn(torch.autograd.Function):
+    """rollout(models, ...): one node over the stack; params are every model's canonical parameters, model-major."""
+
+    @staticmethod
+    def forward(ctx, x0, cfg, *params):
+        xT, hist = rollout_models_fwd_raw(cfg["desc"], cfg["packed"], x0, cfg["schedule"])
+        ctx.cfg, ctx.hist = cfg, hist
+        ctx.param_shapes = [p.shape for p in params]
+        return xT
+
+    @staticmethod
+    def backward(ctx, gT):
+        cfg = ctx.cfg
+        if ctx.hist is None:
+            raise RuntimeError("rollout: the BPTT history was already consumed by an earlier backward")
+        g0, gflat = rollout_models_bwd_raw(cfg["desc"], cfg["packed"], ctx.hist, cfg["schedule"], gT)
+        ctx.hist = None
+        offs = GF.segment_offsets(cfg["desc"])
+        n = len(offs) - 1
+        grads = [gflat[j // n, offs[j % n]:offs[j % n + 1]].view(s) for j, s in enumerate(ctx.param_shapes)]
+        return (g0, None, *grads)
+
+
 def _check_checkpoint_impl(impl: str, what: str) -> None:
     if impl in ("resident", "banded"):
         raise ValueError(f"{what}: checkpoints are recomputed with the streaming kernels, so impl={impl!r} cannot "
@@ -754,7 +836,37 @@ def rollout(model, x0: torch.Tensor, schedule: Schedule, *, checkpoint_every: Op
     history `rollout()` keeps without a budget is kept unchanged when it fits (bit-identical results); else the
     resident BPTT recomputes segments from checkpoints x_{jK} (same dL/dx_0 as the unsegmented resident BPTT), else
     the streaming kernels do (`checkpoint_every`), each with the largest K that fits.  ValueError when nothing fits.
-    `impl="resident"` / `"streaming"` restrict the choice to that backward."""
+    `impl="resident"` / `"streaming"` restrict the choice to that backward.
+
+    `model` may be a list of M models of one architecture (same `model_desc()`, graph offsets and neighbour count, one
+    device), e.g. the seeds or learning rates of a sweep.  x0 is [M*B, C, H, W], model-major: model i runs samples
+    [i*B, (i+1)*B) and x_T keeps that layout.  Build the schedule with `make_schedule(models[0], M*B, ...)`, so that every
+    model sees the same offsets, fire draws and damage.  With grad, the M models train in one resident BPTT
+    (gnca_rollout_fwd_bptt_models / gnca_rollout_bwd_bptt_models, or their _zp forms): one autograd node whose backward
+    gives dL/dx0 and each model's parameter gradients, so `loss.backward()` fills every model's `.grad`.  Model i's
+    gradients come from its own samples only.  Without grad it returns x_T, bit-equal to `record_rollout(models,
+    ...).x_T`.  The stack keeps the records the single-model call keeps for an M*B batch (T*M*B*H*W*1.4 KB at worst,
+    `stack_bptt_bytes`), but has no streaming backward to fall back to: where the single-model call would take the dense
+    history (more than BPTT_MAX_BYTES of records, or a model / shape outside the resident BPTT) it raises ValueError
+    naming the bytes, before any launch.  `checkpoint_every`, `bptt_budget`, `return_history`, impl='streaming' or
+    'banded', and a batch that is not a multiple of M raise ValueError before any launch."""
+    if isinstance(model, (list, tuple)):
+        for name, on in (("checkpoint_every", checkpoint_every is not None), ("bptt_budget", bptt_budget is not None),
+                         ("return_history=True", return_history)):
+            if on:
+                raise ValueError(f"rollout: {name} does not take a list of models (a stack trains on the resident "
+                                 "BPTT only)")
+        if impl == "banded":
+            raise ValueError("rollout: a list of models trains on the replicated-state kernels; impl='banded' cannot "
+                             "take it")
+        desc, models, M = _model_stack(model, x0, "rollout", impl)
+        if not x0.is_cuda:
+            raise RuntimeError(f"rollout: x0 is on {x0.device}; CUDA (sm_100a) only, no CPU fallback")
+        ps = [p for m in models for p in m.canonical_params()]
+        if not (torch.is_grad_enabled() and (x0.requires_grad or any(p.requires_grad for p in ps))):
+            return record_rollout(models, x0, schedule, every=max(schedule.T, 1), impl=impl).x_T
+        cfg = {"desc": desc, "packed": _stack_packed(models), "schedule": schedule}
+        return _RolloutModelsFn.apply(x0, cfg, *ps)
     if bptt_budget is not None:
         if int(bptt_budget) < 0:
             raise ValueError(f"rollout: bptt_budget must be >= 0 bytes, got {bptt_budget}")

@@ -382,6 +382,42 @@ int gnca_rollout_bwd_bptt_zp(const gnca_model* m, const float* packed_dev, int B
                              void* workspace_dev, size_t workspace_bytes, void* stream);
 
 /*
+ * Training many models in one rollout: the resident BPTT (gnca_rollout_fwd_bptt / _bwd_bptt, and the _zp pair for the
+ * zero-padded graph shift) for a stack of n_models models that share the descriptor `m` and the schedule -- e.g. the
+ * seeds or learning rates of a sweep.  packed_dev is [n_models][packed_total] as in gnca_rollout_record_models; B counts
+ * all samples and must be a multiple of n_models: sample b runs model b / (B / n_models), so x0, x_T, gT and g0 keep
+ * their single-model shapes with the model-major B.  The record buffer is that of the single-model call on the total B
+ * (gnca_bptt_bytes / gnca_bptt_zp_bytes).
+ *   - The forward writes no history or frames; x_T equals gnca_rollout_record_models on the same impl 0.
+ *   - The backward ACCUMULATES gparams_dev[n_models][param_total]: model i's gradients in row i, summed over its own
+ *     samples only, in a fixed order (no float atomics: two calls are bit-identical).  With n_models == 1 every output
+ *     is bit-identical to the single-model call.  Model i's block of g0 equals the single-model call of model i on the
+ *     whole batch with gT zero outside block i; its parameter gradients equal that call's up to the summation order.
+ *   - Workspace: gnca_rollout_workspace_models_bytes, which holds at least one weight-gradient partial per model (0 on
+ *     bad arguments).
+ *   - No frame gradients, no checkpoints and no streaming fallback: a batch or shape the resident BPTT has no
+ *     configuration for is GNCA_ERR_UNSUPPORTED.
+ * Errors return before any launch: a NULL required pointer, n_models < 1, B % n_models != 0, B, H or W <= 0 or T < 0 is
+ * GNCA_ERR_ARG; a buffer or workspace too small is GNCA_ERR_WORKSPACE; k outside [0, GNCA_MAX_K] or an unsupported
+ * model, batch or shape is GNCA_ERR_UNSUPPORTED.
+ */
+size_t gnca_rollout_workspace_models_bytes(const gnca_model* m, int n_models, int B, int H, int W, int T);
+int gnca_rollout_fwd_bptt_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                 const gnca_schedule* sched, const float* x0_dev, float* xT_dev, void* bptt_dev,
+                                 size_t bptt_bytes, void* workspace_dev, size_t workspace_bytes, void* stream);
+int gnca_rollout_bwd_bptt_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                 const gnca_schedule* sched, void* bptt_dev, size_t bptt_bytes, const float* gT_dev,
+                                 float* g0_dev, float* gparams_dev, void* workspace_dev, size_t workspace_bytes,
+                                 void* stream);
+int gnca_rollout_fwd_bptt_zp_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                    const gnca_schedule* sched, const float* x0_dev, float* xT_dev, void* bptt_dev,
+                                    size_t bptt_bytes, void* workspace_dev, size_t workspace_bytes, void* stream);
+int gnca_rollout_bwd_bptt_zp_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                    const gnca_schedule* sched, void* bptt_dev, size_t bptt_bytes, const float* gT_dev,
+                                    float* g0_dev, float* gparams_dev, void* workspace_dev, size_t workspace_bytes,
+                                    void* stream);
+
+/*
  * Checkpointed resident BPTT: the resident backward with memory that does not grow with T.  The forward keeps only the
  * states x_{j*every}; the backward recomputes the records of one `every`-step segment at a time, last segment first,
  * with the resident forward kernel, and runs the resident backward over them.  Eligible configurations are those of
