@@ -89,6 +89,20 @@ EXPORTS = {
                                               C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
                                               C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p,
                                               C.c_size_t, C.c_int, C.c_void_p]),
+    "gnca_ssim_rgb_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
+    "gnca_ssim_rgb": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                C.c_size_t, C.c_void_p]),
+    "gnca_metrics_ssim_scratch_bytes": (C.c_size_t, [C.POINTER(GncaModel), C.c_int, C.c_int, C.c_int, C.c_int,
+                                                     C.c_int]),
+    "gnca_rollout_metrics_ssim": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                            C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                            C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                            C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
+    "gnca_rollout_metrics_ssim_models": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                   C.c_int, C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_int,
+                                                   C.c_void_p, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                   C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_int,
+                                                   C.c_void_p]),
     "gnca_rollout_bwd": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
                                    C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),

@@ -79,6 +79,15 @@ struct FrameMetrics {
 // sums / counts of `rows` (frame, sample) pairs from their P partials (gnca_rollout.cu)
 int run_metrics_reduce(int rows, int P, const double* part, double* sums, int* counts, cudaStream_t st);
 
+// SSIM of the same frames (gnca_rollout_metrics_ssim): one double partial per (frame, sample, part), the sum of ssim_cell
+// (gnca_metrics.cuh) over the part's interior cells, reduced in part order by run_ssim_reduce into ssim[F][B].  The
+// cluster kernels take `part` as a trailing kernel parameter of their SSIM instantiations.
+struct SsimFrames {
+  double* part;          // [F][B][P] (cluster kernels) or [B][P] (streaming path, one frame at a time)
+  double* ssim;          // [F][B]
+};
+int run_ssim_reduce(int rows, int P, const double* part, double* ssim, int H, int W, cudaStream_t st);
+
 // A stack of same-architecture models in one launch of the cluster kernels (gnca_rollout_record_models /
 // gnca_rollout_metrics_models): `packed` is [n_models][stride] and sample b runs model b / per_model.  Each kernel
 // rebases `packed` once, before staging the weights into shared memory.  stride = 0: one model for the whole batch.
@@ -93,7 +102,8 @@ struct ModelStack {
 int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                      const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                      float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st, int hist_every = 1,
-                     const FrameMetrics* met = nullptr, ModelStack ms = ModelStack{0, 0});
+                     const FrameMetrics* met = nullptr, ModelStack ms = ModelStack{0, 0},
+                     const SsimFrames* ss = nullptr);
 
 // replicated-state cluster rollout (gnca_rep.cu): every CTA of a sample's cluster holds the whole sample; first
 // choice of the resident path.  scratch: >= B*C*H*W floats of device memory (overflow of the in-smem u buffer).
@@ -103,13 +113,14 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
 // zp (zero-padded graph shift only): with records, also the attention weights and row sums of every message step
 // met: the per-frame metrics of the steps t % met->every == 0 (a whole rollout, t0 = 0)
 // ms: a stack of models, one per block of ms.per_model samples, with or without records
+// ss (with met only): the SSIM of the same frames, by the kernel's SSIM instantiation (run_resident_fwd likewise)
 struct ZpRec;
 struct ZpBwd;
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                 float* u_hist, float* rec, uint32_t* masks, float* scratch, cudaStream_t st, int hist_every = 1,
                 int t0 = 0, const ZpRec* zp = nullptr, const FrameMetrics* met = nullptr,
-                ModelStack ms = ModelStack{0, 0});
+                ModelStack ms = ModelStack{0, 0}, const SsimFrames* ss = nullptr);
 // resident BPTT on the records of run_rep_fwd (gnca_rep_bwd.cu).  g_frames (optional, [F][B][C][H][W]): dL/dx_{f*every}
 // added at step f * every (gnca_rollout_bwd_bptt_frames)
 size_t rep_bptt_bytes(const gnca_model& m, int B, int H, int W, int T);     // 0: configuration not supported

@@ -128,12 +128,45 @@ __device__ __forceinline__ void rep_met_cells(const FrameMetrics& M, const float
 __device__ __forceinline__ void rep_met_flush(const float* sY, int w0, double* dst) {
   met_sum_parts(dst, reinterpret_cast<const double*>(sY), w0, kPW, 3 * 16 * 8 / 2);
 }
-// a whole frame by all warps, outside the tile phase of a step
+
+// SSIM of x_t over the interior cells among [lo, hi), spread over warps [w0, kPW) like rep_met_cells: the 7x7 windows are
+// read from the replica (sX, sAg), which holds all of x_t.  Each warp leaves its sum as the fifth double of its tile head.
+__device__ __forceinline__ void rep_ssim_cells(const float* sX, const float* sAg, float* sY, const float* tgt, int lo,
+                                               int hi, int H, int W, int w0) {
+  constexpr int C = 16, kTile = 3 * C * 8;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  auto state = [&](int yy, int xx) {
+    const int cell = yy * W + xx;
+    float4 v = *reinterpret_cast<const float4*>(sX + (size_t)cell * C);
+    v.w = sAg[cell];
+    return v;
+  };
+  double s = 0.0;
+#pragma unroll 1
+  for (int cell = lo + (warp - w0) * 32 + lane; cell < hi; cell += (kPW - w0) * 32) {
+    const int y = cell / W, x = cell - y * W;
+    if (ssim_interior(y, x, H, W)) s += ssim_cell(state, tgt, y, x, W, H * W);
+  }
+  s = warp_sum_f64(s);
+  if (lane == 0) reinterpret_cast<double*>(sY + warp * kTile)[4] = s;
+}
+__device__ __forceinline__ void rep_ssim_flush(const float* sY, int w0, double* dst) {
+  double s = 0.0;
+  for (int w = w0; w < kPW; ++w) s += reinterpret_cast<const double*>(sY + w * 3 * 16 * 8)[4];
+  *dst = s;
+}
+
+// a whole frame's metrics (SS: and SSIM, into *ss_dst) by all warps, outside the tile phase of a step
+template <bool SS>
 __device__ __forceinline__ void rep_met_frame(const FrameMetrics& M, const float* sX, const float* sAg, float* sY, int lo,
-                                              int hi, int HW, float thr, double* dst) {
+                                              int hi, int HW, float thr, double* dst, double* ss_dst, int H, int W) {
   rep_met_cells(M, sX, sAg, sY, lo, hi, HW, thr, 0);
+  if constexpr (SS) rep_ssim_cells(sX, sAg, sY, M.target, lo, hi, H, W, 0);
   __syncthreads();
-  if (threadIdx.x == 0) rep_met_flush(sY, 0, dst);
+  if (threadIdx.x == 0) {
+    rep_met_flush(sY, 0, dst);
+    if constexpr (SS) rep_ssim_flush(sY, 0, ss_dst);
+  }
   __syncthreads();
 }
 
@@ -144,9 +177,12 @@ __device__ __forceinline__ void rep_met_frame(const FrameMetrics& M, const float
 // Z (ZP with records only, else unused): the softmax weights and row sums of every message step, for k_rep_bwd.
 // MET (gnca_rollout_metrics): at every step t % M.every == 0 each CTA reduces the cells it stores for the history,
 // [my_lo, my_hi), against M.target and writes one partial per (frame, sample, rank); M is unused otherwise.
-template <int C, bool ZP, bool MET>
+// SS (with MET, gnca_rollout_metrics_ssim): at the same steps each CTA also sums the SSIM of its interior cells among
+// [my_lo, my_hi) into ssim_part[frame][b][rank]; ssim_part is unused otherwise.
+template <int C, bool ZP, bool MET, bool SS>
 __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const float* __restrict__ packed, ZpRec Z,
-                                                     FrameMetrics M) {
+                                                     FrameMetrics M, double* ssim_part) {
+  static_assert(MET || !SS, "SSIM rides on the metrics steps");
   static_assert(C == 16, "lane mapping: 2 cells x 16 channels per warp row");
   constexpr int C3 = 3 * C, HID = 128;
   constexpr int CPL = 32 / C;                    // cells per lane row (2)
@@ -268,7 +304,6 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
   // frame metrics: the partial of this CTA's cells of frame t goes to part[frame][b][rank]
   double* met_dst = MET ? M.part + ((size_t)b * NC + rank) * 4 : nullptr;
   const size_t met_frame_stride = MET ? (size_t)a.B * NC * 4 : 0;
-
   // ---- schedule: registers hold step t+2 while step t runs; smem buffers hold t and t+1 ---------------------
   float nx_fr = 0.f, nx_gain = 0.f;
   signed char nx_off = 0;
@@ -461,7 +496,9 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
     if (t >= my_steps) {                         // frozen sample (whole cluster agrees): state passes through
       if (float* h = hist_at(t)) store_state(h, my_lo, my_hi);
       if constexpr (MET)
-        if (t % M.every == 0) rep_met_frame(M, sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr, met_dst + (t / M.every) * met_frame_stride);
+        if (t % M.every == 0)
+          rep_met_frame<SS>(M, sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr, met_dst + (t / M.every) * met_frame_stride,
+                            ssim_part + ((size_t)(t / M.every) * a.B + b) * NC + rank, H, W);
       continue;
     }
     const float gain_m = s_gain[cur];
@@ -783,6 +820,7 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
         }
       }
       if constexpr (MET) if (hist && t % M.every == 0) rep_met_cells(M, sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr, 1);
+      if constexpr (SS) if (hist && t % M.every == 0) rep_ssim_cells(sX, sAg, sY, M.target, my_lo, my_hi, H, W, 1);
     };
     const bool had_tile = n_my <= 32 ? (2 * warp < n_my) : n_my <= 64 ? (4 * warp < n_my) : (((n_my * warp) >> 4) < ((n_my * (warp + 1)) >> 4));
     const bool fire_early = !use_async || !had_tile;
@@ -796,7 +834,10 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
     }
     __syncthreads();
     if constexpr (MET)
-      if (tid == 32 && t % M.every == 0) rep_met_flush(sY, 1, met_dst + (t / M.every) * met_frame_stride);
+      if (tid == 32 && t % M.every == 0) {
+        rep_met_flush(sY, 1, met_dst + (t / M.every) * met_frame_stride);
+        if constexpr (SS) rep_ssim_flush(sY, 1, ssim_part + ((size_t)(t / M.every) * a.B + b) * NC + rank);
+      }
     if (!use_async) {
       if (gn && warp == 0) {
         float t1 = lane < kPW ? s_wred[lane][0] : 0.f, t2 = lane < kPW ? s_wred[lane][1] : 0.f;
@@ -963,7 +1004,9 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
   __syncthreads();
   if (float* h = hist_at(R.T)) store_state(h, my_lo, my_hi);
   if constexpr (MET)
-    if (R.T % M.every == 0) rep_met_frame(M, sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr, met_dst + (R.T / M.every) * met_frame_stride);
+    if (R.T % M.every == 0)
+      rep_met_frame<SS>(M, sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr, met_dst + (R.T / M.every) * met_frame_stride,
+                        ssim_part + ((size_t)(R.T / M.every) * a.B + b) * NC + rank, H, W);
   store_state(R.xT + sample_off, my_lo, my_hi);
   if (R.dbg && blockIdx.x == R.dbg_cta && tid < 24) R.dbg[tid] = s_dbg[tid];
   cluster_arrive(); cluster_wait();      // nobody exits while a peer may still address its shared memory
@@ -1004,7 +1047,7 @@ static size_t rep_smem_bytes(int C, int HW, int ucap, int listcap) {
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                 float* u_hist, float* rec, uint32_t* masks, float* scratch /* >= B*C*H*W floats */, cudaStream_t st,
-                int hist_every, int t0, const ZpRec* zpr, const FrameMetrics* met, ModelStack ms) {
+                int hist_every, int t0, const ZpRec* zpr, const FrameMetrics* met, ModelStack ms, const SsimFrames* ss) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (m.C != 16 || m.hidden != 128) return GNCA_ERR_UNSUPPORTED;
   if (H > kMaxRows || W > kMaxRows || H < 1 || W < 4 || (W & 3)) return GNCA_ERR_UNSUPPORTED;   // quads of 4 cells per row
@@ -1037,10 +1080,13 @@ int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B
   R.KP = k > 8 ? 16 : 8;
   R.zd = zp ? m.d_model : 0;
   R.model_stride = ms.stride; R.model_per = ms.per_model;
-  // the metrics instantiations have the same shared memory and register cap as the plain ones: the same launch
-  // configuration, so x_T is bit-equal to the rollout without metrics
-  const void* kfn = zp ? (met ? (const void*)k_rep_fwd<16, true, true> : (const void*)k_rep_fwd<16, true, false>)
-                       : (met ? (const void*)k_rep_fwd<16, false, true> : (const void*)k_rep_fwd<16, false, false>);
+  // the metrics (and SSIM) instantiations have the same shared memory and register cap as the plain ones: the same
+  // launch configuration, so x_T is bit-equal to the rollout without metrics
+  const bool ssim = met && ss;
+  const void* kfn = zp ? (ssim ? (const void*)k_rep_fwd<16, true, true, true>
+                               : met ? (const void*)k_rep_fwd<16, true, true, false> : (const void*)k_rep_fwd<16, true, false, false>)
+                       : (ssim ? (const void*)k_rep_fwd<16, false, true, true>
+                               : met ? (const void*)k_rep_fwd<16, false, true, false> : (const void*)k_rep_fwd<16, false, false, false>);
   R.HWp = 4 * (((HW >> 2) + 31) & ~31) + 16;      // planes padded to whole warps of quads + one scratch quad
   R.inv_n = (float)(1.0 / ((double)C * (double)H * (double)W));
 
@@ -1108,15 +1154,22 @@ int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B
   prof_begin(PROF_RESIDENT_FWD, st);
   const ZpRec Z = (zp && zpr && rec) ? *zpr : ZpRec{nullptr, nullptr};
   const FrameMetrics M = met ? *met : FrameMetrics{};
-  cudaError_t e = zp ? (met ? cudaLaunchKernelEx(&cfg, k_rep_fwd<16, true, true>, R, P, packed, Z, M)
-                            : cudaLaunchKernelEx(&cfg, k_rep_fwd<16, true, false>, R, P, packed, Z, M))
-                     : (met ? cudaLaunchKernelEx(&cfg, k_rep_fwd<16, false, true>, R, P, packed, Z, M)
-                            : cudaLaunchKernelEx(&cfg, k_rep_fwd<16, false, false>, R, P, packed, Z, M));
+  double* ssp = ssim ? ss->part : nullptr;
+  cudaError_t e = zp ? (ssim ? cudaLaunchKernelEx(&cfg, k_rep_fwd<16, true, true, true>, R, P, packed, Z, M, ssp)
+                        : met ? cudaLaunchKernelEx(&cfg, k_rep_fwd<16, true, true, false>, R, P, packed, Z, M, ssp)
+                              : cudaLaunchKernelEx(&cfg, k_rep_fwd<16, true, false, false>, R, P, packed, Z, M, ssp))
+                     : (ssim ? cudaLaunchKernelEx(&cfg, k_rep_fwd<16, false, true, true>, R, P, packed, Z, M, ssp)
+                        : met ? cudaLaunchKernelEx(&cfg, k_rep_fwd<16, false, true, false>, R, P, packed, Z, M, ssp)
+                              : cudaLaunchKernelEx(&cfg, k_rep_fwd<16, false, false, false>, R, P, packed, Z, M, ssp));
   prof_end(PROF_RESIDENT_FWD, st);
   if (e != cudaSuccess) return (int)e;
   GNCA_LAUNCH_CHECK();
   if (met) {
     const int rc = run_metrics_reduce((R.T / met->every + 1) * B, pick, met->part, met->sums, met->counts, st);
+    if (rc) return rc;
+  }
+  if (ssim) {
+    const int rc = run_ssim_reduce((R.T / met->every + 1) * B, pick, ss->part, ss->ssim, H, W, st);
     if (rc) return rc;
   }
   if (R.dbg) {

@@ -93,10 +93,14 @@ __device__ __noinline__ bool alive_local_ool(const float* plane, int lr, int x, 
 // against M.target and writes one partial per (frame, sample, rank); M is unused otherwise.
 // MS (a stack of models, gnca_rollout_*_models): sample b stages its weights from packed + (b / S.per_model) * S.stride;
 // S is unused otherwise.  A compile-time flag: a runtime field moves the register allocation of the plain kernels.
-template <int C, bool MET, bool MS>
+// SS (with MET, gnca_rollout_metrics_ssim): at the same steps each CTA also sums the SSIM of the interior cells of its
+// own rows into ssim_part[frame][b][rank], reading the window rows it does not own from their owners over DSMEM between
+// two cluster barriers; ssim_part is unused otherwise.
+template <int C, bool MET, bool MS, bool SS>
 __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, Packed P, int hid,
                                                                const float* __restrict__ packed, FrameMetrics M,
-                                                               ModelStack S) {
+                                                               ModelStack S, double* ssim_part) {
+  static_assert(MET || !SS, "SSIM rides on the metrics steps");
   cg::cluster_group cluster = cg::this_cluster();
   constexpr int C3 = 3 * C;
   constexpr int CQ = C / 4;                                     // channel quads (power of two)
@@ -230,6 +234,33 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
     if (tid == 0) met_sum_parts(M.part + (((size_t)(t / M.every) * a.B + b) * NC + rank) * 4, s_met, 0, kRWarps, 4);
     __syncthreads();
   };
+  // SSIM of x_t over the interior cells of the own rows.  A window reaches 3 rows beyond the band, more than the halo
+  // may hold, so every row is read from the CTA that owns it; the first barrier makes every CTA's x_t (after this step's
+  // damage) visible, the second keeps the rows unchanged until every peer has read them.
+  auto ssim_frame = [&](int t) {
+    cluster.sync();
+    auto state = [&](int yy, int xx) {
+      const int q = yy / own;
+      const float* p = cluster.map_shared_rank(sX, q) + (size_t)(HALO + yy - q * own) * W + xx;
+      return make_float4(p[0], p[PL], p[2 * (size_t)PL], p[3 * (size_t)PL]);
+    };
+    double s = 0.0;
+#pragma unroll 1
+    for (int oc = tid; oc < nown; oc += kRThreads) {
+      const int y = r0 + oc / W, x = oc % W;
+      if (ssim_interior(y, x, H, W)) s += ssim_cell(state, M.target, y, x, W, HW);
+    }
+    s = warp_sum_f64(s);
+    double* s_ss = reinterpret_cast<double*>(Ht);
+    if (lane == 0) s_ss[warp] = s;
+    __syncthreads();
+    if (tid == 0) {
+      double v = 0.0;
+      for (int w = 0; w < kRWarps; ++w) v += s_ss[w];
+      ssim_part[((size_t)(t / M.every) * a.B + b) * NC + rank] = v;
+    }
+    cluster.sync();
+  };
   auto alive_local = [&](const float* plane, int lr, int x, int gy, float thr) {
     return alive_local_ool(plane, lr, x, gy, H, W, thr);
   };
@@ -247,6 +278,7 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
     }
     store_hist(t);
     if constexpr (MET) if (t % M.every == 0) met_frame(t);
+    if constexpr (SS) if (t % M.every == 0) ssim_frame(t);
     if (t >= my_steps) continue;               // frozen sample (whole cluster agrees): state passes through
     a.t = t;
     a.fire_u = R.fire_u_base ? R.fire_u_base + (size_t)t * a.B * HW : nullptr;
@@ -627,6 +659,7 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
 
   store_hist(R.T);
   if constexpr (MET) if (R.T % M.every == 0) met_frame(R.T);
+  if constexpr (SS) if (R.T % M.every == 0) ssim_frame(R.T);
   store_own(R.xT + sample_off);
   if (R.dbg && blockIdx.x == R.dbg_cta && tid < 16) R.dbg[tid] = s_dbg[tid];
   cluster_sync_no_acquire();     // nobody exits while a neighbour may still address its shared memory
@@ -654,7 +687,7 @@ static size_t resident_smem_bytes(int C, int hid, bool graph, int own, int halo,
 
 template <int C>
 static int launch_resident(const gnca_model& m, const Packed& P, const float* packed, ResidentArgs& R, int B, int radius,
-                           cudaStream_t st, const FrameMetrics* met, ModelStack S) {
+                           cudaStream_t st, const FrameMetrics* met, ModelStack S, const SsimFrames* ss) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   const int H = R.s.H, W = R.s.W;
   if (m.hidden != 128 || C < 4 || W > 255) return GNCA_ERR_UNSUPPORTED;   // layer 1 + 2 of a tile live in one warp: 32 lanes x 4 units
@@ -667,10 +700,13 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
   // Cluster size: the largest NC in {8,4,2,1} whose bands are at least `halo` rows, that fits shared memory and
   // keeps ALL B clusters co-resident (B <= cudaOccupancyMaxActiveClusters); if the batch is too large for that,
   // the smallest NC that fits (most clusters per wave) and the launch runs in waves.
-  // the metrics instantiation has the plain one's shared memory and register cap: the same launch configuration
-  const bool stack = S.stride != 0;
-  auto kfn = stack ? (met ? k_resident_fwd<C, true, true> : k_resident_fwd<C, false, true>)
-                   : (met ? k_resident_fwd<C, true, false> : k_resident_fwd<C, false, false>);
+  // the metrics (and SSIM) instantiations have the plain one's shared memory and register cap: the same launch
+  // configuration
+  const bool stack = S.stride != 0, ssim = met && ss;
+  auto kfn = stack ? (ssim ? k_resident_fwd<C, true, true, true>
+                           : met ? k_resident_fwd<C, true, true, false> : k_resident_fwd<C, false, true, false>)
+                   : (ssim ? k_resident_fwd<C, true, false, true>
+                           : met ? k_resident_fwd<C, true, false, false> : k_resident_fwd<C, false, false, false>);
   // the dynamic carve shares the opt-in limit with the kernel's static shared memory (about 1.1 KB at C = 32)
   const size_t cap = dynamic_smem_cap((const void*)kfn);
   const int cands[4] = {8, 4, 2, 1};
@@ -732,12 +768,17 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
       R.dbg_cta = atoi(getenv("GNCA_PHASE_TIMING"));
     }
     prof_begin(PROF_RESIDENT_FWD, st);
-    cudaError_t e = cudaLaunchKernelEx(&cfg, kfn, R, P, m.hidden, packed, met ? *met : FrameMetrics{}, S);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, kfn, R, P, m.hidden, packed, met ? *met : FrameMetrics{}, S,
+                                       ssim ? ss->part : nullptr);
     prof_end(PROF_RESIDENT_FWD, st);
     if (e != cudaSuccess) return (int)e;
     GNCA_LAUNCH_CHECK();
     if (met) {
       const int rc = run_metrics_reduce((R.T / met->every + 1) * B, NC, met->part, met->sums, met->counts, st);
+      if (rc) return rc;
+    }
+    if (ssim) {
+      const int rc = run_ssim_reduce((R.T / met->every + 1) * B, NC, ss->part, ss->ssim, H, W, st);
       if (rc) return rc;
     }
     if (R.dbg) {   // development only: synchronous read-back of the phase counters of CTA 0
@@ -759,7 +800,7 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
 int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                      const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                      float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st, int hist_every,
-                     const FrameMetrics* met, ModelStack ms) {
+                     const FrameMetrics* met, ModelStack ms, const SsimFrames* ss) {
   (void)ping; (void)pong; (void)alpha_tmp;
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (graph && !(m.flags & GNCA_F_TORUS) && sched.k > 0) return GNCA_ERR_UNSUPPORTED;   // zero-pad: streaming path
@@ -779,10 +820,10 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
   R.damage = DamageView{sched.damage, sched.damage_layout}; R.damage_step = sched.damage_step;
   const int radius = sched.max_offset;       // largest |dy| / |dx| in the schedule: sets the halo depth
   switch (m.C) {
-    case 4: return launch_resident<4>(m, P, packed, R, B, radius, st, met, ms);
-    case 8: return launch_resident<8>(m, P, packed, R, B, radius, st, met, ms);
-    case 16: return launch_resident<16>(m, P, packed, R, B, radius, st, met, ms);
-    case 32: return launch_resident<32>(m, P, packed, R, B, radius, st, met, ms);
+    case 4: return launch_resident<4>(m, P, packed, R, B, radius, st, met, ms, ss);
+    case 8: return launch_resident<8>(m, P, packed, R, B, radius, st, met, ms, ss);
+    case 16: return launch_resident<16>(m, P, packed, R, B, radius, st, met, ms, ss);
+    case 32: return launch_resident<32>(m, P, packed, R, B, radius, st, met, ms, ss);
   }
   return GNCA_ERR_UNSUPPORTED;
 }

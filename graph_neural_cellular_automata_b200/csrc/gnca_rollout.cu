@@ -76,6 +76,72 @@ static int frame_metrics(const FrameMetrics& met, const float* x, int f, int B, 
   return run_metrics_reduce(B, P, met.part, met.sums + (size_t)f * B * 2, met.counts + (size_t)f * B * 2, st);
 }
 
+// SSIM of one state buffer x ([B][C][HW]): block (p, b) sums ssim_cell over the interior cells among
+// [p * kSsimCells, (p + 1) * kSsimCells) of sample b into part[b][p]; k_ssim_reduce is the second level.  Both in a fixed
+// order.  Backs gnca_ssim_rgb and the kept steps of the streaming path.
+constexpr int kSsimCells = 1024;                   // cells per block of k_frame_ssim
+
+static inline int frame_ssim_parts(int HW) { return (HW + kSsimCells - 1) / kSsimCells; }
+
+__global__ void __launch_bounds__(kMetThreads) k_frame_ssim(const float* __restrict__ x, int C, int H, int W,
+                                                             const float* __restrict__ tgt, double* __restrict__ part) {
+  const int p = blockIdx.x, P = gridDim.x, b = blockIdx.y, HW = H * W;
+  const int lo = p * kSsimCells, hi = min(HW, lo + kSsimCells);
+  const float* xb = x + (size_t)b * C * HW;
+  auto state = [&](int yy, int xx) {
+    const int cell = yy * W + xx;
+    return make_float4(xb[cell], xb[HW + cell], xb[2 * (size_t)HW + cell], xb[3 * (size_t)HW + cell]);
+  };
+  double s = 0.0;
+  for (int cell = lo + (int)threadIdx.x; cell < hi; cell += kMetThreads) {
+    const int y = cell / W, xx = cell - y * W;
+    if (ssim_interior(y, xx, H, W)) s += ssim_cell(state, tgt, y, xx, W, HW);
+  }
+  s = warp_sum_f64(s);
+  __shared__ double s_ss[kMetThreads / 32];
+  if ((threadIdx.x & 31) == 0) s_ss[threadIdx.x >> 5] = s;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double t = 0.0;
+    for (int w = 0; w < kMetThreads / 32; ++w) t += s_ss[w];
+    part[(size_t)b * P + p] = t;
+  }
+}
+
+// ssim[r] = (sum of the P partials of row r, in part order) / (3 (H-6)(W-6))
+__global__ void k_ssim_reduce(int rows, int P, const double* __restrict__ part, double inv_cells,
+                              double* __restrict__ ssim) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= rows) return;
+  double s = 0.0;
+  for (int p = 0; p < P; ++p) s += part[(size_t)r * P + p];
+  ssim[r] = s * inv_cells;
+}
+
+int run_ssim_reduce(int rows, int P, const double* part, double* ssim, int H, int W, cudaStream_t st) {
+  const double inv_cells = 1.0 / (3.0 * (double)(H - 2 * kSsimR) * (double)(W - 2 * kSsimR));
+  k_ssim_reduce<<<(rows + 127) / 128, 128, 0, st>>>(rows, P, part, inv_cells, ssim);
+  GNCA_LAUNCH_CHECK();
+  return 0;
+}
+
+// SSIM of the B samples of x into ssim[B], through part (>= B * frame_ssim_parts(H * W) doubles)
+static int frame_ssim(const float* x, int B, int C, int H, int W, const float* tgt, double* part, double* ssim,
+                      cudaStream_t st) {
+  const int P = frame_ssim_parts(H * W);
+  k_frame_ssim<<<dim3(P, B), kMetThreads, 0, st>>>(x, C, H, W, tgt, part);
+  GNCA_LAUNCH_CHECK();
+  return run_ssim_reduce(B, P, part, ssim, H, W, st);
+}
+
+// the metrics of frame f on the streaming path, with its SSIM when ss is set
+static int frame_quality(const FrameMetrics& met, const SsimFrames* ss, const float* x, int f, int B, int C, int H,
+                         int W, float thr, cudaStream_t st) {
+  int rc = frame_metrics(met, x, f, B, C, H * W, thr, st);
+  if (rc || !ss) return rc;
+  return frame_ssim(x, B, C, H, W, met.target, ss->part, ss->ssim + (size_t)f * B, st);
+}
+
 static int launch_add(size_t n, float* out, const float* a, const float* b, cudaStream_t st) {
   k_add<<<(int)((n + 1023) / 1024 < 2368 ? (n + 1023) / 1024 : 2368), 256, 0, st>>>(n, out, a, b);
   GNCA_LAUNCH_CHECK();
@@ -234,12 +300,14 @@ static Segment carve_segment(void* base, const gnca_model& m, int B, int H, int 
 // gnca_rollout_fwd with a strided history: x_t of every step t % every == 0 goes to x_hist slot t / every
 // (every == 1: the full [T+1] history of gnca_rollout_fwd).
 // met: the per-frame metrics of gnca_rollout_metrics (stride met->every), by the kernel that runs the steps
+// ss (with met only): the SSIM of the same frames (gnca_rollout_metrics_ssim)
 // ms: a stack of models (gnca_rollout_*_models): the steps run on a cluster kernel or not at all, since only those stage
 // their weights per sample.  T = 0 reads no weight and takes the copy path below.
 static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
                        const float* x0_dev, float* xT_dev, float* x_hist_dev, int every, float* stats_hist_dev,
                        float* u_hist_dev, void* workspace_dev, size_t workspace_bytes, int impl, void* stream,
-                       const FrameMetrics* met = nullptr, const ModelStack* ms = nullptr) {
+                       const FrameMetrics* met = nullptr, const ModelStack* ms = nullptr,
+                       const SsimFrames* ss = nullptr) {
   if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !workspace_dev) return GNCA_ERR_ARG;
   if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
   if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
@@ -262,10 +330,10 @@ static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int 
       int rc = GNCA_ERR_UNSUPPORTED;
       if (impl != 3)
         rc = run_rep_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, x_hist_dev, stats_hist_dev, u_hist_dev,
-                         nullptr, nullptr, r.ping, st, every, 0, nullptr, met, ms ? *ms : one);
+                         nullptr, nullptr, r.ping, st, every, 0, nullptr, met, ms ? *ms : one, ss);
       if (rc == GNCA_ERR_UNSUPPORTED)
         rc = run_resident_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, x_hist_dev, stats_hist_dev,
-                              u_hist_dev, r.ping, r.pong, r.alpha_tmp, st, every, met, ms ? *ms : one);
+                              u_hist_dev, r.ping, r.pong, r.alpha_tmp, st, every, met, ms ? *ms : one, ss);
       if (rc != GNCA_ERR_UNSUPPORTED || impl == 2 || impl == 3 || ms) return rc;
     }
   }
@@ -284,7 +352,7 @@ static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int 
       if (rc) return rc;
     }
     if (met && t % met->every == 0) {
-      int rc = frame_metrics(*met, x_at(t), t / met->every, B, m->C, H * W, m->alpha_thr, st);
+      int rc = frame_quality(*met, ss, x_at(t), t / met->every, B, m->C, H, W, m->alpha_thr, st);
       if (rc) return rc;
     }
     StepArgs a;
@@ -300,7 +368,7 @@ static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int 
   }
   if ((x_hist_dev && T % every == 0) || T == 0)
     GNCA_CHECK_CUDA(cudaMemcpyAsync(xT_dev, x_at(T), N * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  if (met && T % met->every == 0) return frame_metrics(*met, xT_dev, T / met->every, B, m->C, H * W, m->alpha_thr, st);
+  if (met && T % met->every == 0) return frame_quality(*met, ss, xT_dev, T / met->every, B, m->C, H, W, m->alpha_thr, st);
   return 0;
 }
 
@@ -457,21 +525,74 @@ size_t gnca_metrics_scratch_bytes(const gnca_model* m, int B, int H, int W, int 
   return (cluster > streaming ? cluster : streaming) * 4 * sizeof(double);
 }
 
+static int model_stack(const gnca_model& m, int n_models, int B, int impl, ModelStack* ms);
+
+// the shared body of gnca_rollout_metrics[_ssim][_models]: n_models = 0 runs one model, ssim_dev = NULL skips SSIM
+static int rollout_metrics(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                           const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                           const float* target_dev, float eps, double* sums_dev, int32_t* counts_dev, double* ssim_dev,
+                           bool want_ssim, void* scratch_dev, size_t scratch_bytes, void* workspace_dev,
+                           size_t workspace_bytes, int impl, void* stream) {
+  if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !target_dev || !sums_dev || !counts_dev || !scratch_dev ||
+      !workspace_dev || (want_ssim && !ssim_dev))
+    return GNCA_ERR_ARG;
+  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0 || every <= 0 || m->C < 4) return GNCA_ERR_ARG;
+  if (want_ssim && (H < kSsimWin || W < kSsimWin)) return GNCA_ERR_ARG;
+  if (!(eps >= 0.f)) return GNCA_ERR_ARG;
+  ModelStack ms{0, 0};
+  if (n_models > 0) {
+    int rc = model_stack(*m, n_models, B, impl, &ms);
+    if (rc) return rc;
+  }
+  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
+  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
+  const size_t met_bytes = gnca_metrics_scratch_bytes(m, B, H, W, sched->T, every);
+  const size_t need = want_ssim ? gnca_metrics_ssim_scratch_bytes(m, B, H, W, sched->T, every) : met_bytes;
+  if (need > scratch_bytes) return GNCA_ERR_WORKSPACE;
+  const FrameMetrics met{target_dev, reinterpret_cast<double*>(scratch_dev), sums_dev, counts_dev, eps, every};
+  const SsimFrames ss{reinterpret_cast<double*>(static_cast<char*>(scratch_dev) + met_bytes), ssim_dev};
+  return rollout_fwd(m, packed_dev, B, H, W, sched, x0_dev, xT_dev, nullptr, 1, nullptr, nullptr, workspace_dev,
+                     workspace_bytes, impl, stream, &met, n_models > 0 ? &ms : nullptr, want_ssim ? &ss : nullptr);
+}
+
 int gnca_rollout_metrics(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
                          const float* x0_dev, float* xT_dev, int every, const float* target_dev, float eps,
                          double* sums_dev, int32_t* counts_dev, void* scratch_dev, size_t scratch_bytes,
                          void* workspace_dev, size_t workspace_bytes, int impl, void* stream) {
-  if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !target_dev || !sums_dev || !counts_dev || !scratch_dev ||
-      !workspace_dev)
-    return GNCA_ERR_ARG;
-  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0 || every <= 0 || m->C < 4) return GNCA_ERR_ARG;
-  if (!(eps >= 0.f)) return GNCA_ERR_ARG;
-  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
-  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
-  if (gnca_metrics_scratch_bytes(m, B, H, W, sched->T, every) > scratch_bytes) return GNCA_ERR_WORKSPACE;
-  const FrameMetrics met{target_dev, reinterpret_cast<double*>(scratch_dev), sums_dev, counts_dev, eps, every};
-  return rollout_fwd(m, packed_dev, B, H, W, sched, x0_dev, xT_dev, nullptr, 1, nullptr, nullptr, workspace_dev,
-                     workspace_bytes, impl, stream, &met);
+  return rollout_metrics(m, packed_dev, 0, B, H, W, sched, x0_dev, xT_dev, every, target_dev, eps, sums_dev, counts_dev,
+                         nullptr, false, scratch_dev, scratch_bytes, workspace_dev, workspace_bytes, impl, stream);
+}
+
+size_t gnca_metrics_ssim_scratch_bytes(const gnca_model* m, int B, int H, int W, int T, int every) {
+  const size_t met = gnca_metrics_scratch_bytes(m, B, H, W, T, every);
+  if (met == 0 || H < kSsimWin || W < kSsimWin) return 0;
+  // one SSIM partial per rank of every frame on the cluster kernels, per block of one frame on the streaming path
+  const size_t F = (size_t)(T / every + 1);
+  const size_t cluster = F * B * 8, streaming = (size_t)B * frame_ssim_parts(H * W);
+  return met + (cluster > streaming ? cluster : streaming) * sizeof(double);
+}
+
+int gnca_rollout_metrics_ssim(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                              const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                              const float* target_dev, float eps, double* sums_dev, int32_t* counts_dev,
+                              double* ssim_dev, void* scratch_dev, size_t scratch_bytes, void* workspace_dev,
+                              size_t workspace_bytes, int impl, void* stream) {
+  return rollout_metrics(m, packed_dev, 0, B, H, W, sched, x0_dev, xT_dev, every, target_dev, eps, sums_dev, counts_dev,
+                         ssim_dev, true, scratch_dev, scratch_bytes, workspace_dev, workspace_bytes, impl, stream);
+}
+
+size_t gnca_ssim_rgb_scratch_bytes(int B, int H, int W) {
+  if (B <= 0 || H < kSsimWin || W < kSsimWin) return 0;
+  return (size_t)B * frame_ssim_parts(H * W) * sizeof(double);
+}
+
+int gnca_ssim_rgb(const float* x_dev, int B, int C, int H, int W, const float* target_dev, double* ssim_dev,
+                  void* scratch_dev, size_t scratch_bytes, void* stream) {
+  if (!x_dev || !target_dev || !ssim_dev || !scratch_dev) return GNCA_ERR_ARG;
+  if (B <= 0 || C < 4 || H < kSsimWin || W < kSsimWin) return GNCA_ERR_ARG;
+  if (gnca_ssim_rgb_scratch_bytes(B, H, W) > scratch_bytes) return GNCA_ERR_WORKSPACE;
+  return frame_ssim(x_dev, B, C, H, W, target_dev, reinterpret_cast<double*>(scratch_dev), ssim_dev,
+                    (cudaStream_t)stream);
 }
 
 /* ---- a stack of same-architecture models in one launch: sample b runs model b / (B / n_models) ---- */
@@ -503,20 +624,21 @@ int gnca_rollout_metrics_models(const gnca_model* m, const float* packed_dev, in
                                 const float* target_dev, float eps, double* sums_dev, int32_t* counts_dev,
                                 void* scratch_dev, size_t scratch_bytes, void* workspace_dev, size_t workspace_bytes,
                                 int impl, void* stream) {
-  if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !target_dev || !sums_dev || !counts_dev || !scratch_dev ||
-      !workspace_dev)
-    return GNCA_ERR_ARG;
-  if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0 || every <= 0 || m->C < 4) return GNCA_ERR_ARG;
-  if (!(eps >= 0.f)) return GNCA_ERR_ARG;
-  ModelStack ms;
-  int rc = model_stack(*m, n_models, B, impl, &ms);
-  if (rc) return rc;
-  if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
-  if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
-  if (gnca_metrics_scratch_bytes(m, B, H, W, sched->T, every) > scratch_bytes) return GNCA_ERR_WORKSPACE;
-  const FrameMetrics met{target_dev, reinterpret_cast<double*>(scratch_dev), sums_dev, counts_dev, eps, every};
-  return rollout_fwd(m, packed_dev, B, H, W, sched, x0_dev, xT_dev, nullptr, 1, nullptr, nullptr, workspace_dev,
-                     workspace_bytes, impl, stream, &met, &ms);
+  if (n_models < 1) return GNCA_ERR_ARG;
+  return rollout_metrics(m, packed_dev, n_models, B, H, W, sched, x0_dev, xT_dev, every, target_dev, eps, sums_dev,
+                         counts_dev, nullptr, false, scratch_dev, scratch_bytes, workspace_dev, workspace_bytes, impl,
+                         stream);
+}
+
+int gnca_rollout_metrics_ssim_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                     const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                                     const float* target_dev, float eps, double* sums_dev, int32_t* counts_dev,
+                                     double* ssim_dev, void* scratch_dev, size_t scratch_bytes, void* workspace_dev,
+                                     size_t workspace_bytes, int impl, void* stream) {
+  if (n_models < 1) return GNCA_ERR_ARG;
+  return rollout_metrics(m, packed_dev, n_models, B, H, W, sched, x0_dev, xT_dev, every, target_dev, eps, sums_dev,
+                         counts_dev, ssim_dev, true, scratch_dev, scratch_bytes, workspace_dev, workspace_bytes, impl,
+                         stream);
 }
 
 int gnca_rollout_bwd_frames(const gnca_model* m, const float* packed_dev, int B, int H, int W,

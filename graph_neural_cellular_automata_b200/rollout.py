@@ -1076,10 +1076,11 @@ class Monitor:
     pixel_perfect: torch.Tensor             # [F,B] f32: utils.metrics.pixel_perfect(frame, target, eps)
     alive: torch.Tensor                     # [F,B] int64: cells with alpha > model.alpha_thr (no dilation)
     x_T: torch.Tensor                       # [B,C,H,W]
+    ssim: Optional[torch.Tensor] = None     # [F,B] f32: utils.metrics.ssim_rgb (monitor_rollout(..., ssim=True))
 
 
 def monitor_rollout(model, x0: torch.Tensor, schedule: Schedule, target: torch.Tensor, *, every: int,
-                    impl: str = "auto", eps: float = 0.05) -> Monitor:
+                    impl: str = "auto", eps: float = 0.05, ssim: bool = False) -> Monitor:
     """Quality curves of a rollout without its states: the T steps of `rollout()` (same `impl` and dispatch, the same
     x_T) in one library call (gnca_rollout_metrics), reducing every `every`-th state against `target` ([4,H,W]
     premultiplied RGBA on x0's device) where the kernel holds it.  Memory is F*B*24 bytes of results plus at most
@@ -1091,8 +1092,17 @@ def monitor_rollout(model, x0: torch.Tensor, schedule: Schedule, target: torch.T
     (gnca_rollout_metrics_models), x0 [M*B, C, H, W] model-major, every [F, M*B] curve and x_T with the sample axis M*B
     long, model i's curves at `[:, i*B:(i+1)*B]`.  Build the schedule with `make_schedule(models[0], M*B, ...)` so that
     every model sees the same offsets, fire draws and damage.  impl='streaming' raises ValueError; a shape neither
-    cluster kernel takes raises the library's RuntimeError.  Picking the best epoch of a run by pixel-perfection after
-    damage is one such call over its checkpoints."""
+    cluster kernel takes raises the library's RuntimeError.
+
+    ssim=True adds `Monitor.ssim`, the SSIM of every frame against the target as `utils.metrics.ssim_rgb` defines it
+    (skimage's structural_similarity on clip(premultiplied RGB, 0, 1), 7x7 uniform windows, data_range 1), computed
+    where the kernel holds the frame (gnca_rollout_metrics_ssim[_models]).  The other curves and x_T are those of the
+    call without it; H or W below 7 raises ValueError.  Picking the best epoch of a run is one such call over its
+    checkpoints::
+
+        mon = monitor_rollout(checkpoints, x0.repeat(M, 1, 1, 1), sched, target, every=10, ssim=True)
+        best = int(mon.ssim[-1].view(M, B).mean(1).argmax())   # the epoch whose final frames score highest
+    """
     every = int(every)
     if every < 1:
         raise ValueError(f"monitor_rollout: every must be >= 1, got {every}")
@@ -1116,6 +1126,8 @@ def monitor_rollout(model, x0: torch.Tensor, schedule: Schedule, target: torch.T
     if tuple(target.shape) != (4, H, W):
         raise ValueError(f"monitor_rollout: target must be [4, {H}, {W}] (premultiplied RGBA), got "
                          f"{list(target.shape)}")
+    if ssim and (H < 7 or W < 7):
+        raise ValueError(f"monitor_rollout: SSIM needs a 7x7 window inside the grid, got H={H}, W={W}")
     x0 = GF._require_cuda_f32(x0.detach(), "x0")
     target = GF._require_cuda_f32(target.detach(), "target")
     if target.device != x0.device:
@@ -1126,11 +1138,22 @@ def monitor_rollout(model, x0: torch.Tensor, schedule: Schedule, target: torch.T
     xT = torch.empty_like(x0)
     sums = torch.empty(F, B, 2, dtype=torch.float64, device=x0.device)
     counts = torch.empty(F, B, 2, dtype=torch.int32, device=x0.device)
-    scratch = torch.empty(lib.gnca_metrics_scratch_bytes(C.byref(desc), B, H, W, T, every), dtype=torch.uint8,
-                          device=x0.device)
+    scratch_bytes = (lib.gnca_metrics_ssim_scratch_bytes if ssim else lib.gnca_metrics_scratch_bytes)
+    scratch = torch.empty(scratch_bytes(C.byref(desc), B, H, W, T, every), dtype=torch.uint8, device=x0.device)
     ws = GF._WS.get(x0.device, lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, T))
     cs = schedule.c_struct()
-    if stack:
+    ss = torch.empty(F, B, dtype=torch.float64, device=x0.device) if ssim else None
+    if ssim and stack:
+        _lib.check(lib.gnca_rollout_metrics_ssim_models(
+            C.byref(desc), GF._ptr(_stack_packed(models)), M, B, H, W, C.byref(cs), GF._ptr(x0), GF._ptr(xT), every,
+            GF._ptr(target), eps, GF._ptr(sums), GF._ptr(counts), GF._ptr(ss), GF._ptr(scratch), scratch.numel(),
+            GF._ptr(ws), ws.numel(), IMPL[impl], GF._stream()), "gnca_rollout_metrics_ssim_models")
+    elif ssim:
+        _lib.check(lib.gnca_rollout_metrics_ssim(
+            C.byref(desc), GF._ptr(model.packed_weights()), B, H, W, C.byref(cs), GF._ptr(x0), GF._ptr(xT), every,
+            GF._ptr(target), eps, GF._ptr(sums), GF._ptr(counts), GF._ptr(ss), GF._ptr(scratch), scratch.numel(),
+            GF._ptr(ws), ws.numel(), IMPL[impl], GF._stream()), "gnca_rollout_metrics_ssim")
+    elif stack:
         _lib.check(lib.gnca_rollout_metrics_models(C.byref(desc), GF._ptr(_stack_packed(models)), M, B, H, W,
                                                    C.byref(cs), GF._ptr(x0), GF._ptr(xT), every, GF._ptr(target), eps,
                                                    GF._ptr(sums), GF._ptr(counts), GF._ptr(scratch), scratch.numel(),
@@ -1144,4 +1167,5 @@ def monitor_rollout(model, x0: torch.Tensor, schedule: Schedule, target: torch.T
     HW = H * W
     return Monitor(t=list(range(0, T + 1, every)), loss=(sums[..., 0] / (4 * HW)).float(),
                    psnr=(10.0 * torch.log10(1.0 / (sums[..., 1] / (3 * HW)))).float(),
-                   pixel_perfect=(counts[..., 0].double() / HW).float(), alive=counts[..., 1].long(), x_T=xT)
+                   pixel_perfect=(counts[..., 0].double() / HW).float(), alive=counts[..., 1].long(), x_T=xT,
+                   ssim=ss.float() if ssim else None)

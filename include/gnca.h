@@ -266,6 +266,41 @@ int gnca_rollout_metrics_models(const gnca_model* m, const float* packed_dev, in
                                 void* scratch_dev, size_t scratch_bytes, void* workspace_dev, size_t workspace_bytes,
                                 int impl, void* stream);
 
+/*
+ * SSIM on the device.  The SSIM of a state is skimage's structural_similarity(pred, tgt, channel_axis=-1,
+ * data_range=1.0) with every other argument at its default, where pred = clip(premultiplied RGB of the state, 0, 1)
+ * (r * alpha rounded as for gnca_rollout_metrics, alpha = channel 3) and tgt = clip(target RGB, 0, 1).  Per channel: 7x7
+ * uniform windows, cov_norm = 49/48, C1 = 0.01^2, C2 = 0.03^2, S = (2 ux uy + C1)(2 vxy + C2) / ((ux^2 + uy^2 + C1)
+ * (vx + vy + C2)) averaged over the (H-6)(W-6) interior cells (the windows that lie inside the grid); SSIM is the mean
+ * of the three channel means.  The window moments are taken in double and summed over a fixed partition in a fixed
+ * order: two calls give bit-identical results.
+ *
+ * gnca_ssim_rgb: ssim_dev[B] (double) of the states x_dev [B][C][H][W] against target_dev [4][H][W] (premultiplied).
+ * scratch_dev: gnca_ssim_rgb_scratch_bytes(B, H, W) bytes (0: bad arguments).
+ *
+ * gnca_rollout_metrics_ssim[_models]: gnca_rollout_metrics[_models] with, in addition, ssim_dev[F][B] (double) = the
+ * SSIM of each frame.  sums, counts and x_T are those of the call without SSIM.  scratch_dev:
+ * gnca_metrics_ssim_scratch_bytes(m, B, H, W, T, every) bytes (0: bad arguments, H or W < 7).
+ *
+ * Argument errors return before any launch: a NULL pointer, C < 4, H or W < 7, every <= 0 (and the other argument
+ * errors of the calls without SSIM) are GNCA_ERR_ARG, a scratch too small is GNCA_ERR_WORKSPACE, k outside
+ * [0, GNCA_MAX_K] or a shape no kernel family takes is GNCA_ERR_UNSUPPORTED.
+ */
+size_t gnca_ssim_rgb_scratch_bytes(int B, int H, int W);
+int gnca_ssim_rgb(const float* x_dev, int B, int C, int H, int W, const float* target_dev, double* ssim_dev,
+                  void* scratch_dev, size_t scratch_bytes, void* stream);
+size_t gnca_metrics_ssim_scratch_bytes(const gnca_model* m, int B, int H, int W, int T, int every);
+int gnca_rollout_metrics_ssim(const gnca_model* m, const float* packed_dev, int B, int H, int W,
+                              const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                              const float* target_dev, float eps, double* sums_dev, int32_t* counts_dev,
+                              double* ssim_dev, void* scratch_dev, size_t scratch_bytes, void* workspace_dev,
+                              size_t workspace_bytes, int impl, void* stream);
+int gnca_rollout_metrics_ssim_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                     const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                                     const float* target_dev, float eps, double* sums_dev, int32_t* counts_dev,
+                                     double* ssim_dev, void* scratch_dev, size_t scratch_bytes, void* workspace_dev,
+                                     size_t workspace_bytes, int impl, void* stream);
+
 /* BPTT: given gT = dL/dx_T and the x_hist of the forward, produce g0 = dL/dx_0 and ACCUMULATE gparams. */
 int gnca_rollout_bwd(const gnca_model* m, const float* packed_dev, int B, int H, int W,
                      const gnca_schedule* sched, const float* x_hist_dev, const float* stats_hist_dev,
