@@ -103,6 +103,10 @@ EXPORTS = {
                                                    C.c_void_p, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p,
                                                    C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_int,
                                                    C.c_void_p]),
+    "gnca_rollout_metrics_targets": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                               C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                               C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                               C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
     "gnca_rollout_bwd": (C.c_int, [C.POINTER(GncaModel), C.c_void_p, C.c_int, C.c_int, C.c_int,
                                    C.POINTER(GncaSchedule), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
@@ -161,6 +165,8 @@ EXPORTS = {
     "gnca_host_sample_offsets_words": (C.c_int, [C.c_char_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                  C.c_void_p, C.POINTER(C.c_int32)]),
     "gnca_loss_premult_rgba": (C.c_int, [C.c_int] * 4 + [C.c_void_p] * 4 + [C.c_float, C.c_void_p]),
+    "gnca_loss_premult_rgba_targets": (C.c_int, [C.c_int] * 4 + [C.c_void_p] * 2 + [C.c_int] + [C.c_void_p] * 2
+                                       + [C.c_float, C.c_void_p]),
     "gnca_normalize_adam": (C.c_int, [C.c_void_p] * 4 + [C.POINTER(C.c_int64), C.POINTER(C.c_int32), C.c_int, C.c_int,
                                       C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_int64, C.c_void_p]),
     "gnca_apply_mask": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -66,9 +66,13 @@ __global__ void k_alive_mask(int B, int C, int H, int W, const float* __restrict
 }
 
 // train_graph_augmented_nca.py:52-61 -- one block per sample, deterministic
+// MT (gnca_loss_premult_rgba_targets): tgt is [B / per][4][H][W] and sample b reads target b / per; per is unused
+// otherwise.  A compile-time flag with a trailing parameter, so the single-target kernel keeps its code.
+template <bool MT>
 __global__ void k_loss_premult(int B, int C, int H, int W, const float* __restrict__ x, const float* __restrict__ tgt,
-                               float* __restrict__ per_sample, float* __restrict__ gx, float scale) {
+                               float* __restrict__ per_sample, float* __restrict__ gx, float scale, int per) {
   const int b = blockIdx.x, HW = H * W;
+  if constexpr (MT) tgt += (size_t)(b / per) * 4 * HW;
   const float* xb = x + (size_t)b * C * HW;
   const float inv = 1.0f / (4.0f * (float)HW);
   double acc = 0.0;
@@ -229,7 +233,18 @@ int gnca_alive_mask(int B, int C, int H, int W, const float* x_dev, float thr, f
 int gnca_loss_premult_rgba(int B, int C, int H, int W, const float* x_dev, const float* target_dev,
                            float* per_sample_dev, float* gx_dev, float scale, void* stream) {
   if (!x_dev || !target_dev || !per_sample_dev || B <= 0 || C < 4 || H <= 0 || W <= 0) return GNCA_ERR_ARG;
-  k_loss_premult<<<B, 256, 0, (cudaStream_t)stream>>>(B, C, H, W, x_dev, target_dev, per_sample_dev, gx_dev, scale);
+  k_loss_premult<false><<<B, 256, 0, (cudaStream_t)stream>>>(B, C, H, W, x_dev, target_dev, per_sample_dev, gx_dev,
+                                                              scale, 0);
+  GNCA_LAUNCH_CHECK();
+  return 0;
+}
+
+int gnca_loss_premult_rgba_targets(int B, int C, int H, int W, const float* x_dev, const float* targets_dev,
+                                   int n_targets, float* per_sample_dev, float* gx_dev, float scale, void* stream) {
+  if (!x_dev || !targets_dev || !per_sample_dev || B <= 0 || C < 4 || H <= 0 || W <= 0) return GNCA_ERR_ARG;
+  if (n_targets < 1 || B % n_targets != 0) return GNCA_ERR_ARG;
+  k_loss_premult<true><<<B, 256, 0, (cudaStream_t)stream>>>(B, C, H, W, x_dev, targets_dev, per_sample_dev, gx_dev,
+                                                             scale, B / n_targets);
   GNCA_LAUNCH_CHECK();
   return 0;
 }

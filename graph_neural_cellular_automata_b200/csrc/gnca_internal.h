@@ -69,7 +69,7 @@ int launch_update_tc(const gnca_model& m, const Packed& P, const float* packed, 
 // T % every == 0): one partial of 4 doubles per (frame, sample, part) -- part = the CTA's rank in the cluster kernels,
 // a block of k_frame_metrics on the streaming path -- summed over the parts in part order by run_metrics_reduce.
 struct FrameMetrics {
-  const float* target;   // [4][H][W] premultiplied RGBA
+  const float* target;   // [4][H][W] premultiplied RGBA ([n_models][4][H][W] with a target stride)
   double* part;          // [F][B][P][4] (gnca_metrics_scratch_bytes)
   double* sums;          // [F][B][2] premultiplied-RGBA and clipped-RGB squared-error sums
   int* counts;           // [F][B][2] pixel-perfect and alive cells
@@ -91,6 +91,11 @@ int run_ssim_reduce(int rows, int P, const double* part, double* ssim, int H, in
 // A stack of same-architecture models in one launch of the cluster kernels (gnca_rollout_record_models /
 // gnca_rollout_metrics_models): `packed` is [n_models][stride] and sample b runs model b / per_model.  Each kernel
 // rebases `packed` once, before staging the weights into shared memory.  stride = 0: one model for the whole batch.
+// A stack's metrics may take one target per model (gnca_rollout_metrics_targets): the forward entry points then take
+// target_stride, the floats between two models' targets in FrameMetrics::target (0 = one target for every sample), and
+// sample b measures against target + (b / per_model) * target_stride.  It is an argument of its own, not a field: both
+// FrameMetrics and ModelStack are kernel parameters by value ahead of or in the plain kernels' parameter lists, and a
+// larger struct would change the code of those kernels.
 struct ModelStack {
   int stride;      // floats between two models' packed buffers (Packed::total)
   int per_model;   // samples per model (B / n_models)
@@ -103,7 +108,7 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
                      const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                      float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st, int hist_every = 1,
                      const FrameMetrics* met = nullptr, ModelStack ms = ModelStack{0, 0},
-                     const SsimFrames* ss = nullptr);
+                     const SsimFrames* ss = nullptr, int target_stride = 0);
 
 // replicated-state cluster rollout (gnca_rep.cu): every CTA of a sample's cluster holds the whole sample; first
 // choice of the resident path.  scratch: >= B*C*H*W floats of device memory (overflow of the in-smem u buffer).
@@ -114,13 +119,14 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
 // met: the per-frame metrics of the steps t % met->every == 0 (a whole rollout, t0 = 0)
 // ms: a stack of models, one per block of ms.per_model samples, with or without records
 // ss (with met only): the SSIM of the same frames, by the kernel's SSIM instantiation (run_resident_fwd likewise)
+// target_stride (with met and ms only): per-model targets, see ModelStack (run_resident_fwd likewise)
 struct ZpRec;
 struct ZpBwd;
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                 float* u_hist, float* rec, uint32_t* masks, float* scratch, cudaStream_t st, int hist_every = 1,
                 int t0 = 0, const ZpRec* zp = nullptr, const FrameMetrics* met = nullptr,
-                ModelStack ms = ModelStack{0, 0}, const SsimFrames* ss = nullptr);
+                ModelStack ms = ModelStack{0, 0}, const SsimFrames* ss = nullptr, int target_stride = 0);
 // resident BPTT on the records of run_rep_fwd (gnca_rep_bwd.cu).  g_frames (optional, [F][B][C][H][W]): dL/dx_{f*every}
 // added at step f * every (gnca_rollout_bwd_bptt_frames)
 size_t rep_bptt_bytes(const gnca_model& m, int B, int H, int W, int T);     // 0: configuration not supported

@@ -71,6 +71,10 @@ struct RepArgs {
   // a stack of models (ModelStack): sample b stages its weights from packed + (b / model_per) * model_stride;
   // model_stride = 0: every sample runs the model at `packed`
   int model_stride, model_per;
+  // MET with per-model targets (run_rep_fwd's target_stride): sample b measures against M.target + (b / model_per) *
+  // target_stride; 0 = one target.  It fills the struct's tail padding, so the parameters of the plain instantiations
+  // keep their offsets.
+  int target_stride;
 };
 
 #ifdef GNCA_PHASE_COUNTERS          /* build with -DGNCA_PHASE_COUNTERS for the per-phase cycle counters */
@@ -112,15 +116,15 @@ __device__ __forceinline__ uint32_t pack_nibbles(uint32_t nib, int lane) {
 // Frame metrics of x_t (cell-major sX, alpha plane sAg) over cells [lo, hi), spread over warps [w0, kPW): each warp
 // leaves its partial as 4 doubles at the head of its own perception tile in sY, which is free from the end of its tiles
 // to the next step's tiles.  rep_met_flush (one thread, after a barrier) adds them in warp order.
-__device__ __forceinline__ void rep_met_cells(const FrameMetrics& M, const float* sX, const float* sAg, float* sY, int lo,
-                                              int hi, int HW, float thr, int w0) {
+__device__ __forceinline__ void rep_met_cells(const FrameMetrics& M, const float* tgt, const float* sX, const float* sAg,
+                                              float* sY, int lo, int hi, int HW, float thr, int w0) {
   constexpr int C = 16, kTile = 3 * C * 8;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   MetAcc acc{0.0, 0.0, 0, 0};
 #pragma unroll 1
   for (int cell = lo + (warp - w0) * 32 + lane; cell < hi; cell += (kPW - w0) * 32) {
     const float4 v = *reinterpret_cast<const float4*>(sX + (size_t)cell * C);
-    met_cell(acc, v.x, v.y, v.z, sAg[cell], M.target, cell, HW, M.eps, thr);
+    met_cell(acc, v.x, v.y, v.z, sAg[cell], tgt, cell, HW, M.eps, thr);
   }
   met_warp_sum(acc);
   if (lane == 0) met_put(reinterpret_cast<double*>(sY + warp * kTile), acc);
@@ -156,12 +160,18 @@ __device__ __forceinline__ void rep_ssim_flush(const float* sY, int w0, double* 
   *dst = s;
 }
 
+// the target sample b is measured against: M.target, or its model's with per-model targets (R.target_stride)
+__device__ __forceinline__ const float* rep_met_target(const RepArgs& R, const FrameMetrics& M, int b) {
+  return R.target_stride ? M.target + (size_t)(b / R.model_per) * R.target_stride : M.target;
+}
+
 // a whole frame's metrics (SS: and SSIM, into *ss_dst) by all warps, outside the tile phase of a step
 template <bool SS>
-__device__ __forceinline__ void rep_met_frame(const FrameMetrics& M, const float* sX, const float* sAg, float* sY, int lo,
-                                              int hi, int HW, float thr, double* dst, double* ss_dst, int H, int W) {
-  rep_met_cells(M, sX, sAg, sY, lo, hi, HW, thr, 0);
-  if constexpr (SS) rep_ssim_cells(sX, sAg, sY, M.target, lo, hi, H, W, 0);
+__device__ __forceinline__ void rep_met_frame(const FrameMetrics& M, const float* tgt, const float* sX, const float* sAg,
+                                              float* sY, int lo, int hi, int HW, float thr, double* dst, double* ss_dst,
+                                              int H, int W) {
+  rep_met_cells(M, tgt, sX, sAg, sY, lo, hi, HW, thr, 0);
+  if constexpr (SS) rep_ssim_cells(sX, sAg, sY, tgt, lo, hi, H, W, 0);
   __syncthreads();
   if (threadIdx.x == 0) {
     rep_met_flush(sY, 0, dst);
@@ -176,7 +186,8 @@ __device__ __forceinline__ void rep_met_frame(const FrameMetrics& M, const float
 // instantiation: the torus kernel (trainer, bench) is compiled exactly as before.
 // Z (ZP with records only, else unused): the softmax weights and row sums of every message step, for k_rep_bwd.
 // MET (gnca_rollout_metrics): at every step t % M.every == 0 each CTA reduces the cells it stores for the history,
-// [my_lo, my_hi), against M.target and writes one partial per (frame, sample, rank); M is unused otherwise.
+// [my_lo, my_hi), against M.target and writes one partial per (frame, sample, rank); M is unused otherwise.  With
+// R.target_stride (a stack with per-model targets) each reduction reads sample b's model's target (rep_met_target).
 // SS (with MET, gnca_rollout_metrics_ssim): at the same steps each CTA also sums the SSIM of its interior cells among
 // [my_lo, my_hi) into ssim_part[frame][b][rank]; ssim_part is unused otherwise.
 template <int C, bool ZP, bool MET, bool SS>
@@ -497,7 +508,8 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
       if (float* h = hist_at(t)) store_state(h, my_lo, my_hi);
       if constexpr (MET)
         if (t % M.every == 0)
-          rep_met_frame<SS>(M, sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr, met_dst + (t / M.every) * met_frame_stride,
+          rep_met_frame<SS>(M, rep_met_target(R, M, b), sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr,
+                            met_dst + (t / M.every) * met_frame_stride,
                             ssim_part + ((size_t)(t / M.every) * a.B + b) * NC + rank, H, W);
       continue;
     }
@@ -819,8 +831,11 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
           }
         }
       }
-      if constexpr (MET) if (hist && t % M.every == 0) rep_met_cells(M, sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr, 1);
-      if constexpr (SS) if (hist && t % M.every == 0) rep_ssim_cells(sX, sAg, sY, M.target, my_lo, my_hi, H, W, 1);
+      if constexpr (MET)
+        if (hist && t % M.every == 0)
+          rep_met_cells(M, rep_met_target(R, M, b), sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr, 1);
+      if constexpr (SS)
+        if (hist && t % M.every == 0) rep_ssim_cells(sX, sAg, sY, rep_met_target(R, M, b), my_lo, my_hi, H, W, 1);
     };
     const bool had_tile = n_my <= 32 ? (2 * warp < n_my) : n_my <= 64 ? (4 * warp < n_my) : (((n_my * warp) >> 4) < ((n_my * (warp + 1)) >> 4));
     const bool fire_early = !use_async || !had_tile;
@@ -1005,7 +1020,8 @@ __global__ void __launch_bounds__(kPT, 1) k_rep_fwd(RepArgs R, Packed P, const f
   if (float* h = hist_at(R.T)) store_state(h, my_lo, my_hi);
   if constexpr (MET)
     if (R.T % M.every == 0)
-      rep_met_frame<SS>(M, sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr, met_dst + (R.T / M.every) * met_frame_stride,
+      rep_met_frame<SS>(M, rep_met_target(R, M, b), sX, sAg, sY, my_lo, my_hi, HW, a.alpha_thr,
+                        met_dst + (R.T / M.every) * met_frame_stride,
                         ssim_part + ((size_t)(R.T / M.every) * a.B + b) * NC + rank, H, W);
   store_state(R.xT + sample_off, my_lo, my_hi);
   if (R.dbg && blockIdx.x == R.dbg_cta && tid < 24) R.dbg[tid] = s_dbg[tid];
@@ -1047,7 +1063,8 @@ static size_t rep_smem_bytes(int C, int HW, int ucap, int listcap) {
 int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                 const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                 float* u_hist, float* rec, uint32_t* masks, float* scratch /* >= B*C*H*W floats */, cudaStream_t st,
-                int hist_every, int t0, const ZpRec* zpr, const FrameMetrics* met, ModelStack ms, const SsimFrames* ss) {
+                int hist_every, int t0, const ZpRec* zpr, const FrameMetrics* met, ModelStack ms, const SsimFrames* ss,
+                int target_stride) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (m.C != 16 || m.hidden != 128) return GNCA_ERR_UNSUPPORTED;
   if (H > kMaxRows || W > kMaxRows || H < 1 || W < 4 || (W & 3)) return GNCA_ERR_UNSUPPORTED;   // quads of 4 cells per row
@@ -1079,7 +1096,7 @@ int run_rep_fwd(const gnca_model& m, const Packed& P, const float* packed, int B
   R.damage = DamageView{sched.damage, sched.damage_layout}; R.damage_step = sched.damage_step;
   R.KP = k > 8 ? 16 : 8;
   R.zd = zp ? m.d_model : 0;
-  R.model_stride = ms.stride; R.model_per = ms.per_model;
+  R.model_stride = ms.stride; R.model_per = ms.per_model; R.target_stride = target_stride;
   // the metrics (and SSIM) instantiations have the same shared memory and register cap as the plain ones: the same
   // launch configuration, so x_T is bit-equal to the rollout without metrics
   const bool ssim = met && ss;

@@ -93,13 +93,15 @@ __device__ __noinline__ bool alive_local_ool(const float* plane, int lr, int x, 
 // against M.target and writes one partial per (frame, sample, rank); M is unused otherwise.
 // MS (a stack of models, gnca_rollout_*_models): sample b stages its weights from packed + (b / S.per_model) * S.stride;
 // S is unused otherwise.  A compile-time flag: a runtime field moves the register allocation of the plain kernels.
+// MET with MS: sample b measures against M.target + (b / S.per_model) * target_stride (0: one target for the stack), a
+// trailing parameter as ssim_part is; unused otherwise.
 // SS (with MET, gnca_rollout_metrics_ssim): at the same steps each CTA also sums the SSIM of the interior cells of its
 // own rows into ssim_part[frame][b][rank], reading the window rows it does not own from their owners over DSMEM between
 // two cluster barriers; ssim_part is unused otherwise.
 template <int C, bool MET, bool MS, bool SS>
 __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, Packed P, int hid,
                                                                const float* __restrict__ packed, FrameMetrics M,
-                                                               ModelStack S, double* ssim_part) {
+                                                               ModelStack S, double* ssim_part, int target_stride) {
   static_assert(MET || !SS, "SSIM rides on the metrics steps");
   cg::cluster_group cluster = cg::this_cluster();
   constexpr int C3 = 3 * C;
@@ -219,12 +221,23 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
   };
   // frame metrics of x_t over the own rows; the warps' partials go through the head of the hidden-layer staging
   // buffer Ht, which is free outside P2
+  // sample b's target, formed at each use from %ctaid.x and the parameters: the volatile read keeps the compiler from
+  // hoisting the rebased pointer out of the step loop, where it would cost two registers (at C = 32 with SSIM, spills)
+  auto met_target = [&]() -> const float* {
+    if constexpr (MS) {
+      unsigned cta;
+      asm volatile("mov.u32 %0, %%ctaid.x;" : "=r"(cta));
+      return M.target + (size_t)((int)cta / NC / S.per_model) * target_stride;
+    }
+    return M.target;
+  };
   auto met_frame = [&](int t) {
+    const float* tgt = met_target();
     MetAcc acc{0.0, 0.0, 0, 0};
 #pragma unroll 1
     for (int oc = tid; oc < nown; oc += kRThreads) {
       const float* px = sX + HALO * W + oc;
-      met_cell(acc, px[0], px[PL], px[2 * (size_t)PL], px[3 * (size_t)PL], M.target, r0 * W + oc, HW, M.eps,
+      met_cell(acc, px[0], px[PL], px[2 * (size_t)PL], px[3 * (size_t)PL], tgt, r0 * W + oc, HW, M.eps,
                a.alpha_thr);
     }
     met_warp_sum(acc);
@@ -239,6 +252,7 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
   // damage) visible, the second keeps the rows unchanged until every peer has read them.
   auto ssim_frame = [&](int t) {
     cluster.sync();
+    const float* tgt = met_target();
     auto state = [&](int yy, int xx) {
       const int q = yy / own;
       const float* p = cluster.map_shared_rank(sX, q) + (size_t)(HALO + yy - q * own) * W + xx;
@@ -248,7 +262,7 @@ __global__ void __launch_bounds__(kRThreads, 1) k_resident_fwd(ResidentArgs R, P
 #pragma unroll 1
     for (int oc = tid; oc < nown; oc += kRThreads) {
       const int y = r0 + oc / W, x = oc % W;
-      if (ssim_interior(y, x, H, W)) s += ssim_cell(state, M.target, y, x, W, HW);
+      if (ssim_interior(y, x, H, W)) s += ssim_cell(state, tgt, y, x, W, HW);
     }
     s = warp_sum_f64(s);
     double* s_ss = reinterpret_cast<double*>(Ht);
@@ -687,7 +701,8 @@ static size_t resident_smem_bytes(int C, int hid, bool graph, int own, int halo,
 
 template <int C>
 static int launch_resident(const gnca_model& m, const Packed& P, const float* packed, ResidentArgs& R, int B, int radius,
-                           cudaStream_t st, const FrameMetrics* met, ModelStack S, const SsimFrames* ss) {
+                           cudaStream_t st, const FrameMetrics* met, ModelStack S, const SsimFrames* ss,
+                           int target_stride) {
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   const int H = R.s.H, W = R.s.W;
   if (m.hidden != 128 || C < 4 || W > 255) return GNCA_ERR_UNSUPPORTED;   // layer 1 + 2 of a tile live in one warp: 32 lanes x 4 units
@@ -769,7 +784,7 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
     }
     prof_begin(PROF_RESIDENT_FWD, st);
     cudaError_t e = cudaLaunchKernelEx(&cfg, kfn, R, P, m.hidden, packed, met ? *met : FrameMetrics{}, S,
-                                       ssim ? ss->part : nullptr);
+                                       ssim ? ss->part : nullptr, target_stride);
     prof_end(PROF_RESIDENT_FWD, st);
     if (e != cudaSuccess) return (int)e;
     GNCA_LAUNCH_CHECK();
@@ -800,7 +815,7 @@ static int launch_resident(const gnca_model& m, const Packed& P, const float* pa
 int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, int B, int H, int W,
                      const gnca_schedule& sched, const float* x0, float* xT, float* hist, float* stats_hist,
                      float* u_hist, float* ping, float* pong, float* alpha_tmp, cudaStream_t st, int hist_every,
-                     const FrameMetrics* met, ModelStack ms, const SsimFrames* ss) {
+                     const FrameMetrics* met, ModelStack ms, const SsimFrames* ss, int target_stride) {
   (void)ping; (void)pong; (void)alpha_tmp;
   const bool graph = (m.flags & GNCA_F_GRAPH) != 0;
   if (graph && !(m.flags & GNCA_F_TORUS) && sched.k > 0) return GNCA_ERR_UNSUPPORTED;   // zero-pad: streaming path
@@ -820,10 +835,10 @@ int run_resident_fwd(const gnca_model& m, const Packed& P, const float* packed, 
   R.damage = DamageView{sched.damage, sched.damage_layout}; R.damage_step = sched.damage_step;
   const int radius = sched.max_offset;       // largest |dy| / |dx| in the schedule: sets the halo depth
   switch (m.C) {
-    case 4: return launch_resident<4>(m, P, packed, R, B, radius, st, met, ms, ss);
-    case 8: return launch_resident<8>(m, P, packed, R, B, radius, st, met, ms, ss);
-    case 16: return launch_resident<16>(m, P, packed, R, B, radius, st, met, ms, ss);
-    case 32: return launch_resident<32>(m, P, packed, R, B, radius, st, met, ms, ss);
+    case 4: return launch_resident<4>(m, P, packed, R, B, radius, st, met, ms, ss, target_stride);
+    case 8: return launch_resident<8>(m, P, packed, R, B, radius, st, met, ms, ss, target_stride);
+    case 16: return launch_resident<16>(m, P, packed, R, B, radius, st, met, ms, ss, target_stride);
+    case 32: return launch_resident<32>(m, P, packed, R, B, radius, st, met, ms, ss, target_stride);
   }
   return GNCA_ERR_UNSUPPORTED;
 }

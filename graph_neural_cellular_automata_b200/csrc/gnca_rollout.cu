@@ -67,12 +67,17 @@ int run_metrics_reduce(int rows, int P, const double* part, double* sums, int* c
   return 0;
 }
 
-// metrics of frame f (the state x) on the streaming path
-static int frame_metrics(const FrameMetrics& met, const float* x, int f, int B, int C, int HW, float thr,
-                         cudaStream_t st) {
+// metrics of frame f (the state x) on the streaming path.  per < B: one launch per block of `per` samples, block i
+// against target + i * tstride (a stack with per-model targets), into the same partial rows
+static int frame_metrics(const FrameMetrics& met, const float* x, int f, int B, int C, int HW, float thr, int per,
+                         int tstride, cudaStream_t st) {
   const int P = frame_metrics_parts(HW);
-  k_frame_metrics<<<dim3(P, B), kMetThreads, 0, st>>>(x, C, HW, met.target, met.eps, thr, met.part);
-  GNCA_LAUNCH_CHECK();
+  for (int b0 = 0; b0 < B; b0 += per) {
+    k_frame_metrics<<<dim3(P, per), kMetThreads, 0, st>>>(x + (size_t)b0 * C * HW, C, HW,
+                                                          met.target + (size_t)(b0 / per) * tstride, met.eps, thr,
+                                                          met.part + (size_t)b0 * P * 4);
+    GNCA_LAUNCH_CHECK();
+  }
   return run_metrics_reduce(B, P, met.part, met.sums + (size_t)f * B * 2, met.counts + (size_t)f * B * 2, st);
 }
 
@@ -125,21 +130,29 @@ int run_ssim_reduce(int rows, int P, const double* part, double* ssim, int H, in
   return 0;
 }
 
-// SSIM of the B samples of x into ssim[B], through part (>= B * frame_ssim_parts(H * W) doubles)
+// SSIM of the B samples of x into ssim[B], through part (>= B * frame_ssim_parts(H * W) doubles); per / tstride as in
+// frame_metrics
 static int frame_ssim(const float* x, int B, int C, int H, int W, const float* tgt, double* part, double* ssim,
-                      cudaStream_t st) {
+                      cudaStream_t st, int per = 0, int tstride = 0) {
   const int P = frame_ssim_parts(H * W);
-  k_frame_ssim<<<dim3(P, B), kMetThreads, 0, st>>>(x, C, H, W, tgt, part);
-  GNCA_LAUNCH_CHECK();
+  if (per == 0) per = B;
+  for (int b0 = 0; b0 < B; b0 += per) {
+    k_frame_ssim<<<dim3(P, per), kMetThreads, 0, st>>>(x + (size_t)b0 * C * H * W, C, H, W,
+                                                       tgt + (size_t)(b0 / per) * tstride, part + (size_t)b0 * P);
+    GNCA_LAUNCH_CHECK();
+  }
   return run_ssim_reduce(B, P, part, ssim, H, W, st);
 }
 
-// the metrics of frame f on the streaming path, with its SSIM when ss is set
+// the metrics of frame f on the streaming path, with its SSIM when ss is set.  A stack with a target stride: each
+// model's samples against its own target (x_0 of a stack at T = 0: a stack runs no streaming step)
 static int frame_quality(const FrameMetrics& met, const SsimFrames* ss, const float* x, int f, int B, int C, int H,
-                         int W, float thr, cudaStream_t st) {
-  int rc = frame_metrics(met, x, f, B, C, H * W, thr, st);
+                         int W, float thr, cudaStream_t st, const ModelStack* ms, int target_stride) {
+  const bool own = ms && target_stride;
+  const int per = own ? ms->per_model : B, tstride = own ? target_stride : 0;
+  int rc = frame_metrics(met, x, f, B, C, H * W, thr, per, tstride, st);
   if (rc || !ss) return rc;
-  return frame_ssim(x, B, C, H, W, met.target, ss->part, ss->ssim + (size_t)f * B, st);
+  return frame_ssim(x, B, C, H, W, met.target, ss->part, ss->ssim + (size_t)f * B, st, per, tstride);
 }
 
 static int launch_add(size_t n, float* out, const float* a, const float* b, cudaStream_t st) {
@@ -303,11 +316,12 @@ static Segment carve_segment(void* base, const gnca_model& m, int B, int H, int 
 // ss (with met only): the SSIM of the same frames (gnca_rollout_metrics_ssim)
 // ms: a stack of models (gnca_rollout_*_models): the steps run on a cluster kernel or not at all, since only those stage
 // their weights per sample.  T = 0 reads no weight and takes the copy path below.
+// target_stride (with met and ms): model i's metrics against met->target + i * target_stride (gnca_rollout_metrics_targets)
 static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
                        const float* x0_dev, float* xT_dev, float* x_hist_dev, int every, float* stats_hist_dev,
                        float* u_hist_dev, void* workspace_dev, size_t workspace_bytes, int impl, void* stream,
                        const FrameMetrics* met = nullptr, const ModelStack* ms = nullptr,
-                       const SsimFrames* ss = nullptr) {
+                       const SsimFrames* ss = nullptr, int target_stride = 0) {
   if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !workspace_dev) return GNCA_ERR_ARG;
   if (B <= 0 || H <= 0 || W <= 0 || sched->T < 0) return GNCA_ERR_ARG;
   if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
@@ -330,10 +344,11 @@ static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int 
       int rc = GNCA_ERR_UNSUPPORTED;
       if (impl != 3)
         rc = run_rep_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, x_hist_dev, stats_hist_dev, u_hist_dev,
-                         nullptr, nullptr, r.ping, st, every, 0, nullptr, met, ms ? *ms : one, ss);
+                         nullptr, nullptr, r.ping, st, every, 0, nullptr, met, ms ? *ms : one, ss, target_stride);
       if (rc == GNCA_ERR_UNSUPPORTED)
         rc = run_resident_fwd(*m, P, packed_dev, B, H, W, *sched, x0_dev, xT_dev, x_hist_dev, stats_hist_dev,
-                              u_hist_dev, r.ping, r.pong, r.alpha_tmp, st, every, met, ms ? *ms : one, ss);
+                              u_hist_dev, r.ping, r.pong, r.alpha_tmp, st, every, met, ms ? *ms : one, ss,
+                              target_stride);
       if (rc != GNCA_ERR_UNSUPPORTED || impl == 2 || impl == 3 || ms) return rc;
     }
   }
@@ -352,7 +367,7 @@ static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int 
       if (rc) return rc;
     }
     if (met && t % met->every == 0) {
-      int rc = frame_quality(*met, ss, x_at(t), t / met->every, B, m->C, H, W, m->alpha_thr, st);
+      int rc = frame_quality(*met, ss, x_at(t), t / met->every, B, m->C, H, W, m->alpha_thr, st, ms, target_stride);
       if (rc) return rc;
     }
     StepArgs a;
@@ -368,7 +383,8 @@ static int rollout_fwd(const gnca_model* m, const float* packed_dev, int B, int 
   }
   if ((x_hist_dev && T % every == 0) || T == 0)
     GNCA_CHECK_CUDA(cudaMemcpyAsync(xT_dev, x_at(T), N * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  if (met && T % met->every == 0) return frame_quality(*met, ss, xT_dev, T / met->every, B, m->C, H, W, m->alpha_thr, st);
+  if (met && T % met->every == 0)
+    return frame_quality(*met, ss, xT_dev, T / met->every, B, m->C, H, W, m->alpha_thr, st, ms, target_stride);
   return 0;
 }
 
@@ -527,12 +543,14 @@ size_t gnca_metrics_scratch_bytes(const gnca_model* m, int B, int H, int W, int 
 
 static int model_stack(const gnca_model& m, int n_models, int B, int impl, ModelStack* ms);
 
-// the shared body of gnca_rollout_metrics[_ssim][_models]: n_models = 0 runs one model, ssim_dev = NULL skips SSIM
+// the shared body of gnca_rollout_metrics[_ssim][_models] and gnca_rollout_metrics_targets: n_models = 0 runs one
+// model, ssim_dev = NULL skips SSIM.  own_targets (a stack only): target_dev is [n_models][4][H][W], one per model;
+// otherwise one [4][H][W] target for every sample
 static int rollout_metrics(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
                            const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
-                           const float* target_dev, float eps, double* sums_dev, int32_t* counts_dev, double* ssim_dev,
-                           bool want_ssim, void* scratch_dev, size_t scratch_bytes, void* workspace_dev,
-                           size_t workspace_bytes, int impl, void* stream) {
+                           const float* target_dev, bool own_targets, float eps, double* sums_dev, int32_t* counts_dev,
+                           double* ssim_dev, bool want_ssim, void* scratch_dev, size_t scratch_bytes,
+                           void* workspace_dev, size_t workspace_bytes, int impl, void* stream) {
   if (!m || !packed_dev || !sched || !x0_dev || !xT_dev || !target_dev || !sums_dev || !counts_dev || !scratch_dev ||
       !workspace_dev || (want_ssim && !ssim_dev))
     return GNCA_ERR_ARG;
@@ -544,6 +562,8 @@ static int rollout_metrics(const gnca_model* m, const float* packed_dev, int n_m
     int rc = model_stack(*m, n_models, B, impl, &ms);
     if (rc) return rc;
   }
+  const long long target_stride = own_targets ? 4LL * H * W : 0;     // an int in the kernels
+  if (target_stride > 0x7fffffffLL) return GNCA_ERR_UNSUPPORTED;
   if (!model_supported(*m)) return GNCA_ERR_UNSUPPORTED;
   if (sched->k < 0 || sched->k > GNCA_MAX_K) return GNCA_ERR_UNSUPPORTED;
   const size_t met_bytes = gnca_metrics_scratch_bytes(m, B, H, W, sched->T, every);
@@ -552,15 +572,17 @@ static int rollout_metrics(const gnca_model* m, const float* packed_dev, int n_m
   const FrameMetrics met{target_dev, reinterpret_cast<double*>(scratch_dev), sums_dev, counts_dev, eps, every};
   const SsimFrames ss{reinterpret_cast<double*>(static_cast<char*>(scratch_dev) + met_bytes), ssim_dev};
   return rollout_fwd(m, packed_dev, B, H, W, sched, x0_dev, xT_dev, nullptr, 1, nullptr, nullptr, workspace_dev,
-                     workspace_bytes, impl, stream, &met, n_models > 0 ? &ms : nullptr, want_ssim ? &ss : nullptr);
+                     workspace_bytes, impl, stream, &met, n_models > 0 ? &ms : nullptr, want_ssim ? &ss : nullptr,
+                     (int)target_stride);
 }
 
 int gnca_rollout_metrics(const gnca_model* m, const float* packed_dev, int B, int H, int W, const gnca_schedule* sched,
                          const float* x0_dev, float* xT_dev, int every, const float* target_dev, float eps,
                          double* sums_dev, int32_t* counts_dev, void* scratch_dev, size_t scratch_bytes,
                          void* workspace_dev, size_t workspace_bytes, int impl, void* stream) {
-  return rollout_metrics(m, packed_dev, 0, B, H, W, sched, x0_dev, xT_dev, every, target_dev, eps, sums_dev, counts_dev,
-                         nullptr, false, scratch_dev, scratch_bytes, workspace_dev, workspace_bytes, impl, stream);
+  return rollout_metrics(m, packed_dev, 0, B, H, W, sched, x0_dev, xT_dev, every, target_dev, false, eps, sums_dev,
+                         counts_dev, nullptr, false, scratch_dev, scratch_bytes, workspace_dev, workspace_bytes, impl,
+                         stream);
 }
 
 size_t gnca_metrics_ssim_scratch_bytes(const gnca_model* m, int B, int H, int W, int T, int every) {
@@ -577,8 +599,9 @@ int gnca_rollout_metrics_ssim(const gnca_model* m, const float* packed_dev, int 
                               const float* target_dev, float eps, double* sums_dev, int32_t* counts_dev,
                               double* ssim_dev, void* scratch_dev, size_t scratch_bytes, void* workspace_dev,
                               size_t workspace_bytes, int impl, void* stream) {
-  return rollout_metrics(m, packed_dev, 0, B, H, W, sched, x0_dev, xT_dev, every, target_dev, eps, sums_dev, counts_dev,
-                         ssim_dev, true, scratch_dev, scratch_bytes, workspace_dev, workspace_bytes, impl, stream);
+  return rollout_metrics(m, packed_dev, 0, B, H, W, sched, x0_dev, xT_dev, every, target_dev, false, eps, sums_dev,
+                         counts_dev, ssim_dev, true, scratch_dev, scratch_bytes, workspace_dev, workspace_bytes, impl,
+                         stream);
 }
 
 size_t gnca_ssim_rgb_scratch_bytes(int B, int H, int W) {
@@ -625,9 +648,9 @@ int gnca_rollout_metrics_models(const gnca_model* m, const float* packed_dev, in
                                 void* scratch_dev, size_t scratch_bytes, void* workspace_dev, size_t workspace_bytes,
                                 int impl, void* stream) {
   if (n_models < 1) return GNCA_ERR_ARG;
-  return rollout_metrics(m, packed_dev, n_models, B, H, W, sched, x0_dev, xT_dev, every, target_dev, eps, sums_dev,
-                         counts_dev, nullptr, false, scratch_dev, scratch_bytes, workspace_dev, workspace_bytes, impl,
-                         stream);
+  return rollout_metrics(m, packed_dev, n_models, B, H, W, sched, x0_dev, xT_dev, every, target_dev, false, eps,
+                         sums_dev, counts_dev, nullptr, false, scratch_dev, scratch_bytes, workspace_dev,
+                         workspace_bytes, impl, stream);
 }
 
 int gnca_rollout_metrics_ssim_models(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
@@ -636,9 +659,20 @@ int gnca_rollout_metrics_ssim_models(const gnca_model* m, const float* packed_de
                                      double* ssim_dev, void* scratch_dev, size_t scratch_bytes, void* workspace_dev,
                                      size_t workspace_bytes, int impl, void* stream) {
   if (n_models < 1) return GNCA_ERR_ARG;
-  return rollout_metrics(m, packed_dev, n_models, B, H, W, sched, x0_dev, xT_dev, every, target_dev, eps, sums_dev,
-                         counts_dev, ssim_dev, true, scratch_dev, scratch_bytes, workspace_dev, workspace_bytes, impl,
-                         stream);
+  return rollout_metrics(m, packed_dev, n_models, B, H, W, sched, x0_dev, xT_dev, every, target_dev, false, eps,
+                         sums_dev, counts_dev, ssim_dev, true, scratch_dev, scratch_bytes, workspace_dev,
+                         workspace_bytes, impl, stream);
+}
+
+int gnca_rollout_metrics_targets(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                 const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                                 const float* targets_dev, float eps, double* sums_dev, int32_t* counts_dev,
+                                 double* ssim_dev, void* scratch_dev, size_t scratch_bytes, void* workspace_dev,
+                                 size_t workspace_bytes, int impl, void* stream) {
+  if (!targets_dev || n_models < 1 || B % n_models != 0) return GNCA_ERR_ARG;
+  return rollout_metrics(m, packed_dev, n_models, B, H, W, sched, x0_dev, xT_dev, every, targets_dev, true, eps,
+                         sums_dev, counts_dev, ssim_dev, ssim_dev != nullptr, scratch_dev, scratch_bytes, workspace_dev,
+                         workspace_bytes, impl, stream);
 }
 
 int gnca_rollout_bwd_frames(const gnca_model* m, const float* packed_dev, int B, int H, int W,

@@ -1069,14 +1069,18 @@ def record_rollout(model, x0: torch.Tensor, schedule: Schedule, *, every: int, a
 @dataclass
 class Monitor:
     """What `monitor_rollout` returns.  Row f of every [F,B] tensor is frame f of `record_rollout(..., every=S)`:
-    x_{t[f]}, after the schedule's damage at `damage_step`, frozen for a sample with steps[b] <= t[f]."""
+    x_{t[f]}, after the schedule's damage at `damage_step`, frozen for a sample with steps[b] <= t[f].
+
+    "The target" of a column is the call's [4,H,W] target, or, for a stack of M models given a [M,4,H,W] target,
+    target[i] for model i's columns i*B:(i+1)*B (B samples per model)."""
     t: List[int]                            # step indices 0, S, 2S, ... <= T
-    loss: torch.Tensor                      # [F,B] f32: premultiplied-RGBA MSE against the target
-    psnr: torch.Tensor                      # [F,B] f32: utils.metrics.psnr_rgb
+    loss: torch.Tensor                      # [F,B] f32: premultiplied-RGBA MSE against the column's target
+    psnr: torch.Tensor                      # [F,B] f32: utils.metrics.psnr_rgb against the column's target
     pixel_perfect: torch.Tensor             # [F,B] f32: utils.metrics.pixel_perfect(frame, target, eps)
     alive: torch.Tensor                     # [F,B] int64: cells with alpha > model.alpha_thr (no dilation)
     x_T: torch.Tensor                       # [B,C,H,W]
-    ssim: Optional[torch.Tensor] = None     # [F,B] f32: utils.metrics.ssim_rgb (monitor_rollout(..., ssim=True))
+    ssim: Optional[torch.Tensor] = None     # [F,B] f32: utils.metrics.ssim_rgb against the column's target
+                                            # (monitor_rollout(..., ssim=True))
 
 
 def monitor_rollout(model, x0: torch.Tensor, schedule: Schedule, target: torch.Tensor, *, every: int,
@@ -1092,7 +1096,10 @@ def monitor_rollout(model, x0: torch.Tensor, schedule: Schedule, target: torch.T
     (gnca_rollout_metrics_models), x0 [M*B, C, H, W] model-major, every [F, M*B] curve and x_T with the sample axis M*B
     long, model i's curves at `[:, i*B:(i+1)*B]`.  Build the schedule with `make_schedule(models[0], M*B, ...)` so that
     every model sees the same offsets, fire draws and damage.  impl='streaming' raises ValueError; a shape neither
-    cluster kernel takes raises the library's RuntimeError.
+    cluster kernel takes raises the library's RuntimeError.  With a list, `target` may also be [M, 4, H, W], one
+    target per model (gnca_rollout_metrics_targets): model i's curves are measured against target[i], so a target
+    sweep (one model trained per image) compares in one call.  A [4, H, W] target is shared by all M; any other count
+    of targets raises ValueError.
 
     ssim=True adds `Monitor.ssim`, the SSIM of every frame against the target as `utils.metrics.ssim_rgb` defines it
     (skimage's structural_similarity on clip(premultiplied RGB, 0, 1), 7x7 uniform windows, data_range 1), computed
@@ -1123,9 +1130,13 @@ def monitor_rollout(model, x0: torch.Tensor, schedule: Schedule, target: torch.T
         raise ValueError(f"x0 has {Cc} channels, model has {desc.C}")
     if desc.C < 4:
         raise ValueError(f"monitor_rollout: the metrics read RGBA (channels 0-3); the model has {desc.C} channels")
-    if tuple(target.shape) != (4, H, W):
-        raise ValueError(f"monitor_rollout: target must be [4, {H}, {W}] (premultiplied RGBA), got "
-                         f"{list(target.shape)}")
+    per_model = stack and target.dim() == 4
+    if per_model and tuple(target.shape[1:]) == (4, H, W) and target.shape[0] != M:
+        raise ValueError(f"monitor_rollout: {target.shape[0]} targets for {M} models; a per-model target is "
+                         f"[{M}, 4, {H}, {W}]")
+    if tuple(target.shape) != ((M, 4, H, W) if per_model else (4, H, W)):
+        want = f"[4, {H}, {W}]" + (f" or [{M}, 4, {H}, {W}]" if stack else "")
+        raise ValueError(f"monitor_rollout: target must be {want} (premultiplied RGBA), got {list(target.shape)}")
     if ssim and (H < 7 or W < 7):
         raise ValueError(f"monitor_rollout: SSIM needs a 7x7 window inside the grid, got H={H}, W={W}")
     x0 = GF._require_cuda_f32(x0.detach(), "x0")
@@ -1143,7 +1154,12 @@ def monitor_rollout(model, x0: torch.Tensor, schedule: Schedule, target: torch.T
     ws = GF._WS.get(x0.device, lib.gnca_rollout_workspace_bytes(C.byref(desc), B, H, W, T))
     cs = schedule.c_struct()
     ss = torch.empty(F, B, dtype=torch.float64, device=x0.device) if ssim else None
-    if ssim and stack:
+    if per_model:
+        _lib.check(lib.gnca_rollout_metrics_targets(
+            C.byref(desc), GF._ptr(_stack_packed(models)), M, B, H, W, C.byref(cs), GF._ptr(x0), GF._ptr(xT), every,
+            GF._ptr(target), eps, GF._ptr(sums), GF._ptr(counts), GF._ptr(ss), GF._ptr(scratch), scratch.numel(),
+            GF._ptr(ws), ws.numel(), IMPL[impl], GF._stream()), "gnca_rollout_metrics_targets")
+    elif ssim and stack:
         _lib.check(lib.gnca_rollout_metrics_ssim_models(
             C.byref(desc), GF._ptr(_stack_packed(models)), M, B, H, W, C.byref(cs), GF._ptr(x0), GF._ptr(xT), every,
             GF._ptr(target), eps, GF._ptr(sums), GF._ptr(counts), GF._ptr(ss), GF._ptr(scratch), scratch.numel(),

@@ -5,7 +5,8 @@ because a sample's cluster of at most 8 CTAs sets the step time; a seed or learn
 
 Each model keeps its own SamplePool and FusedNormalizedAdam, so its checkpoints (utils/checkpoint.py, torch_state_dict)
 are those of a single-model run.  The models share the schedule of an iteration (step counts, fire rates, offsets, the
-Philox stream) and the damage policy draw; the pools are drawn model by model.
+Philox stream) and the damage policy draw; the pools are drawn model by model.  They share the target too, or each
+trains towards its own (a target sweep: one model per image).
 """
 from __future__ import annotations
 
@@ -30,9 +31,12 @@ class PopulationTrainer(GraphNCATrainer):
     pool replace.  With one model it consumes the host RNG exactly as GraphNCATrainer(fire="philox") and gives
     bit-identical parameters, Adam moments, losses and pool.
 
+    `target`: [4, H, W] premultiplied RGBA shared by every model, or [M, 4, H, W], model i training towards target[i]
+    (premult_loss with per-model targets; nothing else about the iteration changes).
+
     `learning_rates`: one base learning rate per model (default cfg.learning_rate for all).  Production mode only:
     fire="torch", a BPTT budget, rollout_impl other than "auto" / "resident", more than one rank, or a learning-rate list
-    whose length is not M raise ValueError."""
+    whose length is not M, or a [M', 4, H, W] target with M' != M raise ValueError."""
 
     def __init__(self, models: Sequence, target: torch.Tensor, cfg: TrainConfig, *,
                  learning_rates: Optional[Sequence[float]] = None, seed_fn=None):
@@ -48,6 +52,8 @@ class PopulationTrainer(GraphNCATrainer):
             raise ValueError("PopulationTrainer: runs on one rank (no data-parallel populations)")
         _model_stack(models, None, "PopulationTrainer", cfg.rollout_impl)
         M = len(models)
+        if target.dim() == 4 and target.shape[0] != M:
+            raise ValueError(f"PopulationTrainer: {target.shape[0]} targets for {M} models")
         lrs = [cfg.learning_rate] * M if learning_rates is None else [float(v) for v in learning_rates]
         if len(lrs) != M:
             raise ValueError(f"PopulationTrainer: {len(lrs)} learning rates for {M} models")

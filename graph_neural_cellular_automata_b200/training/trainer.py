@@ -84,13 +84,32 @@ def scheduled_message_gain(epoch: int, base: float) -> float:
 
 
 def premult_loss(x: torch.Tensor, target: torch.Tensor, scale: float, want_grad: bool = True):
-    """Per-sample premultiplied-RGBA MSE (train...:52-61) and d(scale * sum_b loss_b)/dx, one fused kernel."""
+    """Per-sample premultiplied-RGBA MSE (train...:52-61) and d(scale * sum_b loss_b)/dx, one fused kernel.
+
+    `target` is [4, H, W], or [M, 4, H, W] with M dividing the batch: sample b is then measured against
+    target[b // (B // M)], the per-model targets of a model-major stack (PopulationTrainer)."""
+    stacked = target.dim() == 4
+    if stacked:
+        B, _, H, W = x.shape
+        M = target.shape[0]
+        if tuple(target.shape[1:]) != (4, H, W) or M < 1 or B % M:
+            raise ValueError(f"premult_loss: target must be [4, {H}, {W}] or [M, 4, {H}, {W}] with M dividing the "
+                             f"batch of {B}, got {list(target.shape)}")
+        target = GF._require_cuda_f32(target, "target")
     x = GF._require_cuda_f32(x, "x")
     B, Cc, H, W = x.shape
+    if stacked and target.device != x.device:
+        raise ValueError(f"premult_loss: target is on {target.device}, x on {x.device}")
     per = torch.empty(B, dtype=torch.float32, device=x.device)
     gx = torch.empty_like(x) if want_grad else None
-    _lib.check(_lib.load().gnca_loss_premult_rgba(B, Cc, H, W, GF._ptr(x), GF._ptr(target.contiguous()), GF._ptr(per),
-                                                  GF._ptr(gx), float(scale), GF._stream()), "gnca_loss_premult_rgba")
+    lib = _lib.load()
+    if stacked:
+        _lib.check(lib.gnca_loss_premult_rgba_targets(B, Cc, H, W, GF._ptr(x), GF._ptr(target), M, GF._ptr(per),
+                                                      GF._ptr(gx), float(scale), GF._stream()),
+                   "gnca_loss_premult_rgba_targets")
+    else:
+        _lib.check(lib.gnca_loss_premult_rgba(B, Cc, H, W, GF._ptr(x), GF._ptr(target.contiguous()), GF._ptr(per),
+                                              GF._ptr(gx), float(scale), GF._stream()), "gnca_loss_premult_rgba")
     return per, gx
 
 

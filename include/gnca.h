@@ -301,6 +301,23 @@ int gnca_rollout_metrics_ssim_models(const gnca_model* m, const float* packed_de
                                      double* ssim_dev, void* scratch_dev, size_t scratch_bytes, void* workspace_dev,
                                      size_t workspace_bytes, int impl, void* stream);
 
+/*
+ * A target per model: gnca_rollout_metrics_ssim_models where model i (samples [i * B / n_models, (i + 1) * B /
+ * n_models)) is measured against targets_dev[i] ([n_models][4][H][W], premultiplied RGBA), for a target sweep.
+ * ssim_dev = NULL skips the SSIM (gnca_rollout_metrics_models).  Scratch from gnca_metrics_scratch_bytes, or
+ * gnca_metrics_ssim_scratch_bytes with ssim_dev.  With every targets_dev[i] equal to one target the results are
+ * bit-identical to the _models calls with that target; model i's block equals block i of the _models call with the
+ * target targets_dev[i].
+ * Argument errors return before any launch: a NULL targets_dev, n_models < 1 and B % n_models != 0 are GNCA_ERR_ARG;
+ * every other case is that of the _models calls (GNCA_ERR_UNSUPPORTED for impl 1 and for shapes no cluster kernel
+ * takes).
+ */
+int gnca_rollout_metrics_targets(const gnca_model* m, const float* packed_dev, int n_models, int B, int H, int W,
+                                 const gnca_schedule* sched, const float* x0_dev, float* xT_dev, int every,
+                                 const float* targets_dev, float eps, double* sums_dev, int32_t* counts_dev,
+                                 double* ssim_dev, void* scratch_dev, size_t scratch_bytes, void* workspace_dev,
+                                 size_t workspace_bytes, int impl, void* stream);
+
 /* BPTT: given gT = dL/dx_T and the x_hist of the forward, produce g0 = dL/dx_0 and ACCUMULATE gparams. */
 int gnca_rollout_bwd(const gnca_model* m, const float* packed_dev, int B, int H, int W,
                      const gnca_schedule* sched, const float* x_hist_dev, const float* stats_hist_dev,
@@ -522,6 +539,11 @@ int gnca_host_sample_offsets_words(const uint32_t* words, int n_words, const int
 /* per_sample[b] = mean_{4HW}([rgb*a, a] - target)^2 ; gx (optional) = d(scale * sum_b per_sample[b])/dx, [B,C,H,W] */
 int gnca_loss_premult_rgba(int B, int C, int H, int W, const float* x_dev, const float* target_dev /*[4,H,W]*/,
                            float* per_sample_dev, float* gx_dev, float scale, void* stream);
+/* the same with one target per block of B / n_targets samples: sample b against targets_dev[b / (B / n_targets)]
+ * ([n_targets][4][H][W]); n_targets == 1 is bit-identical to gnca_loss_premult_rgba.  n_targets < 1 or
+ * B % n_targets != 0 is GNCA_ERR_ARG. */
+int gnca_loss_premult_rgba_targets(int B, int C, int H, int W, const float* x_dev, const float* targets_dev,
+                                   int n_targets, float* per_sample_dev, float* gx_dev, float scale, void* stream);
 /*
  * For each of n_seg parameter tensors (seg_off[i]..seg_off[i+1] in the flat buffers, host array of n_seg+1):
  * g /= (||g||_2 + 1e-8) unless seg_has_grad[i]==0 (skipped like a None grad), then torch.optim.Adam
